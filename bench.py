@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- BSMAP hot path on B200: reads (pairs) mapped per second, one JSON line (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config cfg1..cfg5]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config cfg1..cfg5] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Workloads (BASELINE.json configs; default cfg2 = the configuration the metric is quoted on):
@@ -68,8 +68,8 @@ CPU_UNITS_PER_THREAD = {"cfg2": 40_000, "cfg1": 100_000, "cfg3": 6_000, "cfg4": 
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=5)
-    ap.add_argument("--warmup", type=int, default=3)
+    ap.add_argument("--steps", type=int, default=None, help="timed steps (default 5; --reference-binary: 1)")
+    ap.add_argument("--warmup", type=int, default=None, help="untimed steps before them (default 3; --reference-binary: 0)")
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--config", default="cfg2", choices=sorted(CONFIGS))
     ap.add_argument("--reads", type=int, default=0, help="units (reads / pairs) per GPU per step (0 = the config's)")
@@ -78,7 +78,39 @@ def parse():
     ap.add_argument("--no-strong", action="store_true", help="skip the strong-scaling / merge leg (N > 1)")
     ap.add_argument("--batch", type=int, default=1 << 20, help="sub-batch of the end-to-end pipeline")
     ap.add_argument("--reference-binary", action="store_true", help="--impl reference: run the unmodified oracle/_ref/bsmap (cfg2, first 1 M reads)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the records of the last timed step for rank 0's read set as DIR/<array>_<field>.npy (float64; a "
+                         "fixed, seeded sample of the units when all of them would exceed 64 MB, their positions in DIR/unit_index.npy)")
+    a = ap.parse_args()
+    if a.reference_binary:
+        # one run of the binary is one step: every run repeats its FASTA load and seed-table build (minutes at 3.1 Gb)
+        if a.steps not in (None, 1) or a.warmup not in (None, 0):
+            ap.error("--reference-binary times one run of the binary: --steps 1 --warmup 0")
+        a.steps, a.warmup = 1, 0
+    a.steps = 5 if a.steps is None else a.steps
+    a.warmup = 3 if a.warmup is None else a.warmup
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.reference_binary:
+        ap.error("--dump-outputs: the reference binary's output is SAM text, not records")
+    return a
+
+
+DUMP_BYTES = 64_000_000
+
+
+def dump_outputs(path, arrays, first):
+    """Every field of the record arrays (same length, one entry per unit) as float64 .npy files, exact for the u32 / i32 /
+    u8 fields.  When they exceed DUMP_BYTES, a sorted sample of units drawn with a fixed seed: the same units every run,
+    so two builds can be compared output for output.  unit_index.npy holds the units' global indices (first + row)."""
+    n = len(next(iter(arrays.values())))
+    fields = [(name, f) for name, arr in arrays.items() for f in arr.dtype.names]
+    k = min(n, (DUMP_BYTES - 128 * (len(fields) + 1)) // (8 * (len(fields) + 1)))     # 128: the .npy header of a 1-D array
+    rows = np.arange(n) if k == n else np.sort(np.random.default_rng(0).choice(n, size=k, replace=False))
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, "unit_index.npy"), (first + rows).astype(np.float64))
+    for name, f in fields:
+        np.save(os.path.join(path, f"{name}_{f}.npy"), arrays[name][f][rows].astype(np.float64))
 
 
 class _DevBuf:
@@ -303,7 +335,7 @@ def main():
             raise SystemExit("--reference-binary is set up for cfg2")
         info = run_reference_binary(a, cfg, names, genome, make_reads, synth)
         val = info["reads_per_s"]
-        print(json.dumps({"metric": metric, "value": val, "unit": unit, "n_gpus": a.gpus, "steps": 1, "warmup": 0,
+        print(json.dumps({"metric": metric, "value": val, "unit": unit, "n_gpus": a.gpus, "steps": a.steps, "warmup": a.warmup,
                           "ms_per_step": 1e3 * info["mapping_s"], "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "u32",
                           "data": "synthetic", "impl": "reference", "config": {"workload": "cfg2: " + cfg["desc"].format(n=info["reads"])},
                           "cpu_baseline": {"value": val, "unit": unit, "cores": info["threads"], "kind": "reference",
@@ -401,6 +433,8 @@ def main():
             differing += count_diff(orecs, grecs, s0, s0 + sample)
             if it >= a.warmup:
                 times.append(dt)
+        if a.dump_outputs:
+            dump_outputs(a.dump_outputs, dict(zip(("pairs", "recs_a", "recs_b") if pe else ("recs",), orecs)), first_index + s0)
         tot = sum(times)
         val = sample * a.steps / tot
         line = {"metric": metric, "value": val, "unit": unit, "n_gpus": a.gpus, "steps": a.steps,
@@ -593,6 +627,9 @@ def main():
         oref.close()
 
     if rank == 0:
+        if a.dump_outputs:
+            # recs_dev: downloaded after the last launch of the timed packed-resident loop that `value` measures
+            dump_outputs(a.dump_outputs, dict(zip(("pairs", "recs_a", "recs_b") if pe else ("recs",), recs_dev)), first_index)
         h2d = n * mates * (PS + 2)
         d2h = n * (16 if not pe else 28 + 32)
         line = {"metric": metric, "value": value, "unit": unit, "n_gpus": world, "steps": a.steps,

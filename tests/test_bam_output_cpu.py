@@ -1,7 +1,8 @@
 """`-o out.bam`: bsx_sam_to_sorted_bam against the vendored samtools 0.1.7 (what the reference's sam2bam.sh runs):
 `samtools view -bS | samtools sort | samtools index` on the reference's own SAM output.  The BAM must decompress to the
 same bytes; the .bai must hold what `samtools index` computes for our file (bins, chunks, linear index).  Without
-oracle/_ref/samtools (make -C oracle samtools) the decompressed BAM is still checked against committed digests."""
+oracle/_ref/samtools (make -C oracle samtools) both are checked against committed digests of samtools' output
+(bam_output_sha256.json, bam_index_sha256.json; tests/golden/make_reference_digests.py)."""
 from __future__ import annotations
 
 import gzip
@@ -22,6 +23,7 @@ from bsmap_b200 import lib as BL
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 SAMTOOLS = os.path.join(ROOT, "oracle", "_ref", "samtools")
 DIGESTS = os.path.join(ROOT, "tests", "golden", "bam_output_sha256.json")
+BAI_DIGESTS = os.path.join(ROOT, "tests", "golden", "bam_index_sha256.json")
 NAMES = ["se_cfg2_r0_uR", "pe_sam", "pe_sam_v5_R", "pe_readthrough", "rrbs_pe", "rrbs_se_A", "se_n1", "se_cfg1", "se_mixed_A", "se_cfg5"]
 pytestmark = pytest.mark.skipif(not os.path.exists(BL.LIB_PATH), reason="library not built")
 
@@ -44,6 +46,14 @@ def parse_bai(path):
     return out
 
 
+def bai_digest(path):
+    """sha256 of the index parse_bai reads (per reference: bins in key order with their chunks, then the linear index).
+    samtools writes the bins of a reference in hash-table order and this library in key order, so two .bai files that
+    hold the same index need not be the same bytes."""
+    canon = [[sorted((b, [list(c) for c in ch]) for b, ch in bins.items()), list(lin)] for bins, lin in parse_bai(path)]
+    return hashlib.sha256(json.dumps(canon).encode()).hexdigest()
+
+
 @pytest.mark.parametrize("name", NAMES)
 def test_sorted_bam_equals_samtools(tmp_path, name):
     case = CS.BY_NAME[name]
@@ -55,7 +65,9 @@ def test_sorted_bam_equals_samtools(tmp_path, name):
     assert raw[:4] == b"BAM\1" and open(ours, "rb").read()[-28:] == bytes.fromhex("1f8b08040000000000ff0600424302001b0003000000000000000000")
     assert hashlib.sha256(raw).hexdigest() == json.load(open(DIGESTS))[name], "decompressed BAM differs from samtools' (committed digest)"
     if not os.path.exists(SAMTOOLS):
-        pytest.skip("oracle/_ref/samtools not built: live comparison skipped")
+        assert bai_digest(ours + ".bai") == json.load(open(BAI_DIGESTS))[name], \
+            "index differs from what `samtools index` computes for this file (committed digest of its bins, chunks and linear index)"
+        return
     ref = str(tmp_path / "ref")
     subprocess.run(f"{SAMTOOLS} view -bS {sam} > {tmp_path}/tmp.bam 2>/dev/null && {SAMTOOLS} sort {tmp_path}/tmp.bam {ref}", shell=True, check=True)
     assert gzip.open(ref + ".bam", "rb").read() == raw
