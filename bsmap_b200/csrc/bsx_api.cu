@@ -3,7 +3,10 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <map>
+#include <mutex>
 #include <string>
+#include <utility>
 #include <vector>
 #include "bsx_common.cuh"
 #include "bsx_internal.h"
@@ -333,13 +336,20 @@ struct bsx_slot {
     bool packed = false;         // the slot's read buffers hold packed slots (bsx_packed_stride) instead of ASCII
 };
 
+// one of the six mapping kernels with the persistent grid it runs in
+struct map_launch {
+    const void *kernel = nullptr;
+    int n_ctas = 0, warps = BSX_WARPS_PER_CTA;   // warps per CTA: fewer when the plan of a read is large
+    size_t smem = 0;                             // dynamic shared memory per CTA
+};
+
 struct bsx_mapper {
     const bsx_index *ix = nullptr;
     int device = 0;                  // kept here too: a mapper may be destroyed after its index (garbage-collected bindings)
     bsx_params par{};
     uint32_t max_batch = 0, stride = 0;
-    int n_ctas_se = 0, n_ctas_pe = 0, plan_cap = 0, nslot = 1;
-    int warps_se = BSX_WARPS_PER_CTA, warps_pe = BSX_WARPS_PER_CTA;   // warps per CTA (fewer when the plan of a read is large)
+    int plan_cap = 0, nslot = 1;
+    map_launch se, pe;               // single-end and paired-end kernel of this parameter set and index
     uint32_t hit_stride = 0, dd_stride = 0, pair_stride = 0;
     bool pe_ready = false;
     bsx_slot slot[2];
@@ -352,18 +362,57 @@ struct bsx_mapper {
     int meth_sam = 1;
 };
 
-int bsx_map_occupancy_se_wgbs(size_t smem, int warps);   // bsx_map_se.cu
-int bsx_map_occupancy_se_rrbs(size_t smem, int warps);   // bsx_map_se_rrbs.cu
-int bsx_launch_map_se_wgbs(const MapArgs &a, int n_ctas, int warps, cudaStream_t st);
-int bsx_launch_map_se_rrbs(const MapArgs &a, int n_ctas, int warps, cudaStream_t st);
-int bsx_map_occupancy_se_wide(size_t smem, int warps);   // bsx_map_se_wide.cu
-int bsx_launch_map_se_wide(const MapArgs &a, int n_ctas, int warps, cudaStream_t st);
-int bsx_map_occupancy_pe_wgbs(size_t smem, int warps);   // bsx_map_pe.cu
-int bsx_map_occupancy_pe_wide(size_t smem, int warps);   // bsx_map_pe_wide.cu
-int bsx_launch_map_pe_wide(const MapArgs &a, int n_ctas, int warps, cudaStream_t st);
-int bsx_map_occupancy_pe_rrbs(size_t smem, int warps);   // bsx_map_pe_rrbs.cu
-int bsx_launch_map_pe_wgbs(const MapArgs &a, int n_ctas, int warps, cudaStream_t st);
-int bsx_launch_map_pe_rrbs(const MapArgs &a, int n_ctas, int warps, cudaStream_t st);
+// the six mapping kernels (bsx_map_{se,pe}{,_rrbs,_wide}.cu)
+extern const void *const bsx_map_se_wgbs, *const bsx_map_se_rrbs, *const bsx_map_se_wide;
+extern const void *const bsx_map_pe_wgbs, *const bsx_map_pe_rrbs, *const bsx_map_pe_wide;
+
+static const void *map_kernel(bool pe, bool rrbs, bool wide) {
+    if (rrbs) return pe ? bsx_map_pe_rrbs : bsx_map_se_rrbs;
+    if (wide) return pe ? bsx_map_pe_wide : bsx_map_se_wide;
+    return pe ? bsx_map_pe_wgbs : bsx_map_se_wgbs;
+}
+
+// Lets `kernel` launch with `smem` bytes of dynamic shared memory on the current device.  The limit belongs to (kernel,
+// device) and is shared by every mapper and host thread, so it is only ever raised: lowering it for one mapper would
+// make the launches of another that needs more fail.
+static int raise_smem_limit(const void *kernel, size_t smem) {
+    static std::mutex mu;
+    static std::map<std::pair<const void *, int>, size_t> limit;
+    int dev = 0;
+    BSX_CUDA_CHECK(cudaGetDevice(&dev));
+    std::lock_guard<std::mutex> lock(mu);
+    size_t &cur = limit[{kernel, dev}];
+    if (smem > cur) {
+        BSX_CUDA_CHECK(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        cur = smem;
+    }
+    return BSX_OK;
+}
+
+// Chooses the kernel for a parameter set and the CTA shape of its persistent grid: eight warps per CTA; a parameter set
+// whose per-read plan is large (many segments x -I, -n 1, wide context) runs with fewer.  Fails when none fits on an SM.
+static int plan_launch(map_launch &k, bool pe, const bsx_mapper *m, bool wide, int sms) {
+    k.kernel = map_kernel(pe, m->par.rrbs, wide);
+    for (int w = BSX_WARPS_PER_CTA; w >= 1; w >>= 1) {
+        const size_t smem = bsx_cta_smem_bytes(pe ? 2 : 1, m->plan_cap, m->nslot, wide, m->par.rrbs, w);
+        if (smem > BSX_MAX_CTA_SMEM) continue;
+        int occ = 0;   // resident CTAs per SM
+        if (raise_smem_limit(k.kernel, smem) != BSX_OK ||
+            cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k.kernel, w * 32, smem) != cudaSuccess) { cudaGetLastError(); occ = 0; }
+        k.warps = w; k.smem = smem; k.n_ctas = sms * occ;
+        if (occ >= 1) return BSX_OK;
+    }
+    bsx_set_error("mapping kernel does not fit on an SM (shared memory: plan of %d entries x %d chains)", m->plan_cap, m->nslot);
+    return BSX_ERR_CUDA;
+}
+
+static int launch_map(const map_launch &k, const MapArgs &a, cudaStream_t st) {
+    int rc = raise_smem_limit(k.kernel, k.smem); if (rc) return rc;
+    void *args[] = {const_cast<MapArgs *>(&a)};
+    cudaLaunchKernel(k.kernel, dim3(k.n_ctas), dim3(k.warps * 32), args, k.smem, st);
+    BSX_CUDA_CHECK(cudaGetLastError());       // the launch's error, cleared so that it does not surface in a later call
+    return BSX_OK;
+}
 
 static void slot_free(bsx_slot &s) {
     cudaFree(s.d_seq_a); cudaFree(s.d_seq_b); cudaFree(s.d_len_a); cudaFree(s.d_len_b); cudaFree(s.d_out_a); cudaFree(s.d_out_b);
@@ -385,7 +434,7 @@ extern "C" int bsx_mapper_destroy(bsx_mapper *m) {
 static int alloc_pe(bsx_mapper *m) {
     // second mate + pair buckets: allocated on first paired-end use
     if (m->pe_ready) return BSX_OK;
-    const size_t warps = (size_t)m->n_ctas_pe * m->warps_pe;
+    const size_t warps = (size_t)m->pe.n_ctas * m->pe.warps;
     const uint32_t W1 = (uint32_t)m->par.max_num_hits + 1, lv = (uint32_t)m->par.max_snp_num + 1;
     for (int i = 0; i < 2; i++) {
         bsx_slot &s = m->slot[i];
@@ -396,7 +445,7 @@ static int alloc_pe(bsx_mapper *m) {
         BSX_CUDA_CHECK(cudaMalloc(&s.d_out_pair, (size_t)m->max_batch * sizeof(bsx_pair_rec)));
         // all-level hit storage for both mates replaces the SE scratch
         cudaFree(s.d_hits); cudaFree(s.d_dd); s.d_hits = nullptr; s.d_dd = nullptr;
-        const size_t se_warps = (size_t)m->n_ctas_se * m->warps_se;
+        const size_t se_warps = (size_t)m->se.n_ctas * m->se.warps;
         const size_t hit_elems = std::max(warps * 2 * (size_t)(lv * 2 * W1), se_warps * (size_t)(2 * W1));
         const size_t dd_elems = std::max(warps * 2, se_warps) * (size_t)m->dd_stride;
         BSX_CUDA_CHECK(cudaMalloc(&s.d_hits, hit_elems * sizeof(uint2)));
@@ -440,29 +489,15 @@ static int mapper_init(bsx_mapper *m, const bsx_index *ix, const bsx_params *p, 
     BSX_CUDA_CHECK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, ix->device));
     // the kernel follows the index layout: an index built with -v >= 8 holds 16-byte context entries whatever -v the mapper uses
     const bool wide = !p->rrbs && ix->ctx_wide;
-    // eight warps per CTA; a parameter set whose per-read plan is large (many segments x -I, -n 1, wide context) runs with fewer
-    int occ_se = 0, occ_pe = 0;
-    for (int w = BSX_WARPS_PER_CTA; w >= 1 && occ_se < 1; w >>= 1) {
-        const size_t smem = bsx_cta_smem_bytes(1, m->plan_cap, m->nslot, wide, p->rrbs, w);
-        if (smem > BSX_MAX_CTA_SMEM) continue;
-        m->warps_se = w;
-        occ_se = p->rrbs ? bsx_map_occupancy_se_rrbs(smem, w) : (wide ? bsx_map_occupancy_se_wide(smem, w) : bsx_map_occupancy_se_wgbs(smem, w));
-    }
-    for (int w = BSX_WARPS_PER_CTA; w >= 1 && occ_pe < 1; w >>= 1) {
-        const size_t smem = bsx_cta_smem_bytes(2, m->plan_cap, m->nslot, wide, p->rrbs, w);
-        if (smem > BSX_MAX_CTA_SMEM) continue;
-        m->warps_pe = w;
-        occ_pe = p->rrbs ? bsx_map_occupancy_pe_rrbs(smem, w) : (wide ? bsx_map_occupancy_pe_wide(smem, w) : bsx_map_occupancy_pe_wgbs(smem, w));
-    }
-    if (occ_se < 1 || occ_pe < 1) { bsx_set_error("mapping kernel does not fit on an SM (shared memory: plan of %d entries x %d chains)", m->plan_cap, m->nslot); return BSX_ERR_CUDA; }
-    m->n_ctas_se = sms * occ_se; m->n_ctas_pe = sms * occ_pe;
+    int rc = plan_launch(m->se, false, m, wide, sms); if (rc) return rc;
+    rc = plan_launch(m->pe, true, m, wide, sms); if (rc) return rc;
     const uint32_t W1 = (uint32_t)p->max_num_hits + 1, lv = (uint32_t)p->max_snp_num + 1;
     m->hit_stride = 2 * W1;                        // SE: only the best level is kept
     m->dd_stride = lv * (uint32_t)p->max_num_hits + 32;
     m->pair_stride = (2 * (uint32_t)p->max_snp_num + 1) * W1 * 2;   // uint4 units (32-byte PairHit)
-    const size_t se_warps = (size_t)m->n_ctas_se * m->warps_se;
+    const size_t se_warps = (size_t)m->se.n_ctas * m->se.warps;
     // prepared-unit images: 32 per resident warp (phase A of the align kernels, bsx_prep.cuh)
-    const size_t prep_bytes = std::max(se_warps, (size_t)m->n_ctas_pe * m->warps_pe) * 32u * bsx_image_bytes(m->plan_cap, m->nslot);
+    const size_t prep_bytes = std::max(se_warps, (size_t)m->pe.n_ctas * m->pe.warps) * 32u * bsx_image_bytes(m->plan_cap, m->nslot);
     for (int i = 0; i < 2; i++) {
         bsx_slot &s = m->slot[i];
         BSX_CUDA_CHECK(cudaStreamCreateWithFlags(&s.stream, cudaStreamNonBlocking));
@@ -534,6 +569,7 @@ static int run_slot(bsx_mapper *m, int si, uint32_t n, uint32_t first_index, int
     bsx_slot &s = m->slot[si];
     if (n == 0) return BSX_OK;
     if (pe) { int rc = alloc_pe(m); if (rc) return rc; }
+    const map_launch &k = pe ? m->pe : m->se;
     MapArgs a = m->base;
     a.seq_a = s.d_seq_a; a.len_a = s.d_len_a; a.seq_b = s.d_seq_b; a.len_b = s.d_len_b;
     a.n = n; a.first_index = first_index; a.readset = readset;
@@ -544,7 +580,7 @@ static int run_slot(bsx_mapper *m, int si, uint32_t n, uint32_t first_index, int
     {   // 32 units per warp and atomic when the batch is large (>= 2 blocks per resident warp: the prepare phase runs
         // with all lanes busy); small batches take smaller blocks (>= 8 per warp) because there the tail decides --
         // config 5's 200 k heavy reads: 0.62 M reads/s with blocks of 32, 0.86 M with blocks of 4
-        const uint64_t units = (uint64_t)n * (uint64_t)a.mates, warps = (uint64_t)(pe ? m->n_ctas_pe * m->warps_pe : m->n_ctas_se * m->warps_se);
+        const uint64_t units = (uint64_t)n * (uint64_t)a.mates, warps = (uint64_t)(k.n_ctas * k.warps);
         const uint64_t want = units >= (1u << 19) ? 2 : 8;
         uint32_t b = 32;
         while (b > 4 && units / b < want * warps) b >>= 1;
@@ -553,10 +589,7 @@ static int run_slot(bsx_mapper *m, int si, uint32_t n, uint32_t first_index, int
     if (pe) a.hit_stride = ((uint32_t)m->par.max_snp_num + 1) * 2 * ((uint32_t)m->par.max_num_hits + 1);
     BSX_CUDA_CHECK(cudaMemsetAsync(s.d_counter, 0, 4, st));
     m->launches++;
-    int rc = pe ? (a.rrbs ? bsx_launch_map_pe_rrbs(a, m->n_ctas_pe, m->warps_pe, st)
-                          : (a.ctx_wide ? bsx_launch_map_pe_wide(a, m->n_ctas_pe, m->warps_pe, st) : bsx_launch_map_pe_wgbs(a, m->n_ctas_pe, m->warps_pe, st)))
-                : (a.rrbs ? bsx_launch_map_se_rrbs(a, m->n_ctas_se, m->warps_se, st)
-                          : (a.ctx_wide ? bsx_launch_map_se_wide(a, m->n_ctas_se, m->warps_se, st) : bsx_launch_map_se_wgbs(a, m->n_ctas_se, m->warps_se, st)));
+    int rc = launch_map(k, a, st);
     if (rc == BSX_OK && m->meth && !s.packed) {
         rc = bsx_meth_pile_mapped(m->meth, &m->meth_opts, m->meth_sam, m->par.report_repeat_hits, n, pe ? 2 : 1, m->stride,
                                   s.d_seq_a, s.d_seq_b, s.d_out_a, s.d_out_b, s.d_out_pair, st);

@@ -106,23 +106,11 @@ static_assert(sizeof(CtaSm) % 16 == 0, "per-warp shared memory follows CtaSm and
 // rounds spread the per-round work (schedule, staging issue, wait) over more entries but cost shared memory and leave
 // more of a short mode's round empty: measured per kernel family (paired-end, config 3: 8 -> 81.3, 12 -> 84.2, 16 -> 80.3 M pairs/s;
 // single-end WGBS, config 2: 8 -> 356.3, 12 -> 355.4 M reads/s; single-end RRBS, config 4: 12 and 16 gain 2 % resident and lose 4-7 %
-// end to end in 1 M-read sub-batches).
-#ifndef BSX_WIDE_ROUND_HS
-#define BSX_WIDE_ROUND_HS 8
-#endif
-#ifndef BSX_NARROW_ROUND_HS
-#define BSX_NARROW_ROUND_HS 8          // single-end WGBS
-#endif
-#ifndef BSX_NARROW_ROUND_HS_PE
-#define BSX_NARROW_ROUND_HS_PE 12      // paired-end (WGBS and RRBS)
-#endif
-#ifndef BSX_NARROW_ROUND_HS_RRBS
-#define BSX_NARROW_ROUND_HS_RRBS 8     // single-end RRBS
-#endif
+// end to end in 1 M-read sub-batches).  The kernels (bsx_map_impl.cuh) and the host's shared-memory sizing both read it here.
+constexpr __host__ __device__ int bsx_round_hs(int pe, int /*rrbs: 8 either way*/, int wide) { return (pe && !wide) ? 12 : 8; }
 // bytes of the per-warp staging area beyond the PrepCol it aliases (slot[HS*32] entries + HS schedule entries of 32 / 48 bytes)
 static inline __host__ __device__ size_t bsx_stage_extra_bytes(int wide, int pe, int rrbs) {
-    const size_t need = wide ? (size_t)BSX_WIDE_ROUND_HS * (32u * 16u + 48u)
-                             : (size_t)(pe ? BSX_NARROW_ROUND_HS_PE : (rrbs ? BSX_NARROW_ROUND_HS_RRBS : BSX_NARROW_ROUND_HS)) * (32u * 8u + 32u);
+    const size_t need = (size_t)bsx_round_hs(pe, rrbs, wide) * (wide ? 32u * 16u + 48u : 32u * 8u + 32u);
     return need > sizeof(PrepCol) ? ((need - sizeof(PrepCol) + 15u) & ~(size_t)15u) : 0u;
 }
 static inline __host__ __device__ size_t bsx_read_smem_bytes(int plan_cap, int nslot, int wide) {

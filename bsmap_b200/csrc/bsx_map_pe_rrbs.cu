@@ -1,9 +1,12 @@
 // bsx_map_pe_rrbs.cu -- the paired-end RRBS (-D) mapping kernel: same source, RRBS fixed at compile time.
-#define BSX_BUILD_PE 1
-#define BSX_CALLS 0
-#define BSX_RRBS(A) 1
-#define BSX_WIDE(A) 0
-#define BSX_PE_KERNEL bsx_map_pe_rrbs_kernel
-#define BSX_PE_OCC bsx_map_occupancy_pe_rrbs
-#define BSX_PE_LAUNCH bsx_launch_map_pe_rrbs
+struct MapKernel {
+    static constexpr bool pe = true, rrbs = true, wide = false;
+    static constexpr bool owner_sched = false;
+    static constexpr bool run_advance = true;      // long lists, see bsx_map_se_rrbs.cu
+};
 #include "bsx_map_impl.cuh"
+
+namespace {
+__global__ void __launch_bounds__(BSX_WARPS_PER_CTA * 32, 4) bsx_map_pe_rrbs_kernel(const __grid_constant__ MapArgs A) { map_pe(A); }
+}
+extern const void *const bsx_map_pe_rrbs = (const void *)bsx_map_pe_rrbs_kernel;

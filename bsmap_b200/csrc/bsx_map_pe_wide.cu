@@ -1,9 +1,12 @@
 // bsx_map_pe_wide.cu -- the paired-end WGBS kernel for indexes built with -v >= 8 (16-byte context entries).
-#define BSX_BUILD_PE 1
-#define BSX_CALLS 0
-#define BSX_RRBS(A) 0
-#define BSX_WIDE(A) 1
-#define BSX_PE_KERNEL bsx_map_pe_wide_kernel
-#define BSX_PE_OCC bsx_map_occupancy_pe_wide
-#define BSX_PE_LAUNCH bsx_launch_map_pe_wide
+struct MapKernel {
+    static constexpr bool pe = true, rrbs = false, wide = true;
+    static constexpr bool owner_sched = false;
+    static constexpr bool run_advance = true;      // long lists, see bsx_map_se_rrbs.cu
+};
 #include "bsx_map_impl.cuh"
+
+namespace {
+__global__ void __launch_bounds__(BSX_WARPS_PER_CTA * 32, 4) bsx_map_pe_wide_kernel(const __grid_constant__ MapArgs A) { map_pe(A); }
+}
+extern const void *const bsx_map_pe_wide = (const void *)bsx_map_pe_wide_kernel;

@@ -1,9 +1,14 @@
 // bsx_map_se_rrbs.cu -- the single-end RRBS (-D) mapping kernel: same source, RRBS fixed at compile time.
-#define BSX_BUILD_SE 1
-#define BSX_CALLS 0
-#define BSX_RRBS(A) 1
-#define BSX_WIDE(A) 0
-#define BSX_SE_KERNEL bsx_map_se_rrbs_kernel
-#define BSX_SE_OCC bsx_map_occupancy_se_rrbs
-#define BSX_SE_LAUNCH bsx_launch_map_se_rrbs
+struct MapKernel {
+    static constexpr bool pe = false, rrbs = true, wide = false;
+    static constexpr bool owner_sched = false;
+    // rounds that stay inside one long list advance the previous schedule instead of rebuilding it: pays where lists run
+    // to thousands of entries (config 4 +2 %, config 5 +9 %), costs 1-3 % on configs 2 / 3
+    static constexpr bool run_advance = true;
+};
 #include "bsx_map_impl.cuh"
+
+namespace {
+__global__ void __launch_bounds__(BSX_WARPS_PER_CTA * 32, 5) bsx_map_se_rrbs_kernel(const __grid_constant__ MapArgs A) { map_se(A); }
+}
+extern const void *const bsx_map_se_rrbs = (const void *)bsx_map_se_rrbs_kernel;

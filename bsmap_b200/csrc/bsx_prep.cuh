@@ -81,7 +81,7 @@ __device__ __forceinline__ void pack_chain(const uint8_t *sq, uint32_t stride, i
 
 // TrimAdapter (align.cpp:371-425): adapters in -A order, positions ascending, first success wins
 __device__ int trim_adapter(const MapArgs &A, const uint8_t *sq, int len) {
-    const int s = A.s, tail = BSX_RRBS(A) ? 5 : 4;
+    const int s = A.s, tail = MapKernel::rrbs ? 5 : 4;
     #pragma unroll 1
     for (int a = 0; a < A.n_adapter; a++) {
         const int al = A.adapter_len[a];
@@ -94,7 +94,7 @@ __device__ int trim_adapter(const MapArgs &A, const uint8_t *sq, int len) {
                 if (m0 > 4) break;
             }
             bool ok = false;
-            if (!BSX_RRBS(A)) ok = (k >= m0 * 5 && k > 3);
+            if constexpr (!MapKernel::rrbs) ok = (k >= m0 * 5 && k > 3);
             else if (k >= m0 * 5) {
                 // digestion-site remnant just before the adapter (align.cpp:383-404)
                 const int sl = A.site_len, dp = A.digest_pos;
@@ -164,7 +164,7 @@ __device__ __forceinline__ void pack_chain_packed(const uint8_t *pk, uint32_t ma
 // TrimAdapter on a packed slot.  Adapters and the digestion site are upper-case ACGT (checked on the host), so
 // "characters differ" is "invalid base or different code".
 __device__ int trim_adapter_packed(const MapArgs &A, const uint8_t *pk, int len) {
-    const int s = A.s, tail = BSX_RRBS(A) ? 5 : 4;
+    const int s = A.s, tail = MapKernel::rrbs ? 5 : 4;
     const uint32_t mo = A.pk_mask_off;
     #pragma unroll 1
     for (int a = 0; a < A.n_adapter; a++) {
@@ -178,7 +178,7 @@ __device__ int trim_adapter_packed(const MapArgs &A, const uint8_t *pk, int len)
                 if (m0 > 4) break;
             }
             bool ok = false;
-            if (!BSX_RRBS(A)) ok = (k >= m0 * 5 && k > 3);
+            if constexpr (!MapKernel::rrbs) ok = (k >= m0 * 5 && k > 3);
             else if (k >= m0 * 5) {
                 const int sl = A.site_len, dp = A.digest_pos;
                 int m = m0, m2 = m0;
@@ -207,20 +207,12 @@ __device__ __forceinline__ uint32_t seed_key(const MapArgs &A, const uint32_t *r
 // list header of seed key `key`: {list start, reverse-strand start, list end} (tab is the CSR of the seed table)
 // A probe is a random 12-byte read of a 344 MB table: fetch 64 bytes from HBM for it, not the default 128-byte line
 // (measured in round 1: 121 B of HBM traffic per random gather with the default load, 62 B with .L2::64B).
-#ifndef BSX_PROBE_64B
-#define BSX_PROBE_64B 1
-#endif
 __device__ __forceinline__ uint3 probe_tab(const MapArgs &A, uint32_t key) {
-#if BSX_PROBE_64B
     uint3 r;
     const uint32_t *p = A.tab + 2 * (size_t)key;
     asm volatile("ld.global.nc.L2::64B.v2.u32 {%0,%1}, [%2];" : "=r"(r.x), "=r"(r.y) : "l"(p));
     asm volatile("ld.global.nc.L2::64B.u32 %0, [%1];" : "=r"(r.z) : "l"(p + 2));
     return r;
-#else
-    const uint2 a = __ldg(reinterpret_cast<const uint2 *>(A.tab) + key);
-    return make_uint3(a.x, a.y, __ldg(A.tab + 2 * (size_t)key + 2));
-#endif
 }
 
 // RRBS: the table is a CSR over (key, group) (bsx_index.cu); the whole list of a key -- ref.index[key].n1, what
@@ -236,7 +228,7 @@ __device__ __forceinline__ uint32_t probe_rrbs_size(const MapArgs &A, uint32_t k
 __device__ __forceinline__ int select_seeds(const MapArgs &A, const PrepSm *K, const uint32_t *rw, int len, int seg, int chain,
                             uint4 *plan, uint32_t *dbg) {
     const int s = A.s, I = A.I;
-    const bool rrbs = BSX_RRBS(A) != 0;                                           // fixed at compile time in the specialised kernels
+    constexpr bool rrbs = MapKernel::rrbs;
     const int mo = (rrbs || len - I + 1 < 0) ? 0 : (int)K->remof[len - I + 1];   // max_offset = (len-I+1) % s
     const int cso = (rrbs && chain) ? (int)K->remof[len] : 0;                     // cseed_offset (RRBS rc chain)
     const int lim = I - 1 + mo;

@@ -290,6 +290,39 @@ def test_empty_and_ragged_batches():
     mp.close(); mp2.close(); ix.close(); oref.close()
 
 
+def test_mapper_with_less_shared_memory_does_not_break_an_earlier_mapper():
+    """The kernels' dynamic shared-memory limit belongs to (kernel, device), not to a mapper: creating and running a
+    mapper that needs less (-v 0 on a wide -v 12 index) must not leave the earlier mapper unable to launch."""
+    from bsmap_b200 import synth
+    g = synth.make_genome(12, [150_000, 90_000])
+    names, gseqs = ["chr1", "chr2"], [x.numpy().tobytes() for x in g]
+    sim = synth.simulate_pairs(g, 2000, 100, seed=12, subs="cfg1")
+    buf_a, lens_a = B.pack_reads([bytes(r) for r in sim["seq1"].numpy()], stride=160)
+    buf_b, lens_b = B.pack_reads([bytes(r) for r in sim["seq2"].numpy()], stride=160)
+    ix = B.Index(B.make_params(s=12, I=4, v=12), names, gseqs)
+    assert ix.info.ctx_words == 4                    # 16-byte context entries: the wide kernels
+    # single-end
+    a = B.Mapper(ix, B.make_params(s=12, I=4, v=12), max_batch=4096, stride=160)
+    first, _ = a.map_se(buf_a, lens_a)
+    b = B.Mapper(ix, B.make_params(s=12, I=4, v=0), max_batch=4096, stride=160)
+    b.map_se(buf_a, lens_a)
+    again, _ = a.map_se(buf_a, lens_a)
+    assert np.array_equal(first, again)
+    assert (first["nhits"] > 0).mean() > 0.9
+    # paired-end
+    pa = B.Mapper(ix, B.make_params(s=12, I=4, v=12, pairend=1), max_batch=4096, stride=160)
+    first = pa.map_pe(buf_a, lens_a, buf_b, lens_b)
+    pb = B.Mapper(ix, B.make_params(s=12, I=4, v=0, pairend=1), max_batch=4096, stride=160)
+    pb.map_pe(buf_a, lens_a, buf_b, lens_b)
+    again = pa.map_pe(buf_a, lens_a, buf_b, lens_b)
+    for x, y in zip(first, again):
+        assert np.array_equal(x, y)
+    assert (first[0]["paired"] > 0).mean() > 0.9
+    for m in (a, b, pa, pb):
+        m.close()
+    ix.close()
+
+
 @pytest.mark.parametrize("L,opts,n_reads", [
     (100, dict(s=16, v=5, I=4, S=13), 60000),
     (50, dict(s=16, v=2, I=4, S=13), 60000),
