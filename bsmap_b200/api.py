@@ -7,7 +7,7 @@ import os
 import numpy as np
 
 from . import lib as _l
-from .lib import PAIR_REC, REC, BsxError, IndexInfo, MethOpts, Params, Stats, check, load, strs
+from .lib import MBIAS_CYCLES, METH_READ2, PAIR_REC, REC, BsxError, IndexInfo, MethOpts, Params, Stats, check, load, strs
 
 
 def make_params(s=16, I=4, v=2, w=1000, r=1, m=28, x=500, n=0, pairend=0, S=0, f=5, L=144,
@@ -397,9 +397,12 @@ class Meth:
         self.h = h
         self.n_valid = 0
 
-    def add(self, seqs, chr_idx, pos, strand, insert, mate_pos, flags):
-        """seqs: list of bytes (SEQ as printed); strand: bit 0 / 1 = first / second ZS character is '-'"""
+    def add(self, seqs, chr_idx, pos, strand, insert, mate_pos, flags, read2=None):
+        """seqs: list of bytes (SEQ as printed); strand: bit 0 / 1 = first / second ZS character is '-';
+        read2: optional per-alignment truth values (FLAG 0x80), setting BSX_METH_READ2 in flags"""
         n = len(seqs)
+        if read2 is not None:
+            flags = np.asarray(flags, dtype=np.uint8) | np.where(np.asarray(read2, dtype=bool), np.uint8(METH_READ2), np.uint8(0))
         buf, lens = pack_reads(seqs, stride=max(16, (max((len(s) for s in seqs), default=1) + 15) // 16 * 16))
         arr = lambda a, t: np.ascontiguousarray(np.asarray(a, dtype=t))
         c, p, st, ins, mt, fl = arr(chr_idx, np.uint32), arr(pos, np.uint32), arr(strand, np.uint8), arr(insert, np.int32), arr(mate_pos, np.int32), arr(flags, np.uint8)
@@ -425,6 +428,29 @@ class Meth:
         m, d = np.zeros(n, dtype=np.uint32), np.zeros(n, dtype=np.uint32)
         check(load().bsx_meth_download(self.h, C.byref(self.o), k, m.ctypes.data, d.ctypes.data))
         return m, d
+
+    def enable_mbias(self):
+        """track the M-bias (methylation by read, C context and cycle); before the first add / mapped batch"""
+        check(load().bsx_meth_enable_mbias(self.h))
+
+    def set_ignore(self, r1_5p=0, r1_3p=0, r2_5p=0, r2_3p=0):
+        """drop calls in the first / last cycles of read 1 / read 2 from the counters and the M-bias; before the first add"""
+        v = (C.c_int32 * 4)(int(r1_5p), int(r1_3p), int(r2_5p), int(r2_3p))
+        check(load().bsx_meth_set_ignore(self.h, v))
+
+    def mbias(self):
+        """-> (uint64 array [read][context CpG/CHG/CHH][cycle][methylated, unmethylated], calls past the last cycle)"""
+        h = np.zeros((2, 3, MBIAS_CYCLES, 2), dtype=np.uint64)
+        over = C.c_uint64(0)
+        check(load().bsx_meth_mbias(self.h, h.ctypes.data, C.byref(over)))
+        return h, over.value
+
+    def write_mbias(self, fd: int) -> int:
+        """the M-bias report (include/bsmap_b200.h) to fd; returns bytes written"""
+        w = load().bsx_meth_write_mbias(self.h, fd)
+        if w == 0:
+            check(1)
+        return w
 
     def write(self, seqs, fd: int, chroms=None, threads=0):
         keep = [s if isinstance(s, bytes) else bytes(s) for s in seqs]

@@ -591,7 +591,7 @@ static int run_slot(bsx_mapper *m, int si, uint32_t n, uint32_t first_index, int
     m->launches++;
     int rc = launch_map(k, a, st);
     if (rc == BSX_OK && m->meth && !s.packed) {
-        rc = bsx_meth_pile_mapped(m->meth, &m->meth_opts, m->meth_sam, m->par.report_repeat_hits, n, pe ? 2 : 1, m->stride,
+        rc = bsx_meth_pile_mapped(m->meth, &m->meth_opts, m->meth_sam, m->par.report_repeat_hits, n, pe ? 2 : 1, readset, m->stride,
                                   s.d_seq_a, s.d_seq_b, s.d_out_a, s.d_out_b, s.d_out_pair, st);
         m->launches++;
     }

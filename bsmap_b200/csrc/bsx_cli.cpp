@@ -33,6 +33,9 @@ struct Opts {
     std::string bam_out;         // -o x.bam: SAM text goes to a temporary file, then bsx_sam_to_sorted_bam (the reference: sam2bam.sh)
     std::string meth_out;        // --methratio FILE: methylation ratios straight from the device (no SAM needed)
     bsx_meth_opts mo;
+    std::string meth_mbias;      // --meth-mbias FILE: the M-bias report of the same calls
+    bool meth_ignore_set = false;
+    int32_t meth_ignore[4] = {0, 0, 0, 0};   // --meth-ignore A,B,C,D: cycles dropped at the 5' / 3' ends of read 1 / read 2
     unsigned batch = 1u << 17;   // reads per GPU batch: small enough to keep the three host stages overlapped
     std::string gpus;            // -g: number of devices (default: all visible) or a comma list of device ids; output stays in input order
 };
@@ -73,7 +76,10 @@ void usage() {
            "       --methratio <str>   also write methratio.py's table, piled up on the GPU from the mapped batches\n"
            "                           (-o may then be omitted: no alignment text is produced at all)\n"
            "       --meth-unique --meth-pair --meth-zero --meth-cpg --meth-rmdup --meth-trim <int> --meth-min-depth <int>\n"
-           "                           methratio.py's -u -p -z -g -r -t -m\n\n");
+           "                           methratio.py's -u -p -z -g -r -t -m\n"
+           "       --meth-mbias <str>  with --methratio: also write the M-bias report (methylation by read, context and cycle)\n"
+           "       --meth-ignore <A,B,C,D>  with --methratio: drop calls in the first A / last B cycles of read 1 and the\n"
+           "                           first C / last D cycles of read 2, from the table and the M-bias report\n\n");
     exit(1);
 }
 
@@ -103,6 +109,16 @@ int get_options(int argc, char **argv, Opts &o) {
             else if (a == "meth-rmdup") o.mo.rm_dup = 1;
             else if (a == "meth-trim" && i + 1 < argc) o.mo.trim_fillin = atoi(argv[++i]);
             else if (a == "meth-min-depth" && i + 1 < argc) o.mo.min_depth = atoi(argv[++i]);
+            else if (a == "meth-mbias" && i + 1 < argc) o.meth_mbias = argv[++i];
+            else if (a == "meth-ignore" && i + 1 < argc) {
+                const char *q = argv[++i];
+                for (int k = 0; k < 4; k++) {
+                    char *e; const long x = strtol(q, &e, 10);
+                    if (e == q || x < 0 || x > 0x7fffffff || *e != (k < 3 ? ',' : '\0')) return i;   // "unknown option: <value>"
+                    o.meth_ignore[k] = (int32_t)x; q = e + 1;
+                }
+                o.meth_ignore_set = true;
+            }
             else return i;
             continue;
         }
@@ -258,6 +274,7 @@ extern "C" int bsx_cli_main(int argc, char **argv) {
     { time_t t = time(nullptr); printf("Start at:  %s\n", ctime(&t)); }
     Opts o; bsx_params_default(&o.p); bsx_meth_opts_default(&o.mo);
     if (int bad = get_options(argc, argv, o)) { printf("unknown option: %s\n", argv[bad]); exit(bad); }
+    if (o.meth_out.empty() && (!o.meth_mbias.empty() || o.meth_ignore_set)) { fprintf(stderr, "--meth-mbias and --meth-ignore need --methratio\n"); return 1; }
     if (o.qual_threshold != 0) { fprintf(stderr, "-q quality trimming is not supported by the GPU path\n"); return 1; }
     if (o.o.size() > 4) {
         if (o.o.compare(o.o.size() - 4, 4, ".sam") == 0) o.p.out_sam = 1;
@@ -355,7 +372,9 @@ extern "C" int bsx_cli_main(int argc, char **argv) {
     bsx_meth *mh = nullptr;
     if (!o.meth_out.empty()) {
         // SAM rules (mate-overlap removal) unless the alignment output is BSP: the table then equals methratio.py run on -o
-        if (bsx_meth_create(ix, &mh) != BSX_OK || bsx_mapper_attach_meth(mp, mh, &o.mo, (p.out_sam || no_text) ? 1 : 0) != BSX_OK) {
+        if (bsx_meth_create(ix, &mh) != BSX_OK || (!o.meth_mbias.empty() && bsx_meth_enable_mbias(mh) != BSX_OK) ||
+            (o.meth_ignore_set && bsx_meth_set_ignore(mh, o.meth_ignore) != BSX_OK) ||
+            bsx_mapper_attach_meth(mp, mh, &o.mo, (p.out_sam || no_text) ? 1 : 0) != BSX_OK) {
             fprintf(stderr, "%s\n", bsx_last_error()); return 1; }
     }
     bsx_reads_skip(ra, o.read_start - 1); if (pe) bsx_reads_skip(rb, o.read_start - 1);
@@ -509,6 +528,7 @@ extern "C" int bsx_cli_main(int argc, char **argv) {
         fclose(fm);
         printf("total %llu valid mappings, %llu covered cytosines, average coverage: %.2f fold.\n", (unsigned long long)nv, (unsigned long long)st[0],
                st[0] ? (double)st[1] / (double)st[0] : 0.0);
+        if (!o.meth_mbias.empty() && bsx_meth_write_mbias_file(mh, o.meth_mbias.c_str()) != BSX_OK) return 1;
         if (timing) fprintf(stderr, "[bsx timing] methratio report %.3f s\n", now() - t);
         bsx_meth_destroy(mh);
     }

@@ -97,9 +97,12 @@ void bsx_format_pe_chunks(const bsx_index *ix, const bsx_params *p, uint32_t n, 
                           std::vector<std::string> &chunks_unpair, uint32_t *n_stats);
 int bsx_load_fasta(const char *path, std::vector<std::string> &names, std::vector<std::string> &seqs);   // bsx_reads.cpp
 struct bsx_meth;
-int bsx_meth_pile_mapped(bsx_meth *m, const bsx_meth_opts *o, int sam, int report_repeat_hits, uint32_t n, int mates, uint32_t stride,
+int bsx_meth_pile_mapped(bsx_meth *m, const bsx_meth_opts *o, int sam, int report_repeat_hits, uint32_t n, int mates, int readset, uint32_t stride,
                          const uint8_t *seq_a, const uint8_t *seq_b, const bsx_rec *out_a, const bsx_rec *out_b, const bsx_pair_rec *out_pair,
                          cudaStream_t st);   // bsx_meth.cu
+// the command lines' M-bias output: bsx_meth_write_mbias to a new file at path, a warning on stderr for calls past
+// BSX_MBIAS_CYCLES; errors are printed (bsx_meth.cu)
+int bsx_meth_write_mbias_file(bsx_meth *m, const char *path);
 int bsx_inflate_file(const char *path, std::vector<char> &out);   // gzip / BGZF members -> bytes (bsx_reads.cpp)
 int bsx_host_threads(int requested);   // 0 = BSX_THREADS env or hardware concurrency (capped at 32)
 

@@ -12,12 +12,20 @@
 // atomicMin(first[key], order + 1), then the pile-up kernel lets the alignment through whose claim stands and marks
 // the key 0 = taken for good, so later batches lose against earlier ones.  8 bytes per reference position, allocated
 // on first use.
+//
+// M-bias (bsx_meth_enable_mbias) and per-cycle exclusion (bsx_meth_set_ignore) switch both pile-up kernels to their
+// `Cycles` instantiation: each call also gets its cycle (position in the read as sequenced), read (1 / 2) and C context
+// (CpG / CHG / CHH), excluded calls are dropped from the counters, and the others go into a per-CTA shared-memory
+// histogram [read][context][cycle][meth|unmeth] that is flushed (non-zero bins only) into a device-global u64 one.  That
+// grid is capped at the resident CTAs and strides over the alignments, so one flush serves many alignments.  With both
+// off the kernels are the plain instantiation, which compiles to the same code as before these options existed.
 #include <algorithm>
 #include <cmath>
 #include <cstdio>
 #include <cstring>
 #include <string>
 #include <vector>
+#include <fcntl.h>
 #include <unistd.h>
 #include "bsx_internal.h"
 #include "bsx_common.cuh"
@@ -33,18 +41,37 @@ struct bsx_meth {
     size_t cap = 0; uint32_t stride = 0;
     char *d_seq = nullptr; uint16_t *d_len = nullptr; uint32_t *d_chr = nullptr, *d_pos = nullptr;
     uint8_t *d_strand = nullptr, *d_flags = nullptr; int32_t *d_ins = nullptr, *d_mate = nullptr;
+    // M-bias / exclusion: fixed before the first alignment is piled up
+    bool mbias = false, started = false;
+    int32_t ignore[4] = {0, 0, 0, 0};                 // r1_5p, r1_3p, r2_5p, r2_3p
+    unsigned long long *d_mbias = nullptr;            // MBIAS_BINS counters, then the overflow counter
+    int resident[2] = {0, 0};                         // CTAs of the Cycles pile-up kernels (text, mapped) the device holds at once
 };
 
 namespace {
+
+constexpr int MBIAS_BINS = 2 * 3 * BSX_MBIAS_CYCLES * 2;
+
+// what the Cycles instantiation needs beyond the plain one
+struct MbiasArgs {
+    unsigned long long *hist;     // MBIAS_BINS counters, then the overflow counter (calls at cycle >= BSX_MBIAS_CYCLES);
+                                  // NULL: exclusion only, no histogram to keep
+    int32_t ignore[4];            // r1_5p, r1_3p, r2_5p, r2_3p
+    int readset;                  // mapped single-end batches: 2 = these are read 2
+};
 
 __device__ __forceinline__ uint32_t ref_code(const uint32_t *refcat, uint32_t q) { return (refcat[q >> 4] >> (30 - 2 * (q & 15))) & 3u; }
 
 // One alignment, executed by a warp: get_alignment's trimming (methratio.py:56-64), the bounds test (105) and the
 // pile-up (107-118).  getc(i) = i-th character of SEQ as printed.  Filters (-u / -p) were applied by the caller.
-template <class GetC>
+// Cycles: the call's cycle is its offset in printed SEQ, counted from the far end when SEQ is printed reversed (the two
+// ZS characters differ); calls of read `read2` outside [5p, L - 3p) are dropped; the rest also go into `hist` (shared).
+template <bool Cycles, class GetC>
 __device__ __forceinline__ void pile_alignment(const uint32_t *__restrict__ refcat, const uint32_t *__restrict__ seqinfo, uint32_t n_seq,
                                                uint32_t *meth, uint32_t *depth, unsigned long long *n_valid, const bsx_meth_opts &o,
-                                               uint32_t k, long long pos, long long len, int st, int ins, long long mate_pos, bool sam, int lane, GetC getc) {
+                                               uint32_t k, long long pos, long long len, int st, int ins, long long mate_pos, bool sam, int lane, GetC getc,
+                                               const MbiasArgs &mb = MbiasArgs{}, int read2 = 0, uint32_t *hist = nullptr) {
+    const int L = (int)len;                                  // printed length, before trimming
     const uint32_t *anchor = seqinfo, *size = seqinfo + n_seq + 1;
     long long start = 0;
     const int N = o.trim_fillin;
@@ -67,12 +94,52 @@ __device__ __forceinline__ void pile_alignment(const uint32_t *__restrict__ refc
     const uint32_t base = anchor[k] + (uint32_t)pos;
     const uint32_t match = first_minus ? 2u : 1u;           // '+': C (converted reads show T), '-': G (A)
     const char cm = first_minus ? 'G' : 'C', cc = first_minus ? 'A' : 'T';
-    for (int i = lane; i < (int)len; i += 32) {
-        if (ref_code(refcat, base + (uint32_t)i) != match) continue;
-        const char c = getc((int)start + i);
-        if (c == cc) atomicAdd(depth + base + i, 1u);
-        else if (c == cm) { atomicAdd(meth + base + i, 1u); atomicAdd(depth + base + i, 1u); }
+    if constexpr (!Cycles) {
+        for (int i = lane; i < (int)len; i += 32) {
+            if (ref_code(refcat, base + (uint32_t)i) != match) continue;
+            const char c = getc((int)start + i);
+            if (c == cc) atomicAdd(depth + base + i, 1u);
+            else if (c == cm) { atomicAdd(meth + base + i, 1u); atomicAdd(depth + base + i, 1u); }
+        }
+    } else {
+        const bool rev = ((st ^ (st >> 1)) & 1) != 0;
+        const int lo = read2 ? mb.ignore[2] : mb.ignore[0], hi = L - (read2 ? mb.ignore[3] : mb.ignore[1]);
+        uint32_t *h = hist + read2 * (3 * BSX_MBIAS_CYCLES * 2);
+        for (int i = lane; i < (int)len; i += 32) {
+            const uint32_t q = base + (uint32_t)i;
+            if (ref_code(refcat, q) != match) continue;
+            const int j = (int)start + i;
+            const char c = getc(j);
+            const bool is_m = c == cm;
+            if (!is_m && c != cc) continue;
+            const int cyc = rev ? L - 1 - j : j;
+            if (cyc < lo || cyc >= hi) continue;
+            atomicAdd(depth + q, 1u);
+            if (is_m) atomicAdd(meth + q, 1u);
+            // context on the call's strand: '+' looks at q+1, q+2 for G, '-' at q-1, q-2 for C; non-ACGT and the zero
+            // margins / pads read as A, i.e. H
+            const uint32_t want = 3u - match;
+            const uint32_t c1 = first_minus ? ref_code(refcat, q - 1u) : ref_code(refcat, q + 1u);
+            const uint32_t c2 = first_minus ? ref_code(refcat, q - 2u) : ref_code(refcat, q + 2u);
+            const int ctx = c1 == want ? 0 : (c2 == want ? 1 : 2);
+            if (!mb.hist) continue;
+            if (cyc < BSX_MBIAS_CYCLES) atomicAdd(h + (ctx * BSX_MBIAS_CYCLES + cyc) * 2 + (is_m ? 0 : 1), 1u);
+            else atomicAdd(mb.hist + MBIAS_BINS, 1ull);
+        }
     }
+}
+
+// Cycles: the per-CTA histogram, zeroed before and flushed (non-zero bins) after the CTA's alignments; out == NULL
+// (exclusion without M-bias) skips both
+__device__ __forceinline__ void hist_zero(uint32_t *hist, const unsigned long long *out) {
+    if (!out) return;
+    for (int b = threadIdx.x; b < MBIAS_BINS; b += blockDim.x) hist[b] = 0u;
+    __syncthreads();
+}
+__device__ __forceinline__ void hist_flush(uint32_t *hist, unsigned long long *out) {
+    if (!out) return;
+    __syncthreads();
+    for (int b = threadIdx.x; b < MBIAS_BINS; b += blockDim.x) { const uint32_t v = hist[b]; if (v) atomicAdd(out + b, (unsigned long long)v); }
 }
 
 // what get_alignment hands on (before trimming): sequence index, 0-based position, printed length, strand bits, ...
@@ -124,21 +191,33 @@ __global__ void __launch_bounds__(256) meth_claim_kernel(const uint32_t *__restr
     if (a < n && parsed_alignment(o, n_seq, a, lens, chr, pos0, strand, insert, mate_pos, flags, v) && dup_key(seqinfo, n_seq, v, key)) atomicMin(first + key, a + 1u);
 }
 
-// alignments parsed from SAM / BSP text on the host: one warp per alignment
+// alignments parsed from SAM / BSP text on the host: one warp per alignment (Cycles: a grid-stride loop of them)
+template <bool Cycles>
 __global__ void __launch_bounds__(256) meth_pileup_kernel(const uint32_t *__restrict__ refcat, const uint32_t *__restrict__ seqinfo, uint32_t n_seq,
                                                           uint32_t *meth, uint32_t *depth, unsigned long long *n_valid, uint32_t *first, bsx_meth_opts o, uint32_t n,
                                                           const char *__restrict__ seqs, uint32_t stride, const uint16_t *__restrict__ lens,
                                                           const uint32_t *__restrict__ chr, const uint32_t *__restrict__ pos0,
                                                           const uint8_t *__restrict__ strand, const int32_t *__restrict__ insert,
-                                                          const int32_t *__restrict__ mate_pos, const uint8_t *__restrict__ flags) {
-    const uint32_t a = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+                                                          const int32_t *__restrict__ mate_pos, const uint8_t *__restrict__ flags, MbiasArgs mb) {
+    const uint32_t w = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     const int lane = threadIdx.x & 31;
-    if (a >= n) return;
-    AlnView v;
-    if (!parsed_alignment(o, n_seq, a, lens, chr, pos0, strand, insert, mate_pos, flags, v)) return;
-    if (first && !dup_holds(first, seqinfo, n_seq, v, a, lane)) return;
-    const char *sq = seqs + (size_t)a * stride;
-    pile_alignment(refcat, seqinfo, n_seq, meth, depth, n_valid, o, v.k, v.pos, v.len, v.st, v.ins, v.mate_pos, v.sam, lane, [sq](int i) { return sq[i]; });
+    auto one = [&](uint32_t a, uint32_t *hist) {
+        AlnView v;
+        if (!parsed_alignment(o, n_seq, a, lens, chr, pos0, strand, insert, mate_pos, flags, v)) return;
+        if (first && !dup_holds(first, seqinfo, n_seq, v, a, lane)) return;
+        const char *sq = seqs + (size_t)a * stride;
+        pile_alignment<Cycles>(refcat, seqinfo, n_seq, meth, depth, n_valid, o, v.k, v.pos, v.len, v.st, v.ins, v.mate_pos, v.sam, lane,
+                               [sq](int i) { return sq[i]; }, mb, (flags[a] & BSX_METH_READ2) ? 1 : 0, hist);
+    };
+    if constexpr (!Cycles) {
+        if (w >= n) return;
+        one(w, nullptr);
+    } else {
+        __shared__ uint32_t hist[MBIAS_BINS];
+        hist_zero(hist, mb.hist);
+        for (uint32_t a = w; a < n; a += (gridDim.x * blockDim.x) >> 5) one(a, hist);
+        hist_flush(hist, mb.hist);
+    }
 }
 
 __device__ __forceinline__ char comp_char(char c) {   // rev_char[] (param.cpp:166-177)
@@ -195,24 +274,45 @@ __global__ void __launch_bounds__(256) meth_claim_mapped_kernel(const uint32_t *
         atomicMin(first + key, u + 1u);
 }
 
-// pile-up of the mapped batch: one warp per read (PE: per mate)
+// pile-up of the mapped batch: one warp per read (PE: per mate; Cycles: a grid-stride loop of them)
+template <bool Cycles>
 __global__ void __launch_bounds__(256) meth_pileup_mapped_kernel(const uint32_t *__restrict__ refcat, const uint32_t *__restrict__ seqinfo, uint32_t n_seq,
                                                                  uint32_t *meth, uint32_t *depth, unsigned long long *n_valid, uint32_t *first, bsx_meth_opts o,
                                                                  int sam, int report_repeat_hits, uint32_t n, int mates, uint32_t stride,
                                                                  const uint8_t *__restrict__ seq_a, const uint8_t *__restrict__ seq_b,
                                                                  const bsx_rec *__restrict__ out_a, const bsx_rec *__restrict__ out_b,
-                                                                 const bsx_pair_rec *__restrict__ out_pair) {
-    const uint32_t u = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+                                                                 const bsx_pair_rec *__restrict__ out_pair, MbiasArgs mb) {
+    const uint32_t w = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     const int lane = threadIdx.x & 31;
-    if (u >= n * (uint32_t)mates) return;
-    AlnView v; bool rev;
-    if (!mapped_alignment(o, sam, report_repeat_hits, u, mates, out_a, out_b, out_pair, v, rev)) return;
-    if (first && !dup_holds(first, seqinfo, n_seq, v, u, lane)) return;
-    const uint32_t r = mates == 2 ? u >> 1 : u;
-    const uint8_t *rd = ((mates == 2 && (u & 1u)) ? seq_b : seq_a) + (size_t)r * stride;
-    const int lp = (int)v.len;
-    pile_alignment(refcat, seqinfo, n_seq, meth, depth, n_valid, o, v.k, v.pos, v.len, v.st, v.ins, v.mate_pos, v.sam, lane,
-                   [rd, rev, lp](int i) { return rev ? comp_char((char)rd[lp - 1 - i]) : (char)rd[i]; });
+    auto one = [&](uint32_t u, uint32_t *hist) {
+        AlnView v; bool rev;
+        if (!mapped_alignment(o, sam, report_repeat_hits, u, mates, out_a, out_b, out_pair, v, rev)) return;
+        if (first && !dup_holds(first, seqinfo, n_seq, v, u, lane)) return;
+        const uint32_t r = mates == 2 ? u >> 1 : u;
+        const uint8_t *rd = ((mates == 2 && (u & 1u)) ? seq_b : seq_a) + (size_t)r * stride;
+        const int lp = (int)v.len;
+        const int read2 = mates == 2 ? (int)(u & 1u) : (mb.readset == 2 ? 1 : 0);     // mate b / readset 2 print FLAG 0x80
+        pile_alignment<true>(refcat, seqinfo, n_seq, meth, depth, n_valid, o, v.k, v.pos, v.len, v.st, v.ins, v.mate_pos, v.sam, lane,
+                             [rd, rev, lp](int i) { return rev ? comp_char((char)rd[lp - 1 - i]) : (char)rd[i]; }, mb, read2, hist);
+    };
+    if constexpr (!Cycles) {
+        // the same steps as `one`, written out: through the lambda, ptxas allocates this instantiation differently
+        const uint32_t u = w;
+        if (u >= n * (uint32_t)mates) return;
+        AlnView v; bool rev;
+        if (!mapped_alignment(o, sam, report_repeat_hits, u, mates, out_a, out_b, out_pair, v, rev)) return;
+        if (first && !dup_holds(first, seqinfo, n_seq, v, u, lane)) return;
+        const uint32_t r = mates == 2 ? u >> 1 : u;
+        const uint8_t *rd = ((mates == 2 && (u & 1u)) ? seq_b : seq_a) + (size_t)r * stride;
+        const int lp = (int)v.len;
+        pile_alignment<false>(refcat, seqinfo, n_seq, meth, depth, n_valid, o, v.k, v.pos, v.len, v.st, v.ins, v.mate_pos, v.sam, lane,
+                              [rd, rev, lp](int i) { return rev ? comp_char((char)rd[lp - 1 - i]) : (char)rd[i]; });
+    } else {
+        __shared__ uint32_t hist[MBIAS_BINS];
+        hist_zero(hist, mb.hist);
+        for (uint32_t u = w; u < n * (uint32_t)mates; u += (gridDim.x * blockDim.x) >> 5) one(u, hist);
+        hist_flush(hist, mb.hist);
+    }
 }
 
 // -g: every reference "CG": both counters of the C take the G's, the G's become 0 (methratio.py:122-131)
@@ -249,6 +349,31 @@ int ensure_dup_table(bsx_meth *m) {
     BSX_CUDA_CHECK(cudaEventCreateWithFlags(&m->dup_order, cudaEventDisableTiming));
     BSX_CUDA_CHECK(cudaDeviceSynchronize());
     return BSX_OK;
+}
+
+bool cycles_on(const bsx_meth *m) { return m->mbias || m->ignore[0] || m->ignore[1] || m->ignore[2] || m->ignore[3]; }
+
+// the Cycles kernels' grid cap and, with M-bias on, their histogram (zeroed), on the first pile-up that needs them
+int ensure_cycles(bsx_meth *m) {
+    if (m->resident[0]) return BSX_OK;
+    if (m->mbias) {
+        BSX_CUDA_CHECK(cudaMalloc(&m->d_mbias, (MBIAS_BINS + 1) * sizeof(unsigned long long)));
+        BSX_CUDA_CHECK(cudaMemset(m->d_mbias, 0, (MBIAS_BINS + 1) * sizeof(unsigned long long)));
+    }
+    int dev = 0, sms = 0, per_sm[2] = {0, 0};
+    BSX_CUDA_CHECK(cudaGetDevice(&dev));
+    BSX_CUDA_CHECK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+    BSX_CUDA_CHECK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm[0], meth_pileup_kernel<true>, 256, 0));
+    BSX_CUDA_CHECK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm[1], meth_pileup_mapped_kernel<true>, 256, 0));
+    for (int i = 0; i < 2; i++) m->resident[i] = std::max(per_sm[i], 1) * sms;
+    BSX_CUDA_CHECK(cudaDeviceSynchronize());
+    return BSX_OK;
+}
+MbiasArgs mbias_args(const bsx_meth *m, int readset) {
+    MbiasArgs a{};
+    a.hist = m->d_mbias; a.readset = readset;          // NULL without M-bias: the kernels keep no histogram
+    for (int i = 0; i < 4; i++) a.ignore[i] = m->ignore[i];
+    return a;
 }
 
 int combine_once(bsx_meth *m, const bsx_meth_opts *o) {
@@ -295,7 +420,7 @@ extern "C" int bsx_meth_create(const bsx_index *ix, bsx_meth **out) {
 
 extern "C" int bsx_meth_destroy(bsx_meth *m) {
     if (!m) return BSX_OK;
-    cudaFree(m->d_meth); cudaFree(m->d_depth); cudaFree(m->d_valid); cudaFree(m->d_first);
+    cudaFree(m->d_meth); cudaFree(m->d_depth); cudaFree(m->d_valid); cudaFree(m->d_first); cudaFree(m->d_mbias);
     if (m->dup_order) cudaEventDestroy(m->dup_order);
     cudaFree(m->d_seq); cudaFree(m->d_len); cudaFree(m->d_chr); cudaFree(m->d_pos); cudaFree(m->d_strand); cudaFree(m->d_flags); cudaFree(m->d_ins); cudaFree(m->d_mate);
     delete m;
@@ -309,6 +434,7 @@ extern "C" int bsx_meth_add(bsx_meth *m, const bsx_meth_opts *o, uint32_t n, con
     if (m->combined) { bsx_set_error("bsx_meth_add: counters were already combined (-g); create a new bsx_meth"); return BSX_ERR_ARG; }
     BSX_CUDA_CHECK(cudaSetDevice(m->ix->device));
     if (n) {
+        m->started = true;
         int rc = ensure_staging(m, n, stride); if (rc) return rc;
         BSX_CUDA_CHECK(cudaMemcpy2D(m->d_seq, m->stride, seqs, stride, stride, n, cudaMemcpyHostToDevice));
         BSX_CUDA_CHECK(cudaMemcpy(m->d_len, lens, (size_t)n * 2, cudaMemcpyHostToDevice));
@@ -325,8 +451,16 @@ extern "C" int bsx_meth_add(bsx_meth *m, const bsx_meth_opts *o, uint32_t n, con
             BSX_CUDA_CHECK(cudaGetLastError());
         }
         const unsigned blocks = (unsigned)(((uint64_t)n * 32 + 255) / 256);
-        meth_pileup_kernel<<<blocks, 256>>>(m->ix->d_refcat, m->ix->d_seqinfo, m->ix->n_seq, m->d_meth, m->d_depth, m->d_valid,
-                                            o->rm_dup ? m->d_first : nullptr, *o, n, m->d_seq, m->stride, m->d_len, m->d_chr, m->d_pos, m->d_strand, m->d_ins, m->d_mate, m->d_flags);
+        if (!cycles_on(m)) {
+            meth_pileup_kernel<false><<<blocks, 256>>>(m->ix->d_refcat, m->ix->d_seqinfo, m->ix->n_seq, m->d_meth, m->d_depth, m->d_valid,
+                                                       o->rm_dup ? m->d_first : nullptr, *o, n, m->d_seq, m->stride, m->d_len, m->d_chr, m->d_pos, m->d_strand,
+                                                       m->d_ins, m->d_mate, m->d_flags, MbiasArgs{});
+        } else {
+            rc = ensure_cycles(m); if (rc) return rc;
+            meth_pileup_kernel<true><<<std::min<unsigned>(blocks, (unsigned)m->resident[0]), 256>>>(
+                m->ix->d_refcat, m->ix->d_seqinfo, m->ix->n_seq, m->d_meth, m->d_depth, m->d_valid, o->rm_dup ? m->d_first : nullptr, *o, n, m->d_seq,
+                m->stride, m->d_len, m->d_chr, m->d_pos, m->d_strand, m->d_ins, m->d_mate, m->d_flags, mbias_args(m, 0));
+        }
         BSX_CUDA_CHECK(cudaGetLastError());
     }
     if (n_valid) {
@@ -338,11 +472,13 @@ extern "C" int bsx_meth_add(bsx_meth *m, const bsx_meth_opts *o, uint32_t n, con
 }
 
 // pile up the batch a mapper has just mapped (called by bsx_api.cu::run_slot on the batch's stream)
-int bsx_meth_pile_mapped(bsx_meth *m, const bsx_meth_opts *o, int sam, int report_repeat_hits, uint32_t n, int mates, uint32_t stride,
+int bsx_meth_pile_mapped(bsx_meth *m, const bsx_meth_opts *o, int sam, int report_repeat_hits, uint32_t n, int mates, int readset, uint32_t stride,
                          const uint8_t *seq_a, const uint8_t *seq_b, const bsx_rec *out_a, const bsx_rec *out_b, const bsx_pair_rec *out_pair,
                          cudaStream_t st) {
     if (!m || !o || n == 0) return BSX_OK;
     if (m->combined) { bsx_set_error("bsx_meth: counters were already combined (-g); create a new bsx_meth"); return BSX_ERR_ARG; }
+    m->started = true;
+    if (cycles_on(m)) { int rc = ensure_cycles(m); if (rc) return rc; }
     if (o->rm_dup) {
         // file order = batch order: this batch's claims start when the previous batch has resolved its own (the batches
         // alternate between two streams).  Paired-end BSP output goes to two files, whose concatenation is the script's
@@ -354,9 +490,14 @@ int bsx_meth_pile_mapped(bsx_meth *m, const bsx_meth_opts *o, int sam, int repor
         BSX_CUDA_CHECK(cudaGetLastError());
     }
     const unsigned blocks = (unsigned)(((uint64_t)n * (uint64_t)mates * 32 + 255) / 256);
-    meth_pileup_mapped_kernel<<<blocks, 256, 0, st>>>(m->ix->d_refcat, m->ix->d_seqinfo, m->ix->n_seq, m->d_meth, m->d_depth, m->d_valid,
-                                                       o->rm_dup ? m->d_first : nullptr, *o, sam, report_repeat_hits, n, mates, stride, seq_a, seq_b,
-                                                       out_a, out_b, out_pair);
+    if (!cycles_on(m))
+        meth_pileup_mapped_kernel<false><<<blocks, 256, 0, st>>>(m->ix->d_refcat, m->ix->d_seqinfo, m->ix->n_seq, m->d_meth, m->d_depth, m->d_valid,
+                                                                 o->rm_dup ? m->d_first : nullptr, *o, sam, report_repeat_hits, n, mates, stride, seq_a, seq_b,
+                                                                 out_a, out_b, out_pair, MbiasArgs{});
+    else
+        meth_pileup_mapped_kernel<true><<<std::min<unsigned>(blocks, (unsigned)m->resident[1]), 256, 0, st>>>(
+            m->ix->d_refcat, m->ix->d_seqinfo, m->ix->n_seq, m->d_meth, m->d_depth, m->d_valid, o->rm_dup ? m->d_first : nullptr, *o, sam,
+            report_repeat_hits, n, mates, stride, seq_a, seq_b, out_a, out_b, out_pair, mbias_args(m, readset));
     BSX_CUDA_CHECK(cudaGetLastError());
     if (o->rm_dup) BSX_CUDA_CHECK(cudaEventRecord(m->dup_order, st));
     return BSX_OK;
@@ -431,4 +572,66 @@ extern "C" size_t bsx_meth_write(bsx_meth *m, const bsx_meth_opts *o, const char
     }
     if (stats) { stats[0] = nc; stats[1] = nd; }
     return written;
+}
+
+extern "C" int bsx_meth_enable_mbias(bsx_meth *m) {
+    if (!m) { bsx_set_error("bsx_meth_enable_mbias: bad argument"); return BSX_ERR_ARG; }
+    if (m->started) { bsx_set_error("bsx_meth_enable_mbias: alignments were already piled up; enable M-bias first"); return BSX_ERR_ARG; }
+    m->mbias = true;
+    return BSX_OK;
+}
+
+extern "C" int bsx_meth_set_ignore(bsx_meth *m, const int32_t ignore[4]) {
+    if (!m || !ignore) { bsx_set_error("bsx_meth_set_ignore: bad argument"); return BSX_ERR_ARG; }
+    if (m->started) { bsx_set_error("bsx_meth_set_ignore: alignments were already piled up; set the exclusion first"); return BSX_ERR_ARG; }
+    for (int i = 0; i < 4; i++)
+        if (ignore[i] < 0) { bsx_set_error("bsx_meth_set_ignore: cycle counts must be >= 0 (got %d)", ignore[i]); return BSX_ERR_ARG; }
+    for (int i = 0; i < 4; i++) m->ignore[i] = ignore[i];
+    return BSX_OK;
+}
+
+extern "C" int bsx_meth_mbias(bsx_meth *m, uint64_t *out, uint64_t *overflow) {
+    if (!m || !out) { bsx_set_error("bsx_meth_mbias: bad argument"); return BSX_ERR_ARG; }
+    if (!m->mbias) { bsx_set_error("bsx_meth_mbias: M-bias was not enabled (bsx_meth_enable_mbias)"); return BSX_ERR_ARG; }
+    BSX_CUDA_CHECK(cudaSetDevice(m->ix->device));
+    BSX_CUDA_CHECK(cudaDeviceSynchronize());           // in-process batches flush from two streams
+    std::vector<unsigned long long> h(MBIAS_BINS + 1, 0ull);
+    if (m->d_mbias) BSX_CUDA_CHECK(cudaMemcpy(h.data(), m->d_mbias, h.size() * sizeof(unsigned long long), cudaMemcpyDeviceToHost));
+    for (int b = 0; b < MBIAS_BINS; b++) out[b] = h[b];
+    if (overflow) *overflow = h[MBIAS_BINS];
+    return BSX_OK;
+}
+
+// the report to fd; *overflow (may be NULL) from the same download
+static size_t write_mbias(bsx_meth *m, int fd, uint64_t *overflow) {
+    std::vector<uint64_t> h(MBIAS_BINS);
+    if (bsx_meth_mbias(m, h.data(), overflow) != BSX_OK) return 0;
+    std::string s = "context\tread\tcycle\tmethylated\tunmethylated\tratio\n";
+    Sink o{&s};
+    static const char *const ctx[3] = {"CpG", "CHG", "CHH"};
+    for (int c = 0; c < 3; c++)
+        for (int r = 0; r < 2; r++)
+            for (int y = 0; y < BSX_MBIAS_CYCLES; y++) {
+                const uint64_t *b = &h[((size_t)(r * 3 + c) * BSX_MBIAS_CYCLES + y) * 2];
+                if (b[0] + b[1] == 0) continue;
+                o.put(ctx[c], 3); o.putc('\t'); o.putc((char)('1' + r)); o.putc('\t'); o.putu((unsigned long long)y + 1); o.putc('\t');
+                o.putu(b[0]); o.putc('\t'); o.putu(b[1]); o.putc('\t'); o.putf3((double)b[0] / (double)(b[0] + b[1])); o.putc('\n');
+            }
+    size_t off = 0;
+    while (off < s.size()) { const ssize_t w = write(fd, s.data() + off, s.size() - off); if (w <= 0) break; off += (size_t)w; }
+    return off;
+}
+
+extern "C" size_t bsx_meth_write_mbias(bsx_meth *m, int fd) { return write_mbias(m, fd, nullptr); }
+
+int bsx_meth_write_mbias_file(bsx_meth *m, const char *path) {
+    const int fd = open(path, O_WRONLY | O_CREAT | O_TRUNC, 0644);
+    if (fd < 0) { fprintf(stderr, "failed to open M-bias output file: %s\n", path); return BSX_ERR_IO; }
+    uint64_t over = 0;
+    const size_t w = write_mbias(m, fd, &over);
+    close(fd);
+    if (w == 0) { fprintf(stderr, "%s\n", bsx_last_error()); return BSX_ERR_IO; }
+    if (over) fprintf(stderr, "warning: %llu methylation calls at cycle %d or later are in the table but not in the M-bias report\n",
+                      (unsigned long long)over, BSX_MBIAS_CYCLES + 1);
+    return BSX_OK;
 }

@@ -7,6 +7,10 @@
 // `samtools view -X`) or BSP output; the format follows the file suffix like the script does.  Text files are
 // memory-mapped and parsed on all host threads; the pile-up, and -r's "first alignment in file order wins", run on the
 // GPU (bsx_meth.cu).  -s (path to samtools) is accepted and ignored: nothing here shells out.
+//
+// Extensions (SAM and BAM input only: BSP records carry no read number):
+//   --mbias FILE               M-bias report (methylation by read, C context and cycle; include/bsmap_b200.h)
+//   --mbias-ignore A,B,C,D     drop calls in the first A / last B cycles of read 1 and first C / last D of read 2
 #include <chrono>
 #include <cstdio>
 #include <cstdlib>
@@ -27,6 +31,9 @@ struct MOpts {
     std::string out, ref, chroms;
     bsx_meth_opts o;
     bool quiet = false;
+    std::string mbias;                       // --mbias FILE
+    bool ignore_set = false;
+    int32_t ignore[4] = {0, 0, 0, 0};        // --mbias-ignore
     std::vector<std::string> files;
 };
 
@@ -47,7 +54,8 @@ void parse(int argc, char **argv, MOpts &m) {
     struct Def { char s; const char *l; bool val; };
     static const Def defs[] = {{'o', "out", true}, {'d', "ref", true}, {'c', "chr", true}, {'s', "sam-path", true}, {'u', "unique", false},
                                {'p', "pair", false}, {'z', "zero-meth", false}, {'q', "quiet", false}, {'r', "remove-duplicate", false},
-                               {'t', "trim-fillin", true}, {'g', "combine-CpG", false}, {'m', "min-depth", true}, {'h', "help", false}};
+                               {'t', "trim-fillin", true}, {'g', "combine-CpG", false}, {'m', "min-depth", true}, {'h', "help", false},
+                               {'\1', "mbias", true}, {'\2', "mbias-ignore", true}};   // long only
     auto apply = [&](char c, const char *v) {
         if (!v) v = "";
         switch (c) {
@@ -63,7 +71,17 @@ void parse(int argc, char **argv, MOpts &m) {
             case 't': { char *e; long x = strtol(v, &e, 10); if (*e || e == v) usage_error("option -t: invalid integer value"); m.o.trim_fillin = (int)x; } break;
             case 'g': m.o.combine_cpg = 1; break;
             case 'm': { char *e; long x = strtol(v, &e, 10); if (*e || e == v) usage_error("option -m: invalid integer value"); m.o.min_depth = (int)x; } break;
-            case 'h': printf("Usage: methratio [options] BSMAP_MAPPING_FILES\n  -o FILE -d FILE [-c CHR] [-u] [-p] [-z] [-q] [-r] [-t N] [-g] [-m FOLD]\n"); exit(0);
+            case '\1': m.mbias = v; break;
+            case '\2': {
+                const char *q = v;
+                for (int k = 0; k < 4; k++) {
+                    char *e; const long x = strtol(q, &e, 10);
+                    if (e == q || x < 0 || x > 0x7fffffff || *e != (k < 3 ? ',' : '\0')) usage_error("option --mbias-ignore: expected four non-negative integers A,B,C,D");
+                    m.ignore[k] = (int32_t)x; q = e + 1;
+                }
+                m.ignore_set = true;
+            } break;
+            case 'h': printf("Usage: methratio [options] BSMAP_MAPPING_FILES\n  -o FILE -d FILE [-c CHR] [-u] [-p] [-z] [-q] [-r] [-t N] [-g] [-m FOLD] [--mbias FILE] [--mbias-ignore A,B,C,D]\n"); exit(0);
         }
     };
     for (int i = 1; i < argc; i++) {
@@ -82,7 +100,7 @@ void parse(int argc, char **argv, MOpts &m) {
         }
         for (const char *c = a + 1; *c; c++) {
             const Def *d = nullptr;
-            for (const Def &x : defs) if (*c == x.s) d = &x;
+            for (const Def &x : defs) if (*c == x.s && *c > ' ') d = &x;
             if (!d) usage_error((std::string("no such option: -") + *c).c_str());
             if (d->val) { const char *v = c[1] ? c + 1 : (i + 1 < argc ? argv[++i] : nullptr); if (!v) usage_error("option requires an argument"); apply(d->s, v); break; }
             apply(d->s, nullptr);
@@ -121,8 +139,15 @@ bool parse_line(const char *b, const char *e, bool sam, const std::unordered_map
             if (v & 0x4) return false;
             if (v & 0x100) fl |= BSX_METH_SECONDARY;
             if (v & 0x2) fl |= BSX_METH_PROPER;
+            if (v & 0x80) fl |= BSX_METH_READ2;
         } else {
-            for (uint32_t i = 0; i < f[1].n; i++) { const char c = f[1].p[i]; if (c == 'u') return false; if (c == 's') fl |= BSX_METH_SECONDARY; if (c == 'P') fl |= BSX_METH_PROPER; }
+            for (uint32_t i = 0; i < f[1].n; i++) {
+                const char c = f[1].p[i];
+                if (c == 'u') return false;
+                if (c == 's') fl |= BSX_METH_SECONDARY;
+                if (c == 'P') fl |= BSX_METH_PROPER;
+                if (c == '2') fl |= BSX_METH_READ2;
+            }
         }
         auto it = chrom.find(std::string(f[2].p, f[2].n));
         if (it == chrom.end()) return false;
@@ -200,7 +225,8 @@ bool pile_bam(const std::string &path, const std::unordered_map<std::string, uin
                 if (flag & 0x4) continue;                                    // 'u'
                 if (ref_id < 0 || ref_id >= (int32_t)ref_to_chr.size() || ref_to_chr[(size_t)ref_id] < 0) continue;   // cr not in options.chroms
                 Aln a;
-                a.flags = (uint8_t)(BSX_METH_SAM | ((flag & 0x100) ? BSX_METH_SECONDARY : 0u) | ((flag & 0x2) ? BSX_METH_PROPER : 0u));
+                a.flags = (uint8_t)(BSX_METH_SAM | ((flag & 0x100) ? BSX_METH_SECONDARY : 0u) | ((flag & 0x2) ? BSX_METH_PROPER : 0u) |
+                                   ((flag & 0x80) ? BSX_METH_READ2 : 0u));
                 a.chr = (uint32_t)ref_to_chr[(size_t)ref_id]; a.pos = (uint32_t)pos; a.insert = tlen; a.mate = next_pos;
                 char *sq = bases[t].data() + used;
                 for (int32_t i = 0; i < l_seq; i++) sq[i] = nt16[(q[off_seq + ((size_t)i >> 1)] >> ((~i & 1) << 2)) & 15];
@@ -246,6 +272,13 @@ extern "C" int bsx_methratio_main(int argc, char **argv) {
     if (m.ref.empty()) usage_error("Missing reference file, use -d or --ref option.");
     if (m.out.empty()) usage_error("Missing output file name, use -o or --out option.");
     if (m.files.empty()) usage_error("Require at least one BSMAP_MAPPING_FILE.");
+    const bool cycles = !m.mbias.empty() || m.ignore_set;
+    if (cycles)
+        for (const std::string &f : m.files) {
+            std::string suf = f.size() >= 4 ? f.substr(f.size() - 4) : "";
+            for (char &c : suf) c = (char)toupper((unsigned char)c);
+            if (suf != ".SAM" && suf != ".BAM") usage_error(("--mbias / --mbias-ignore need SAM or BAM input (BSP records carry no read number): " + f).c_str());
+        }
     const int threads = bsx_host_threads(0);
 
     disp(m, ("reading reference " + m.ref + " ...").c_str());
@@ -275,6 +308,8 @@ extern "C" int bsx_methratio_main(int argc, char **argv) {
     for (size_t k = 0; k < seqs.size(); k++) { np.push_back(names[k].c_str()); sp.push_back(seqs[k].data()); ln.push_back((uint32_t)seqs[k].size()); }
     bsx_index *ix = nullptr; bsx_meth *mh = nullptr;
     if (bsx_index_create_packed((int)seqs.size(), np.data(), sp.data(), ln.data(), 0, &ix) != BSX_OK || bsx_meth_create(ix, &mh) != BSX_OK) {
+        fprintf(stderr, "%s\n", bsx_last_error()); return 1; }
+    if ((!m.mbias.empty() && bsx_meth_enable_mbias(mh) != BSX_OK) || (m.ignore_set && bsx_meth_set_ignore(mh, m.ignore) != BSX_OK)) {
         fprintf(stderr, "%s\n", bsx_last_error()); return 1; }
 
     const double t_ix = now_s();
@@ -358,6 +393,10 @@ extern "C" int bsx_methratio_main(int argc, char **argv) {
     uint64_t stats[2] = {0, 0};
     bsx_meth_write(mh, &m.o, sp.data(), ln.data(), selected.data(), threads, ofd, stats);
     close(ofd);
+    if (!m.mbias.empty()) {
+        disp(m, ("writing " + m.mbias + " ...").c_str());
+        if (bsx_meth_write_mbias_file(mh, m.mbias.c_str()) != BSX_OK) return 1;
+    }
     if (getenv("BSX_CLI_TIMING"))
         fprintf(stderr, "[bsx timing] reference FASTA %.3f s || CUDA context (ready at %.3f s), packed reference + counters %.3f s, parse + pile-up %.3f s, report %.3f s\n",
                 t_fa - t_start, t_ctx - t_start, t_ix - t_ctx, t_pile - t_ix, now_s() - t_pile);

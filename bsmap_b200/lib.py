@@ -66,7 +66,11 @@ EXPORTS = [
     "bsx_index_create_packed", "bsx_index_save_packed", "bsx_index_create_from_packed", "bsx_meth_opts_default", "bsx_meth_create", "bsx_meth_destroy", "bsx_meth_add", "bsx_meth_download",
     "bsx_meth_write", "bsx_methratio_main", "bsx_sam_to_sorted_bam", "bsx_mapper_attach_meth", "bsx_meth_valid_count",
     "bsx_packed_stride", "bsx_pack_reads", "bsx_map_se_packed", "bsx_map_pe_packed", "bsx_batch_upload_packed",
+    "bsx_meth_enable_mbias", "bsx_meth_set_ignore", "bsx_meth_mbias", "bsx_meth_write_mbias",
 ]
+
+METH_READ2 = 8        # BSX_METH_READ2: alignment flag, read 2 (FLAG 0x80)
+MBIAS_CYCLES = 512    # BSX_MBIAS_CYCLES
 
 _lib = None
 
@@ -147,6 +151,11 @@ def load():
     L.bsx_meth_valid_count.argtypes = [vp, C.POINTER(C.c_uint64)]
     L.bsx_meth_write.restype = sz
     L.bsx_meth_write.argtypes = [vp, C.POINTER(MethOpts), pp, vp, vp, i32, i32, C.POINTER(C.c_uint64)]
+    L.bsx_meth_enable_mbias.argtypes = [vp]
+    L.bsx_meth_set_ignore.argtypes = [vp, C.POINTER(C.c_int32)]
+    L.bsx_meth_mbias.argtypes = [vp, vp, C.POINTER(C.c_uint64)]
+    L.bsx_meth_write_mbias.restype = sz
+    L.bsx_meth_write_mbias.argtypes = [vp, i32]
     L.bsx_packed_stride.restype = sz
     L.bsx_packed_stride.argtypes = [u32]
     L.bsx_pack_reads.argtypes = [u32, vp, u32, vp, vp, C.POINTER(C.c_uint64), i32]

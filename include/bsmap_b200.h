@@ -288,7 +288,31 @@ int bsx_meth_download(bsx_meth *m, const bsx_meth_opts *o, uint32_t k, uint32_t 
  * stats: covered cytosines, their summed depth.  Returns bytes written. */
 size_t bsx_meth_write(bsx_meth *m, const bsx_meth_opts *o, const char *const *seqs, const uint32_t *lens,
                       const uint8_t *chroms /* n_seq flags or NULL */, int threads, int fd, uint64_t *stats);
-/* the methratio.py command line: -o -d [-c -u -p -z -q -r -t -g -m -s] files... (SAM, BAM and BSP; -s is ignored) */
+/* --- M-bias: methylation level by position in the read, and per-cycle exclusion of calls ----------
+ * A call is one increment of the counters above (after -u / -p, -r, -t, mate-overlap removal and the bounds test).
+ * Its cycle is its 0-based offset j in SEQ as printed, or L-1-j when SEQ is printed reversed (the two ZS characters
+ * differ), L being the printed length; its read is 2 when the printed FLAG has 0x80 (bsx_meth_add: BSX_METH_READ2;
+ * in process: mate b of bsx_map_pe, or readset 2 of bsx_map_se), else 1; its context is CpG / CHG / CHH from the
+ * reference on the call's strand (non-ACGT and positions off the sequence count as H). */
+#define BSX_METH_READ2     8u   /* alignment flag: read 2 (FLAG 0x80) -- M-bias and exclusion only       */
+#define BSX_MBIAS_CYCLES   512  /* cycles tracked; calls at later cycles count in the table and in *overflow */
+/* track M-bias from now on.  Must precede the first alignment piled up (BSX_ERR_ARG otherwise). */
+int bsx_meth_enable_mbias(bsx_meth *m);
+/* drop every call of read 1 with cycle < ignore[0] or cycle >= L - ignore[1], and of read 2 with cycle < ignore[2]
+ * or cycle >= L - ignore[3], from the counters and from the M-bias ("valid mappings" and -r are unaffected).  All
+ * zero (the default) drops nothing.  Must precede the first alignment piled up; negative values: BSX_ERR_ARG. */
+int bsx_meth_set_ignore(bsx_meth *m, const int32_t ignore[4] /* r1_5p, r1_3p, r2_5p, r2_3p */);
+/* the M-bias so far (synchronises the device): out has 2 x 3 x BSX_MBIAS_CYCLES x 2 counters, index
+ * ((read * 3 + ctx) * BSX_MBIAS_CYCLES + cycle) * 2 + {0 methylated, 1 unmethylated} with read 0 / 1 = read 1 / 2 and
+ * ctx 0 / 1 / 2 = CpG / CHG / CHH; *overflow (may be NULL): calls at cycle >= BSX_MBIAS_CYCLES.  BSX_ERR_ARG when
+ * M-bias was not enabled. */
+int bsx_meth_mbias(bsx_meth *m, uint64_t *out, uint64_t *overflow);
+/* write the M-bias report to fd: a header line "context read cycle methylated unmethylated ratio" (tab-separated),
+ * then per context CpG, CHG, CHH, per read 1, 2, per 1-based cycle ascending, a row when methylated + unmethylated
+ * > 0, ratio = %.3f of methylated / (methylated + unmethylated).  Returns bytes written (0 on error). */
+size_t bsx_meth_write_mbias(bsx_meth *m, int fd);
+/* the methratio.py command line: -o -d [-c -u -p -z -q -r -t -g -m -s] files... (SAM, BAM and BSP; -s is ignored);
+ * extensions: --mbias FILE (the M-bias report) and --mbias-ignore A,B,C,D (bsx_meth_set_ignore), SAM and BAM only */
 int bsx_methratio_main(int argc, char **argv);
 
 /* --- the bsmap command line (main.cpp:441-476): same options, same output files -------------- */
