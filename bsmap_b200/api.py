@@ -7,7 +7,7 @@ import os
 import numpy as np
 
 from . import lib as _l
-from .lib import MBIAS_CYCLES, METH_READ2, PAIR_REC, REC, BsxError, IndexInfo, MethOpts, Params, Stats, check, load, strs
+from .lib import CT_SNP_MODES, MBIAS_CYCLES, METH_READ2, PAIR_REC, REC, BsxError, IndexInfo, MethOpts, Params, Stats, check, load, strs
 
 
 def make_params(s=16, I=4, v=2, w=1000, r=1, m=28, x=500, n=0, pairend=0, S=0, f=5, L=144,
@@ -451,6 +451,20 @@ class Meth:
         if w == 0:
             check(1)
         return w
+
+    def enable_ct_snp(self, mode: str):
+        """count C/T SNP evidence from the opposite strand and write the 12-column table; mode "no-action",
+        "correct" or "skip" (include/bsmap_b200.h); before the first add / mapped batch"""
+        if mode not in CT_SNP_MODES:
+            raise ValueError("ct-snp mode must be one of %s, not %r" % (", ".join(CT_SNP_MODES), mode))
+        check(load().bsx_meth_enable_ct_snp(self.h, CT_SNP_MODES[mode]))
+
+    def ct_snp_counters(self, k: int):
+        """(confirm, snp) evidence of reference sequence k, after -g combining"""
+        n = load().bsx_index_seq_size(self.index.h, k)
+        c, s = np.zeros(n, dtype=np.uint32), np.zeros(n, dtype=np.uint32)
+        check(load().bsx_meth_download_ct_snp(self.h, C.byref(self.o), k, c.ctypes.data, s.ctypes.data))
+        return c, s
 
     def write(self, seqs, fd: int, chroms=None, threads=0):
         keep = [s if isinstance(s, bytes) else bytes(s) for s in seqs]

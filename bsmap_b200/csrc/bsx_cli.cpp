@@ -36,6 +36,7 @@ struct Opts {
     std::string meth_mbias;      // --meth-mbias FILE: the M-bias report of the same calls
     bool meth_ignore_set = false;
     int32_t meth_ignore[4] = {0, 0, 0, 0};   // --meth-ignore A,B,C,D: cycles dropped at the 5' / 3' ends of read 1 / read 2
+    int meth_ct_snp = 0;                     // --meth-ct-snp MODE: BSX_CT_SNP_*
     unsigned batch = 1u << 17;   // reads per GPU batch: small enough to keep the three host stages overlapped
     std::string gpus;            // -g: number of devices (default: all visible) or a comma list of device ids; output stays in input order
 };
@@ -79,7 +80,9 @@ void usage() {
            "                           methratio.py's -u -p -z -g -r -t -m\n"
            "       --meth-mbias <str>  with --methratio: also write the M-bias report (methylation by read, context and cycle)\n"
            "       --meth-ignore <A,B,C,D>  with --methratio: drop calls in the first A / last B cycles of read 1 and the\n"
-           "                           first C / last D cycles of read 2, from the table and the M-bias report\n\n");
+           "                           first C / last D cycles of read 2, from the table and the M-bias report\n"
+           "       --meth-ct-snp <no-action|correct|skip>  with --methratio: count C/T SNP evidence from the opposite\n"
+           "                           strand and write the table with eff_CT_count, rev_G_count and rev_GA_count\n\n");
     exit(1);
 }
 
@@ -118,6 +121,10 @@ int get_options(int argc, char **argv, Opts &o) {
                     o.meth_ignore[k] = (int32_t)x; q = e + 1;
                 }
                 o.meth_ignore_set = true;
+            }
+            else if (a == "meth-ct-snp" && i + 1 < argc) {
+                o.meth_ct_snp = bsx_ct_snp_mode(argv[++i]);
+                if (!o.meth_ct_snp) return i;                                                            // "unknown option: <value>"
             }
             else return i;
             continue;
@@ -275,6 +282,7 @@ extern "C" int bsx_cli_main(int argc, char **argv) {
     Opts o; bsx_params_default(&o.p); bsx_meth_opts_default(&o.mo);
     if (int bad = get_options(argc, argv, o)) { printf("unknown option: %s\n", argv[bad]); exit(bad); }
     if (o.meth_out.empty() && (!o.meth_mbias.empty() || o.meth_ignore_set)) { fprintf(stderr, "--meth-mbias and --meth-ignore need --methratio\n"); return 1; }
+    if (o.meth_out.empty() && o.meth_ct_snp) { fprintf(stderr, "--meth-ct-snp needs --methratio\n"); return 1; }
     if (o.qual_threshold != 0) { fprintf(stderr, "-q quality trimming is not supported by the GPU path\n"); return 1; }
     if (o.o.size() > 4) {
         if (o.o.compare(o.o.size() - 4, 4, ".sam") == 0) o.p.out_sam = 1;
@@ -374,6 +382,7 @@ extern "C" int bsx_cli_main(int argc, char **argv) {
         // SAM rules (mate-overlap removal) unless the alignment output is BSP: the table then equals methratio.py run on -o
         if (bsx_meth_create(ix, &mh) != BSX_OK || (!o.meth_mbias.empty() && bsx_meth_enable_mbias(mh) != BSX_OK) ||
             (o.meth_ignore_set && bsx_meth_set_ignore(mh, o.meth_ignore) != BSX_OK) ||
+            (o.meth_ct_snp && bsx_meth_enable_ct_snp(mh, o.meth_ct_snp) != BSX_OK) ||
             bsx_mapper_attach_meth(mp, mh, &o.mo, (p.out_sam || no_text) ? 1 : 0) != BSX_OK) {
             fprintf(stderr, "%s\n", bsx_last_error()); return 1; }
     }

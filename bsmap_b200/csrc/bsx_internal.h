@@ -103,6 +103,8 @@ int bsx_meth_pile_mapped(bsx_meth *m, const bsx_meth_opts *o, int sam, int repor
 // the command lines' M-bias output: bsx_meth_write_mbias to a new file at path, a warning on stderr for calls past
 // BSX_MBIAS_CYCLES; errors are printed (bsx_meth.cu)
 int bsx_meth_write_mbias_file(bsx_meth *m, const char *path);
+// "no-action" / "correct" / "skip" -> BSX_CT_SNP_*, anything else 0 (bsx_meth.cu)
+int bsx_ct_snp_mode(const char *name);
 int bsx_inflate_file(const char *path, std::vector<char> &out);   // gzip / BGZF members -> bytes (bsx_reads.cpp)
 int bsx_host_threads(int requested);   // 0 = BSX_THREADS env or hardware concurrency (capped at 32)
 

@@ -19,6 +19,12 @@
 // histogram [read][context][cycle][meth|unmeth] that is flushed (non-zero bins only) into a device-global u64 one.  That
 // grid is capped at the resident CTAs and strides over the alignments, so one flush serves many alignments.  With both
 // off the kernels are the plain instantiation, which compiles to the same code as before these options existed.
+//
+// C/T SNP evidence (bsx_meth_enable_ct_snp) switches them to their `Snp` instantiation: a base under the read whose
+// reference code is the complement of the call's (G under a '+' hit, C under a '-' hit) is opposite-strand evidence,
+// untouched by bisulfite: the read shows G / C when the genome has the reference C, A / T when it has a T (a C/T SNP).
+// Two more u32 arrays over the same positions count those bases, `confirm` and `snp`, one global atomic per counted
+// base.  The writer then scales or drops a C's line by that evidence.
 #include <algorithm>
 #include <cmath>
 #include <cstdio>
@@ -46,6 +52,9 @@ struct bsx_meth {
     int32_t ignore[4] = {0, 0, 0, 0};                 // r1_5p, r1_3p, r2_5p, r2_3p
     unsigned long long *d_mbias = nullptr;            // MBIAS_BINS counters, then the overflow counter
     int resident[2] = {0, 0};                         // CTAs of the Cycles pile-up kernels (text, mapped) the device holds at once
+    // C/T SNP evidence: fixed before the first alignment is piled up
+    int ct_snp = 0;                                   // BSX_CT_SNP_*, 0 = off
+    uint32_t *d_confirm = nullptr, *d_snp = nullptr;  // n_words * 16 counters each, like d_meth / d_depth
 };
 
 namespace {
@@ -66,11 +75,14 @@ __device__ __forceinline__ uint32_t ref_code(const uint32_t *refcat, uint32_t q)
 // pile-up (107-118).  getc(i) = i-th character of SEQ as printed.  Filters (-u / -p) were applied by the caller.
 // Cycles: the call's cycle is its offset in printed SEQ, counted from the far end when SEQ is printed reversed (the two
 // ZS characters differ); calls of read `read2` outside [5p, L - 3p) are dropped; the rest also go into `hist` (shared).
-template <bool Cycles, class GetC>
+// Snp: a base over the complementary reference code counts into `confirm` (read G on '+' / C on '-') or `snp` (A / T),
+// after the same trimming, bounds test and (Cycles) exclusion as a call.
+template <bool Cycles, bool Snp, class GetC>
 __device__ __forceinline__ void pile_alignment(const uint32_t *__restrict__ refcat, const uint32_t *__restrict__ seqinfo, uint32_t n_seq,
                                                uint32_t *meth, uint32_t *depth, unsigned long long *n_valid, const bsx_meth_opts &o,
                                                uint32_t k, long long pos, long long len, int st, int ins, long long mate_pos, bool sam, int lane, GetC getc,
-                                               const MbiasArgs &mb = MbiasArgs{}, int read2 = 0, uint32_t *hist = nullptr) {
+                                               const MbiasArgs &mb = MbiasArgs{}, int read2 = 0, uint32_t *hist = nullptr,
+                                               uint32_t *confirm = nullptr, uint32_t *snp = nullptr) {
     const int L = (int)len;                                  // printed length, before trimming
     const uint32_t *anchor = seqinfo, *size = seqinfo + n_seq + 1;
     long long start = 0;
@@ -94,9 +106,20 @@ __device__ __forceinline__ void pile_alignment(const uint32_t *__restrict__ refc
     const uint32_t base = anchor[k] + (uint32_t)pos;
     const uint32_t match = first_minus ? 2u : 1u;           // '+': C (converted reads show T), '-': G (A)
     const char cm = first_minus ? 'G' : 'C', cc = first_minus ? 'A' : 'T';
+    const char ec = first_minus ? 'C' : 'G', es = first_minus ? 'T' : 'A';   // Snp: the opposite strand's base as printed
     if constexpr (!Cycles) {
         for (int i = lane; i < (int)len; i += 32) {
-            if (ref_code(refcat, base + (uint32_t)i) != match) continue;
+            const uint32_t r = ref_code(refcat, base + (uint32_t)i);
+            if (r != match) {
+                if constexpr (Snp) {
+                    if (r == 3u - match) {
+                        const char c = getc((int)start + i);
+                        if (c == ec) atomicAdd(confirm + base + i, 1u);
+                        else if (c == es) atomicAdd(snp + base + i, 1u);
+                    }
+                }
+                continue;
+            }
             const char c = getc((int)start + i);
             if (c == cc) atomicAdd(depth + base + i, 1u);
             else if (c == cm) { atomicAdd(meth + base + i, 1u); atomicAdd(depth + base + i, 1u); }
@@ -107,7 +130,19 @@ __device__ __forceinline__ void pile_alignment(const uint32_t *__restrict__ refc
         uint32_t *h = hist + read2 * (3 * BSX_MBIAS_CYCLES * 2);
         for (int i = lane; i < (int)len; i += 32) {
             const uint32_t q = base + (uint32_t)i;
-            if (ref_code(refcat, q) != match) continue;
+            const uint32_t r = ref_code(refcat, q);
+            if (r != match) {
+                if constexpr (Snp) {
+                    if (r == 3u - match) {
+                        const int j = (int)start + i;
+                        const char c = getc(j);
+                        uint32_t *ctr = c == ec ? confirm : (c == es ? snp : nullptr);
+                        const int cyc = rev ? L - 1 - j : j;
+                        if (ctr && cyc >= lo && cyc < hi) atomicAdd(ctr + q, 1u);
+                    }
+                }
+                continue;
+            }
             const int j = (int)start + i;
             const char c = getc(j);
             const bool is_m = c == cm;
@@ -192,13 +227,14 @@ __global__ void __launch_bounds__(256) meth_claim_kernel(const uint32_t *__restr
 }
 
 // alignments parsed from SAM / BSP text on the host: one warp per alignment (Cycles: a grid-stride loop of them)
-template <bool Cycles>
+template <bool Cycles, bool Snp>
 __global__ void __launch_bounds__(256) meth_pileup_kernel(const uint32_t *__restrict__ refcat, const uint32_t *__restrict__ seqinfo, uint32_t n_seq,
                                                           uint32_t *meth, uint32_t *depth, unsigned long long *n_valid, uint32_t *first, bsx_meth_opts o, uint32_t n,
                                                           const char *__restrict__ seqs, uint32_t stride, const uint16_t *__restrict__ lens,
                                                           const uint32_t *__restrict__ chr, const uint32_t *__restrict__ pos0,
                                                           const uint8_t *__restrict__ strand, const int32_t *__restrict__ insert,
-                                                          const int32_t *__restrict__ mate_pos, const uint8_t *__restrict__ flags, MbiasArgs mb) {
+                                                          const int32_t *__restrict__ mate_pos, const uint8_t *__restrict__ flags, MbiasArgs mb,
+                                                          uint32_t *confirm, uint32_t *snp) {
     const uint32_t w = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     const int lane = threadIdx.x & 31;
     auto one = [&](uint32_t a, uint32_t *hist) {
@@ -206,8 +242,8 @@ __global__ void __launch_bounds__(256) meth_pileup_kernel(const uint32_t *__rest
         if (!parsed_alignment(o, n_seq, a, lens, chr, pos0, strand, insert, mate_pos, flags, v)) return;
         if (first && !dup_holds(first, seqinfo, n_seq, v, a, lane)) return;
         const char *sq = seqs + (size_t)a * stride;
-        pile_alignment<Cycles>(refcat, seqinfo, n_seq, meth, depth, n_valid, o, v.k, v.pos, v.len, v.st, v.ins, v.mate_pos, v.sam, lane,
-                               [sq](int i) { return sq[i]; }, mb, (flags[a] & BSX_METH_READ2) ? 1 : 0, hist);
+        pile_alignment<Cycles, Snp>(refcat, seqinfo, n_seq, meth, depth, n_valid, o, v.k, v.pos, v.len, v.st, v.ins, v.mate_pos, v.sam, lane,
+                                    [sq](int i) { return sq[i]; }, mb, (flags[a] & BSX_METH_READ2) ? 1 : 0, hist, confirm, snp);
     };
     if constexpr (!Cycles) {
         if (w >= n) return;
@@ -275,13 +311,13 @@ __global__ void __launch_bounds__(256) meth_claim_mapped_kernel(const uint32_t *
 }
 
 // pile-up of the mapped batch: one warp per read (PE: per mate; Cycles: a grid-stride loop of them)
-template <bool Cycles>
+template <bool Cycles, bool Snp>
 __global__ void __launch_bounds__(256) meth_pileup_mapped_kernel(const uint32_t *__restrict__ refcat, const uint32_t *__restrict__ seqinfo, uint32_t n_seq,
                                                                  uint32_t *meth, uint32_t *depth, unsigned long long *n_valid, uint32_t *first, bsx_meth_opts o,
                                                                  int sam, int report_repeat_hits, uint32_t n, int mates, uint32_t stride,
                                                                  const uint8_t *__restrict__ seq_a, const uint8_t *__restrict__ seq_b,
                                                                  const bsx_rec *__restrict__ out_a, const bsx_rec *__restrict__ out_b,
-                                                                 const bsx_pair_rec *__restrict__ out_pair, MbiasArgs mb) {
+                                                                 const bsx_pair_rec *__restrict__ out_pair, MbiasArgs mb, uint32_t *confirm, uint32_t *snp) {
     const uint32_t w = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     const int lane = threadIdx.x & 31;
     auto one = [&](uint32_t u, uint32_t *hist) {
@@ -292,8 +328,8 @@ __global__ void __launch_bounds__(256) meth_pileup_mapped_kernel(const uint32_t 
         const uint8_t *rd = ((mates == 2 && (u & 1u)) ? seq_b : seq_a) + (size_t)r * stride;
         const int lp = (int)v.len;
         const int read2 = mates == 2 ? (int)(u & 1u) : (mb.readset == 2 ? 1 : 0);     // mate b / readset 2 print FLAG 0x80
-        pile_alignment<true>(refcat, seqinfo, n_seq, meth, depth, n_valid, o, v.k, v.pos, v.len, v.st, v.ins, v.mate_pos, v.sam, lane,
-                             [rd, rev, lp](int i) { return rev ? comp_char((char)rd[lp - 1 - i]) : (char)rd[i]; }, mb, read2, hist);
+        pile_alignment<true, Snp>(refcat, seqinfo, n_seq, meth, depth, n_valid, o, v.k, v.pos, v.len, v.st, v.ins, v.mate_pos, v.sam, lane,
+                                  [rd, rev, lp](int i) { return rev ? comp_char((char)rd[lp - 1 - i]) : (char)rd[i]; }, mb, read2, hist, confirm, snp);
     };
     if constexpr (!Cycles) {
         // the same steps as `one`, written out: through the lambda, ptxas allocates this instantiation differently
@@ -305,8 +341,8 @@ __global__ void __launch_bounds__(256) meth_pileup_mapped_kernel(const uint32_t 
         const uint32_t r = mates == 2 ? u >> 1 : u;
         const uint8_t *rd = ((mates == 2 && (u & 1u)) ? seq_b : seq_a) + (size_t)r * stride;
         const int lp = (int)v.len;
-        pile_alignment<false>(refcat, seqinfo, n_seq, meth, depth, n_valid, o, v.k, v.pos, v.len, v.st, v.ins, v.mate_pos, v.sam, lane,
-                              [rd, rev, lp](int i) { return rev ? comp_char((char)rd[lp - 1 - i]) : (char)rd[i]; });
+        pile_alignment<false, Snp>(refcat, seqinfo, n_seq, meth, depth, n_valid, o, v.k, v.pos, v.len, v.st, v.ins, v.mate_pos, v.sam, lane,
+                                   [rd, rev, lp](int i) { return rev ? comp_char((char)rd[lp - 1 - i]) : (char)rd[i]; }, MbiasArgs{}, 0, nullptr, confirm, snp);
     } else {
         __shared__ uint32_t hist[MBIAS_BINS];
         hist_zero(hist, mb.hist);
@@ -315,13 +351,19 @@ __global__ void __launch_bounds__(256) meth_pileup_mapped_kernel(const uint32_t 
     }
 }
 
-// -g: every reference "CG": both counters of the C take the G's, the G's become 0 (methratio.py:122-131)
-__global__ void meth_combine_kernel(const uint32_t *__restrict__ refcat, uint64_t n_pos, uint32_t *meth, uint32_t *depth) {
+// -g: every reference "CG": both counters of the C take the G's, the G's become 0 (methratio.py:122-131); Snp: the
+// evidence counters the same way
+template <bool Snp>
+__global__ void meth_combine_kernel(const uint32_t *__restrict__ refcat, uint64_t n_pos, uint32_t *meth, uint32_t *depth, uint32_t *confirm, uint32_t *snp) {
     const uint64_t q = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (q + 1 >= n_pos) return;
     if (ref_code(refcat, (uint32_t)q) == 1u && ref_code(refcat, (uint32_t)q + 1u) == 2u) {
         depth[q] += depth[q + 1]; meth[q] += meth[q + 1];
         depth[q + 1] = 0; meth[q + 1] = 0;
+        if constexpr (Snp) {
+            confirm[q] += confirm[q + 1]; snp[q] += snp[q + 1];
+            confirm[q + 1] = 0; snp[q + 1] = 0;
+        }
     }
 }
 
@@ -351,6 +393,15 @@ int ensure_dup_table(bsx_meth *m) {
     return BSX_OK;
 }
 
+// the instantiation for a combination of options (the kernels of one combination share a signature)
+auto text_kernel(bool cycles, bool snp) {
+    return cycles ? (snp ? meth_pileup_kernel<true, true> : meth_pileup_kernel<true, false>) : (snp ? meth_pileup_kernel<false, true> : meth_pileup_kernel<false, false>);
+}
+auto mapped_kernel(bool cycles, bool snp) {
+    return cycles ? (snp ? meth_pileup_mapped_kernel<true, true> : meth_pileup_mapped_kernel<true, false>)
+                  : (snp ? meth_pileup_mapped_kernel<false, true> : meth_pileup_mapped_kernel<false, false>);
+}
+
 bool cycles_on(const bsx_meth *m) { return m->mbias || m->ignore[0] || m->ignore[1] || m->ignore[2] || m->ignore[3]; }
 
 // the Cycles kernels' grid cap and, with M-bias on, their histogram (zeroed), on the first pile-up that needs them
@@ -363,8 +414,8 @@ int ensure_cycles(bsx_meth *m) {
     int dev = 0, sms = 0, per_sm[2] = {0, 0};
     BSX_CUDA_CHECK(cudaGetDevice(&dev));
     BSX_CUDA_CHECK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
-    BSX_CUDA_CHECK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm[0], meth_pileup_kernel<true>, 256, 0));
-    BSX_CUDA_CHECK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm[1], meth_pileup_mapped_kernel<true>, 256, 0));
+    BSX_CUDA_CHECK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm[0], text_kernel(true, m->ct_snp != 0), 256, 0));
+    BSX_CUDA_CHECK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm[1], mapped_kernel(true, m->ct_snp != 0), 256, 0));
     for (int i = 0; i < 2; i++) m->resident[i] = std::max(per_sm[i], 1) * sms;
     BSX_CUDA_CHECK(cudaDeviceSynchronize());
     return BSX_OK;
@@ -379,7 +430,8 @@ MbiasArgs mbias_args(const bsx_meth *m, int readset) {
 int combine_once(bsx_meth *m, const bsx_meth_opts *o) {
     if (!o->combine_cpg || m->combined) return BSX_OK;
     const uint64_t n_pos = m->ix->n_words * 16;
-    meth_combine_kernel<<<(unsigned)((n_pos + 255) / 256), 256>>>(m->ix->d_refcat, n_pos, m->d_meth, m->d_depth);
+    (m->ct_snp ? meth_combine_kernel<true> : meth_combine_kernel<false>)<<<(unsigned)((n_pos + 255) / 256), 256>>>(m->ix->d_refcat, n_pos, m->d_meth, m->d_depth,
+                                                                                                              m->d_confirm, m->d_snp);
     BSX_CUDA_CHECK(cudaGetLastError());
     BSX_CUDA_CHECK(cudaDeviceSynchronize());
     m->combined = true;
@@ -392,6 +444,7 @@ struct Sink {
     void putc(char c) { s->push_back(c); }
     void putu(unsigned long long v) { char b[24]; char *e = b + 24, *q = e; do { *--q = (char)('0' + v % 10); v /= 10; } while (v); put(q, (size_t)(e - q)); }
     void putf3(double v) { char b[48]; const int l = snprintf(b, sizeof b, "%.3f", v); put(b, (size_t)l); }
+    void putf2(double v) { char b[48]; const int l = snprintf(b, sizeof b, "%.2f", v); put(b, (size_t)l); }
 };
 
 }  // namespace
@@ -420,7 +473,7 @@ extern "C" int bsx_meth_create(const bsx_index *ix, bsx_meth **out) {
 
 extern "C" int bsx_meth_destroy(bsx_meth *m) {
     if (!m) return BSX_OK;
-    cudaFree(m->d_meth); cudaFree(m->d_depth); cudaFree(m->d_valid); cudaFree(m->d_first); cudaFree(m->d_mbias);
+    cudaFree(m->d_meth); cudaFree(m->d_depth); cudaFree(m->d_valid); cudaFree(m->d_first); cudaFree(m->d_mbias); cudaFree(m->d_confirm); cudaFree(m->d_snp);
     if (m->dup_order) cudaEventDestroy(m->dup_order);
     cudaFree(m->d_seq); cudaFree(m->d_len); cudaFree(m->d_chr); cudaFree(m->d_pos); cudaFree(m->d_strand); cudaFree(m->d_flags); cudaFree(m->d_ins); cudaFree(m->d_mate);
     delete m;
@@ -451,16 +504,11 @@ extern "C" int bsx_meth_add(bsx_meth *m, const bsx_meth_opts *o, uint32_t n, con
             BSX_CUDA_CHECK(cudaGetLastError());
         }
         const unsigned blocks = (unsigned)(((uint64_t)n * 32 + 255) / 256);
-        if (!cycles_on(m)) {
-            meth_pileup_kernel<false><<<blocks, 256>>>(m->ix->d_refcat, m->ix->d_seqinfo, m->ix->n_seq, m->d_meth, m->d_depth, m->d_valid,
-                                                       o->rm_dup ? m->d_first : nullptr, *o, n, m->d_seq, m->stride, m->d_len, m->d_chr, m->d_pos, m->d_strand,
-                                                       m->d_ins, m->d_mate, m->d_flags, MbiasArgs{});
-        } else {
-            rc = ensure_cycles(m); if (rc) return rc;
-            meth_pileup_kernel<true><<<std::min<unsigned>(blocks, (unsigned)m->resident[0]), 256>>>(
-                m->ix->d_refcat, m->ix->d_seqinfo, m->ix->n_seq, m->d_meth, m->d_depth, m->d_valid, o->rm_dup ? m->d_first : nullptr, *o, n, m->d_seq,
-                m->stride, m->d_len, m->d_chr, m->d_pos, m->d_strand, m->d_ins, m->d_mate, m->d_flags, mbias_args(m, 0));
-        }
+        const bool cyc = cycles_on(m);
+        if (cyc) { rc = ensure_cycles(m); if (rc) return rc; }
+        text_kernel(cyc, m->ct_snp != 0)<<<cyc ? std::min<unsigned>(blocks, (unsigned)m->resident[0]) : blocks, 256>>>(
+            m->ix->d_refcat, m->ix->d_seqinfo, m->ix->n_seq, m->d_meth, m->d_depth, m->d_valid, o->rm_dup ? m->d_first : nullptr, *o, n, m->d_seq,
+            m->stride, m->d_len, m->d_chr, m->d_pos, m->d_strand, m->d_ins, m->d_mate, m->d_flags, cyc ? mbias_args(m, 0) : MbiasArgs{}, m->d_confirm, m->d_snp);
         BSX_CUDA_CHECK(cudaGetLastError());
     }
     if (n_valid) {
@@ -478,7 +526,8 @@ int bsx_meth_pile_mapped(bsx_meth *m, const bsx_meth_opts *o, int sam, int repor
     if (!m || !o || n == 0) return BSX_OK;
     if (m->combined) { bsx_set_error("bsx_meth: counters were already combined (-g); create a new bsx_meth"); return BSX_ERR_ARG; }
     m->started = true;
-    if (cycles_on(m)) { int rc = ensure_cycles(m); if (rc) return rc; }
+    const bool cyc = cycles_on(m);
+    if (cyc) { int rc = ensure_cycles(m); if (rc) return rc; }
     if (o->rm_dup) {
         // file order = batch order: this batch's claims start when the previous batch has resolved its own (the batches
         // alternate between two streams).  Paired-end BSP output goes to two files, whose concatenation is the script's
@@ -490,14 +539,9 @@ int bsx_meth_pile_mapped(bsx_meth *m, const bsx_meth_opts *o, int sam, int repor
         BSX_CUDA_CHECK(cudaGetLastError());
     }
     const unsigned blocks = (unsigned)(((uint64_t)n * (uint64_t)mates * 32 + 255) / 256);
-    if (!cycles_on(m))
-        meth_pileup_mapped_kernel<false><<<blocks, 256, 0, st>>>(m->ix->d_refcat, m->ix->d_seqinfo, m->ix->n_seq, m->d_meth, m->d_depth, m->d_valid,
-                                                                 o->rm_dup ? m->d_first : nullptr, *o, sam, report_repeat_hits, n, mates, stride, seq_a, seq_b,
-                                                                 out_a, out_b, out_pair, MbiasArgs{});
-    else
-        meth_pileup_mapped_kernel<true><<<std::min<unsigned>(blocks, (unsigned)m->resident[1]), 256, 0, st>>>(
-            m->ix->d_refcat, m->ix->d_seqinfo, m->ix->n_seq, m->d_meth, m->d_depth, m->d_valid, o->rm_dup ? m->d_first : nullptr, *o, sam,
-            report_repeat_hits, n, mates, stride, seq_a, seq_b, out_a, out_b, out_pair, mbias_args(m, readset));
+    mapped_kernel(cyc, m->ct_snp != 0)<<<cyc ? std::min<unsigned>(blocks, (unsigned)m->resident[1]) : blocks, 256, 0, st>>>(
+        m->ix->d_refcat, m->ix->d_seqinfo, m->ix->n_seq, m->d_meth, m->d_depth, m->d_valid, o->rm_dup ? m->d_first : nullptr, *o, sam,
+        report_repeat_hits, n, mates, stride, seq_a, seq_b, out_a, out_b, out_pair, cyc ? mbias_args(m, readset) : MbiasArgs{}, m->d_confirm, m->d_snp);
     BSX_CUDA_CHECK(cudaGetLastError());
     if (o->rm_dup) BSX_CUDA_CHECK(cudaEventRecord(m->dup_order, st));
     return BSX_OK;
@@ -530,18 +574,21 @@ extern "C" size_t bsx_meth_write(bsx_meth *m, const bsx_meth_opts *o, const char
     threads = bsx_host_threads(threads);
     size_t written = 0;
     auto out = [&](const std::string &s) { size_t off = 0; while (off < s.size()) { ssize_t w = write(fd, s.data() + off, s.size() - off); if (w <= 0) return; off += (size_t)w; written += (size_t)w; } };
-    out("chr\tpos\tstrand\tcontext\tratio\ttotal_C\tmethy_C\tCI_lower\tCI_upper\n");
+    const int snp_mode = m->ct_snp;
+    out(snp_mode ? "chr\tpos\tstrand\tcontext\tratio\teff_CT_count\tC_count\tCT_count\trev_G_count\trev_GA_count\tCI_lower\tCI_upper\n"
+                 : "chr\tpos\tstrand\tcontext\tratio\ttotal_C\tmethy_C\tCI_lower\tCI_upper\n");
     std::vector<uint32_t> order;
     for (uint32_t k = 0; k < ix->n_seq; k++) if (!chroms || chroms[k]) order.push_back(k);
     std::sort(order.begin(), order.end(), [&](uint32_t a, uint32_t b) { return ix->names[a] < ix->names[b]; });   // sorted(depth.keys())
     uint64_t nc = 0, nd = 0;
     const double z95 = 1.96, z95sq = 1.96 * 1.96;
-    std::vector<uint32_t> hm, hd;
+    std::vector<uint32_t> hm, hd, hc, hs;
     for (uint32_t k : order) {
         const uint32_t L = ix->size[k];
         if (lens[k] != L) { bsx_set_error("bsx_meth_write: sequence %u has %u bases, the index %u", k, lens[k], L); return written; }
         hm.resize(L); hd.resize(L);
         if (bsx_meth_download(m, o, k, hm.data(), hd.data()) != BSX_OK) return written;
+        if (snp_mode) { hc.resize(L); hs.resize(L); if (bsx_meth_download_ct_snp(m, o, k, hc.data(), hs.data()) != BSX_OK) return written; }
         const char *rs = seqs[k];
         const std::string &name = ix->names[k];
         std::vector<std::string> chunk((size_t)threads);
@@ -555,15 +602,26 @@ extern "C" size_t bsx_meth_write(bsx_meth *m, const bsx_meth_opts *o, const char
                 lc++; ld += d;
                 const uint32_t mm = hm[i];
                 if (mm == 0 && !o->meth0) continue;
-                const double ratio = (double)mm / d;
+                // C/T SNP: the depth the ratio divides by; the line is dropped by `skip` at any SNP evidence and by
+                // `correct` when no confirming evidence is left
+                double eff = (double)d;
+                uint64_t rg = 0, rga = 0;
+                if (snp_mode) {
+                    rg = hc[i]; rga = rg + hs[i];
+                    if (snp_mode == BSX_CT_SNP_CORRECT) { if (rga) eff = (double)d * (double)rg / (double)rga; if (eff == 0) continue; }
+                    else if (snp_mode == BSX_CT_SNP_SKIP && rg < rga) continue;
+                }
+                const double ratio = std::min((double)mm, eff) / eff;
                 s.put(name.data(), name.size()); s.putc('\t'); s.putu(i + 1); s.putc('\t');
                 const char rc = (char)(rs[i] >= 'a' && rs[i] <= 'z' ? rs[i] - 32 : rs[i]);
                 s.putc(rc == 'C' ? '+' : '-'); s.putc('\t');
                 if (i >= 2) for (size_t j = i - 2; j < i + 3 && j < L; j++) s.putc((char)(rs[j] >= 'a' && rs[j] <= 'z' ? rs[j] - 32 : rs[j]));   // refcr[i-2:i+3] ('' when i < 2)
-                s.putc('\t'); s.putf3(ratio); s.putc('\t'); s.putu(d); s.putc('\t'); s.putu(mm); s.putc('\t');
-                const double pmid = ratio + z95sq / (2 * (double)d);
-                const double sd = z95 * pow(ratio * (1 - ratio) / d + z95sq / (4 * (double)d * d), 0.5);
-                const double nm = 1 + z95sq / d;
+                s.putc('\t'); s.putf3(ratio); s.putc('\t');
+                if (snp_mode) { s.putf2(eff); s.putc('\t'); s.putu(mm); s.putc('\t'); s.putu(d); s.putc('\t'); s.putu(rg); s.putc('\t'); s.putu(rga); s.putc('\t'); }
+                else { s.putu(d); s.putc('\t'); s.putu(mm); s.putc('\t'); }
+                const double pmid = ratio + z95sq / (2 * eff);
+                const double sd = z95 * pow(ratio * (1 - ratio) / eff + z95sq / (4 * eff * eff), 0.5);
+                const double nm = 1 + z95sq / eff;
                 s.putf3((pmid - sd) / nm); s.putc('\t'); s.putf3((pmid + sd) / nm); s.putc('\n');
             }
             cnc[t] = lc; cnd[t] = ld;
@@ -572,6 +630,39 @@ extern "C" size_t bsx_meth_write(bsx_meth *m, const bsx_meth_opts *o, const char
     }
     if (stats) { stats[0] = nc; stats[1] = nd; }
     return written;
+}
+
+extern "C" int bsx_meth_enable_ct_snp(bsx_meth *m, int mode) {
+    if (!m) { bsx_set_error("bsx_meth_enable_ct_snp: bad argument"); return BSX_ERR_ARG; }
+    if (m->started) { bsx_set_error("bsx_meth_enable_ct_snp: alignments were already piled up; enable C/T SNP evidence first"); return BSX_ERR_ARG; }
+    if (mode != BSX_CT_SNP_NO_ACTION && mode != BSX_CT_SNP_CORRECT && mode != BSX_CT_SNP_SKIP) {
+        bsx_set_error("bsx_meth_enable_ct_snp: mode must be BSX_CT_SNP_NO_ACTION, _CORRECT or _SKIP (got %d)", mode); return BSX_ERR_ARG; }
+    if (!m->d_confirm) {
+        BSX_CUDA_CHECK(cudaSetDevice(m->ix->device));
+        const size_t bytes = m->ix->n_words * 16 * sizeof(uint32_t);
+        if (cudaMalloc(&m->d_confirm, bytes) != cudaSuccess || cudaMalloc(&m->d_snp, bytes) != cudaSuccess) {
+            cudaGetLastError(); cudaFree(m->d_confirm); cudaFree(m->d_snp); m->d_confirm = m->d_snp = nullptr;
+            bsx_set_error("C/T SNP evidence: out of device memory (%zu bytes per evidence array, two arrays)", bytes); return BSX_ERR_CUDA; }
+        BSX_CUDA_CHECK(cudaMemset(m->d_confirm, 0, bytes));
+        BSX_CUDA_CHECK(cudaMemset(m->d_snp, 0, bytes));
+    }
+    m->ct_snp = mode;
+    return BSX_OK;
+}
+
+int bsx_ct_snp_mode(const char *name) {
+    return !strcmp(name, "no-action") ? BSX_CT_SNP_NO_ACTION : !strcmp(name, "correct") ? BSX_CT_SNP_CORRECT : !strcmp(name, "skip") ? BSX_CT_SNP_SKIP : 0;
+}
+
+extern "C" int bsx_meth_download_ct_snp(bsx_meth *m, const bsx_meth_opts *o, uint32_t k, uint32_t *confirm, uint32_t *snp) {
+    if (!m || !o || k >= m->ix->n_seq) { bsx_set_error("bsx_meth_download_ct_snp: bad argument"); return BSX_ERR_ARG; }
+    if (!m->ct_snp) { bsx_set_error("bsx_meth_download_ct_snp: C/T SNP evidence was not enabled (bsx_meth_enable_ct_snp)"); return BSX_ERR_ARG; }
+    BSX_CUDA_CHECK(cudaSetDevice(m->ix->device));
+    int rc = combine_once(m, o); if (rc) return rc;
+    const size_t off = m->ix->anchor[k], cnt = m->ix->size[k];
+    if (confirm) BSX_CUDA_CHECK(cudaMemcpy(confirm, m->d_confirm + off, cnt * 4, cudaMemcpyDeviceToHost));
+    if (snp) BSX_CUDA_CHECK(cudaMemcpy(snp, m->d_snp + off, cnt * 4, cudaMemcpyDeviceToHost));
+    return BSX_OK;
 }
 
 extern "C" int bsx_meth_enable_mbias(bsx_meth *m) {

@@ -11,6 +11,9 @@
 // Extensions (SAM and BAM input only: BSP records carry no read number):
 //   --mbias FILE               M-bias report (methylation by read, C context and cycle; include/bsmap_b200.h)
 //   --mbias-ignore A,B,C,D     drop calls in the first A / last B cycles of read 1 and first C / last D of read 2
+// Extension (SAM, BAM and BSP input):
+//   --ct-snp MODE              count C/T SNP evidence from the opposite strand and write the 12-column table with
+//                              eff_CT_count, rev_G_count and rev_GA_count; MODE no-action, correct or skip
 #include <chrono>
 #include <cstdio>
 #include <cstdlib>
@@ -34,6 +37,7 @@ struct MOpts {
     std::string mbias;                       // --mbias FILE
     bool ignore_set = false;
     int32_t ignore[4] = {0, 0, 0, 0};        // --mbias-ignore
+    int ct_snp = 0;                          // --ct-snp: BSX_CT_SNP_*
     std::vector<std::string> files;
 };
 
@@ -55,7 +59,7 @@ void parse(int argc, char **argv, MOpts &m) {
     static const Def defs[] = {{'o', "out", true}, {'d', "ref", true}, {'c', "chr", true}, {'s', "sam-path", true}, {'u', "unique", false},
                                {'p', "pair", false}, {'z', "zero-meth", false}, {'q', "quiet", false}, {'r', "remove-duplicate", false},
                                {'t', "trim-fillin", true}, {'g', "combine-CpG", false}, {'m', "min-depth", true}, {'h', "help", false},
-                               {'\1', "mbias", true}, {'\2', "mbias-ignore", true}};   // long only
+                               {'\1', "mbias", true}, {'\2', "mbias-ignore", true}, {'\3', "ct-snp", true}};   // long only
     auto apply = [&](char c, const char *v) {
         if (!v) v = "";
         switch (c) {
@@ -81,7 +85,12 @@ void parse(int argc, char **argv, MOpts &m) {
                 }
                 m.ignore_set = true;
             } break;
-            case 'h': printf("Usage: methratio [options] BSMAP_MAPPING_FILES\n  -o FILE -d FILE [-c CHR] [-u] [-p] [-z] [-q] [-r] [-t N] [-g] [-m FOLD] [--mbias FILE] [--mbias-ignore A,B,C,D]\n"); exit(0);
+            case '\3':
+                m.ct_snp = bsx_ct_snp_mode(v);
+                if (!m.ct_snp) usage_error((std::string("option --ct-snp: invalid choice: '") + v + "' (choose from 'no-action', 'correct', 'skip')").c_str());
+                break;
+            case 'h': printf("Usage: methratio [options] BSMAP_MAPPING_FILES\n  -o FILE -d FILE [-c CHR] [-u] [-p] [-z] [-q] [-r] [-t N] [-g] [-m FOLD] [--mbias FILE] [--mbias-ignore A,B,C,D]\n"
+                             "  [--ct-snp no-action|correct|skip]\n"); exit(0);
         }
     };
     for (int i = 1; i < argc; i++) {
@@ -309,7 +318,8 @@ extern "C" int bsx_methratio_main(int argc, char **argv) {
     bsx_index *ix = nullptr; bsx_meth *mh = nullptr;
     if (bsx_index_create_packed((int)seqs.size(), np.data(), sp.data(), ln.data(), 0, &ix) != BSX_OK || bsx_meth_create(ix, &mh) != BSX_OK) {
         fprintf(stderr, "%s\n", bsx_last_error()); return 1; }
-    if ((!m.mbias.empty() && bsx_meth_enable_mbias(mh) != BSX_OK) || (m.ignore_set && bsx_meth_set_ignore(mh, m.ignore) != BSX_OK)) {
+    if ((!m.mbias.empty() && bsx_meth_enable_mbias(mh) != BSX_OK) || (m.ignore_set && bsx_meth_set_ignore(mh, m.ignore) != BSX_OK) ||
+        (m.ct_snp && bsx_meth_enable_ct_snp(mh, m.ct_snp) != BSX_OK)) {
         fprintf(stderr, "%s\n", bsx_last_error()); return 1; }
 
     const double t_ix = now_s();

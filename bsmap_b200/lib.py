@@ -67,10 +67,12 @@ EXPORTS = [
     "bsx_meth_write", "bsx_methratio_main", "bsx_sam_to_sorted_bam", "bsx_mapper_attach_meth", "bsx_meth_valid_count",
     "bsx_packed_stride", "bsx_pack_reads", "bsx_map_se_packed", "bsx_map_pe_packed", "bsx_batch_upload_packed",
     "bsx_meth_enable_mbias", "bsx_meth_set_ignore", "bsx_meth_mbias", "bsx_meth_write_mbias",
+    "bsx_meth_enable_ct_snp", "bsx_meth_download_ct_snp",
 ]
 
 METH_READ2 = 8        # BSX_METH_READ2: alignment flag, read 2 (FLAG 0x80)
 MBIAS_CYCLES = 512    # BSX_MBIAS_CYCLES
+CT_SNP_MODES = {"no-action": 1, "correct": 2, "skip": 3}   # BSX_CT_SNP_*
 
 _lib = None
 
@@ -156,6 +158,8 @@ def load():
     L.bsx_meth_mbias.argtypes = [vp, vp, C.POINTER(C.c_uint64)]
     L.bsx_meth_write_mbias.restype = sz
     L.bsx_meth_write_mbias.argtypes = [vp, i32]
+    L.bsx_meth_enable_ct_snp.argtypes = [vp, i32]
+    L.bsx_meth_download_ct_snp.argtypes = [vp, C.POINTER(MethOpts), u32, vp, vp]
     L.bsx_packed_stride.restype = sz
     L.bsx_packed_stride.argtypes = [u32]
     L.bsx_pack_reads.argtypes = [u32, vp, u32, vp, vp, C.POINTER(C.c_uint64), i32]

@@ -311,8 +311,35 @@ int bsx_meth_mbias(bsx_meth *m, uint64_t *out, uint64_t *overflow);
  * then per context CpG, CHG, CHH, per read 1, 2, per 1-based cycle ascending, a row when methylated + unmethylated
  * > 0, ratio = %.3f of methylated / (methylated + unmethylated).  Returns bytes written (0 on error). */
 size_t bsx_meth_write_mbias(bsx_meth *m, int fd);
+/* --- C/T SNP evidence from the opposite strand, and SNP-corrected ratios ---------------------------------------------
+ * Bisulfite leaves the opposite strand's base untouched, so it tells a genomic T at a reference C (which reads like an
+ * unmethylated C) from a real C.  Evidence bases are those of an alignment that survive every step a call survives
+ * (-u / -p, -r, -t, mate-overlap removal, the bounds test, and bsx_meth_set_ignore's cycle rule); q = reference position.
+ *   '+' alignment (first ZS character '+'), reference G at q: read G -> confirm[q] += 1, read A -> snp[q] += 1
+ *   '-' alignment, reference C at q:                          read C -> confirm[q] += 1, read T -> snp[q] += 1
+ * Other read characters count nothing (compared in upper case, as the calls are); non-ACGT reference bases count nothing.
+ * Calls, the M-bias and "valid mappings" are unchanged.  -g adds a CpG's G evidence to its C and zeroes the G.
+ * With the option set, bsx_meth_write writes 12 columns:
+ *   chr pos strand context ratio eff_CT_count C_count CT_count rev_G_count rev_GA_count CI_lower CI_upper
+ * with C_count = meth, CT_count = depth, rev_G_count = confirm, rev_GA_count = confirm + snp, over the lines the plain
+ * table prints (depth >= min_depth, depth > 0, meth > 0 unless -z); the mode then sets eff or drops the line:
+ *   BSX_CT_SNP_NO_ACTION  eff = CT
+ *   BSX_CT_SNP_CORRECT    eff = CT when rev_GA == 0, else (double)CT * rev_G / rev_GA; the line is dropped when eff == 0
+ *   BSX_CT_SNP_SKIP       the line is dropped when rev_G < rev_GA, else eff = CT
+ * ratio = min(C, eff) / eff and the Wilson interval with eff for the depth; eff prints as %.2f.  The summary (covered
+ * cytosines, their summed depth) is the plain table's in every mode.  8 more bytes of HBM per position. */
+#define BSX_CT_SNP_NO_ACTION 1
+#define BSX_CT_SNP_CORRECT   2
+#define BSX_CT_SNP_SKIP      3
+/* count the evidence from now on and write the 12-column table in `mode`.  Must precede the first alignment piled up;
+ * a bad mode or a late call: BSX_ERR_ARG; no device memory for the two arrays: BSX_ERR_CUDA. */
+int bsx_meth_enable_ct_snp(bsx_meth *m, int mode);
+/* copy the evidence of sequence k to the host (after -g combining when o->combine_cpg, like bsx_meth_download);
+ * BSX_ERR_ARG when the evidence was not enabled */
+int bsx_meth_download_ct_snp(bsx_meth *m, const bsx_meth_opts *o, uint32_t k, uint32_t *confirm, uint32_t *snp);
 /* the methratio.py command line: -o -d [-c -u -p -z -q -r -t -g -m -s] files... (SAM, BAM and BSP; -s is ignored);
- * extensions: --mbias FILE (the M-bias report) and --mbias-ignore A,B,C,D (bsx_meth_set_ignore), SAM and BAM only */
+ * extensions: --mbias FILE (the M-bias report) and --mbias-ignore A,B,C,D (bsx_meth_set_ignore), SAM and BAM only;
+ * --ct-snp no-action|correct|skip (bsx_meth_enable_ct_snp) */
 int bsx_methratio_main(int argc, char **argv);
 
 /* --- the bsmap command line (main.cpp:441-476): same options, same output files -------------- */
