@@ -7,7 +7,7 @@ import os
 import numpy as np
 
 from . import lib as _l
-from .lib import CT_SNP_MODES, MBIAS_CYCLES, METH_READ2, PAIR_REC, REC, BsxError, IndexInfo, MethOpts, Params, Stats, check, load, strs
+from .lib import CONV_BINS, CT_SNP_MODES, MBIAS_CYCLES, METH_READ2, PAIR_REC, REC, BsxError, IndexInfo, MethOpts, Params, Stats, check, load, strs
 
 
 def make_params(s=16, I=4, v=2, w=1000, r=1, m=28, x=500, n=0, pairend=0, S=0, f=5, L=144,
@@ -465,6 +465,25 @@ class Meth:
         c, s = np.zeros(n, dtype=np.uint32), np.zeros(n, dtype=np.uint32)
         check(load().bsx_meth_download_ct_snp(self.h, C.byref(self.o), k, c.ctypes.data, s.ctypes.data))
         return c, s
+
+    def enable_conversion_filter(self, threshold: int = 3):
+        """score every alignment by its methylated non-CpG calls and drop those scoring `threshold` or more (0..255;
+        0 only counts them), include/bsmap_b200.h; before the first add / mapped batch"""
+        check(load().bsx_meth_enable_conversion_filter(self.h, int(threshold)))
+
+    def conversion(self):
+        """-> (uint64 array [CONV_BINS]: valid alignments by score, the last bin 255 or more; alignments dropped)"""
+        h = np.zeros(CONV_BINS, dtype=np.uint64)
+        dropped = C.c_uint64(0)
+        check(load().bsx_meth_conversion(self.h, h.ctypes.data, C.byref(dropped)))
+        return h, dropped.value
+
+    def write_conversion(self, fd: int) -> int:
+        """the conversion report (include/bsmap_b200.h) to fd; returns bytes written"""
+        w = load().bsx_meth_write_conversion(self.h, fd)
+        if w == 0:
+            check(1)
+        return w
 
     def write(self, seqs, fd: int, chroms=None, threads=0):
         keep = [s if isinstance(s, bytes) else bytes(s) for s in seqs]

@@ -5,6 +5,9 @@
 // reference's token semantics (reads.cpp:83-146), mapped in large batches on the GPU, formatted on
 // the host and written in input order (= the reference with -p 1, SURVEY.md App. A14).
 // `-o x.bam` writes a coordinate-sorted BAM and its .bai in process (bsx_bam.cpp).
+// Extensions: --methratio T and its --meth-* options pile methratio.py's table up on the device from the mapped batches,
+// with the M-bias report (--meth-mbias, --meth-ignore), C/T SNP evidence (--meth-ct-snp) and the conversion filter
+// (--meth-conversion-filter N, --meth-conversion-report FILE: drop alignments with N or more methylated non-CpG calls).
 // Out of scope (errors out): SAM text input (broken in the reference too: it is opened as BAM), -q quality
 // trimming, -M other than TC.
 #include <cerrno>
@@ -37,6 +40,8 @@ struct Opts {
     bool meth_ignore_set = false;
     int32_t meth_ignore[4] = {0, 0, 0, 0};   // --meth-ignore A,B,C,D: cycles dropped at the 5' / 3' ends of read 1 / read 2
     int meth_ct_snp = 0;                     // --meth-ct-snp MODE: BSX_CT_SNP_*
+    int meth_conv = -1;                      // --meth-conversion-filter N (0..255); -1 = off
+    std::string meth_conv_report;            // --meth-conversion-report FILE (alone: N = 0)
     unsigned batch = 1u << 17;   // reads per GPU batch: small enough to keep the three host stages overlapped
     std::string gpus;            // -g: number of devices (default: all visible) or a comma list of device ids; output stays in input order
 };
@@ -82,7 +87,11 @@ void usage() {
            "       --meth-ignore <A,B,C,D>  with --methratio: drop calls in the first A / last B cycles of read 1 and the\n"
            "                           first C / last D cycles of read 2, from the table and the M-bias report\n"
            "       --meth-ct-snp <no-action|correct|skip>  with --methratio: count C/T SNP evidence from the opposite\n"
-           "                           strand and write the table with eff_CT_count, rev_G_count and rev_GA_count\n\n");
+           "                           strand and write the table with eff_CT_count, rev_G_count and rev_GA_count\n"
+           "       --meth-conversion-filter <int>  with --methratio: drop alignments with this many or more methylated\n"
+           "                           non-CpG calls (incompletely converted reads), 0..255; 0 only counts them\n"
+           "       --meth-conversion-report <str>  with --methratio: write the alignments by their number of methylated\n"
+           "                           non-CpG calls (alone: --meth-conversion-filter 0)\n\n");
     exit(1);
 }
 
@@ -126,6 +135,12 @@ int get_options(int argc, char **argv, Opts &o) {
                 o.meth_ct_snp = bsx_ct_snp_mode(argv[++i]);
                 if (!o.meth_ct_snp) return i;                                                            // "unknown option: <value>"
             }
+            else if (a == "meth-conversion-filter" && i + 1 < argc) {
+                const char *v = argv[++i]; char *e; const long x = strtol(v, &e, 10);
+                if (*e || e == v || x < 0 || x > BSX_CONV_BINS - 1) return i;                             // "unknown option: <value>"
+                o.meth_conv = (int)x;
+            }
+            else if (a == "meth-conversion-report" && i + 1 < argc) o.meth_conv_report = argv[++i];
             else return i;
             continue;
         }
@@ -283,6 +298,9 @@ extern "C" int bsx_cli_main(int argc, char **argv) {
     if (int bad = get_options(argc, argv, o)) { printf("unknown option: %s\n", argv[bad]); exit(bad); }
     if (o.meth_out.empty() && (!o.meth_mbias.empty() || o.meth_ignore_set)) { fprintf(stderr, "--meth-mbias and --meth-ignore need --methratio\n"); return 1; }
     if (o.meth_out.empty() && o.meth_ct_snp) { fprintf(stderr, "--meth-ct-snp needs --methratio\n"); return 1; }
+    if (o.meth_out.empty() && (o.meth_conv >= 0 || !o.meth_conv_report.empty())) {
+        fprintf(stderr, "--meth-conversion-filter and --meth-conversion-report need --methratio\n"); return 1; }
+    if (!o.meth_conv_report.empty() && o.meth_conv < 0) o.meth_conv = 0;
     if (o.qual_threshold != 0) { fprintf(stderr, "-q quality trimming is not supported by the GPU path\n"); return 1; }
     if (o.o.size() > 4) {
         if (o.o.compare(o.o.size() - 4, 4, ".sam") == 0) o.p.out_sam = 1;
@@ -383,6 +401,7 @@ extern "C" int bsx_cli_main(int argc, char **argv) {
         if (bsx_meth_create(ix, &mh) != BSX_OK || (!o.meth_mbias.empty() && bsx_meth_enable_mbias(mh) != BSX_OK) ||
             (o.meth_ignore_set && bsx_meth_set_ignore(mh, o.meth_ignore) != BSX_OK) ||
             (o.meth_ct_snp && bsx_meth_enable_ct_snp(mh, o.meth_ct_snp) != BSX_OK) ||
+            (o.meth_conv >= 0 && bsx_meth_enable_conversion_filter(mh, o.meth_conv) != BSX_OK) ||
             bsx_mapper_attach_meth(mp, mh, &o.mo, (p.out_sam || no_text) ? 1 : 0) != BSX_OK) {
             fprintf(stderr, "%s\n", bsx_last_error()); return 1; }
     }
@@ -538,6 +557,7 @@ extern "C" int bsx_cli_main(int argc, char **argv) {
         printf("total %llu valid mappings, %llu covered cytosines, average coverage: %.2f fold.\n", (unsigned long long)nv, (unsigned long long)st[0],
                st[0] ? (double)st[1] / (double)st[0] : 0.0);
         if (!o.meth_mbias.empty() && bsx_meth_write_mbias_file(mh, o.meth_mbias.c_str()) != BSX_OK) return 1;
+        if (o.meth_conv >= 0 && bsx_meth_write_conversion_file(mh, o.meth_conv_report.empty() ? nullptr : o.meth_conv_report.c_str()) != BSX_OK) return 1;
         if (timing) fprintf(stderr, "[bsx timing] methratio report %.3f s\n", now() - t);
         bsx_meth_destroy(mh);
     }

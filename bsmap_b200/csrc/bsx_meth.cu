@@ -25,6 +25,11 @@
 // untouched by bisulfite: the read shows G / C when the genome has the reference C, A / T when it has a T (a C/T SNP).
 // Two more u32 arrays over the same positions count those bases, `confirm` and `snp`, one global atomic per counted
 // base.  The writer then scales or drops a C's line by that evidence.
+//
+// The conversion filter (bsx_meth_enable_conversion_filter) switches them to their `Conv` instantiation, which exists only
+// with `Cycles` (it needs the call's cycle and context, and its histogram the capped grid): before an alignment's calls are
+// deposited, the warp counts its methylated non-CpG calls (its score), lane 0 adds the alignment to a per-CTA shared
+// histogram of scores, and an alignment whose score reaches the threshold returns without depositing anything.
 #include <algorithm>
 #include <cmath>
 #include <cstdio>
@@ -55,6 +60,9 @@ struct bsx_meth {
     // C/T SNP evidence: fixed before the first alignment is piled up
     int ct_snp = 0;                                   // BSX_CT_SNP_*, 0 = off
     uint32_t *d_confirm = nullptr, *d_snp = nullptr;  // n_words * 16 counters each, like d_meth / d_depth
+    // conversion filter: fixed before the first alignment is piled up
+    int conv_threshold = 0;                           // 0 = report only
+    unsigned long long *d_conv = nullptr;             // BSX_CONV_BINS alignments by score; NULL = filter off
 };
 
 namespace {
@@ -69,6 +77,16 @@ struct MbiasArgs {
     int readset;                  // mapped single-end batches: 2 = these are read 2
 };
 
+// what the Conv instantiation needs beyond the Cycles one
+struct ConvArgs {
+    unsigned long long *hist;     // BSX_CONV_BINS valid alignments by score (the last bin: BSX_CONV_BINS - 1 or more)
+    uint32_t threshold;           // an alignment with score >= threshold is dropped; 0 = none is
+};
+
+// Conv: the CTA's alignments by score, zeroed before and flushed (non-zero bins) after them.  At file scope, so that the
+// pile-up addresses it directly; only the Conv kernels reference it, and only they are given its 1 KB.
+__shared__ uint32_t conv_hist[BSX_CONV_BINS];
+
 __device__ __forceinline__ uint32_t ref_code(const uint32_t *refcat, uint32_t q) { return (refcat[q >> 4] >> (30 - 2 * (q & 15))) & 3u; }
 
 // One alignment, executed by a warp: get_alignment's trimming (methratio.py:56-64), the bounds test (105) and the
@@ -77,12 +95,14 @@ __device__ __forceinline__ uint32_t ref_code(const uint32_t *refcat, uint32_t q)
 // ZS characters differ); calls of read `read2` outside [5p, L - 3p) are dropped; the rest also go into `hist` (shared).
 // Snp: a base over the complementary reference code counts into `confirm` (read G on '+' / C on '-') or `snp` (A / T),
 // after the same trimming, bounds test and (Cycles) exclusion as a call.
-template <bool Cycles, bool Snp, class GetC>
+// Conv (with Cycles): a first pass scores the alignment, its methylated calls whose context is not CpG, into conv_hist;
+// an alignment scoring cv.threshold or more (when non-zero) returns before the second pass deposits anything.
+template <bool Cycles, bool Snp, bool Conv, class GetC>
 __device__ __forceinline__ void pile_alignment(const uint32_t *__restrict__ refcat, const uint32_t *__restrict__ seqinfo, uint32_t n_seq,
                                                uint32_t *meth, uint32_t *depth, unsigned long long *n_valid, const bsx_meth_opts &o,
                                                uint32_t k, long long pos, long long len, int st, int ins, long long mate_pos, bool sam, int lane, GetC getc,
                                                const MbiasArgs &mb = MbiasArgs{}, int read2 = 0, uint32_t *hist = nullptr,
-                                               uint32_t *confirm = nullptr, uint32_t *snp = nullptr) {
+                                               uint32_t *confirm = nullptr, uint32_t *snp = nullptr, const ConvArgs &cv = ConvArgs{}) {
     const int L = (int)len;                                  // printed length, before trimming
     const uint32_t *anchor = seqinfo, *size = seqinfo + n_seq + 1;
     long long start = 0;
@@ -127,6 +147,24 @@ __device__ __forceinline__ void pile_alignment(const uint32_t *__restrict__ refc
     } else {
         const bool rev = ((st ^ (st >> 1)) & 1) != 0;
         const int lo = read2 ? mb.ignore[2] : mb.ignore[0], hi = L - (read2 ? mb.ignore[3] : mb.ignore[1]);
+        if constexpr (Conv) {
+            // the score: a methylated call (read C on '+', G on '-') inside the cycle bounds whose next base on the call's
+            // strand is not the CpG partner (CHG and CHH alike, so the second context code is not needed).  The bounds
+            // [lo, hi) on the cycle are a range of i: cycle j = start + i, or L - 1 - j when reversed.
+            const int s0 = (int)start;
+            const int i_end = min(rev ? L - s0 - lo : hi - s0, (int)len);
+            uint32_t score = 0;
+#pragma unroll 1
+            for (int i = max(rev ? L - s0 - hi : lo - s0, 0) + lane; i < i_end; i += 32) {
+                const uint32_t q = base + (uint32_t)i;
+                if (ref_code(refcat, q) != match || getc(s0 + i) != cm) continue;
+                const uint32_t c1 = first_minus ? ref_code(refcat, q - 1u) : ref_code(refcat, q + 1u);
+                score += c1 != 3u - match;
+            }
+            score = __reduce_add_sync(0xffffffffu, score);
+            if (lane == 0) atomicAdd(&conv_hist[min(score, (uint32_t)BSX_CONV_BINS - 1u)], 1u);
+            if (cv.threshold && score >= cv.threshold) return;
+        }
         uint32_t *h = hist + read2 * (3 * BSX_MBIAS_CYCLES * 2);
         for (int i = lane; i < (int)len; i += 32) {
             const uint32_t q = base + (uint32_t)i;
@@ -164,17 +202,19 @@ __device__ __forceinline__ void pile_alignment(const uint32_t *__restrict__ refc
     }
 }
 
-// Cycles: the per-CTA histogram, zeroed before and flushed (non-zero bins) after the CTA's alignments; out == NULL
-// (exclusion without M-bias) skips both
+// Cycles: a per-CTA histogram (M-bias; Conv: the scores), zeroed before and flushed (non-zero bins) after the CTA's
+// alignments; out == NULL (exclusion without M-bias) skips both
+template <int Bins>
 __device__ __forceinline__ void hist_zero(uint32_t *hist, const unsigned long long *out) {
     if (!out) return;
-    for (int b = threadIdx.x; b < MBIAS_BINS; b += blockDim.x) hist[b] = 0u;
+    for (int b = threadIdx.x; b < Bins; b += blockDim.x) hist[b] = 0u;
     __syncthreads();
 }
+template <int Bins>
 __device__ __forceinline__ void hist_flush(uint32_t *hist, unsigned long long *out) {
     if (!out) return;
     __syncthreads();
-    for (int b = threadIdx.x; b < MBIAS_BINS; b += blockDim.x) { const uint32_t v = hist[b]; if (v) atomicAdd(out + b, (unsigned long long)v); }
+    for (int b = threadIdx.x; b < Bins; b += blockDim.x) { const uint32_t v = hist[b]; if (v) atomicAdd(out + b, (unsigned long long)v); }
 }
 
 // what get_alignment hands on (before trimming): sequence index, 0-based position, printed length, strand bits, ...
@@ -226,15 +266,18 @@ __global__ void __launch_bounds__(256) meth_claim_kernel(const uint32_t *__restr
     if (a < n && parsed_alignment(o, n_seq, a, lens, chr, pos0, strand, insert, mate_pos, flags, v) && dup_key(seqinfo, n_seq, v, key)) atomicMin(first + key, a + 1u);
 }
 
-// alignments parsed from SAM / BSP text on the host: one warp per alignment (Cycles: a grid-stride loop of them)
-template <bool Cycles, bool Snp>
-__global__ void __launch_bounds__(256) meth_pileup_kernel(const uint32_t *__restrict__ refcat, const uint32_t *__restrict__ seqinfo, uint32_t n_seq,
+// alignments parsed from SAM / BSP text on the host: one warp per alignment (Cycles: a grid-stride loop of them).
+// Conv asks for 4 resident CTAs per SM: without that floor, ptxas squeezes its instantiations to 32 or 40 registers
+// and spills; with it they take 38 - 44 and none.  The other instantiations keep the plain bound (0 = none).
+template <bool Cycles, bool Snp, bool Conv>
+__global__ void __launch_bounds__(256, Conv ? 4 : 0) meth_pileup_kernel(const uint32_t *__restrict__ refcat, const uint32_t *__restrict__ seqinfo, uint32_t n_seq,
                                                           uint32_t *meth, uint32_t *depth, unsigned long long *n_valid, uint32_t *first, bsx_meth_opts o, uint32_t n,
                                                           const char *__restrict__ seqs, uint32_t stride, const uint16_t *__restrict__ lens,
                                                           const uint32_t *__restrict__ chr, const uint32_t *__restrict__ pos0,
                                                           const uint8_t *__restrict__ strand, const int32_t *__restrict__ insert,
                                                           const int32_t *__restrict__ mate_pos, const uint8_t *__restrict__ flags, MbiasArgs mb,
-                                                          uint32_t *confirm, uint32_t *snp) {
+                                                          uint32_t *confirm, uint32_t *snp, ConvArgs cv) {
+    static_assert(Cycles || !Conv, "the conversion filter runs in the Cycles kernels");
     const uint32_t w = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     const int lane = threadIdx.x & 31;
     auto one = [&](uint32_t a, uint32_t *hist) {
@@ -242,17 +285,19 @@ __global__ void __launch_bounds__(256) meth_pileup_kernel(const uint32_t *__rest
         if (!parsed_alignment(o, n_seq, a, lens, chr, pos0, strand, insert, mate_pos, flags, v)) return;
         if (first && !dup_holds(first, seqinfo, n_seq, v, a, lane)) return;
         const char *sq = seqs + (size_t)a * stride;
-        pile_alignment<Cycles, Snp>(refcat, seqinfo, n_seq, meth, depth, n_valid, o, v.k, v.pos, v.len, v.st, v.ins, v.mate_pos, v.sam, lane,
-                                    [sq](int i) { return sq[i]; }, mb, (flags[a] & BSX_METH_READ2) ? 1 : 0, hist, confirm, snp);
+        pile_alignment<Cycles, Snp, Conv>(refcat, seqinfo, n_seq, meth, depth, n_valid, o, v.k, v.pos, v.len, v.st, v.ins, v.mate_pos, v.sam, lane,
+                                          [sq](int i) { return sq[i]; }, mb, (flags[a] & BSX_METH_READ2) ? 1 : 0, hist, confirm, snp, cv);
     };
     if constexpr (!Cycles) {
         if (w >= n) return;
         one(w, nullptr);
     } else {
         __shared__ uint32_t hist[MBIAS_BINS];
-        hist_zero(hist, mb.hist);
+        hist_zero<MBIAS_BINS>(hist, mb.hist);
+        if constexpr (Conv) hist_zero<BSX_CONV_BINS>(conv_hist, cv.hist);
         for (uint32_t a = w; a < n; a += (gridDim.x * blockDim.x) >> 5) one(a, hist);
-        hist_flush(hist, mb.hist);
+        hist_flush<MBIAS_BINS>(hist, mb.hist);
+        if constexpr (Conv) hist_flush<BSX_CONV_BINS>(conv_hist, cv.hist);
     }
 }
 
@@ -310,14 +355,16 @@ __global__ void __launch_bounds__(256) meth_claim_mapped_kernel(const uint32_t *
         atomicMin(first + key, u + 1u);
 }
 
-// pile-up of the mapped batch: one warp per read (PE: per mate; Cycles: a grid-stride loop of them)
-template <bool Cycles, bool Snp>
-__global__ void __launch_bounds__(256) meth_pileup_mapped_kernel(const uint32_t *__restrict__ refcat, const uint32_t *__restrict__ seqinfo, uint32_t n_seq,
+// pile-up of the mapped batch: one warp per read (PE: per mate; Cycles: a grid-stride loop of them); Conv's bound as above
+template <bool Cycles, bool Snp, bool Conv>
+__global__ void __launch_bounds__(256, Conv ? 4 : 0) meth_pileup_mapped_kernel(const uint32_t *__restrict__ refcat, const uint32_t *__restrict__ seqinfo, uint32_t n_seq,
                                                                  uint32_t *meth, uint32_t *depth, unsigned long long *n_valid, uint32_t *first, bsx_meth_opts o,
                                                                  int sam, int report_repeat_hits, uint32_t n, int mates, uint32_t stride,
                                                                  const uint8_t *__restrict__ seq_a, const uint8_t *__restrict__ seq_b,
                                                                  const bsx_rec *__restrict__ out_a, const bsx_rec *__restrict__ out_b,
-                                                                 const bsx_pair_rec *__restrict__ out_pair, MbiasArgs mb, uint32_t *confirm, uint32_t *snp) {
+                                                                 const bsx_pair_rec *__restrict__ out_pair, MbiasArgs mb, uint32_t *confirm, uint32_t *snp,
+                                                                 ConvArgs cv) {
+    static_assert(Cycles || !Conv, "the conversion filter runs in the Cycles kernels");
     const uint32_t w = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     const int lane = threadIdx.x & 31;
     auto one = [&](uint32_t u, uint32_t *hist) {
@@ -328,8 +375,8 @@ __global__ void __launch_bounds__(256) meth_pileup_mapped_kernel(const uint32_t 
         const uint8_t *rd = ((mates == 2 && (u & 1u)) ? seq_b : seq_a) + (size_t)r * stride;
         const int lp = (int)v.len;
         const int read2 = mates == 2 ? (int)(u & 1u) : (mb.readset == 2 ? 1 : 0);     // mate b / readset 2 print FLAG 0x80
-        pile_alignment<true, Snp>(refcat, seqinfo, n_seq, meth, depth, n_valid, o, v.k, v.pos, v.len, v.st, v.ins, v.mate_pos, v.sam, lane,
-                                  [rd, rev, lp](int i) { return rev ? comp_char((char)rd[lp - 1 - i]) : (char)rd[i]; }, mb, read2, hist, confirm, snp);
+        pile_alignment<true, Snp, Conv>(refcat, seqinfo, n_seq, meth, depth, n_valid, o, v.k, v.pos, v.len, v.st, v.ins, v.mate_pos, v.sam, lane,
+                                        [rd, rev, lp](int i) { return rev ? comp_char((char)rd[lp - 1 - i]) : (char)rd[i]; }, mb, read2, hist, confirm, snp, cv);
     };
     if constexpr (!Cycles) {
         // the same steps as `one`, written out: through the lambda, ptxas allocates this instantiation differently
@@ -341,13 +388,15 @@ __global__ void __launch_bounds__(256) meth_pileup_mapped_kernel(const uint32_t 
         const uint32_t r = mates == 2 ? u >> 1 : u;
         const uint8_t *rd = ((mates == 2 && (u & 1u)) ? seq_b : seq_a) + (size_t)r * stride;
         const int lp = (int)v.len;
-        pile_alignment<false, Snp>(refcat, seqinfo, n_seq, meth, depth, n_valid, o, v.k, v.pos, v.len, v.st, v.ins, v.mate_pos, v.sam, lane,
+        pile_alignment<false, Snp, false>(refcat, seqinfo, n_seq, meth, depth, n_valid, o, v.k, v.pos, v.len, v.st, v.ins, v.mate_pos, v.sam, lane,
                                    [rd, rev, lp](int i) { return rev ? comp_char((char)rd[lp - 1 - i]) : (char)rd[i]; }, MbiasArgs{}, 0, nullptr, confirm, snp);
     } else {
         __shared__ uint32_t hist[MBIAS_BINS];
-        hist_zero(hist, mb.hist);
+        hist_zero<MBIAS_BINS>(hist, mb.hist);
+        if constexpr (Conv) hist_zero<BSX_CONV_BINS>(conv_hist, cv.hist);
         for (uint32_t u = w; u < n * (uint32_t)mates; u += (gridDim.x * blockDim.x) >> 5) one(u, hist);
-        hist_flush(hist, mb.hist);
+        hist_flush<MBIAS_BINS>(hist, mb.hist);
+        if constexpr (Conv) hist_flush<BSX_CONV_BINS>(conv_hist, cv.hist);
     }
 }
 
@@ -393,16 +442,21 @@ int ensure_dup_table(bsx_meth *m) {
     return BSX_OK;
 }
 
-// the instantiation for a combination of options (the kernels of one combination share a signature)
-auto text_kernel(bool cycles, bool snp) {
-    return cycles ? (snp ? meth_pileup_kernel<true, true> : meth_pileup_kernel<true, false>) : (snp ? meth_pileup_kernel<false, true> : meth_pileup_kernel<false, false>);
+// the instantiation for a combination of options (the kernels of one combination share a signature); conv implies cycles
+auto text_kernel(bool cycles, bool snp, bool conv) {
+    if (conv) return snp ? meth_pileup_kernel<true, true, true> : meth_pileup_kernel<true, false, true>;
+    return cycles ? (snp ? meth_pileup_kernel<true, true, false> : meth_pileup_kernel<true, false, false>)
+                  : (snp ? meth_pileup_kernel<false, true, false> : meth_pileup_kernel<false, false, false>);
 }
-auto mapped_kernel(bool cycles, bool snp) {
-    return cycles ? (snp ? meth_pileup_mapped_kernel<true, true> : meth_pileup_mapped_kernel<true, false>)
-                  : (snp ? meth_pileup_mapped_kernel<false, true> : meth_pileup_mapped_kernel<false, false>);
+auto mapped_kernel(bool cycles, bool snp, bool conv) {
+    if (conv) return snp ? meth_pileup_mapped_kernel<true, true, true> : meth_pileup_mapped_kernel<true, false, true>;
+    return cycles ? (snp ? meth_pileup_mapped_kernel<true, true, false> : meth_pileup_mapped_kernel<true, false, false>)
+                  : (snp ? meth_pileup_mapped_kernel<false, true, false> : meth_pileup_mapped_kernel<false, false, false>);
 }
 
-bool cycles_on(const bsx_meth *m) { return m->mbias || m->ignore[0] || m->ignore[1] || m->ignore[2] || m->ignore[3]; }
+// the Cycles kernels run for M-bias, exclusion or the conversion filter (with M-bias and exclusion off, Cycles is the
+// classification alone: no histogram, bounds [0, L))
+bool cycles_on(const bsx_meth *m) { return m->mbias || m->ignore[0] || m->ignore[1] || m->ignore[2] || m->ignore[3] || m->d_conv; }
 
 // the Cycles kernels' grid cap and, with M-bias on, their histogram (zeroed), on the first pile-up that needs them
 int ensure_cycles(bsx_meth *m) {
@@ -414,8 +468,8 @@ int ensure_cycles(bsx_meth *m) {
     int dev = 0, sms = 0, per_sm[2] = {0, 0};
     BSX_CUDA_CHECK(cudaGetDevice(&dev));
     BSX_CUDA_CHECK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
-    BSX_CUDA_CHECK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm[0], text_kernel(true, m->ct_snp != 0), 256, 0));
-    BSX_CUDA_CHECK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm[1], mapped_kernel(true, m->ct_snp != 0), 256, 0));
+    BSX_CUDA_CHECK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm[0], text_kernel(true, m->ct_snp != 0, m->d_conv != nullptr), 256, 0));
+    BSX_CUDA_CHECK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm[1], mapped_kernel(true, m->ct_snp != 0, m->d_conv != nullptr), 256, 0));
     for (int i = 0; i < 2; i++) m->resident[i] = std::max(per_sm[i], 1) * sms;
     BSX_CUDA_CHECK(cudaDeviceSynchronize());
     return BSX_OK;
@@ -426,6 +480,7 @@ MbiasArgs mbias_args(const bsx_meth *m, int readset) {
     for (int i = 0; i < 4; i++) a.ignore[i] = m->ignore[i];
     return a;
 }
+ConvArgs conv_args(const bsx_meth *m) { return ConvArgs{m->d_conv, (uint32_t)m->conv_threshold}; }
 
 int combine_once(bsx_meth *m, const bsx_meth_opts *o) {
     if (!o->combine_cpg || m->combined) return BSX_OK;
@@ -473,7 +528,7 @@ extern "C" int bsx_meth_create(const bsx_index *ix, bsx_meth **out) {
 
 extern "C" int bsx_meth_destroy(bsx_meth *m) {
     if (!m) return BSX_OK;
-    cudaFree(m->d_meth); cudaFree(m->d_depth); cudaFree(m->d_valid); cudaFree(m->d_first); cudaFree(m->d_mbias); cudaFree(m->d_confirm); cudaFree(m->d_snp);
+    cudaFree(m->d_meth); cudaFree(m->d_depth); cudaFree(m->d_valid); cudaFree(m->d_first); cudaFree(m->d_mbias); cudaFree(m->d_confirm); cudaFree(m->d_snp); cudaFree(m->d_conv);
     if (m->dup_order) cudaEventDestroy(m->dup_order);
     cudaFree(m->d_seq); cudaFree(m->d_len); cudaFree(m->d_chr); cudaFree(m->d_pos); cudaFree(m->d_strand); cudaFree(m->d_flags); cudaFree(m->d_ins); cudaFree(m->d_mate);
     delete m;
@@ -506,9 +561,10 @@ extern "C" int bsx_meth_add(bsx_meth *m, const bsx_meth_opts *o, uint32_t n, con
         const unsigned blocks = (unsigned)(((uint64_t)n * 32 + 255) / 256);
         const bool cyc = cycles_on(m);
         if (cyc) { rc = ensure_cycles(m); if (rc) return rc; }
-        text_kernel(cyc, m->ct_snp != 0)<<<cyc ? std::min<unsigned>(blocks, (unsigned)m->resident[0]) : blocks, 256>>>(
+        text_kernel(cyc, m->ct_snp != 0, m->d_conv != nullptr)<<<cyc ? std::min<unsigned>(blocks, (unsigned)m->resident[0]) : blocks, 256>>>(
             m->ix->d_refcat, m->ix->d_seqinfo, m->ix->n_seq, m->d_meth, m->d_depth, m->d_valid, o->rm_dup ? m->d_first : nullptr, *o, n, m->d_seq,
-            m->stride, m->d_len, m->d_chr, m->d_pos, m->d_strand, m->d_ins, m->d_mate, m->d_flags, cyc ? mbias_args(m, 0) : MbiasArgs{}, m->d_confirm, m->d_snp);
+            m->stride, m->d_len, m->d_chr, m->d_pos, m->d_strand, m->d_ins, m->d_mate, m->d_flags, cyc ? mbias_args(m, 0) : MbiasArgs{}, m->d_confirm, m->d_snp,
+            conv_args(m));
         BSX_CUDA_CHECK(cudaGetLastError());
     }
     if (n_valid) {
@@ -539,9 +595,10 @@ int bsx_meth_pile_mapped(bsx_meth *m, const bsx_meth_opts *o, int sam, int repor
         BSX_CUDA_CHECK(cudaGetLastError());
     }
     const unsigned blocks = (unsigned)(((uint64_t)n * (uint64_t)mates * 32 + 255) / 256);
-    mapped_kernel(cyc, m->ct_snp != 0)<<<cyc ? std::min<unsigned>(blocks, (unsigned)m->resident[1]) : blocks, 256, 0, st>>>(
+    mapped_kernel(cyc, m->ct_snp != 0, m->d_conv != nullptr)<<<cyc ? std::min<unsigned>(blocks, (unsigned)m->resident[1]) : blocks, 256, 0, st>>>(
         m->ix->d_refcat, m->ix->d_seqinfo, m->ix->n_seq, m->d_meth, m->d_depth, m->d_valid, o->rm_dup ? m->d_first : nullptr, *o, sam,
-        report_repeat_hits, n, mates, stride, seq_a, seq_b, out_a, out_b, out_pair, cyc ? mbias_args(m, readset) : MbiasArgs{}, m->d_confirm, m->d_snp);
+        report_repeat_hits, n, mates, stride, seq_a, seq_b, out_a, out_b, out_pair, cyc ? mbias_args(m, readset) : MbiasArgs{}, m->d_confirm, m->d_snp,
+        conv_args(m));
     BSX_CUDA_CHECK(cudaGetLastError());
     if (o->rm_dup) BSX_CUDA_CHECK(cudaEventRecord(m->dup_order, st));
     return BSX_OK;
@@ -724,5 +781,65 @@ int bsx_meth_write_mbias_file(bsx_meth *m, const char *path) {
     if (w == 0) { fprintf(stderr, "%s\n", bsx_last_error()); return BSX_ERR_IO; }
     if (over) fprintf(stderr, "warning: %llu methylation calls at cycle %d or later are in the table but not in the M-bias report\n",
                       (unsigned long long)over, BSX_MBIAS_CYCLES + 1);
+    return BSX_OK;
+}
+
+extern "C" int bsx_meth_enable_conversion_filter(bsx_meth *m, int32_t threshold) {
+    if (!m) { bsx_set_error("bsx_meth_enable_conversion_filter: bad argument"); return BSX_ERR_ARG; }
+    if (m->started) { bsx_set_error("bsx_meth_enable_conversion_filter: alignments were already piled up; enable the conversion filter first"); return BSX_ERR_ARG; }
+    if (threshold < 0 || threshold > BSX_CONV_BINS - 1) {
+        bsx_set_error("bsx_meth_enable_conversion_filter: threshold must be 0..%d (got %d)", BSX_CONV_BINS - 1, (int)threshold); return BSX_ERR_ARG; }
+    if (!m->d_conv) {
+        BSX_CUDA_CHECK(cudaSetDevice(m->ix->device));
+        BSX_CUDA_CHECK(cudaMalloc(&m->d_conv, BSX_CONV_BINS * sizeof(unsigned long long)));
+        BSX_CUDA_CHECK(cudaMemset(m->d_conv, 0, BSX_CONV_BINS * sizeof(unsigned long long)));
+    }
+    m->conv_threshold = threshold;
+    return BSX_OK;
+}
+
+extern "C" int bsx_meth_conversion(bsx_meth *m, uint64_t *out, uint64_t *dropped) {
+    if (!m || !out) { bsx_set_error("bsx_meth_conversion: bad argument"); return BSX_ERR_ARG; }
+    if (!m->d_conv) { bsx_set_error("bsx_meth_conversion: the conversion filter was not enabled (bsx_meth_enable_conversion_filter)"); return BSX_ERR_ARG; }
+    BSX_CUDA_CHECK(cudaSetDevice(m->ix->device));
+    BSX_CUDA_CHECK(cudaDeviceSynchronize());           // in-process batches flush from two streams
+    unsigned long long h[BSX_CONV_BINS];
+    BSX_CUDA_CHECK(cudaMemcpy(h, m->d_conv, sizeof h, cudaMemcpyDeviceToHost));
+    uint64_t d = 0;
+    for (int b = 0; b < BSX_CONV_BINS; b++) { out[b] = h[b]; if (m->conv_threshold && b >= m->conv_threshold) d += h[b]; }
+    if (dropped) *dropped = d;
+    return BSX_OK;
+}
+
+extern "C" size_t bsx_meth_write_conversion(bsx_meth *m, int fd) {
+    uint64_t h[BSX_CONV_BINS];
+    if (bsx_meth_conversion(m, h, nullptr) != BSX_OK) return 0;
+    std::string s = "methylated_nonCpG_calls\talignments\tdropped\n";
+    Sink o{&s};
+    for (int b = 0; b < BSX_CONV_BINS; b++) {
+        if (!h[b]) continue;
+        o.putu((unsigned long long)b);
+        if (b == BSX_CONV_BINS - 1) o.putc('+');
+        o.putc('\t'); o.putu(h[b]); o.putc('\t'); o.putc(m->conv_threshold && b >= m->conv_threshold ? '1' : '0'); o.putc('\n');
+    }
+    size_t off = 0;
+    while (off < s.size()) { const ssize_t w = write(fd, s.data() + off, s.size() - off); if (w <= 0) return 0; off += (size_t)w; }
+    return off;
+}
+
+int bsx_meth_write_conversion_file(bsx_meth *m, const char *path) {
+    if (path) {
+        const int fd = open(path, O_WRONLY | O_CREAT | O_TRUNC, 0644);
+        if (fd < 0) { fprintf(stderr, "failed to open conversion report file: %s\n", path); return BSX_ERR_IO; }
+        const size_t w = bsx_meth_write_conversion(m, fd);
+        close(fd);
+        if (w == 0) { fprintf(stderr, "%s\n", bsx_last_error()); return BSX_ERR_IO; }
+    }
+    uint64_t h[BSX_CONV_BINS], dropped = 0, valid = 0;
+    if (bsx_meth_conversion(m, h, &dropped) != BSX_OK || bsx_meth_valid_count(m, &valid) != BSX_OK) { fprintf(stderr, "%s\n", bsx_last_error()); return BSX_ERR_CUDA; }
+    if (m->conv_threshold)
+        fprintf(stderr, "conversion filter: %llu of %llu valid mappings dropped (>= %d methylated non-CpG calls)\n", (unsigned long long)dropped,
+                (unsigned long long)valid, m->conv_threshold);
+    else fprintf(stderr, "conversion filter: 0 of %llu valid mappings dropped (report only)\n", (unsigned long long)valid);
     return BSX_OK;
 }

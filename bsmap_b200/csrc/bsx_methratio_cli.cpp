@@ -14,6 +14,9 @@
 // Extension (SAM, BAM and BSP input):
 //   --ct-snp MODE              count C/T SNP evidence from the opposite strand and write the 12-column table with
 //                              eff_CT_count, rev_G_count and rev_GA_count; MODE no-action, correct or skip
+//   --conversion-filter N      drop alignments with N or more methylated non-CpG calls (incompletely converted reads);
+//                              N 0..255, 0 = count only; prints "conversion filter: D of V valid mappings dropped" to stderr
+//   --conversion-report FILE   the alignments by their number of methylated non-CpG calls (alone: N = 0)
 #include <chrono>
 #include <cstdio>
 #include <cstdlib>
@@ -38,6 +41,8 @@ struct MOpts {
     bool ignore_set = false;
     int32_t ignore[4] = {0, 0, 0, 0};        // --mbias-ignore
     int ct_snp = 0;                          // --ct-snp: BSX_CT_SNP_*
+    int conv = -1;                           // --conversion-filter N; -1 = off
+    std::string conv_report;                 // --conversion-report FILE
     std::vector<std::string> files;
 };
 
@@ -59,7 +64,8 @@ void parse(int argc, char **argv, MOpts &m) {
     static const Def defs[] = {{'o', "out", true}, {'d', "ref", true}, {'c', "chr", true}, {'s', "sam-path", true}, {'u', "unique", false},
                                {'p', "pair", false}, {'z', "zero-meth", false}, {'q', "quiet", false}, {'r', "remove-duplicate", false},
                                {'t', "trim-fillin", true}, {'g', "combine-CpG", false}, {'m', "min-depth", true}, {'h', "help", false},
-                               {'\1', "mbias", true}, {'\2', "mbias-ignore", true}, {'\3', "ct-snp", true}};   // long only
+                               {'\1', "mbias", true}, {'\2', "mbias-ignore", true}, {'\3', "ct-snp", true},
+                               {'\4', "conversion-filter", true}, {'\5', "conversion-report", true}};   // long only
     auto apply = [&](char c, const char *v) {
         if (!v) v = "";
         switch (c) {
@@ -89,8 +95,12 @@ void parse(int argc, char **argv, MOpts &m) {
                 m.ct_snp = bsx_ct_snp_mode(v);
                 if (!m.ct_snp) usage_error((std::string("option --ct-snp: invalid choice: '") + v + "' (choose from 'no-action', 'correct', 'skip')").c_str());
                 break;
+            case '\4': { char *e; const long x = strtol(v, &e, 10);
+                if (*e || e == v || x < 0 || x > BSX_CONV_BINS - 1) usage_error("option --conversion-filter: expected an integer 0..255");
+                m.conv = (int)x; } break;
+            case '\5': m.conv_report = v; break;
             case 'h': printf("Usage: methratio [options] BSMAP_MAPPING_FILES\n  -o FILE -d FILE [-c CHR] [-u] [-p] [-z] [-q] [-r] [-t N] [-g] [-m FOLD] [--mbias FILE] [--mbias-ignore A,B,C,D]\n"
-                             "  [--ct-snp no-action|correct|skip]\n"); exit(0);
+                             "  [--ct-snp no-action|correct|skip] [--conversion-filter N] [--conversion-report FILE]\n"); exit(0);
         }
     };
     for (int i = 1; i < argc; i++) {
@@ -281,6 +291,7 @@ extern "C" int bsx_methratio_main(int argc, char **argv) {
     if (m.ref.empty()) usage_error("Missing reference file, use -d or --ref option.");
     if (m.out.empty()) usage_error("Missing output file name, use -o or --out option.");
     if (m.files.empty()) usage_error("Require at least one BSMAP_MAPPING_FILE.");
+    if (!m.conv_report.empty() && m.conv < 0) m.conv = 0;
     const bool cycles = !m.mbias.empty() || m.ignore_set;
     if (cycles)
         for (const std::string &f : m.files) {
@@ -319,7 +330,7 @@ extern "C" int bsx_methratio_main(int argc, char **argv) {
     if (bsx_index_create_packed((int)seqs.size(), np.data(), sp.data(), ln.data(), 0, &ix) != BSX_OK || bsx_meth_create(ix, &mh) != BSX_OK) {
         fprintf(stderr, "%s\n", bsx_last_error()); return 1; }
     if ((!m.mbias.empty() && bsx_meth_enable_mbias(mh) != BSX_OK) || (m.ignore_set && bsx_meth_set_ignore(mh, m.ignore) != BSX_OK) ||
-        (m.ct_snp && bsx_meth_enable_ct_snp(mh, m.ct_snp) != BSX_OK)) {
+        (m.ct_snp && bsx_meth_enable_ct_snp(mh, m.ct_snp) != BSX_OK) || (m.conv >= 0 && bsx_meth_enable_conversion_filter(mh, m.conv) != BSX_OK)) {
         fprintf(stderr, "%s\n", bsx_last_error()); return 1; }
 
     const double t_ix = now_s();
@@ -406,6 +417,10 @@ extern "C" int bsx_methratio_main(int argc, char **argv) {
     if (!m.mbias.empty()) {
         disp(m, ("writing " + m.mbias + " ...").c_str());
         if (bsx_meth_write_mbias_file(mh, m.mbias.c_str()) != BSX_OK) return 1;
+    }
+    if (m.conv >= 0) {
+        if (!m.conv_report.empty()) disp(m, ("writing " + m.conv_report + " ...").c_str());
+        if (bsx_meth_write_conversion_file(mh, m.conv_report.empty() ? nullptr : m.conv_report.c_str()) != BSX_OK) return 1;
     }
     if (getenv("BSX_CLI_TIMING"))
         fprintf(stderr, "[bsx timing] reference FASTA %.3f s || CUDA context (ready at %.3f s), packed reference + counters %.3f s, parse + pile-up %.3f s, report %.3f s\n",

@@ -337,9 +337,36 @@ int bsx_meth_enable_ct_snp(bsx_meth *m, int mode);
 /* copy the evidence of sequence k to the host (after -g combining when o->combine_cpg, like bsx_meth_download);
  * BSX_ERR_ARG when the evidence was not enabled */
 int bsx_meth_download_ct_snp(bsx_meth *m, const bsx_meth_opts *o, uint32_t k, uint32_t *confirm, uint32_t *snp);
+/* --- conversion filter: drop incompletely bisulfite-converted alignments ---------------------------------------------
+ * A fragment that bisulfite did not convert reads C at every C it covers, so its non-CpG Cs, almost never methylated
+ * in mammals, look methylated.  The filter scores each alignment and drops those that look unconverted.
+ *   call     one increment of the counters, after every other rule: -u / -p, -r, -t, mate-overlap removal, the bounds
+ *            test and bsx_meth_set_ignore's cycle rule (excluded cycles, trimmed bases and the mate overlap hold none)
+ *   context  the M-bias rule: a '+' C at q is CpG if q+1 is G, else CHG if q+2 is G, else CHH; a '-' G at q the same
+ *            with q-1, q-2 and C; non-ACGT bases and positions off the sequence count as H
+ *   score    the alignment's calls that are methylated (read C on '+', read G on '-') in CHG or CHH context
+ *   filter   threshold N, 1 <= N <= 255: an alignment with score >= N adds nothing to meth / depth, the M-bias or the
+ *            C/T SNP evidence; it is still a valid mapping (bsx_meth_valid_count and the summary line are unchanged).
+ *            N = 0 drops nothing: the scores are only counted.  The filter is per alignment: each mate on its own calls.
+ *   -r       the claim is decided before the filter: a dropped alignment still holds its (position, direction), so its
+ *            later duplicates still lose (the outcome does not depend on how the alignments are cut into batches)
+ *   report   a histogram of the valid mappings by score, BSX_CONV_BINS bins, bin b = score b, the last 255 or more; the
+ *            bins sum to the valid mappings, and the dropped alignments are the bins >= N. */
+#define BSX_CONV_BINS 256
+/* score every alignment from now on and drop those scoring threshold or more (0..255; 0 = report only).  Must precede
+ * the first alignment piled up; a bad threshold or a late call: BSX_ERR_ARG.  2 KB of device memory. */
+int bsx_meth_enable_conversion_filter(bsx_meth *m, int32_t threshold);
+/* the score histogram so far (synchronises the device): out has BSX_CONV_BINS counters; *dropped (may be NULL): the
+ * alignments dropped.  BSX_ERR_ARG when the filter was not enabled. */
+int bsx_meth_conversion(bsx_meth *m, uint64_t *out /* BSX_CONV_BINS */, uint64_t *dropped);
+/* write the report to fd: a header line "methylated_nonCpG_calls alignments dropped" (tab-separated), then one row per
+ * non-empty bin, ascending, the last labelled "255+"; dropped is 1 when the bin's alignments were dropped, else 0.
+ * Returns bytes written (0 on error). */
+size_t bsx_meth_write_conversion(bsx_meth *m, int fd);
 /* the methratio.py command line: -o -d [-c -u -p -z -q -r -t -g -m -s] files... (SAM, BAM and BSP; -s is ignored);
  * extensions: --mbias FILE (the M-bias report) and --mbias-ignore A,B,C,D (bsx_meth_set_ignore), SAM and BAM only;
- * --ct-snp no-action|correct|skip (bsx_meth_enable_ct_snp) */
+ * --ct-snp no-action|correct|skip (bsx_meth_enable_ct_snp); --conversion-filter N and --conversion-report FILE
+ * (bsx_meth_enable_conversion_filter, bsx_meth_write_conversion) */
 int bsx_methratio_main(int argc, char **argv);
 
 /* --- the bsmap command line (main.cpp:441-476): same options, same output files -------------- */
