@@ -485,6 +485,30 @@ class Meth:
             check(1)
         return w
 
+    @staticmethod
+    def _regions(chr_idx, start, end):
+        arr = lambda a, t: np.ascontiguousarray(np.asarray(a, dtype=t).reshape(-1))
+        c, s, e = arr(chr_idx, np.uint32), arr(start, np.uint64), arr(end, np.uint64)
+        if not len(c) == len(s) == len(e):
+            raise ValueError("chr_idx, start and end differ in length (%d, %d, %d)" % (len(c), len(s), len(e)))
+        return c, s, e
+
+    def regions(self, chr_idx, start, end) -> np.ndarray:
+        """-> uint64 array [region][context CpG/CHG/CHH][sites, covered, C, CT] over the 0-based half-open regions
+        (sequence chr_idx[r], start[r], end[r]); the rules are in include/bsmap_b200.h"""
+        c, s, e = self._regions(chr_idx, start, end)
+        out = np.zeros((len(c), 3, 4), dtype=np.uint64)
+        check(load().bsx_meth_regions(self.h, C.byref(self.o), len(c), c.ctypes.data, s.ctypes.data, e.ctypes.data, out.ctypes.data))
+        return out
+
+    def write_regions(self, fd: int, chr_idx, start, end) -> int:
+        """the region report (include/bsmap_b200.h) to fd; returns bytes written"""
+        c, s, e = self._regions(chr_idx, start, end)
+        w = load().bsx_meth_write_regions(self.h, C.byref(self.o), len(c), c.ctypes.data, s.ctypes.data, e.ctypes.data, fd)
+        if w == 0:
+            check(1)
+        return w
+
     def write(self, seqs, fd: int, chroms=None, threads=0):
         keep = [s if isinstance(s, bytes) else bytes(s) for s in seqs]
         lens = np.array([len(s) for s in keep], dtype=np.uint32)

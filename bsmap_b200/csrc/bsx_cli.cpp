@@ -7,7 +7,9 @@
 // `-o x.bam` writes a coordinate-sorted BAM and its .bai in process (bsx_bam.cpp).
 // Extensions: --methratio T and its --meth-* options pile methratio.py's table up on the device from the mapped batches,
 // with the M-bias report (--meth-mbias, --meth-ignore), C/T SNP evidence (--meth-ct-snp) and the conversion filter
-// (--meth-conversion-filter N, --meth-conversion-report FILE: drop alignments with N or more methylated non-CpG calls).
+// (--meth-conversion-filter N, --meth-conversion-report FILE: drop alignments with N or more methylated non-CpG calls),
+// and methylation levels per region and context reduced on the device (--meth-region-report FILE with --meth-regions BED
+// or --meth-tiles W).
 // Out of scope (errors out): SAM text input (broken in the reference too: it is opened as BAM), -q quality
 // trimming, -M other than TC.
 #include <cerrno>
@@ -42,6 +44,8 @@ struct Opts {
     int meth_ct_snp = 0;                     // --meth-ct-snp MODE: BSX_CT_SNP_*
     int meth_conv = -1;                      // --meth-conversion-filter N (0..255); -1 = off
     std::string meth_conv_report;            // --meth-conversion-report FILE (alone: N = 0)
+    std::string meth_region_report, meth_regions;   // --meth-region-report FILE, --meth-regions BED
+    long long meth_tiles = 0;                // --meth-tiles W; 0 = none
     unsigned batch = 1u << 17;   // reads per GPU batch: small enough to keep the three host stages overlapped
     std::string gpus;            // -g: number of devices (default: all visible) or a comma list of device ids; output stays in input order
 };
@@ -91,7 +95,10 @@ void usage() {
            "       --meth-conversion-filter <int>  with --methratio: drop alignments with this many or more methylated\n"
            "                           non-CpG calls (incompletely converted reads), 0..255; 0 only counts them\n"
            "       --meth-conversion-report <str>  with --methratio: write the alignments by their number of methylated\n"
-           "                           non-CpG calls (alone: --meth-conversion-filter 0)\n\n");
+           "                           non-CpG calls (alone: --meth-conversion-filter 0)\n"
+           "       --meth-region-report <str>  with --methratio: write methylation levels per region and context, over\n"
+           "       --meth-regions <str>  the regions of a BED file (columns 1-3), or\n"
+           "       --meth-tiles <int>  tiles of this many bases over every sequence\n\n");
     exit(1);
 }
 
@@ -141,6 +148,13 @@ int get_options(int argc, char **argv, Opts &o) {
                 o.meth_conv = (int)x;
             }
             else if (a == "meth-conversion-report" && i + 1 < argc) o.meth_conv_report = argv[++i];
+            else if (a == "meth-region-report" && i + 1 < argc) o.meth_region_report = argv[++i];
+            else if (a == "meth-regions" && i + 1 < argc) o.meth_regions = argv[++i];
+            else if (a == "meth-tiles" && i + 1 < argc) {
+                const char *v = argv[++i]; char *e; const long long x = strtoll(v, &e, 10);
+                if (*e || e == v || x < 1) return i;                                                      // "unknown option: <value>"
+                o.meth_tiles = x;
+            }
             else return i;
             continue;
         }
@@ -301,6 +315,11 @@ extern "C" int bsx_cli_main(int argc, char **argv) {
     if (o.meth_out.empty() && (o.meth_conv >= 0 || !o.meth_conv_report.empty())) {
         fprintf(stderr, "--meth-conversion-filter and --meth-conversion-report need --methratio\n"); return 1; }
     if (!o.meth_conv_report.empty() && o.meth_conv < 0) o.meth_conv = 0;
+    const bool region_opts = !o.meth_region_report.empty() || !o.meth_regions.empty() || o.meth_tiles;
+    if (o.meth_out.empty() && region_opts) { fprintf(stderr, "--meth-region-report, --meth-regions and --meth-tiles need --methratio\n"); return 1; }
+    if (!o.meth_regions.empty() && o.meth_tiles) { fprintf(stderr, "--meth-regions and --meth-tiles exclude each other\n"); return 1; }
+    if (region_opts && o.meth_region_report.empty()) { fprintf(stderr, "--meth-regions / --meth-tiles need --meth-region-report FILE\n"); return 1; }
+    if (region_opts && o.meth_regions.empty() && !o.meth_tiles) { fprintf(stderr, "--meth-region-report needs --meth-regions BED or --meth-tiles W\n"); return 1; }
     if (o.qual_threshold != 0) { fprintf(stderr, "-q quality trimming is not supported by the GPU path\n"); return 1; }
     if (o.o.size() > 4) {
         if (o.o.compare(o.o.size() - 4, 4, ".sam") == 0) o.p.out_sam = 1;
@@ -341,6 +360,10 @@ extern "C" int bsx_cli_main(int argc, char **argv) {
         if (!cache_path.empty() && bsx_index_save_packed(ix, cache_path.c_str()) != BSX_OK) fprintf(stderr, "warning: %s\n", bsx_last_error());
     }
     if (o.meth_out.empty()) std::vector<std::string>().swap(ref_seqs);   // the methratio report prints reference context
+    bsx_regions regions;                                                 // read before mapping, so that a bad BED fails early
+    if ((!o.meth_regions.empty() && bsx_regions_bed(ix, nullptr, o.meth_regions.c_str(), regions) != BSX_OK) ||
+        (o.meth_tiles && bsx_regions_tiles(ix, nullptr, (uint64_t)o.meth_tiles, regions) != BSX_OK)) {
+        fprintf(stderr, "%s\n", bsx_last_error()); return 1; }
     bsx_index_info info; bsx_index_get_info(ix, &info);
     unsigned long long sum_len = 0; for (uint32_t k = 0; k < info.n_seq; k++) sum_len += bsx_index_seq_size(ix, k);
     printf("Load in %u db seqs, total size %llu bp. %ld secs passed\n", info.n_seq, sum_len, (long)(time(nullptr) - t0));
@@ -558,6 +581,7 @@ extern "C" int bsx_cli_main(int argc, char **argv) {
                st[0] ? (double)st[1] / (double)st[0] : 0.0);
         if (!o.meth_mbias.empty() && bsx_meth_write_mbias_file(mh, o.meth_mbias.c_str()) != BSX_OK) return 1;
         if (o.meth_conv >= 0 && bsx_meth_write_conversion_file(mh, o.meth_conv_report.empty() ? nullptr : o.meth_conv_report.c_str()) != BSX_OK) return 1;
+        if (!o.meth_region_report.empty() && bsx_meth_write_regions_file(mh, &o.mo, regions, o.meth_region_report.c_str()) != BSX_OK) return 1;
         if (timing) fprintf(stderr, "[bsx timing] methratio report %.3f s\n", now() - t);
         bsx_meth_destroy(mh);
     }

@@ -107,6 +107,18 @@ int bsx_meth_write_mbias_file(bsx_meth *m, const char *path);
 // on stderr "conversion filter: D of V valid mappings dropped (>= N methylated non-CpG calls)", or "(report only)" for
 // N = 0; errors are printed (bsx_meth.cu)
 int bsx_meth_write_conversion_file(bsx_meth *m, const char *path);
+// the regions of the command lines' region report: (sequence, start, end) as given; `skipped` counts the BED regions on a
+// sequence that is not in the reference or not selected (bsx_meth.cu)
+struct bsx_regions { std::vector<uint32_t> seq; std::vector<uint64_t> start, end; uint64_t skipped = 0; };
+// BED columns 1-3 against ix's names, the sequences with selected[k] != 0 (NULL = all); further columns, '#' / track /
+// browser / blank lines are ignored, CRLF is accepted; fewer than 3 columns, a coordinate that is not a non-negative
+// integer and start > end are errors naming the line (BSX_ERR_ARG; BSX_ERR_IO when the file cannot be read)
+int bsx_regions_bed(const bsx_index *ix, const uint8_t *selected, const char *path, bsx_regions &rg);
+// tiles [i*W, min((i+1)*W, len)) over every selected sequence, sequences sorted by name (the table's order)
+int bsx_regions_tiles(const bsx_index *ix, const uint8_t *selected, uint64_t width, bsx_regions &rg);
+// the region report (bsx_meth_write_regions) to a new file at path, and "regions: S of R skipped (...)" on stderr when
+// the BED named sequences that are not there; errors are printed
+int bsx_meth_write_regions_file(bsx_meth *m, const bsx_meth_opts *o, const bsx_regions &rg, const char *path);
 // "no-action" / "correct" / "skip" -> BSX_CT_SNP_*, anything else 0 (bsx_meth.cu)
 int bsx_ct_snp_mode(const char *name);
 int bsx_inflate_file(const char *path, std::vector<char> &out);   // gzip / BGZF members -> bytes (bsx_reads.cpp)

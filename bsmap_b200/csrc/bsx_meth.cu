@@ -35,6 +35,7 @@
 #include <cstdio>
 #include <cstring>
 #include <string>
+#include <unordered_map>
 #include <vector>
 #include <fcntl.h>
 #include <unistd.h>
@@ -414,6 +415,86 @@ __global__ void meth_combine_kernel(const uint32_t *__restrict__ refcat, uint64_
             confirm[q + 1] = 0; snp[q + 1] = 0;
         }
     }
+}
+
+// Region reduction (bsx_meth_regions).  Every region is cut into chunks of REGION_CHUNK positions; scan[r] is the
+// exclusive sum of chunks over the regions before r (scan[n] = all), so a warp takes one chunk whatever the regions'
+// sizes.  4096 positions = 128 per lane: the 12 atomics and the reduction of a chunk cost little next to its 32 KB of
+// counters, and a 1 kb tile is still one chunk.
+constexpr uint32_t REGION_CHUNK = 4096;
+constexpr uint64_t REGION_SLICE = 1u << 20;     // regions per launch: bounds the device buffers (scan, spans, 96 MB of sums)
+
+// One warp per chunk (a grid-stride loop of them).  Lanes read meth / depth (and the evidence the mode needs)
+// coalesced, and the reference codes q-2..q+2 from two refcat words; the pads between sequences are zero (A), so
+// positions off the sequence read as H.  Per lane: sites, covered, C and CT of the three contexts in registers, reduced
+// over the warp, then lanes 0-11 add them to out[(r * 3 + ctx) * 4 + {sites, covered, C, CT}] (u64: exact, and
+// independent of the schedule).  Combine: -g's site rule (a G after a C is no site).  Snp: BSX_CT_SNP_SKIP drops a
+// covered site with any SNP evidence, BSX_CT_SNP_CORRECT one whose SNP-corrected depth is 0; 0 = no drop rule.
+template <bool Combine, int Snp>
+__global__ void __launch_bounds__(256) meth_region_kernel(const uint32_t *__restrict__ refcat, const uint32_t *__restrict__ meth,
+                                                          const uint32_t *__restrict__ depth, const uint32_t *__restrict__ confirm,
+                                                          const uint32_t *__restrict__ snp, uint32_t min_depth,
+                                                          const unsigned long long *__restrict__ scan, const uint2 *__restrict__ span, uint32_t n,
+                                                          unsigned long long *out) {
+    const int lane = threadIdx.x & 31;
+    const unsigned long long total = scan[n], warps = ((unsigned long long)gridDim.x * blockDim.x) >> 5;
+    for (unsigned long long c = ((unsigned long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5; c < total; c += warps) {
+        // the chunk's region: the last r with scan[r] <= c, by a 32-way search (scan[lo] <= c < scan[hi] throughout)
+        uint32_t lo = 0, hi = n;
+        while (hi - lo > 1) {
+            const uint32_t step = (hi - lo + 31) / 32, idx = lo + (uint32_t)lane * step;
+            const unsigned ball = __ballot_sync(0xffffffffu, idx < hi && scan[idx] <= c);
+            lo += (uint32_t)(31 - __clz(ball)) * step;
+            hi = min(hi, lo + step);
+        }
+        const uint2 s = span[lo];
+        const uint32_t b = s.x + (uint32_t)(c - scan[lo]) * REGION_CHUNK, e = min(b + REGION_CHUNK, s.y);
+        uint32_t sites[3] = {0u, 0u, 0u}, cov[3] = {0u, 0u, 0u};
+        unsigned long long cm[3] = {0ull, 0ull, 0ull}, ct[3] = {0ull, 0ull, 0ull};
+        for (uint32_t q = b + (uint32_t)lane; q < e; q += 32) {
+            const uint32_t a = (q - 2u) >> 4, sh = (q - 2u) & 15u;     // bases q-2 .. q+2 lie in words a, a+1
+            const unsigned long long w = ((unsigned long long)__ldg(refcat + a) << 32) | __ldg(refcat + a + 1);
+            auto code = [&](uint32_t k) { return (uint32_t)(w >> (62u - 2u * (sh + k))) & 3u; };
+            const uint32_t r = code(2), before = code(1);
+            const bool plus = r == 1u;
+            bool site = plus || r == 2u;
+            if constexpr (Combine) site = site && !(r == 2u && before == 1u);
+            const uint32_t want = plus ? 2u : 1u, c1 = plus ? code(3) : before, c2 = plus ? code(4) : code(0);
+            const int ctx = c1 == want ? 0 : (c2 == want ? 1 : 2);
+            const uint32_t d = depth[q], mm = meth[q];
+            bool covered = site && d >= min_depth;
+            if constexpr (Snp == BSX_CT_SNP_SKIP) covered = covered && snp[q] == 0u;
+            if constexpr (Snp == BSX_CT_SNP_CORRECT) covered = covered && (snp[q] == 0u || confirm[q] != 0u);
+#pragma unroll
+            for (int k = 0; k < 3; k++) {
+                const bool in = ctx == k;
+                sites[k] += (site && in) ? 1u : 0u;
+                if (covered && in) { cov[k] += 1u; cm[k] += mm; ct[k] += d; }
+            }
+        }
+#pragma unroll
+        for (int k = 0; k < 3; k++) {
+            sites[k] = __reduce_add_sync(0xffffffffu, sites[k]);
+            cov[k] = __reduce_add_sync(0xffffffffu, cov[k]);
+#pragma unroll
+            for (int o = 16; o > 0; o >>= 1) { cm[k] += __shfl_xor_sync(0xffffffffu, cm[k], o); ct[k] += __shfl_xor_sync(0xffffffffu, ct[k], o); }
+        }
+        unsigned long long v = 0;
+#pragma unroll
+        for (int k = 0; k < 3; k++) {
+            if (lane == 4 * k) v = sites[k];
+            if (lane == 4 * k + 1) v = cov[k];
+            if (lane == 4 * k + 2) v = cm[k];
+            if (lane == 4 * k + 3) v = ct[k];
+        }
+        if (lane < 12 && v) atomicAdd(out + (size_t)lo * 12 + lane, v);
+    }
+}
+
+auto region_kernel(bool combine, int snp_mode) {
+    if (snp_mode == BSX_CT_SNP_SKIP) return combine ? meth_region_kernel<true, BSX_CT_SNP_SKIP> : meth_region_kernel<false, BSX_CT_SNP_SKIP>;
+    if (snp_mode == BSX_CT_SNP_CORRECT) return combine ? meth_region_kernel<true, BSX_CT_SNP_CORRECT> : meth_region_kernel<false, BSX_CT_SNP_CORRECT>;
+    return combine ? meth_region_kernel<true, 0> : meth_region_kernel<false, 0>;
 }
 
 int ensure_staging(bsx_meth *m, size_t n, uint32_t stride) {
@@ -841,5 +922,179 @@ int bsx_meth_write_conversion_file(bsx_meth *m, const char *path) {
         fprintf(stderr, "conversion filter: %llu of %llu valid mappings dropped (>= %d methylated non-CpG calls)\n", (unsigned long long)dropped,
                 (unsigned long long)valid, m->conv_threshold);
     else fprintf(stderr, "conversion filter: 0 of %llu valid mappings dropped (report only)\n", (unsigned long long)valid);
+    return BSX_OK;
+}
+
+extern "C" int bsx_meth_regions(bsx_meth *m, const bsx_meth_opts *o, uint64_t n, const uint32_t *seq, const uint64_t *start, const uint64_t *end,
+                                uint64_t *out) {
+    if (!m || !o || (n && (!seq || !start || !end || !out))) { bsx_set_error("bsx_meth_regions: bad argument"); return BSX_ERR_ARG; }
+    const bsx_index *ix = m->ix;
+    for (uint64_t r = 0; r < n; r++) {
+        if (seq[r] >= ix->n_seq) { bsx_set_error("bsx_meth_regions: region %llu: sequence %u of %u", (unsigned long long)r, seq[r], ix->n_seq); return BSX_ERR_ARG; }
+        if (start[r] > end[r]) { bsx_set_error("bsx_meth_regions: region %llu: start %llu > end %llu", (unsigned long long)r, (unsigned long long)start[r],
+                                               (unsigned long long)end[r]); return BSX_ERR_ARG; }
+    }
+    BSX_CUDA_CHECK(cudaSetDevice(ix->device));
+    BSX_CUDA_CHECK(cudaDeviceSynchronize());           // in-process batches pile up on the mapper's streams
+    int rc = combine_once(m, o); if (rc) return rc;
+    if (n == 0) return BSX_OK;
+    const uint64_t cap = std::min<uint64_t>(n, REGION_SLICE);
+    unsigned long long *d_scan = nullptr, *d_out = nullptr; uint2 *d_span = nullptr;
+    if (cudaMalloc(&d_scan, (cap + 1) * 8) != cudaSuccess || cudaMalloc(&d_span, cap * 8) != cudaSuccess || cudaMalloc(&d_out, cap * 12 * 8) != cudaSuccess) {
+        cudaGetLastError(); cudaFree(d_scan); cudaFree(d_span); bsx_set_error("bsx_meth_regions: out of device memory"); return BSX_ERR_CUDA; }
+    int dev = 0, sms = 0, per_sm = 0;
+    const int snp_mode = m->ct_snp == BSX_CT_SNP_SKIP || m->ct_snp == BSX_CT_SNP_CORRECT ? m->ct_snp : 0;
+    const auto kern = region_kernel(o->combine_cpg != 0, snp_mode);
+    cudaGetDevice(&dev);
+    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, 256, 0);
+    const uint32_t min_depth = (uint32_t)std::max(o->min_depth, 1);
+    std::vector<unsigned long long> scan;
+    std::vector<uint2> span;
+    int err = BSX_OK;
+    for (uint64_t r0 = 0; r0 < n && err == BSX_OK; r0 += cap) {
+        const uint32_t k = (uint32_t)std::min(cap, n - r0);
+        scan.assign(k + 1, 0ull); span.resize(k);
+        for (uint32_t i = 0; i < k; i++) {
+            const uint32_t sq = seq[r0 + i], len = ix->size[sq];
+            const uint64_t lo = std::min<uint64_t>(start[r0 + i], len), hi = std::min<uint64_t>(end[r0 + i], len);   // clipped to the sequence
+            span[i] = make_uint2(ix->anchor[sq] + (uint32_t)lo, ix->anchor[sq] + (uint32_t)hi);
+            scan[i + 1] = scan[i] + (hi - lo + REGION_CHUNK - 1) / REGION_CHUNK;
+        }
+        auto step = [&]() -> int {
+            BSX_CUDA_CHECK(cudaMemcpy(d_scan, scan.data(), (k + 1) * 8, cudaMemcpyHostToDevice));
+            BSX_CUDA_CHECK(cudaMemcpy(d_span, span.data(), (size_t)k * 8, cudaMemcpyHostToDevice));
+            BSX_CUDA_CHECK(cudaMemset(d_out, 0, (size_t)k * 12 * 8));
+            if (scan[k]) {
+                const unsigned blocks = (unsigned)std::min<unsigned long long>((scan[k] + 7) / 8, (unsigned long long)std::max(per_sm, 1) * (unsigned)sms);
+                kern<<<blocks, 256>>>(ix->d_refcat, m->d_meth, m->d_depth, m->d_confirm, m->d_snp, min_depth, d_scan, d_span, k, d_out);
+                BSX_CUDA_CHECK(cudaGetLastError());
+            }
+            BSX_CUDA_CHECK(cudaMemcpy(out + r0 * 12, d_out, (size_t)k * 12 * 8, cudaMemcpyDeviceToHost));
+            return BSX_OK;
+        };
+        err = step();
+    }
+    cudaFree(d_scan); cudaFree(d_span); cudaFree(d_out);
+    return err;
+}
+
+extern "C" size_t bsx_meth_write_regions(bsx_meth *m, const bsx_meth_opts *o, uint64_t n, const uint32_t *seq, const uint64_t *start,
+                                         const uint64_t *end, int fd) {
+    if (!m || !o || (n && (!seq || !start || !end))) { bsx_set_error("bsx_meth_write_regions: bad argument"); return 0; }
+    const bsx_index *ix = m->ix;
+    static const char *const ctx[3] = {"CpG", "CHG", "CHH"};
+    const int threads = bsx_host_threads(0);
+    size_t written = 0;
+    auto put = [&](const std::string &s) {
+        size_t off = 0;
+        while (off < s.size()) { const ssize_t w = write(fd, s.data() + off, s.size() - off); if (w <= 0) return false; off += (size_t)w; written += (size_t)w; }
+        return true;
+    };
+    if (!put("chr\tstart\tend\tcontext\tsites\tcovered\tC_count\tCT_count\tlevel\n")) return 0;
+    std::vector<uint64_t> sums;
+    for (uint64_t r0 = 0; r0 < n; r0 += REGION_SLICE) {
+        const uint64_t k = std::min<uint64_t>(REGION_SLICE, n - r0);
+        sums.resize(k * 12);
+        if (bsx_meth_regions(m, o, k, seq + r0, start + r0, end + r0, sums.data()) != BSX_OK) return 0;
+        std::vector<std::string> chunk((size_t)threads);
+        bsx_parallel(threads, (size_t)k, [&](int t, size_t b, size_t e) {
+            Sink s{&chunk[t]};
+            for (size_t i = b; i < e; i++) {
+                const std::string &name = ix->names[seq[r0 + i]];
+                for (int c = 0; c < 3; c++) {
+                    const uint64_t *v = &sums[(i * 3 + c) * 4];
+                    s.put(name.data(), name.size()); s.putc('\t'); s.putu(start[r0 + i]); s.putc('\t'); s.putu(end[r0 + i]); s.putc('\t');
+                    s.put(ctx[c], 3);
+                    for (int f = 0; f < 4; f++) { s.putc('\t'); s.putu(v[f]); }
+                    s.putc('\t');
+                    if (v[3]) { char buf[48]; const int l = snprintf(buf, sizeof buf, "%.4f", (double)v[2] / (double)v[3]); s.put(buf, (size_t)l); }
+                    else s.put("NA", 2);
+                    s.putc('\n');
+                }
+            }
+        });
+        for (const std::string &c : chunk) if (!put(c)) return 0;
+    }
+    return written;
+}
+
+// name -> index of the selected sequences (a repeated name: the last record, as the command lines' own lookup)
+static std::unordered_map<std::string, uint32_t> selected_names(const bsx_index *ix, const uint8_t *selected) {
+    std::unordered_map<std::string, uint32_t> by;
+    for (uint32_t k = 0; k < ix->n_seq; k++) if (!selected || selected[k]) by[ix->names[k]] = k;
+    return by;
+}
+
+int bsx_regions_bed(const bsx_index *ix, const uint8_t *selected, const char *path, bsx_regions &rg) {
+    rg = bsx_regions{};
+    FILE *f = fopen(path, "rb");
+    if (!f) { bsx_set_error("failed to open BED file: %s", path); return BSX_ERR_IO; }
+    std::string text;
+    char buf[1 << 16];
+    for (size_t got; (got = fread(buf, 1, sizeof buf, f)) > 0;) text.append(buf, got);
+    const bool io_err = ferror(f) != 0;
+    fclose(f);
+    if (io_err) { bsx_set_error("failed to read BED file: %s", path); return BSX_ERR_IO; }
+    const auto by = selected_names(ix, selected);
+    auto number = [](const char *p, const char *e, uint64_t &v) {
+        if (p == e) return false;
+        v = 0;
+        for (; p < e; p++) {
+            if (*p < '0' || *p > '9' || v > (UINT64_MAX - 9) / 10) return false;
+            v = v * 10 + (uint64_t)(*p - '0');
+        }
+        return true;
+    };
+    uint64_t line = 0;
+    for (size_t b = 0; b < text.size();) {
+        size_t e = text.find('\n', b);
+        if (e == std::string::npos) e = text.size();
+        const size_t next = e + 1;
+        line++;
+        if (e > b && text[e - 1] == '\r') e--;
+        const char *p = text.data() + b, *q = text.data() + e;
+        b = next;
+        if (std::all_of(p, q, [](char c) { return c == ' ' || c == '\t'; })) continue;
+        auto starts = [&](const char *w) { const size_t l = strlen(w); return (size_t)(q - p) >= l && !memcmp(p, w, l) && ((size_t)(q - p) == l || p[l] == ' ' || p[l] == '\t'); };
+        if (*p == '#' || starts("track") || starts("browser")) continue;
+        const char *col[4] = {p, nullptr, nullptr, nullptr};
+        int nc = 1;
+        for (const char *x = p; x < q && nc < 4; x++) if (*x == '\t') col[nc++] = x + 1;
+        if (nc < 3) { bsx_set_error("%s:%llu: fewer than 3 columns", path, (unsigned long long)line); return BSX_ERR_ARG; }
+        const char *end3 = nc == 4 ? col[3] - 1 : q;
+        uint64_t s = 0, t = 0;
+        if (!number(col[1], col[2] - 1, s) || !number(col[2], end3, t)) {
+            bsx_set_error("%s:%llu: start and end must be non-negative integers", path, (unsigned long long)line); return BSX_ERR_ARG; }
+        if (s > t) { bsx_set_error("%s:%llu: start %llu > end %llu", path, (unsigned long long)line, (unsigned long long)s, (unsigned long long)t); return BSX_ERR_ARG; }
+        const auto it = by.find(std::string(col[0], col[1] - 1));
+        if (it == by.end()) { rg.skipped++; continue; }
+        rg.seq.push_back(it->second); rg.start.push_back(s); rg.end.push_back(t);
+    }
+    return BSX_OK;
+}
+
+int bsx_regions_tiles(const bsx_index *ix, const uint8_t *selected, uint64_t width, bsx_regions &rg) {
+    rg = bsx_regions{};
+    if (width < 1) { bsx_set_error("tile width must be >= 1"); return BSX_ERR_ARG; }
+    std::vector<uint32_t> order;
+    for (uint32_t k = 0; k < ix->n_seq; k++) if (!selected || selected[k]) order.push_back(k);
+    std::stable_sort(order.begin(), order.end(), [&](uint32_t a, uint32_t b) { return ix->names[a] < ix->names[b]; });   // the table's order
+    for (uint32_t k : order)
+        for (uint64_t s = 0; s < ix->size[k]; s += width) {
+            rg.seq.push_back(k); rg.start.push_back(s); rg.end.push_back(std::min<uint64_t>(s + width, ix->size[k]));
+        }
+    return BSX_OK;
+}
+
+int bsx_meth_write_regions_file(bsx_meth *m, const bsx_meth_opts *o, const bsx_regions &rg, const char *path) {
+    const int fd = open(path, O_WRONLY | O_CREAT | O_TRUNC, 0644);
+    if (fd < 0) { fprintf(stderr, "failed to open region report file: %s\n", path); return BSX_ERR_IO; }
+    const size_t w = bsx_meth_write_regions(m, o, rg.seq.size(), rg.seq.data(), rg.start.data(), rg.end.data(), fd);
+    close(fd);
+    if (w == 0) { fprintf(stderr, "%s\n", bsx_last_error()); return BSX_ERR_IO; }
+    if (rg.skipped)
+        fprintf(stderr, "regions: %llu of %llu skipped (sequence not in the reference or not selected)\n", (unsigned long long)rg.skipped,
+                (unsigned long long)(rg.skipped + rg.seq.size()));
     return BSX_OK;
 }

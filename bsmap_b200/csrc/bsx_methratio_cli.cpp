@@ -17,6 +17,10 @@
 //   --conversion-filter N      drop alignments with N or more methylated non-CpG calls (incompletely converted reads);
 //                              N 0..255, 0 = count only; prints "conversion filter: D of V valid mappings dropped" to stderr
 //   --conversion-report FILE   the alignments by their number of methylated non-CpG calls (alone: N = 0)
+//   --region-report FILE       methylation levels per region and context (sites, covered, C_count, CT_count, level),
+//                              reduced on the device from the same counters as the table, over
+//   --regions BED                the regions of a BED file (columns 1-3), in the file's order, or
+//   --tiles W                    tiles of W bases over every selected sequence, in the table's order
 #include <chrono>
 #include <cstdio>
 #include <cstdlib>
@@ -43,6 +47,8 @@ struct MOpts {
     int ct_snp = 0;                          // --ct-snp: BSX_CT_SNP_*
     int conv = -1;                           // --conversion-filter N; -1 = off
     std::string conv_report;                 // --conversion-report FILE
+    std::string region_report, regions;      // --region-report FILE, --regions BED
+    long long tiles = 0;                     // --tiles W; 0 = none
     std::vector<std::string> files;
 };
 
@@ -65,7 +71,8 @@ void parse(int argc, char **argv, MOpts &m) {
                                {'p', "pair", false}, {'z', "zero-meth", false}, {'q', "quiet", false}, {'r', "remove-duplicate", false},
                                {'t', "trim-fillin", true}, {'g', "combine-CpG", false}, {'m', "min-depth", true}, {'h', "help", false},
                                {'\1', "mbias", true}, {'\2', "mbias-ignore", true}, {'\3', "ct-snp", true},
-                               {'\4', "conversion-filter", true}, {'\5', "conversion-report", true}};   // long only
+                               {'\4', "conversion-filter", true}, {'\5', "conversion-report", true}, {'\6', "region-report", true},
+                               {'\7', "regions", true}, {'\10', "tiles", true}};   // long only
     auto apply = [&](char c, const char *v) {
         if (!v) v = "";
         switch (c) {
@@ -99,8 +106,14 @@ void parse(int argc, char **argv, MOpts &m) {
                 if (*e || e == v || x < 0 || x > BSX_CONV_BINS - 1) usage_error("option --conversion-filter: expected an integer 0..255");
                 m.conv = (int)x; } break;
             case '\5': m.conv_report = v; break;
+            case '\6': m.region_report = v; break;
+            case '\7': m.regions = v; break;
+            case '\10': { char *e; const long long x = strtoll(v, &e, 10);
+                if (*e || e == v || x < 1) usage_error("option --tiles: expected an integer >= 1");
+                m.tiles = x; } break;
             case 'h': printf("Usage: methratio [options] BSMAP_MAPPING_FILES\n  -o FILE -d FILE [-c CHR] [-u] [-p] [-z] [-q] [-r] [-t N] [-g] [-m FOLD] [--mbias FILE] [--mbias-ignore A,B,C,D]\n"
-                             "  [--ct-snp no-action|correct|skip] [--conversion-filter N] [--conversion-report FILE]\n"); exit(0);
+                             "  [--ct-snp no-action|correct|skip] [--conversion-filter N] [--conversion-report FILE]\n"
+                             "  [--region-report FILE (--regions BED | --tiles W)]\n"); exit(0);
         }
     };
     for (int i = 1; i < argc; i++) {
@@ -292,6 +305,9 @@ extern "C" int bsx_methratio_main(int argc, char **argv) {
     if (m.out.empty()) usage_error("Missing output file name, use -o or --out option.");
     if (m.files.empty()) usage_error("Require at least one BSMAP_MAPPING_FILE.");
     if (!m.conv_report.empty() && m.conv < 0) m.conv = 0;
+    if (!m.regions.empty() && m.tiles) usage_error("--regions and --tiles exclude each other");
+    if (m.region_report.empty() && (!m.regions.empty() || m.tiles)) usage_error("--regions / --tiles need --region-report FILE");
+    if (!m.region_report.empty() && m.regions.empty() && !m.tiles) usage_error("--region-report needs --regions BED or --tiles W");
     const bool cycles = !m.mbias.empty() || m.ignore_set;
     if (cycles)
         for (const std::string &f : m.files) {
@@ -331,6 +347,10 @@ extern "C" int bsx_methratio_main(int argc, char **argv) {
         fprintf(stderr, "%s\n", bsx_last_error()); return 1; }
     if ((!m.mbias.empty() && bsx_meth_enable_mbias(mh) != BSX_OK) || (m.ignore_set && bsx_meth_set_ignore(mh, m.ignore) != BSX_OK) ||
         (m.ct_snp && bsx_meth_enable_ct_snp(mh, m.ct_snp) != BSX_OK) || (m.conv >= 0 && bsx_meth_enable_conversion_filter(mh, m.conv) != BSX_OK)) {
+        fprintf(stderr, "%s\n", bsx_last_error()); return 1; }
+    bsx_regions regions;                                      // read before the pile-up, so that a bad BED fails early
+    if ((!m.regions.empty() && bsx_regions_bed(ix, selected.data(), m.regions.c_str(), regions) != BSX_OK) ||
+        (m.tiles && bsx_regions_tiles(ix, selected.data(), (uint64_t)m.tiles, regions) != BSX_OK)) {
         fprintf(stderr, "%s\n", bsx_last_error()); return 1; }
 
     const double t_ix = now_s();
@@ -421,6 +441,10 @@ extern "C" int bsx_methratio_main(int argc, char **argv) {
     if (m.conv >= 0) {
         if (!m.conv_report.empty()) disp(m, ("writing " + m.conv_report + " ...").c_str());
         if (bsx_meth_write_conversion_file(mh, m.conv_report.empty() ? nullptr : m.conv_report.c_str()) != BSX_OK) return 1;
+    }
+    if (!m.region_report.empty()) {
+        disp(m, ("writing " + m.region_report + " ...").c_str());
+        if (bsx_meth_write_regions_file(mh, &m.o, regions, m.region_report.c_str()) != BSX_OK) return 1;
     }
     if (getenv("BSX_CLI_TIMING"))
         fprintf(stderr, "[bsx timing] reference FASTA %.3f s || CUDA context (ready at %.3f s), packed reference + counters %.3f s, parse + pile-up %.3f s, report %.3f s\n",

@@ -69,6 +69,7 @@ EXPORTS = [
     "bsx_meth_enable_mbias", "bsx_meth_set_ignore", "bsx_meth_mbias", "bsx_meth_write_mbias",
     "bsx_meth_enable_ct_snp", "bsx_meth_download_ct_snp",
     "bsx_meth_enable_conversion_filter", "bsx_meth_conversion", "bsx_meth_write_conversion",
+    "bsx_meth_regions", "bsx_meth_write_regions",
 ]
 
 METH_READ2 = 8        # BSX_METH_READ2: alignment flag, read 2 (FLAG 0x80)
@@ -166,6 +167,9 @@ def load():
     L.bsx_meth_conversion.argtypes = [vp, vp, C.POINTER(C.c_uint64)]
     L.bsx_meth_write_conversion.restype = sz
     L.bsx_meth_write_conversion.argtypes = [vp, i32]
+    L.bsx_meth_regions.argtypes = [vp, C.POINTER(MethOpts), C.c_uint64, vp, vp, vp, vp]
+    L.bsx_meth_write_regions.restype = sz
+    L.bsx_meth_write_regions.argtypes = [vp, C.POINTER(MethOpts), C.c_uint64, vp, vp, vp, i32]
     L.bsx_packed_stride.restype = sz
     L.bsx_packed_stride.argtypes = [u32]
     L.bsx_pack_reads.argtypes = [u32, vp, u32, vp, vp, C.POINTER(C.c_uint64), i32]

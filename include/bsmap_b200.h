@@ -363,10 +363,36 @@ int bsx_meth_conversion(bsx_meth *m, uint64_t *out /* BSX_CONV_BINS */, uint64_t
  * non-empty bin, ascending, the last labelled "255+"; dropped is 1 when the bin's alignments were dropped, else 0.
  * Returns bytes written (0 on error). */
 size_t bsx_meth_write_conversion(bsx_meth *m, int fd);
+/* --- methylation levels over regions, reduced on the device from the counters ----------------------------------------
+ *   region   (sequence, start, end), 0-based and half-open as in BED; start == end is empty; an end past the sequence end
+ *            is clipped when counting.  Each region is reported for the contexts CpG, CHG, CHH (ctx 0, 1, 2).
+ *   site     a reference C (strand '+') or G (strand '-') at a position q with start <= q < end.  Its context is the
+ *            M-bias rule on its strand: '+' CpG if q+1 is G, else CHG if q+2 is G, else CHH; '-' the same with q-1, q-2
+ *            and C; non-ACGT bases and positions off the sequence count as H.  With -g a G that follows a C is not a
+ *            site: its counts sit on the C, and the CpG is one site.
+ *   sites    the number of sites
+ *   covered  the sites whose line the table would print with -z: depth >= max(-m, 1), and, with C/T SNP evidence, not
+ *            dropped by the mode (BSX_CT_SNP_SKIP: any SNP evidence; BSX_CT_SNP_CORRECT: eff == 0)
+ *   C, CT    over the covered sites, the sums of the table's methylated count (methy_C / C_count) and of its depth
+ *            (total_C / the raw CT_count)
+ * So covered, C and CT are the count and the sums of the -z table's lines in the region, by context.  -z itself is
+ * ignored (leaving out unmethylated sites would bias the levels up), and `correct`'s scaled eff_CT_count is not summed:
+ * the sums stay exact integers. */
+/* out[(r * 3 + ctx) * 4 + {0 sites, 1 covered, 2 C, 3 CT}] for the n regions (seq: sequence index; a bad index or
+ * start > end: BSX_ERR_ARG).  Synchronises the device.  -g combines the counters first, like bsx_meth_download; without
+ * -g the counters are not changed, so more alignments may be added afterwards. */
+int bsx_meth_regions(bsx_meth *m, const bsx_meth_opts *o, uint64_t n, const uint32_t *seq, const uint64_t *start, const uint64_t *end,
+                     uint64_t *out);
+/* write the region report to fd: a header line "chr start end context sites covered C_count CT_count level"
+ * (tab-separated), then three lines per region, CpG, CHG, CHH, in region order, start and end as given; level = %.4f
+ * of C / CT, or NA when CT == 0.  Returns bytes written (0 on error). */
+size_t bsx_meth_write_regions(bsx_meth *m, const bsx_meth_opts *o, uint64_t n, const uint32_t *seq, const uint64_t *start, const uint64_t *end,
+                              int fd);
 /* the methratio.py command line: -o -d [-c -u -p -z -q -r -t -g -m -s] files... (SAM, BAM and BSP; -s is ignored);
  * extensions: --mbias FILE (the M-bias report) and --mbias-ignore A,B,C,D (bsx_meth_set_ignore), SAM and BAM only;
  * --ct-snp no-action|correct|skip (bsx_meth_enable_ct_snp); --conversion-filter N and --conversion-report FILE
- * (bsx_meth_enable_conversion_filter, bsx_meth_write_conversion) */
+ * (bsx_meth_enable_conversion_filter, bsx_meth_write_conversion); --region-report FILE with --regions BED or --tiles W
+ * (bsx_meth_write_regions) */
 int bsx_methratio_main(int argc, char **argv);
 
 /* --- the bsmap command line (main.cpp:441-476): same options, same output files -------------- */
