@@ -401,6 +401,9 @@ class Meth:
         """seqs: list of bytes (SEQ as printed); strand: bit 0 / 1 = first / second ZS character is '-';
         read2: optional per-alignment truth values (FLAG 0x80), setting BSX_METH_READ2 in flags"""
         n = len(seqs)
+        longest = max((len(s) for s in seqs), default=0)
+        if longest > 65535:                                  # the lengths bsx_meth_add takes are 16-bit
+            raise ValueError("Meth.add: a SEQ of %d bases; at most 65535 are supported" % longest)
         if read2 is not None:
             flags = np.asarray(flags, dtype=np.uint8) | np.where(np.asarray(read2, dtype=bool), np.uint8(METH_READ2), np.uint8(0))
         buf, lens = pack_reads(seqs, stride=max(16, (max((len(s) for s in seqs), default=1) + 15) // 16 * 16))

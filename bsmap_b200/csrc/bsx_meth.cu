@@ -753,7 +753,10 @@ extern "C" size_t bsx_meth_write(bsx_meth *m, const bsx_meth_opts *o, const char
                 s.put(name.data(), name.size()); s.putc('\t'); s.putu(i + 1); s.putc('\t');
                 const char rc = (char)(rs[i] >= 'a' && rs[i] <= 'z' ? rs[i] - 32 : rs[i]);
                 s.putc(rc == 'C' ? '+' : '-'); s.putc('\t');
-                if (i >= 2) for (size_t j = i - 2; j < i + 3 && j < L; j++) s.putc((char)(rs[j] >= 'a' && rs[j] <= 'z' ? rs[j] - 32 : rs[j]));   // refcr[i-2:i+3] ('' when i < 2)
+                // refcr[i-2:i+3] with Python's slice rules: for i < 2 the start counts from the sequence end, so a
+                // sequence of 4 bases or fewer prints some of its last bases there, a longer one nothing
+                const size_t c0 = i >= 2 ? i - 2 : (i + L >= 2 ? i + L - 2 : 0), c1 = std::min<size_t>(i + 3, L);
+                for (size_t j = c0; j < c1; j++) s.putc((char)(rs[j] >= 'a' && rs[j] <= 'z' ? rs[j] - 32 : rs[j]));
                 s.putc('\t'); s.putf3(ratio); s.putc('\t');
                 if (snp_mode) { s.putf2(eff); s.putc('\t'); s.putu(mm); s.putc('\t'); s.putu(d); s.putc('\t'); s.putu(rg); s.putc('\t'); s.putu(rga); s.putc('\t'); }
                 else { s.putu(d); s.putc('\t'); s.putu(mm); s.putc('\t'); }

@@ -166,7 +166,10 @@ bool parse_line(const char *b, const char *e, bool sam, const std::unordered_map
         const int n = split(b, e, f, 64);
         if (n < 11) return false;
         uint32_t fl = 0;
-        if (f[1].n && f[1].p[0] >= '0' && f[1].p[0] <= '9') {
+        // numeric when every character is a digit: the letters of 0x40 / 0x80 ('1', '2') may open a lettered FLAG ("2s")
+        bool numeric = f[1].n > 0;
+        for (uint32_t i = 0; i < f[1].n; i++) numeric = numeric && f[1].p[i] >= '0' && f[1].p[i] <= '9';
+        if (numeric) {
             const long long v = to_int(f[1]);
             if (v & 0x4) return false;
             if (v & 0x100) fl |= BSX_METH_SECONDARY;
@@ -263,6 +266,7 @@ bool pile_bam(const std::string &path, const std::unordered_map<std::string, uin
                 char *sq = bases[t].data() + used;
                 for (int32_t i = 0; i < l_seq; i++) sq[i] = nt16[(q[off_seq + ((size_t)i >> 1)] >> ((~i & 1) << 2)) & 15];
                 a.seq = sq; a.len = (uint32_t)l_seq; used += (size_t)l_seq;
+                if (l_seq == 0) { a.seq = "*"; a.len = 1; }                 // no SEQ: `samtools view` prints '*', one character to the script
                 // tags: two letters, a type, a value
                 int strand = -1;
                 size_t x = off_seq + ((size_t)l_seq + 1) / 2 + (size_t)l_seq;
@@ -355,6 +359,7 @@ extern "C" int bsx_methratio_main(int argc, char **argv) {
 
     const double t_ix = now_s();
     uint64_t nmap = 0;
+    const char *cur_path = "";
     // one piece of alignments (file order = thread 0's, then thread 1's, ...) -> staging arrays -> the device
     auto pile = [&](const std::vector<std::vector<Aln>> &part) -> bool {
         size_t tot = 0; uint32_t maxlen = 16;
@@ -362,15 +367,16 @@ extern "C" int bsx_methratio_main(int argc, char **argv) {
         for (int t = 0; t < threads; t++) { off[t] = tot; tot += part[t].size(); for (const Aln &a : part[t]) maxlen = std::max(maxlen, a.len); }
         off[threads] = tot;
         if (tot > 0xffffffffull) { fprintf(stderr, "too many alignments in one piece\n"); return false; }
-        const uint32_t stride = (std::min<uint32_t>(maxlen, 65535u) + 15u) & ~15u;
+        // bsx_meth_add takes 16-bit lengths: a longer SEQ is refused rather than piled up cut short
+        if (maxlen > 65535u) { fprintf(stderr, "%s: SEQ longer than 65535 bases (%u): not supported\n", cur_path, maxlen); return false; }
+        const uint32_t stride = (maxlen + 15u) & ~15u;
         std::vector<char> sq(tot * stride); std::vector<uint16_t> len(tot); std::vector<uint32_t> chr(tot), pos(tot);
         std::vector<uint8_t> strand(tot), flags(tot); std::vector<int32_t> ins(tot), mate(tot);
         bsx_parallel(threads, (size_t)threads, [&](int t, size_t, size_t) {
             size_t i = off[t];
             for (const Aln &a : part[t]) {
-                const uint32_t l = std::min(a.len, stride);
-                memcpy(&sq[i * stride], a.seq, l);
-                len[i] = (uint16_t)l; chr[i] = a.chr; pos[i] = a.pos; strand[i] = a.strand; flags[i] = a.flags; ins[i] = a.insert; mate[i] = a.mate;
+                memcpy(&sq[i * stride], a.seq, a.len);
+                len[i] = (uint16_t)a.len; chr[i] = a.chr; pos[i] = a.pos; strand[i] = a.strand; flags[i] = a.flags; ins[i] = a.insert; mate[i] = a.mate;
                 i++;
             }
         });
@@ -380,6 +386,7 @@ extern "C" int bsx_methratio_main(int argc, char **argv) {
     };
     for (const std::string &path : m.files) {
         disp(m, ("reading " + path + " ...").c_str());
+        cur_path = path.c_str();
         const size_t pl = path.size();
         std::string suf = pl >= 4 ? path.substr(pl - 4) : "";
         for (char &c : suf) c = (char)toupper((unsigned char)c);

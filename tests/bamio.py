@@ -49,6 +49,43 @@ def write_sam(path, records):
             f.write("\t".join([name, str(flag), "*", "0", "0", "*", "*", "0", "0", seq or "*", qual if qual is not None else "*"]) + "\n")
 
 
+def aligned_bam_from_sam(path, sam: str, extra_names=()):
+    """SAM text (numeric FLAG, @SQ header; Z and i tags) -> an aligned, unsorted BAM file in the same record order.
+    Reference names are the @SQ names, then extra_names (records on names outside the FASTA).  BAM stores no lowercase:
+    SEQ is upper-cased; SEQ '*' becomes l_seq 0."""
+    names, recs = [], []
+    for line in sam.splitlines():
+        if line.startswith("@SQ"):
+            f = dict(x.split(":", 1) for x in line.split("\t")[1:])
+            names.append((f["SN"], int(f["LN"])))
+    names += [(n, 1) for n in extra_names]
+    rid = {n: i for i, (n, _) in enumerate(names)}
+    for line in sam.splitlines():
+        if line.startswith("@") or not line:
+            continue
+        c = line.split("\t")
+        seq = "" if c[9] == "*" else c[9]
+        l = len(seq)
+        codes = [NT16.index(ch.upper()) if ch.upper() in NT16 else 15 for ch in seq] + ([0] if l & 1 else [])
+        packed = bytes((codes[i] << 4) | codes[i + 1] for i in range(0, len(codes), 2))
+        cig = b"" if c[5] == "*" else struct.pack("<I", int(c[5][:-1]) << 4)
+        tags = b""
+        for t in c[11:]:
+            tg, ty, v = t.split(":", 2)
+            tags += tg.encode() + (b"Z" + v.encode() + b"\0" if ty == "Z" else b"i" + struct.pack("<i", int(v)))
+        qn = c[0].encode() + b"\0"
+        ref = rid[c[2]]
+        core = struct.pack("<iiBBHHHiiii", ref, int(c[3]) - 1, len(qn), 255, 4680, len(cig) // 4, int(c[1]), l,
+                           ref if c[6] != "*" else -1, int(c[7]) - 1, int(c[8]))
+        body = core + qn + cig + packed + bytes([0xff] * l) + tags
+        recs.append(struct.pack("<i", len(body)) + body)
+    head = "@HD\tVN:1.0\tSO:unsorted\n"
+    raw = b"BAM\1" + struct.pack("<i", len(head)) + head.encode() + struct.pack("<i", len(names))
+    for n, ln in names:
+        raw += struct.pack("<i", len(n) + 1) + n.encode() + b"\0" + struct.pack("<i", ln)
+    open(path, "wb").write(bgzf(raw + b"".join(recs)))
+
+
 def bam_to_sam_text(path) -> str:
     """an aligned BAM file as headerless SAM text (what `samtools view` prints, numeric FLAG; Z / A / integer tags only):
     lets the methratio oracle, which reads text, see the records of a BAM file in the file's own order"""
