@@ -488,6 +488,34 @@ class Meth:
             check(1)
         return w
 
+    def enable_pdr(self, min_cpg: int = 4):
+        """score every alignment by its CpG calls for the proportion of discordant reads: an alignment with `min_cpg`
+        (1..255) or more CpG calls is concordant or discordant (include/bsmap_b200.h); before the first add / mapped batch"""
+        check(load().bsx_meth_enable_pdr(self.h, int(min_cpg)))
+
+    def pdr_counters(self, k: int):
+        """(concordant, discordant) CpG calls of informative alignments on reference sequence k, after -g combining"""
+        n = load().bsx_index_seq_size(self.index.h, k)
+        c, d = np.zeros(n, dtype=np.uint32), np.zeros(n, dtype=np.uint32)
+        check(load().bsx_meth_download_pdr(self.h, C.byref(self.o), k, c.ctypes.data, d.ctypes.data))
+        return c, d
+
+    def pdr(self):
+        """-> (informative alignments, discordant alignments)"""
+        inf, disc = C.c_uint64(0), C.c_uint64(0)
+        check(load().bsx_meth_pdr(self.h, C.byref(inf), C.byref(disc)))
+        return inf.value, disc.value
+
+    def write_pdr(self, seqs, fd: int, chroms=None, threads=0) -> int:
+        """the PDR file (include/bsmap_b200.h) to fd; seqs and chroms as in write; returns bytes written"""
+        keep = [s if isinstance(s, bytes) else bytes(s) for s in seqs]
+        lens = np.array([len(s) for s in keep], dtype=np.uint32)
+        sel = None if chroms is None else np.ascontiguousarray(np.asarray(chroms, dtype=np.uint8))
+        w = load().bsx_meth_write_pdr(self.h, C.byref(self.o), strs(keep), lens.ctypes.data, _ptr(sel), threads, fd)
+        if w == 0:
+            check(1)
+        return w
+
     @staticmethod
     def _regions(chr_idx, start, end):
         arr = lambda a, t: np.ascontiguousarray(np.asarray(a, dtype=t).reshape(-1))
@@ -503,6 +531,15 @@ class Meth:
         out = np.zeros((len(c), 3, 4), dtype=np.uint64)
         check(load().bsx_meth_regions(self.h, C.byref(self.o), len(c), c.ctypes.data, s.ctypes.data, e.ctypes.data, out.ctypes.data))
         return out
+
+    def regions_pdr(self, chr_idx, start, end):
+        """-> (regions' array as in regions, uint64 array [region][concordant, discordant]: the sums over the PDR file's
+        lines in each region); needs enable_pdr"""
+        c, s, e = self._regions(chr_idx, start, end)
+        out, pdr = np.zeros((len(c), 3, 4), dtype=np.uint64), np.zeros((len(c), 2), dtype=np.uint64)
+        check(load().bsx_meth_regions_pdr(self.h, C.byref(self.o), len(c), c.ctypes.data, s.ctypes.data, e.ctypes.data, out.ctypes.data,
+                                          pdr.ctypes.data))
+        return out, pdr
 
     def write_regions(self, fd: int, chr_idx, start, end) -> int:
         """the region report (include/bsmap_b200.h) to fd; returns bytes written"""

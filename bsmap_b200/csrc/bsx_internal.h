@@ -119,6 +119,10 @@ int bsx_regions_tiles(const bsx_index *ix, const uint8_t *selected, uint64_t wid
 // the region report (bsx_meth_write_regions) to a new file at path, and "regions: S of R skipped (...)" on stderr when
 // the BED named sequences that are not there; errors are printed
 int bsx_meth_write_regions_file(bsx_meth *m, const bsx_meth_opts *o, const bsx_regions &rg, const char *path);
+// the command lines' PDR output: bsx_meth_write_pdr to a new file at path, and on stderr "PDR: I of V valid mappings
+// informative (>= K CpG calls), D discordant"; errors are printed (bsx_meth.cu)
+int bsx_meth_write_pdr_file(bsx_meth *m, const bsx_meth_opts *o, const char *const *seqs, const uint32_t *lens, const uint8_t *chroms, int threads,
+                            const char *path);
 // "no-action" / "correct" / "skip" -> BSX_CT_SNP_*, anything else 0 (bsx_meth.cu)
 int bsx_ct_snp_mode(const char *name);
 int bsx_inflate_file(const char *path, std::vector<char> &out);   // gzip / BGZF members -> bytes (bsx_reads.cpp)

@@ -30,6 +30,12 @@
 // with `Cycles` (it needs the call's cycle and context, and its histogram the capped grid): before an alignment's calls are
 // deposited, the warp counts its methylated non-CpG calls (its score), lane 0 adds the alignment to a per-CTA shared
 // histogram of scores, and an alignment whose score reaches the threshold returns without depositing anything.
+//
+// The proportion of discordant reads (bsx_meth_enable_pdr) switches them to their `Pdr` instantiation, again only with
+// `Cycles`: the same first pass also counts the alignment's methylated and unmethylated CpG calls, and when there are at
+// least K of them the second pass adds every CpG call to `concordant` (all methylated or all unmethylated) or
+// `discordant`, two more u32 arrays over the positions.  The informative and discordant alignments go into two per-CTA
+// shared counters, flushed like the histograms.
 #include <algorithm>
 #include <cmath>
 #include <cstdio>
@@ -64,6 +70,10 @@ struct bsx_meth {
     // conversion filter: fixed before the first alignment is piled up
     int conv_threshold = 0;                           // 0 = report only
     unsigned long long *d_conv = nullptr;             // BSX_CONV_BINS alignments by score; NULL = filter off
+    // PDR: fixed before the first alignment is piled up
+    uint32_t pdr_min_cpg = 0;                         // K; 0 = off
+    uint32_t *d_conc = nullptr, *d_disc = nullptr;    // n_words * 16 counters each, like d_meth / d_depth
+    unsigned long long *d_pdr = nullptr;              // informative, discordant alignments; NULL = PDR off
 };
 
 namespace {
@@ -84,9 +94,18 @@ struct ConvArgs {
     uint32_t threshold;           // an alignment with score >= threshold is dropped; 0 = none is
 };
 
+// what the Pdr instantiation needs beyond the Cycles one
+struct PdrArgs {
+    uint32_t *concordant, *discordant;   // per position: CpG calls of informative alignments, by the alignment's class
+    unsigned long long *count;           // informative, discordant alignments
+    uint32_t min_cpg;                    // K: an alignment with K or more CpG calls is informative
+};
+
 // Conv: the CTA's alignments by score, zeroed before and flushed (non-zero bins) after them.  At file scope, so that the
 // pile-up addresses it directly; only the Conv kernels reference it, and only they are given its 1 KB.
 __shared__ uint32_t conv_hist[BSX_CONV_BINS];
+// Pdr: the CTA's informative and discordant alignments, zeroed and flushed the same way
+__shared__ uint32_t pdr_count[2];
 
 __device__ __forceinline__ uint32_t ref_code(const uint32_t *refcat, uint32_t q) { return (refcat[q >> 4] >> (30 - 2 * (q & 15))) & 3u; }
 
@@ -98,12 +117,16 @@ __device__ __forceinline__ uint32_t ref_code(const uint32_t *refcat, uint32_t q)
 // after the same trimming, bounds test and (Cycles) exclusion as a call.
 // Conv (with Cycles): a first pass scores the alignment, its methylated calls whose context is not CpG, into conv_hist;
 // an alignment scoring cv.threshold or more (when non-zero) returns before the second pass deposits anything.
-template <bool Cycles, bool Snp, bool Conv, class GetC>
+// Pdr (with Cycles): the first pass also counts the methylated (pm) and unmethylated (pu) CpG calls; when the alignment is
+// kept and pm + pu >= pd.min_cpg, the second pass adds each CpG call to pd.concordant (pm == 0 or pu == 0) or
+// pd.discordant, and lane 0 counts the alignment in pdr_count (shared).
+template <bool Cycles, bool Snp, bool Conv, bool Pdr, class GetC>
 __device__ __forceinline__ void pile_alignment(const uint32_t *__restrict__ refcat, const uint32_t *__restrict__ seqinfo, uint32_t n_seq,
                                                uint32_t *meth, uint32_t *depth, unsigned long long *n_valid, const bsx_meth_opts &o,
                                                uint32_t k, long long pos, long long len, int st, int ins, long long mate_pos, bool sam, int lane, GetC getc,
                                                const MbiasArgs &mb = MbiasArgs{}, int read2 = 0, uint32_t *hist = nullptr,
-                                               uint32_t *confirm = nullptr, uint32_t *snp = nullptr, const ConvArgs &cv = ConvArgs{}) {
+                                               uint32_t *confirm = nullptr, uint32_t *snp = nullptr, const ConvArgs &cv = ConvArgs{},
+                                               const PdrArgs &pd = PdrArgs{}) {
     const int L = (int)len;                                  // printed length, before trimming
     const uint32_t *anchor = seqinfo, *size = seqinfo + n_seq + 1;
     long long start = 0;
@@ -148,23 +171,46 @@ __device__ __forceinline__ void pile_alignment(const uint32_t *__restrict__ refc
     } else {
         const bool rev = ((st ^ (st >> 1)) & 1) != 0;
         const int lo = read2 ? mb.ignore[2] : mb.ignore[0], hi = L - (read2 ? mb.ignore[3] : mb.ignore[1]);
-        if constexpr (Conv) {
+        uint32_t *pdr_to = nullptr;                          // Pdr: where the second pass adds the CpG calls; NULL = nowhere
+        if constexpr (Conv || Pdr) {
             // the score: a methylated call (read C on '+', G on '-') inside the cycle bounds whose next base on the call's
             // strand is not the CpG partner (CHG and CHH alike, so the second context code is not needed).  The bounds
-            // [lo, hi) on the cycle are a range of i: cycle j = start + i, or L - 1 - j when reversed.
+            // [lo, hi) on the cycle are a range of i: cycle j = start + i, or L - 1 - j when reversed.  Pdr counts the
+            // calls whose next base is the partner in the same loop, so it reads that base for unmethylated calls too.
             const int s0 = (int)start;
             const int i_end = min(rev ? L - s0 - lo : hi - s0, (int)len);
-            uint32_t score = 0;
+            uint32_t score = 0, pm = 0, pu = 0;
 #pragma unroll 1
             for (int i = max(rev ? L - s0 - hi : lo - s0, 0) + lane; i < i_end; i += 32) {
                 const uint32_t q = base + (uint32_t)i;
-                if (ref_code(refcat, q) != match || getc(s0 + i) != cm) continue;
-                const uint32_t c1 = first_minus ? ref_code(refcat, q - 1u) : ref_code(refcat, q + 1u);
-                score += c1 != 3u - match;
+                if constexpr (!Pdr) {
+                    if (ref_code(refcat, q) != match || getc(s0 + i) != cm) continue;
+                    const uint32_t c1 = first_minus ? ref_code(refcat, q - 1u) : ref_code(refcat, q + 1u);
+                    score += c1 != 3u - match;
+                } else {
+                    if (ref_code(refcat, q) != match) continue;
+                    const char c = getc(s0 + i);
+                    const bool is_m = c == cm;
+                    if (!is_m && c != cc) continue;
+                    const uint32_t c1 = first_minus ? ref_code(refcat, q - 1u) : ref_code(refcat, q + 1u);
+                    if (c1 == 3u - match) { pm += is_m; pu += !is_m; }
+                    else if constexpr (Conv) score += is_m;
+                }
             }
-            score = __reduce_add_sync(0xffffffffu, score);
-            if (lane == 0) atomicAdd(&conv_hist[min(score, (uint32_t)BSX_CONV_BINS - 1u)], 1u);
-            if (cv.threshold && score >= cv.threshold) return;
+            if constexpr (Conv) {
+                score = __reduce_add_sync(0xffffffffu, score);
+                if (lane == 0) atomicAdd(&conv_hist[min(score, (uint32_t)BSX_CONV_BINS - 1u)], 1u);
+                if (cv.threshold && score >= cv.threshold) return;
+            }
+            if constexpr (Pdr) {                             // the drop is decided, now the class
+                pm = __reduce_add_sync(0xffffffffu, pm);
+                pu = __reduce_add_sync(0xffffffffu, pu);
+                if (pm + pu >= pd.min_cpg) {
+                    const bool disc = pm != 0 && pu != 0;
+                    pdr_to = disc ? pd.discordant : pd.concordant;
+                    if (lane == 0) { atomicAdd(&pdr_count[0], 1u); if (disc) atomicAdd(&pdr_count[1], 1u); }
+                }
+            }
         }
         uint32_t *h = hist + read2 * (3 * BSX_MBIAS_CYCLES * 2);
         for (int i = lane; i < (int)len; i += 32) {
@@ -196,6 +242,7 @@ __device__ __forceinline__ void pile_alignment(const uint32_t *__restrict__ refc
             const uint32_t c1 = first_minus ? ref_code(refcat, q - 1u) : ref_code(refcat, q + 1u);
             const uint32_t c2 = first_minus ? ref_code(refcat, q - 2u) : ref_code(refcat, q + 2u);
             const int ctx = c1 == want ? 0 : (c2 == want ? 1 : 2);
+            if constexpr (Pdr) { if (pdr_to && ctx == 0) atomicAdd(pdr_to + q, 1u); }
             if (!mb.hist) continue;
             if (cyc < BSX_MBIAS_CYCLES) atomicAdd(h + (ctx * BSX_MBIAS_CYCLES + cyc) * 2 + (is_m ? 0 : 1), 1u);
             else atomicAdd(mb.hist + MBIAS_BINS, 1ull);
@@ -269,16 +316,18 @@ __global__ void __launch_bounds__(256) meth_claim_kernel(const uint32_t *__restr
 
 // alignments parsed from SAM / BSP text on the host: one warp per alignment (Cycles: a grid-stride loop of them).
 // Conv asks for 4 resident CTAs per SM: without that floor, ptxas squeezes its instantiations to 32 or 40 registers
-// and spills; with it they take 38 - 44 and none.  The other instantiations keep the plain bound (0 = none).
-template <bool Cycles, bool Snp, bool Conv>
-__global__ void __launch_bounds__(256, Conv ? 4 : 0) meth_pileup_kernel(const uint32_t *__restrict__ refcat, const uint32_t *__restrict__ seqinfo, uint32_t n_seq,
+// and spills; with it they take 38 - 44 and none.  Pdr takes the same floor.  The other instantiations keep the plain
+// bound (0 = none).
+template <bool Cycles, bool Snp, bool Conv, bool Pdr>
+__global__ void __launch_bounds__(256, (Conv || Pdr) ? 4 : 0) meth_pileup_kernel(const uint32_t *__restrict__ refcat, const uint32_t *__restrict__ seqinfo, uint32_t n_seq,
                                                           uint32_t *meth, uint32_t *depth, unsigned long long *n_valid, uint32_t *first, bsx_meth_opts o, uint32_t n,
                                                           const char *__restrict__ seqs, uint32_t stride, const uint16_t *__restrict__ lens,
                                                           const uint32_t *__restrict__ chr, const uint32_t *__restrict__ pos0,
                                                           const uint8_t *__restrict__ strand, const int32_t *__restrict__ insert,
                                                           const int32_t *__restrict__ mate_pos, const uint8_t *__restrict__ flags, MbiasArgs mb,
-                                                          uint32_t *confirm, uint32_t *snp, ConvArgs cv) {
+                                                          uint32_t *confirm, uint32_t *snp, ConvArgs cv, PdrArgs pd) {
     static_assert(Cycles || !Conv, "the conversion filter runs in the Cycles kernels");
+    static_assert(Cycles || !Pdr, "PDR runs in the Cycles kernels");
     const uint32_t w = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     const int lane = threadIdx.x & 31;
     auto one = [&](uint32_t a, uint32_t *hist) {
@@ -286,8 +335,8 @@ __global__ void __launch_bounds__(256, Conv ? 4 : 0) meth_pileup_kernel(const ui
         if (!parsed_alignment(o, n_seq, a, lens, chr, pos0, strand, insert, mate_pos, flags, v)) return;
         if (first && !dup_holds(first, seqinfo, n_seq, v, a, lane)) return;
         const char *sq = seqs + (size_t)a * stride;
-        pile_alignment<Cycles, Snp, Conv>(refcat, seqinfo, n_seq, meth, depth, n_valid, o, v.k, v.pos, v.len, v.st, v.ins, v.mate_pos, v.sam, lane,
-                                          [sq](int i) { return sq[i]; }, mb, (flags[a] & BSX_METH_READ2) ? 1 : 0, hist, confirm, snp, cv);
+        pile_alignment<Cycles, Snp, Conv, Pdr>(refcat, seqinfo, n_seq, meth, depth, n_valid, o, v.k, v.pos, v.len, v.st, v.ins, v.mate_pos, v.sam, lane,
+                                               [sq](int i) { return sq[i]; }, mb, (flags[a] & BSX_METH_READ2) ? 1 : 0, hist, confirm, snp, cv, pd);
     };
     if constexpr (!Cycles) {
         if (w >= n) return;
@@ -296,9 +345,11 @@ __global__ void __launch_bounds__(256, Conv ? 4 : 0) meth_pileup_kernel(const ui
         __shared__ uint32_t hist[MBIAS_BINS];
         hist_zero<MBIAS_BINS>(hist, mb.hist);
         if constexpr (Conv) hist_zero<BSX_CONV_BINS>(conv_hist, cv.hist);
+        if constexpr (Pdr) hist_zero<2>(pdr_count, pd.count);
         for (uint32_t a = w; a < n; a += (gridDim.x * blockDim.x) >> 5) one(a, hist);
         hist_flush<MBIAS_BINS>(hist, mb.hist);
         if constexpr (Conv) hist_flush<BSX_CONV_BINS>(conv_hist, cv.hist);
+        if constexpr (Pdr) hist_flush<2>(pdr_count, pd.count);
     }
 }
 
@@ -356,16 +407,18 @@ __global__ void __launch_bounds__(256) meth_claim_mapped_kernel(const uint32_t *
         atomicMin(first + key, u + 1u);
 }
 
-// pile-up of the mapped batch: one warp per read (PE: per mate; Cycles: a grid-stride loop of them); Conv's bound as above
-template <bool Cycles, bool Snp, bool Conv>
-__global__ void __launch_bounds__(256, Conv ? 4 : 0) meth_pileup_mapped_kernel(const uint32_t *__restrict__ refcat, const uint32_t *__restrict__ seqinfo, uint32_t n_seq,
+// pile-up of the mapped batch: one warp per read (PE: per mate; Cycles: a grid-stride loop of them); Conv's and Pdr's
+// bound as above
+template <bool Cycles, bool Snp, bool Conv, bool Pdr>
+__global__ void __launch_bounds__(256, (Conv || Pdr) ? 4 : 0) meth_pileup_mapped_kernel(const uint32_t *__restrict__ refcat, const uint32_t *__restrict__ seqinfo, uint32_t n_seq,
                                                                  uint32_t *meth, uint32_t *depth, unsigned long long *n_valid, uint32_t *first, bsx_meth_opts o,
                                                                  int sam, int report_repeat_hits, uint32_t n, int mates, uint32_t stride,
                                                                  const uint8_t *__restrict__ seq_a, const uint8_t *__restrict__ seq_b,
                                                                  const bsx_rec *__restrict__ out_a, const bsx_rec *__restrict__ out_b,
                                                                  const bsx_pair_rec *__restrict__ out_pair, MbiasArgs mb, uint32_t *confirm, uint32_t *snp,
-                                                                 ConvArgs cv) {
+                                                                 ConvArgs cv, PdrArgs pd) {
     static_assert(Cycles || !Conv, "the conversion filter runs in the Cycles kernels");
+    static_assert(Cycles || !Pdr, "PDR runs in the Cycles kernels");
     const uint32_t w = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     const int lane = threadIdx.x & 31;
     auto one = [&](uint32_t u, uint32_t *hist) {
@@ -376,8 +429,9 @@ __global__ void __launch_bounds__(256, Conv ? 4 : 0) meth_pileup_mapped_kernel(c
         const uint8_t *rd = ((mates == 2 && (u & 1u)) ? seq_b : seq_a) + (size_t)r * stride;
         const int lp = (int)v.len;
         const int read2 = mates == 2 ? (int)(u & 1u) : (mb.readset == 2 ? 1 : 0);     // mate b / readset 2 print FLAG 0x80
-        pile_alignment<true, Snp, Conv>(refcat, seqinfo, n_seq, meth, depth, n_valid, o, v.k, v.pos, v.len, v.st, v.ins, v.mate_pos, v.sam, lane,
-                                        [rd, rev, lp](int i) { return rev ? comp_char((char)rd[lp - 1 - i]) : (char)rd[i]; }, mb, read2, hist, confirm, snp, cv);
+        pile_alignment<true, Snp, Conv, Pdr>(refcat, seqinfo, n_seq, meth, depth, n_valid, o, v.k, v.pos, v.len, v.st, v.ins, v.mate_pos, v.sam, lane,
+                                             [rd, rev, lp](int i) { return rev ? comp_char((char)rd[lp - 1 - i]) : (char)rd[i]; }, mb, read2, hist, confirm, snp, cv,
+                                             pd);
     };
     if constexpr (!Cycles) {
         // the same steps as `one`, written out: through the lambda, ptxas allocates this instantiation differently
@@ -389,22 +443,25 @@ __global__ void __launch_bounds__(256, Conv ? 4 : 0) meth_pileup_mapped_kernel(c
         const uint32_t r = mates == 2 ? u >> 1 : u;
         const uint8_t *rd = ((mates == 2 && (u & 1u)) ? seq_b : seq_a) + (size_t)r * stride;
         const int lp = (int)v.len;
-        pile_alignment<false, Snp, false>(refcat, seqinfo, n_seq, meth, depth, n_valid, o, v.k, v.pos, v.len, v.st, v.ins, v.mate_pos, v.sam, lane,
+        pile_alignment<false, Snp, false, false>(refcat, seqinfo, n_seq, meth, depth, n_valid, o, v.k, v.pos, v.len, v.st, v.ins, v.mate_pos, v.sam, lane,
                                    [rd, rev, lp](int i) { return rev ? comp_char((char)rd[lp - 1 - i]) : (char)rd[i]; }, MbiasArgs{}, 0, nullptr, confirm, snp);
     } else {
         __shared__ uint32_t hist[MBIAS_BINS];
         hist_zero<MBIAS_BINS>(hist, mb.hist);
         if constexpr (Conv) hist_zero<BSX_CONV_BINS>(conv_hist, cv.hist);
+        if constexpr (Pdr) hist_zero<2>(pdr_count, pd.count);
         for (uint32_t u = w; u < n * (uint32_t)mates; u += (gridDim.x * blockDim.x) >> 5) one(u, hist);
         hist_flush<MBIAS_BINS>(hist, mb.hist);
         if constexpr (Conv) hist_flush<BSX_CONV_BINS>(conv_hist, cv.hist);
+        if constexpr (Pdr) hist_flush<2>(pdr_count, pd.count);
     }
 }
 
 // -g: every reference "CG": both counters of the C take the G's, the G's become 0 (methratio.py:122-131); Snp: the
-// evidence counters the same way
-template <bool Snp>
-__global__ void meth_combine_kernel(const uint32_t *__restrict__ refcat, uint64_t n_pos, uint32_t *meth, uint32_t *depth, uint32_t *confirm, uint32_t *snp) {
+// evidence counters the same way; Pdr: the concordance counters too
+template <bool Snp, bool Pdr>
+__global__ void meth_combine_kernel(const uint32_t *__restrict__ refcat, uint64_t n_pos, uint32_t *meth, uint32_t *depth, uint32_t *confirm, uint32_t *snp,
+                                    uint32_t *conc, uint32_t *disc) {
     const uint64_t q = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (q + 1 >= n_pos) return;
     if (ref_code(refcat, (uint32_t)q) == 1u && ref_code(refcat, (uint32_t)q + 1u) == 2u) {
@@ -413,6 +470,10 @@ __global__ void meth_combine_kernel(const uint32_t *__restrict__ refcat, uint64_
         if constexpr (Snp) {
             confirm[q] += confirm[q + 1]; snp[q] += snp[q + 1];
             confirm[q + 1] = 0; snp[q + 1] = 0;
+        }
+        if constexpr (Pdr) {
+            conc[q] += conc[q + 1]; disc[q] += disc[q + 1];
+            conc[q + 1] = 0; disc[q + 1] = 0;
         }
     }
 }
@@ -430,12 +491,15 @@ constexpr uint64_t REGION_SLICE = 1u << 20;     // regions per launch: bounds th
 // over the warp, then lanes 0-11 add them to out[(r * 3 + ctx) * 4 + {sites, covered, C, CT}] (u64: exact, and
 // independent of the schedule).  Combine: -g's site rule (a G after a C is no site).  Snp: BSX_CT_SNP_SKIP drops a
 // covered site with any SNP evidence, BSX_CT_SNP_CORRECT one whose SNP-corrected depth is 0; 0 = no drop rule.
-template <bool Combine, int Snp>
+// Pdr: also the sums of conc and disc over the positions the PDR file prints (conc + disc >= min_depth, the same drop
+// rule), which lane 0 adds to pdr_out[r * 2 + {0, 1}].
+template <bool Combine, int Snp, bool Pdr>
 __global__ void __launch_bounds__(256) meth_region_kernel(const uint32_t *__restrict__ refcat, const uint32_t *__restrict__ meth,
                                                           const uint32_t *__restrict__ depth, const uint32_t *__restrict__ confirm,
                                                           const uint32_t *__restrict__ snp, uint32_t min_depth,
                                                           const unsigned long long *__restrict__ scan, const uint2 *__restrict__ span, uint32_t n,
-                                                          unsigned long long *out) {
+                                                          unsigned long long *out, const uint32_t *__restrict__ conc,
+                                                          const uint32_t *__restrict__ disc, unsigned long long *pdr_out) {
     const int lane = threadIdx.x & 31;
     const unsigned long long total = scan[n], warps = ((unsigned long long)gridDim.x * blockDim.x) >> 5;
     for (unsigned long long c = ((unsigned long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5; c < total; c += warps) {
@@ -451,6 +515,7 @@ __global__ void __launch_bounds__(256) meth_region_kernel(const uint32_t *__rest
         const uint32_t b = s.x + (uint32_t)(c - scan[lo]) * REGION_CHUNK, e = min(b + REGION_CHUNK, s.y);
         uint32_t sites[3] = {0u, 0u, 0u}, cov[3] = {0u, 0u, 0u};
         unsigned long long cm[3] = {0ull, 0ull, 0ull}, ct[3] = {0ull, 0ull, 0ull};
+        unsigned long long pc = 0, pdd = 0;
         for (uint32_t q = b + (uint32_t)lane; q < e; q += 32) {
             const uint32_t a = (q - 2u) >> 4, sh = (q - 2u) & 15u;     // bases q-2 .. q+2 lie in words a, a+1
             const unsigned long long w = ((unsigned long long)__ldg(refcat + a) << 32) | __ldg(refcat + a + 1);
@@ -471,6 +536,13 @@ __global__ void __launch_bounds__(256) meth_region_kernel(const uint32_t *__rest
                 sites[k] += (site && in) ? 1u : 0u;
                 if (covered && in) { cov[k] += 1u; cm[k] += mm; ct[k] += d; }
             }
+            if constexpr (Pdr) {
+                const unsigned long long x = conc[q], y = disc[q];
+                bool shown = x + y >= min_depth;
+                if constexpr (Snp == BSX_CT_SNP_SKIP) shown = shown && snp[q] == 0u;
+                if constexpr (Snp == BSX_CT_SNP_CORRECT) shown = shown && (snp[q] == 0u || confirm[q] != 0u);
+                if (shown) { pc += x; pdd += y; }
+            }
         }
 #pragma unroll
         for (int k = 0; k < 3; k++) {
@@ -488,14 +560,22 @@ __global__ void __launch_bounds__(256) meth_region_kernel(const uint32_t *__rest
             if (lane == 4 * k + 3) v = ct[k];
         }
         if (lane < 12 && v) atomicAdd(out + (size_t)lo * 12 + lane, v);
+        if constexpr (Pdr) {
+#pragma unroll
+            for (int o = 16; o > 0; o >>= 1) { pc += __shfl_xor_sync(0xffffffffu, pc, o); pdd += __shfl_xor_sync(0xffffffffu, pdd, o); }
+            if (lane == 0 && pc) atomicAdd(pdr_out + (size_t)lo * 2, pc);
+            if (lane == 0 && pdd) atomicAdd(pdr_out + (size_t)lo * 2 + 1, pdd);
+        }
     }
 }
 
-auto region_kernel(bool combine, int snp_mode) {
-    if (snp_mode == BSX_CT_SNP_SKIP) return combine ? meth_region_kernel<true, BSX_CT_SNP_SKIP> : meth_region_kernel<false, BSX_CT_SNP_SKIP>;
-    if (snp_mode == BSX_CT_SNP_CORRECT) return combine ? meth_region_kernel<true, BSX_CT_SNP_CORRECT> : meth_region_kernel<false, BSX_CT_SNP_CORRECT>;
-    return combine ? meth_region_kernel<true, 0> : meth_region_kernel<false, 0>;
+template <bool Pdr>
+auto region_kernel_of(bool combine, int snp_mode) {
+    if (snp_mode == BSX_CT_SNP_SKIP) return combine ? meth_region_kernel<true, BSX_CT_SNP_SKIP, Pdr> : meth_region_kernel<false, BSX_CT_SNP_SKIP, Pdr>;
+    if (snp_mode == BSX_CT_SNP_CORRECT) return combine ? meth_region_kernel<true, BSX_CT_SNP_CORRECT, Pdr> : meth_region_kernel<false, BSX_CT_SNP_CORRECT, Pdr>;
+    return combine ? meth_region_kernel<true, 0, Pdr> : meth_region_kernel<false, 0, Pdr>;
 }
+auto region_kernel(bool combine, int snp_mode, bool pdr) { return pdr ? region_kernel_of<true>(combine, snp_mode) : region_kernel_of<false>(combine, snp_mode); }
 
 int ensure_staging(bsx_meth *m, size_t n, uint32_t stride) {
     if (n <= m->cap && stride <= m->stride) return BSX_OK;
@@ -523,21 +603,26 @@ int ensure_dup_table(bsx_meth *m) {
     return BSX_OK;
 }
 
-// the instantiation for a combination of options (the kernels of one combination share a signature); conv implies cycles
-auto text_kernel(bool cycles, bool snp, bool conv) {
-    if (conv) return snp ? meth_pileup_kernel<true, true, true> : meth_pileup_kernel<true, false, true>;
-    return cycles ? (snp ? meth_pileup_kernel<true, true, false> : meth_pileup_kernel<true, false, false>)
-                  : (snp ? meth_pileup_kernel<false, true, false> : meth_pileup_kernel<false, false, false>);
+// the instantiation for a combination of options (the kernels of one combination share a signature); conv and pdr
+// imply cycles
+auto text_kernel(bool cycles, bool snp, bool conv, bool pdr) {
+    if (pdr) return conv ? (snp ? meth_pileup_kernel<true, true, true, true> : meth_pileup_kernel<true, false, true, true>)
+                         : (snp ? meth_pileup_kernel<true, true, false, true> : meth_pileup_kernel<true, false, false, true>);
+    if (conv) return snp ? meth_pileup_kernel<true, true, true, false> : meth_pileup_kernel<true, false, true, false>;
+    return cycles ? (snp ? meth_pileup_kernel<true, true, false, false> : meth_pileup_kernel<true, false, false, false>)
+                  : (snp ? meth_pileup_kernel<false, true, false, false> : meth_pileup_kernel<false, false, false, false>);
 }
-auto mapped_kernel(bool cycles, bool snp, bool conv) {
-    if (conv) return snp ? meth_pileup_mapped_kernel<true, true, true> : meth_pileup_mapped_kernel<true, false, true>;
-    return cycles ? (snp ? meth_pileup_mapped_kernel<true, true, false> : meth_pileup_mapped_kernel<true, false, false>)
-                  : (snp ? meth_pileup_mapped_kernel<false, true, false> : meth_pileup_mapped_kernel<false, false, false>);
+auto mapped_kernel(bool cycles, bool snp, bool conv, bool pdr) {
+    if (pdr) return conv ? (snp ? meth_pileup_mapped_kernel<true, true, true, true> : meth_pileup_mapped_kernel<true, false, true, true>)
+                         : (snp ? meth_pileup_mapped_kernel<true, true, false, true> : meth_pileup_mapped_kernel<true, false, false, true>);
+    if (conv) return snp ? meth_pileup_mapped_kernel<true, true, true, false> : meth_pileup_mapped_kernel<true, false, true, false>;
+    return cycles ? (snp ? meth_pileup_mapped_kernel<true, true, false, false> : meth_pileup_mapped_kernel<true, false, false, false>)
+                  : (snp ? meth_pileup_mapped_kernel<false, true, false, false> : meth_pileup_mapped_kernel<false, false, false, false>);
 }
 
-// the Cycles kernels run for M-bias, exclusion or the conversion filter (with M-bias and exclusion off, Cycles is the
-// classification alone: no histogram, bounds [0, L))
-bool cycles_on(const bsx_meth *m) { return m->mbias || m->ignore[0] || m->ignore[1] || m->ignore[2] || m->ignore[3] || m->d_conv; }
+// the Cycles kernels run for M-bias, exclusion, the conversion filter or PDR (with M-bias and exclusion off, Cycles is
+// the classification alone: no histogram, bounds [0, L))
+bool cycles_on(const bsx_meth *m) { return m->mbias || m->ignore[0] || m->ignore[1] || m->ignore[2] || m->ignore[3] || m->d_conv || m->d_pdr; }
 
 // the Cycles kernels' grid cap and, with M-bias on, their histogram (zeroed), on the first pile-up that needs them
 int ensure_cycles(bsx_meth *m) {
@@ -549,8 +634,8 @@ int ensure_cycles(bsx_meth *m) {
     int dev = 0, sms = 0, per_sm[2] = {0, 0};
     BSX_CUDA_CHECK(cudaGetDevice(&dev));
     BSX_CUDA_CHECK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
-    BSX_CUDA_CHECK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm[0], text_kernel(true, m->ct_snp != 0, m->d_conv != nullptr), 256, 0));
-    BSX_CUDA_CHECK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm[1], mapped_kernel(true, m->ct_snp != 0, m->d_conv != nullptr), 256, 0));
+    BSX_CUDA_CHECK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm[0], text_kernel(true, m->ct_snp != 0, m->d_conv != nullptr, m->d_pdr != nullptr), 256, 0));
+    BSX_CUDA_CHECK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm[1], mapped_kernel(true, m->ct_snp != 0, m->d_conv != nullptr, m->d_pdr != nullptr), 256, 0));
     for (int i = 0; i < 2; i++) m->resident[i] = std::max(per_sm[i], 1) * sms;
     BSX_CUDA_CHECK(cudaDeviceSynchronize());
     return BSX_OK;
@@ -562,12 +647,14 @@ MbiasArgs mbias_args(const bsx_meth *m, int readset) {
     return a;
 }
 ConvArgs conv_args(const bsx_meth *m) { return ConvArgs{m->d_conv, (uint32_t)m->conv_threshold}; }
+PdrArgs pdr_args(const bsx_meth *m) { return PdrArgs{m->d_conc, m->d_disc, m->d_pdr, m->pdr_min_cpg}; }
 
 int combine_once(bsx_meth *m, const bsx_meth_opts *o) {
     if (!o->combine_cpg || m->combined) return BSX_OK;
     const uint64_t n_pos = m->ix->n_words * 16;
-    (m->ct_snp ? meth_combine_kernel<true> : meth_combine_kernel<false>)<<<(unsigned)((n_pos + 255) / 256), 256>>>(m->ix->d_refcat, n_pos, m->d_meth, m->d_depth,
-                                                                                                              m->d_confirm, m->d_snp);
+    const auto kern = m->d_pdr ? (m->ct_snp ? meth_combine_kernel<true, true> : meth_combine_kernel<false, true>)
+                               : (m->ct_snp ? meth_combine_kernel<true, false> : meth_combine_kernel<false, false>);
+    kern<<<(unsigned)((n_pos + 255) / 256), 256>>>(m->ix->d_refcat, n_pos, m->d_meth, m->d_depth, m->d_confirm, m->d_snp, m->d_conc, m->d_disc);
     BSX_CUDA_CHECK(cudaGetLastError());
     BSX_CUDA_CHECK(cudaDeviceSynchronize());
     m->combined = true;
@@ -610,6 +697,7 @@ extern "C" int bsx_meth_create(const bsx_index *ix, bsx_meth **out) {
 extern "C" int bsx_meth_destroy(bsx_meth *m) {
     if (!m) return BSX_OK;
     cudaFree(m->d_meth); cudaFree(m->d_depth); cudaFree(m->d_valid); cudaFree(m->d_first); cudaFree(m->d_mbias); cudaFree(m->d_confirm); cudaFree(m->d_snp); cudaFree(m->d_conv);
+    cudaFree(m->d_conc); cudaFree(m->d_disc); cudaFree(m->d_pdr);
     if (m->dup_order) cudaEventDestroy(m->dup_order);
     cudaFree(m->d_seq); cudaFree(m->d_len); cudaFree(m->d_chr); cudaFree(m->d_pos); cudaFree(m->d_strand); cudaFree(m->d_flags); cudaFree(m->d_ins); cudaFree(m->d_mate);
     delete m;
@@ -642,10 +730,10 @@ extern "C" int bsx_meth_add(bsx_meth *m, const bsx_meth_opts *o, uint32_t n, con
         const unsigned blocks = (unsigned)(((uint64_t)n * 32 + 255) / 256);
         const bool cyc = cycles_on(m);
         if (cyc) { rc = ensure_cycles(m); if (rc) return rc; }
-        text_kernel(cyc, m->ct_snp != 0, m->d_conv != nullptr)<<<cyc ? std::min<unsigned>(blocks, (unsigned)m->resident[0]) : blocks, 256>>>(
+        text_kernel(cyc, m->ct_snp != 0, m->d_conv != nullptr, m->d_pdr != nullptr)<<<cyc ? std::min<unsigned>(blocks, (unsigned)m->resident[0]) : blocks, 256>>>(
             m->ix->d_refcat, m->ix->d_seqinfo, m->ix->n_seq, m->d_meth, m->d_depth, m->d_valid, o->rm_dup ? m->d_first : nullptr, *o, n, m->d_seq,
             m->stride, m->d_len, m->d_chr, m->d_pos, m->d_strand, m->d_ins, m->d_mate, m->d_flags, cyc ? mbias_args(m, 0) : MbiasArgs{}, m->d_confirm, m->d_snp,
-            conv_args(m));
+            conv_args(m), pdr_args(m));
         BSX_CUDA_CHECK(cudaGetLastError());
     }
     if (n_valid) {
@@ -676,10 +764,10 @@ int bsx_meth_pile_mapped(bsx_meth *m, const bsx_meth_opts *o, int sam, int repor
         BSX_CUDA_CHECK(cudaGetLastError());
     }
     const unsigned blocks = (unsigned)(((uint64_t)n * (uint64_t)mates * 32 + 255) / 256);
-    mapped_kernel(cyc, m->ct_snp != 0, m->d_conv != nullptr)<<<cyc ? std::min<unsigned>(blocks, (unsigned)m->resident[1]) : blocks, 256, 0, st>>>(
+    mapped_kernel(cyc, m->ct_snp != 0, m->d_conv != nullptr, m->d_pdr != nullptr)<<<cyc ? std::min<unsigned>(blocks, (unsigned)m->resident[1]) : blocks, 256, 0, st>>>(
         m->ix->d_refcat, m->ix->d_seqinfo, m->ix->n_seq, m->d_meth, m->d_depth, m->d_valid, o->rm_dup ? m->d_first : nullptr, *o, sam,
         report_repeat_hits, n, mates, stride, seq_a, seq_b, out_a, out_b, out_pair, cyc ? mbias_args(m, readset) : MbiasArgs{}, m->d_confirm, m->d_snp,
-        conv_args(m));
+        conv_args(m), pdr_args(m));
     BSX_CUDA_CHECK(cudaGetLastError());
     if (o->rm_dup) BSX_CUDA_CHECK(cudaEventRecord(m->dup_order, st));
     return BSX_OK;
@@ -928,9 +1016,112 @@ int bsx_meth_write_conversion_file(bsx_meth *m, const char *path) {
     return BSX_OK;
 }
 
-extern "C" int bsx_meth_regions(bsx_meth *m, const bsx_meth_opts *o, uint64_t n, const uint32_t *seq, const uint64_t *start, const uint64_t *end,
-                                uint64_t *out) {
-    if (!m || !o || (n && (!seq || !start || !end || !out))) { bsx_set_error("bsx_meth_regions: bad argument"); return BSX_ERR_ARG; }
+extern "C" int bsx_meth_enable_pdr(bsx_meth *m, int32_t min_cpg) {
+    if (!m) { bsx_set_error("bsx_meth_enable_pdr: bad argument"); return BSX_ERR_ARG; }
+    if (m->started) { bsx_set_error("bsx_meth_enable_pdr: alignments were already piled up; enable PDR first"); return BSX_ERR_ARG; }
+    if (min_cpg < 1 || min_cpg > 255) { bsx_set_error("bsx_meth_enable_pdr: the minimum of CpG calls must be 1..255 (got %d)", (int)min_cpg); return BSX_ERR_ARG; }
+    if (!m->d_pdr) {
+        BSX_CUDA_CHECK(cudaSetDevice(m->ix->device));
+        const size_t bytes = m->ix->n_words * 16 * sizeof(uint32_t);
+        if (cudaMalloc(&m->d_conc, bytes) != cudaSuccess || cudaMalloc(&m->d_disc, bytes) != cudaSuccess ||
+            cudaMalloc(&m->d_pdr, 2 * sizeof(unsigned long long)) != cudaSuccess) {
+            cudaGetLastError(); cudaFree(m->d_conc); cudaFree(m->d_disc); cudaFree(m->d_pdr); m->d_conc = m->d_disc = nullptr; m->d_pdr = nullptr;
+            bsx_set_error("PDR: out of device memory (%zu bytes per concordance array, two arrays)", bytes); return BSX_ERR_CUDA; }
+        BSX_CUDA_CHECK(cudaMemset(m->d_conc, 0, bytes));
+        BSX_CUDA_CHECK(cudaMemset(m->d_disc, 0, bytes));
+        BSX_CUDA_CHECK(cudaMemset(m->d_pdr, 0, 2 * sizeof(unsigned long long)));
+    }
+    m->pdr_min_cpg = (uint32_t)min_cpg;
+    return BSX_OK;
+}
+
+extern "C" int bsx_meth_download_pdr(bsx_meth *m, const bsx_meth_opts *o, uint32_t k, uint32_t *concordant, uint32_t *discordant) {
+    if (!m || !o || k >= m->ix->n_seq) { bsx_set_error("bsx_meth_download_pdr: bad argument"); return BSX_ERR_ARG; }
+    if (!m->d_pdr) { bsx_set_error("bsx_meth_download_pdr: PDR was not enabled (bsx_meth_enable_pdr)"); return BSX_ERR_ARG; }
+    BSX_CUDA_CHECK(cudaSetDevice(m->ix->device));
+    int rc = combine_once(m, o); if (rc) return rc;
+    const size_t off = m->ix->anchor[k], cnt = m->ix->size[k];
+    if (concordant) BSX_CUDA_CHECK(cudaMemcpy(concordant, m->d_conc + off, cnt * 4, cudaMemcpyDeviceToHost));
+    if (discordant) BSX_CUDA_CHECK(cudaMemcpy(discordant, m->d_disc + off, cnt * 4, cudaMemcpyDeviceToHost));
+    return BSX_OK;
+}
+
+extern "C" int bsx_meth_pdr(bsx_meth *m, uint64_t *informative, uint64_t *discordant) {
+    if (!m) { bsx_set_error("bsx_meth_pdr: bad argument"); return BSX_ERR_ARG; }
+    if (!m->d_pdr) { bsx_set_error("bsx_meth_pdr: PDR was not enabled (bsx_meth_enable_pdr)"); return BSX_ERR_ARG; }
+    BSX_CUDA_CHECK(cudaSetDevice(m->ix->device));
+    BSX_CUDA_CHECK(cudaDeviceSynchronize());           // in-process batches flush from two streams
+    unsigned long long h[2];
+    BSX_CUDA_CHECK(cudaMemcpy(h, m->d_pdr, sizeof h, cudaMemcpyDeviceToHost));
+    if (informative) *informative = h[0];
+    if (discordant) *discordant = h[1];
+    return BSX_OK;
+}
+
+extern "C" size_t bsx_meth_write_pdr(bsx_meth *m, const bsx_meth_opts *o, const char *const *seqs, const uint32_t *lens, const uint8_t *chroms,
+                                     int threads, int fd) {
+    if (!m || !o || !seqs || !lens) { bsx_set_error("bsx_meth_write_pdr: bad argument"); return 0; }
+    if (!m->d_pdr) { bsx_set_error("bsx_meth_write_pdr: PDR was not enabled (bsx_meth_enable_pdr)"); return 0; }
+    const bsx_index *ix = m->ix;
+    threads = bsx_host_threads(threads);
+    size_t written = 0;
+    auto out = [&](const std::string &s) {
+        size_t off = 0;
+        while (off < s.size()) { const ssize_t w = write(fd, s.data() + off, s.size() - off); if (w <= 0) return false; off += (size_t)w; written += (size_t)w; }
+        return true;
+    };
+    if (!out("chr\tpos\tstrand\tconcordant\tdiscordant\tPDR\n")) return 0;
+    std::vector<uint32_t> order;
+    for (uint32_t k = 0; k < ix->n_seq; k++) if (!chroms || chroms[k]) order.push_back(k);
+    std::sort(order.begin(), order.end(), [&](uint32_t a, uint32_t b) { return ix->names[a] < ix->names[b]; });   // the table's order
+    const int snp_mode = m->ct_snp == BSX_CT_SNP_SKIP || m->ct_snp == BSX_CT_SNP_CORRECT ? m->ct_snp : 0;
+    const uint64_t min_n = (uint64_t)std::max(o->min_depth, 1);
+    std::vector<uint32_t> hc, hd, ec, es;
+    for (uint32_t k : order) {
+        const uint32_t L = ix->size[k];
+        if (lens[k] != L) { bsx_set_error("bsx_meth_write_pdr: sequence %u has %u bases, the index %u", k, lens[k], L); return 0; }
+        hc.resize(L); hd.resize(L);
+        if (bsx_meth_download_pdr(m, o, k, hc.data(), hd.data()) != BSX_OK) return 0;
+        if (snp_mode) { ec.resize(L); es.resize(L); if (bsx_meth_download_ct_snp(m, o, k, ec.data(), es.data()) != BSX_OK) return 0; }
+        const char *rs = seqs[k];
+        const std::string &name = ix->names[k];
+        std::vector<std::string> chunk((size_t)threads);
+        bsx_parallel(threads, L, [&](int t, size_t b, size_t e) {
+            Sink s{&chunk[t]};
+            for (size_t i = b; i < e; i++) {
+                const uint64_t c = hc[i], d = hd[i];
+                if (c + d < min_n) continue;
+                // the C/T SNP mode drops the line as it drops the table's: `skip` at any SNP evidence, `correct` when eff == 0
+                if (snp_mode == BSX_CT_SNP_SKIP && es[i]) continue;
+                if (snp_mode == BSX_CT_SNP_CORRECT && es[i] && !ec[i]) continue;
+                s.put(name.data(), name.size()); s.putc('\t'); s.putu(i + 1); s.putc('\t');
+                const char rc = (char)(rs[i] >= 'a' && rs[i] <= 'z' ? rs[i] - 32 : rs[i]);
+                s.putc(rc == 'C' ? '+' : '-'); s.putc('\t');
+                s.putu(c); s.putc('\t'); s.putu(d); s.putc('\t'); s.putf3((double)d / (double)(c + d)); s.putc('\n');
+            }
+        });
+        for (int t = 0; t < threads; t++) if (!out(chunk[t])) return 0;
+    }
+    return written;
+}
+
+int bsx_meth_write_pdr_file(bsx_meth *m, const bsx_meth_opts *o, const char *const *seqs, const uint32_t *lens, const uint8_t *chroms, int threads,
+                            const char *path) {
+    const int fd = open(path, O_WRONLY | O_CREAT | O_TRUNC, 0644);
+    if (fd < 0) { fprintf(stderr, "failed to open PDR output file: %s\n", path); return BSX_ERR_IO; }
+    const size_t w = bsx_meth_write_pdr(m, o, seqs, lens, chroms, threads, fd);
+    close(fd);
+    if (w == 0) { fprintf(stderr, "%s\n", bsx_last_error()); return BSX_ERR_IO; }
+    uint64_t inf = 0, disc = 0, valid = 0;
+    if (bsx_meth_pdr(m, &inf, &disc) != BSX_OK || bsx_meth_valid_count(m, &valid) != BSX_OK) { fprintf(stderr, "%s\n", bsx_last_error()); return BSX_ERR_CUDA; }
+    fprintf(stderr, "PDR: %llu of %llu valid mappings informative (>= %u CpG calls), %llu discordant\n", (unsigned long long)inf, (unsigned long long)valid,
+            m->pdr_min_cpg, (unsigned long long)disc);
+    return BSX_OK;
+}
+
+// bsx_meth_regions, and with pdr != NULL bsx_meth_regions_pdr: one reduction fills both
+static int meth_regions(bsx_meth *m, const bsx_meth_opts *o, uint64_t n, const uint32_t *seq, const uint64_t *start, const uint64_t *end,
+                        uint64_t *out, uint64_t *pdr) {
     const bsx_index *ix = m->ix;
     for (uint64_t r = 0; r < n; r++) {
         if (seq[r] >= ix->n_seq) { bsx_set_error("bsx_meth_regions: region %llu: sequence %u of %u", (unsigned long long)r, seq[r], ix->n_seq); return BSX_ERR_ARG; }
@@ -942,12 +1133,13 @@ extern "C" int bsx_meth_regions(bsx_meth *m, const bsx_meth_opts *o, uint64_t n,
     int rc = combine_once(m, o); if (rc) return rc;
     if (n == 0) return BSX_OK;
     const uint64_t cap = std::min<uint64_t>(n, REGION_SLICE);
-    unsigned long long *d_scan = nullptr, *d_out = nullptr; uint2 *d_span = nullptr;
-    if (cudaMalloc(&d_scan, (cap + 1) * 8) != cudaSuccess || cudaMalloc(&d_span, cap * 8) != cudaSuccess || cudaMalloc(&d_out, cap * 12 * 8) != cudaSuccess) {
-        cudaGetLastError(); cudaFree(d_scan); cudaFree(d_span); bsx_set_error("bsx_meth_regions: out of device memory"); return BSX_ERR_CUDA; }
+    unsigned long long *d_scan = nullptr, *d_out = nullptr, *d_pdr = nullptr; uint2 *d_span = nullptr;
+    if (cudaMalloc(&d_scan, (cap + 1) * 8) != cudaSuccess || cudaMalloc(&d_span, cap * 8) != cudaSuccess || cudaMalloc(&d_out, cap * 12 * 8) != cudaSuccess ||
+        (pdr && cudaMalloc(&d_pdr, cap * 2 * 8) != cudaSuccess)) {
+        cudaGetLastError(); cudaFree(d_scan); cudaFree(d_span); cudaFree(d_out); bsx_set_error("bsx_meth_regions: out of device memory"); return BSX_ERR_CUDA; }
     int dev = 0, sms = 0, per_sm = 0;
     const int snp_mode = m->ct_snp == BSX_CT_SNP_SKIP || m->ct_snp == BSX_CT_SNP_CORRECT ? m->ct_snp : 0;
-    const auto kern = region_kernel(o->combine_cpg != 0, snp_mode);
+    const auto kern = region_kernel(o->combine_cpg != 0, snp_mode, pdr != nullptr);
     cudaGetDevice(&dev);
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
     cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, 256, 0);
@@ -968,18 +1160,33 @@ extern "C" int bsx_meth_regions(bsx_meth *m, const bsx_meth_opts *o, uint64_t n,
             BSX_CUDA_CHECK(cudaMemcpy(d_scan, scan.data(), (k + 1) * 8, cudaMemcpyHostToDevice));
             BSX_CUDA_CHECK(cudaMemcpy(d_span, span.data(), (size_t)k * 8, cudaMemcpyHostToDevice));
             BSX_CUDA_CHECK(cudaMemset(d_out, 0, (size_t)k * 12 * 8));
+            if (pdr) BSX_CUDA_CHECK(cudaMemset(d_pdr, 0, (size_t)k * 2 * 8));
             if (scan[k]) {
                 const unsigned blocks = (unsigned)std::min<unsigned long long>((scan[k] + 7) / 8, (unsigned long long)std::max(per_sm, 1) * (unsigned)sms);
-                kern<<<blocks, 256>>>(ix->d_refcat, m->d_meth, m->d_depth, m->d_confirm, m->d_snp, min_depth, d_scan, d_span, k, d_out);
+                kern<<<blocks, 256>>>(ix->d_refcat, m->d_meth, m->d_depth, m->d_confirm, m->d_snp, min_depth, d_scan, d_span, k, d_out, m->d_conc, m->d_disc, d_pdr);
                 BSX_CUDA_CHECK(cudaGetLastError());
             }
             BSX_CUDA_CHECK(cudaMemcpy(out + r0 * 12, d_out, (size_t)k * 12 * 8, cudaMemcpyDeviceToHost));
+            if (pdr) BSX_CUDA_CHECK(cudaMemcpy(pdr + r0 * 2, d_pdr, (size_t)k * 2 * 8, cudaMemcpyDeviceToHost));
             return BSX_OK;
         };
         err = step();
     }
-    cudaFree(d_scan); cudaFree(d_span); cudaFree(d_out);
+    cudaFree(d_scan); cudaFree(d_span); cudaFree(d_out); cudaFree(d_pdr);
     return err;
+}
+
+extern "C" int bsx_meth_regions(bsx_meth *m, const bsx_meth_opts *o, uint64_t n, const uint32_t *seq, const uint64_t *start, const uint64_t *end,
+                                uint64_t *out) {
+    if (!m || !o || (n && (!seq || !start || !end || !out))) { bsx_set_error("bsx_meth_regions: bad argument"); return BSX_ERR_ARG; }
+    return meth_regions(m, o, n, seq, start, end, out, nullptr);
+}
+
+extern "C" int bsx_meth_regions_pdr(bsx_meth *m, const bsx_meth_opts *o, uint64_t n, const uint32_t *seq, const uint64_t *start, const uint64_t *end,
+                                    uint64_t *out, uint64_t *pdr) {
+    if (!m || !o || (n && (!seq || !start || !end || !out || !pdr))) { bsx_set_error("bsx_meth_regions_pdr: bad argument"); return BSX_ERR_ARG; }
+    if (!m->d_pdr) { bsx_set_error("bsx_meth_regions_pdr: PDR was not enabled (bsx_meth_enable_pdr)"); return BSX_ERR_ARG; }
+    return meth_regions(m, o, n, seq, start, end, out, pdr);
 }
 
 extern "C" size_t bsx_meth_write_regions(bsx_meth *m, const bsx_meth_opts *o, uint64_t n, const uint32_t *seq, const uint64_t *start,
@@ -994,12 +1201,15 @@ extern "C" size_t bsx_meth_write_regions(bsx_meth *m, const bsx_meth_opts *o, ui
         while (off < s.size()) { const ssize_t w = write(fd, s.data() + off, s.size() - off); if (w <= 0) return false; off += (size_t)w; written += (size_t)w; }
         return true;
     };
-    if (!put("chr\tstart\tend\tcontext\tsites\tcovered\tC_count\tCT_count\tlevel\n")) return 0;
-    std::vector<uint64_t> sums;
+    const bool pdr_on = m->d_pdr != nullptr;             // PDR: three more columns on every line
+    if (!put(pdr_on ? "chr\tstart\tend\tcontext\tsites\tcovered\tC_count\tCT_count\tlevel\tconcordant\tdiscordant\tPDR\n"
+                    : "chr\tstart\tend\tcontext\tsites\tcovered\tC_count\tCT_count\tlevel\n")) return 0;
+    std::vector<uint64_t> sums, pdr;
     for (uint64_t r0 = 0; r0 < n; r0 += REGION_SLICE) {
         const uint64_t k = std::min<uint64_t>(REGION_SLICE, n - r0);
-        sums.resize(k * 12);
-        if (bsx_meth_regions(m, o, k, seq + r0, start + r0, end + r0, sums.data()) != BSX_OK) return 0;
+        sums.resize(k * 12); pdr.resize(k * 2);
+        if (pdr_on ? bsx_meth_regions_pdr(m, o, k, seq + r0, start + r0, end + r0, sums.data(), pdr.data()) != BSX_OK
+                   : bsx_meth_regions(m, o, k, seq + r0, start + r0, end + r0, sums.data()) != BSX_OK) return 0;
         std::vector<std::string> chunk((size_t)threads);
         bsx_parallel(threads, (size_t)k, [&](int t, size_t b, size_t e) {
             Sink s{&chunk[t]};
@@ -1013,6 +1223,12 @@ extern "C" size_t bsx_meth_write_regions(bsx_meth *m, const bsx_meth_opts *o, ui
                     s.putc('\t');
                     if (v[3]) { char buf[48]; const int l = snprintf(buf, sizeof buf, "%.4f", (double)v[2] / (double)v[3]); s.put(buf, (size_t)l); }
                     else s.put("NA", 2);
+                    if (pdr_on) {                                // the CpG line: the PDR file's lines in the region; CHG / CHH: none
+                        const uint64_t pc = c == 0 ? pdr[i * 2] : 0, pd = c == 0 ? pdr[i * 2 + 1] : 0;
+                        s.putc('\t'); s.putu(pc); s.putc('\t'); s.putu(pd); s.putc('\t');
+                        if (pc + pd) { char buf[48]; const int l = snprintf(buf, sizeof buf, "%.4f", (double)pd / (double)(pc + pd)); s.put(buf, (size_t)l); }
+                        else s.put("NA", 2);
+                    }
                     s.putc('\n');
                 }
             }

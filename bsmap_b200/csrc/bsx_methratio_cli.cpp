@@ -21,6 +21,12 @@
 //                              reduced on the device from the same counters as the table, over
 //   --regions BED                the regions of a BED file (columns 1-3), in the file's order, or
 //   --tiles W                    tiles of W bases over every selected sequence, in the table's order
+//   --pdr FILE                 read-level CpG concordance: per CpG position the CpG calls of informative alignments
+//                              (at least K CpG calls) that are concordant (all methylated or all unmethylated) or
+//                              discordant, and PDR = discordant / (concordant + discordant); prints "PDR: I of V valid
+//                              mappings informative (>= K CpG calls), D discordant" to stderr; with --region-report the
+//                              report gains the columns concordant, discordant and PDR
+//   --pdr-min-cpg K            CpG calls an alignment needs to be informative, 1..255 (default 4)
 #include <chrono>
 #include <cstdio>
 #include <cstdlib>
@@ -49,6 +55,8 @@ struct MOpts {
     std::string conv_report;                 // --conversion-report FILE
     std::string region_report, regions;      // --region-report FILE, --regions BED
     long long tiles = 0;                     // --tiles W; 0 = none
+    std::string pdr;                         // --pdr FILE
+    int pdr_min_cpg = 0;                     // --pdr-min-cpg K; 0 = not given (4)
     std::vector<std::string> files;
 };
 
@@ -72,7 +80,7 @@ void parse(int argc, char **argv, MOpts &m) {
                                {'t', "trim-fillin", true}, {'g', "combine-CpG", false}, {'m', "min-depth", true}, {'h', "help", false},
                                {'\1', "mbias", true}, {'\2', "mbias-ignore", true}, {'\3', "ct-snp", true},
                                {'\4', "conversion-filter", true}, {'\5', "conversion-report", true}, {'\6', "region-report", true},
-                               {'\7', "regions", true}, {'\10', "tiles", true}};   // long only
+                               {'\7', "regions", true}, {'\10', "tiles", true}, {'\11', "pdr", true}, {'\12', "pdr-min-cpg", true}};   // long only
     auto apply = [&](char c, const char *v) {
         if (!v) v = "";
         switch (c) {
@@ -111,9 +119,13 @@ void parse(int argc, char **argv, MOpts &m) {
             case '\10': { char *e; const long long x = strtoll(v, &e, 10);
                 if (*e || e == v || x < 1) usage_error("option --tiles: expected an integer >= 1");
                 m.tiles = x; } break;
+            case '\11': m.pdr = v; break;
+            case '\12': { char *e; const long x = strtol(v, &e, 10);
+                if (*e || e == v || x < 1 || x > 255) usage_error("option --pdr-min-cpg: expected an integer 1..255");
+                m.pdr_min_cpg = (int)x; } break;
             case 'h': printf("Usage: methratio [options] BSMAP_MAPPING_FILES\n  -o FILE -d FILE [-c CHR] [-u] [-p] [-z] [-q] [-r] [-t N] [-g] [-m FOLD] [--mbias FILE] [--mbias-ignore A,B,C,D]\n"
                              "  [--ct-snp no-action|correct|skip] [--conversion-filter N] [--conversion-report FILE]\n"
-                             "  [--region-report FILE (--regions BED | --tiles W)]\n"); exit(0);
+                             "  [--region-report FILE (--regions BED | --tiles W)] [--pdr FILE [--pdr-min-cpg K]]\n"); exit(0);
         }
     };
     for (int i = 1; i < argc; i++) {
@@ -312,6 +324,8 @@ extern "C" int bsx_methratio_main(int argc, char **argv) {
     if (!m.regions.empty() && m.tiles) usage_error("--regions and --tiles exclude each other");
     if (m.region_report.empty() && (!m.regions.empty() || m.tiles)) usage_error("--regions / --tiles need --region-report FILE");
     if (!m.region_report.empty() && m.regions.empty() && !m.tiles) usage_error("--region-report needs --regions BED or --tiles W");
+    if (m.pdr_min_cpg && m.pdr.empty()) usage_error("--pdr-min-cpg needs --pdr FILE");
+    if (!m.pdr.empty() && !m.pdr_min_cpg) m.pdr_min_cpg = 4;
     const bool cycles = !m.mbias.empty() || m.ignore_set;
     if (cycles)
         for (const std::string &f : m.files) {
@@ -350,7 +364,8 @@ extern "C" int bsx_methratio_main(int argc, char **argv) {
     if (bsx_index_create_packed((int)seqs.size(), np.data(), sp.data(), ln.data(), 0, &ix) != BSX_OK || bsx_meth_create(ix, &mh) != BSX_OK) {
         fprintf(stderr, "%s\n", bsx_last_error()); return 1; }
     if ((!m.mbias.empty() && bsx_meth_enable_mbias(mh) != BSX_OK) || (m.ignore_set && bsx_meth_set_ignore(mh, m.ignore) != BSX_OK) ||
-        (m.ct_snp && bsx_meth_enable_ct_snp(mh, m.ct_snp) != BSX_OK) || (m.conv >= 0 && bsx_meth_enable_conversion_filter(mh, m.conv) != BSX_OK)) {
+        (m.ct_snp && bsx_meth_enable_ct_snp(mh, m.ct_snp) != BSX_OK) || (m.conv >= 0 && bsx_meth_enable_conversion_filter(mh, m.conv) != BSX_OK) ||
+        (!m.pdr.empty() && bsx_meth_enable_pdr(mh, m.pdr_min_cpg) != BSX_OK)) {
         fprintf(stderr, "%s\n", bsx_last_error()); return 1; }
     bsx_regions regions;                                      // read before the pile-up, so that a bad BED fails early
     if ((!m.regions.empty() && bsx_regions_bed(ix, selected.data(), m.regions.c_str(), regions) != BSX_OK) ||
@@ -448,6 +463,10 @@ extern "C" int bsx_methratio_main(int argc, char **argv) {
     if (m.conv >= 0) {
         if (!m.conv_report.empty()) disp(m, ("writing " + m.conv_report + " ...").c_str());
         if (bsx_meth_write_conversion_file(mh, m.conv_report.empty() ? nullptr : m.conv_report.c_str()) != BSX_OK) return 1;
+    }
+    if (!m.pdr.empty()) {
+        disp(m, ("writing " + m.pdr + " ...").c_str());
+        if (bsx_meth_write_pdr_file(mh, &m.o, sp.data(), ln.data(), selected.data(), threads, m.pdr.c_str()) != BSX_OK) return 1;
     }
     if (!m.region_report.empty()) {
         disp(m, ("writing " + m.region_report + " ...").c_str());

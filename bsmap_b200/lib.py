@@ -70,6 +70,7 @@ EXPORTS = [
     "bsx_meth_enable_ct_snp", "bsx_meth_download_ct_snp",
     "bsx_meth_enable_conversion_filter", "bsx_meth_conversion", "bsx_meth_write_conversion",
     "bsx_meth_regions", "bsx_meth_write_regions",
+    "bsx_meth_enable_pdr", "bsx_meth_download_pdr", "bsx_meth_pdr", "bsx_meth_write_pdr", "bsx_meth_regions_pdr",
 ]
 
 METH_READ2 = 8        # BSX_METH_READ2: alignment flag, read 2 (FLAG 0x80)
@@ -170,6 +171,12 @@ def load():
     L.bsx_meth_regions.argtypes = [vp, C.POINTER(MethOpts), C.c_uint64, vp, vp, vp, vp]
     L.bsx_meth_write_regions.restype = sz
     L.bsx_meth_write_regions.argtypes = [vp, C.POINTER(MethOpts), C.c_uint64, vp, vp, vp, i32]
+    L.bsx_meth_enable_pdr.argtypes = [vp, i32]
+    L.bsx_meth_download_pdr.argtypes = [vp, C.POINTER(MethOpts), u32, vp, vp]
+    L.bsx_meth_pdr.argtypes = [vp, C.POINTER(C.c_uint64), C.POINTER(C.c_uint64)]
+    L.bsx_meth_write_pdr.restype = sz
+    L.bsx_meth_write_pdr.argtypes = [vp, C.POINTER(MethOpts), pp, vp, vp, i32, i32]
+    L.bsx_meth_regions_pdr.argtypes = [vp, C.POINTER(MethOpts), C.c_uint64, vp, vp, vp, vp, vp]
     L.bsx_packed_stride.restype = sz
     L.bsx_packed_stride.argtypes = [u32]
     L.bsx_pack_reads.argtypes = [u32, vp, u32, vp, vp, C.POINTER(C.c_uint64), i32]

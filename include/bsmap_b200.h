@@ -363,6 +363,42 @@ int bsx_meth_conversion(bsx_meth *m, uint64_t *out /* BSX_CONV_BINS */, uint64_t
  * non-empty bin, ascending, the last labelled "255+"; dropped is 1 when the bin's alignments were dropped, else 0.
  * Returns bytes written (0 on error). */
 size_t bsx_meth_write_conversion(bsx_meth *m, int fd);
+/* --- read-level CpG concordance: the proportion of discordant reads (PDR) --------------------------------------------
+ * A level of 0.5 at a CpG may come from half the molecules fully methylated and half unmethylated, or from every molecule
+ * methylated at random.  PDR tells these apart by the CpG calls each read carries.
+ *   call         one increment of the counters, after every other rule (as for the conversion filter): -u / -p, -r, -t,
+ *                mate-overlap removal, the bounds test and bsx_meth_set_ignore's cycle rule
+ *   context      the M-bias rule: a '+' C at q is CpG if q+1 is G; a '-' G at q is CpG if q-1 is C
+ *   pattern      m = the alignment's methylated CpG calls, u = its unmethylated ones; a read character that is neither
+ *                the methylated nor the converted letter (N, lower case) is no call.  Each mate on its own calls.
+ *   informative  m + u >= K, 1 <= K <= 255 (default 4); an informative alignment is concordant when m == 0 or u == 0,
+ *                else discordant
+ *   counters     every CpG call of an informative alignment adds 1 to concordant[q] or discordant[q], by the alignment's
+ *                class; other alignments add nothing.  -g adds a CpG's G counts to its C and zeroes the G.
+ *   other rules  an alignment dropped by the conversion filter and a -r loser are not scored; calls, the M-bias, the C/T
+ *                SNP evidence, the conversion histogram and "valid mappings" do not change
+ *   summary      the informative alignments and the discordant ones
+ *   file         header "chr pos strand concordant discordant PDR" (tab-separated), one line per position with
+ *                concordant + discordant >= max(-m, 1) that the C/T SNP mode would not drop (BSX_CT_SNP_SKIP: any SNP
+ *                evidence; BSX_CT_SNP_CORRECT: eff == 0), sequences selected and sorted by name, positions ascending;
+ *                strand from the reference base as in the table; PDR = discordant / (concordant + discordant) as %.3f;
+ *                -z is ignored
+ *   regions      bsx_meth_write_regions adds the columns "concordant discordant PDR" to every line: on the CpG line the
+ *                sums over the PDR file's lines in the region and PDR = %.4f (NA at 0), on the CHG and CHH lines 0 0 NA
+ * 8 more bytes of HBM per position. */
+/* score every alignment from now on; min_cpg = K.  Must precede the first alignment piled up; K outside 1..255 or a late
+ * call: BSX_ERR_ARG; no device memory for the two arrays: BSX_ERR_CUDA. */
+int bsx_meth_enable_pdr(bsx_meth *m, int32_t min_cpg);
+/* copy the concordance counters of sequence k to the host (after -g combining when o->combine_cpg, like
+ * bsx_meth_download); BSX_ERR_ARG when PDR was not enabled */
+int bsx_meth_download_pdr(bsx_meth *m, const bsx_meth_opts *o, uint32_t k, uint32_t *concordant, uint32_t *discordant);
+/* the informative and discordant alignments so far (synchronises the device; either may be NULL); BSX_ERR_ARG when PDR
+ * was not enabled */
+int bsx_meth_pdr(bsx_meth *m, uint64_t *informative, uint64_t *discordant);
+/* write the PDR file to fd for the sequences selected by `chroms` (NULL = all); seqs / lens as in bsx_meth_write.
+ * Returns bytes written (0 on error). */
+size_t bsx_meth_write_pdr(bsx_meth *m, const bsx_meth_opts *o, const char *const *seqs, const uint32_t *lens,
+                          const uint8_t *chroms /* n_seq flags or NULL */, int threads, int fd);
 /* --- methylation levels over regions, reduced on the device from the counters ----------------------------------------
  *   region   (sequence, start, end), 0-based and half-open as in BED; start == end is empty; an end past the sequence end
  *            is clipped when counting.  Each region is reported for the contexts CpG, CHG, CHH (ctx 0, 1, 2).
@@ -385,14 +421,19 @@ int bsx_meth_regions(bsx_meth *m, const bsx_meth_opts *o, uint64_t n, const uint
                      uint64_t *out);
 /* write the region report to fd: a header line "chr start end context sites covered C_count CT_count level"
  * (tab-separated), then three lines per region, CpG, CHG, CHH, in region order, start and end as given; level = %.4f
- * of C / CT, or NA when CT == 0.  Returns bytes written (0 on error). */
+ * of C / CT, or NA when CT == 0.  With PDR enabled, "concordant discordant PDR" follow on every line (see above).
+ * Returns bytes written (0 on error). */
 size_t bsx_meth_write_regions(bsx_meth *m, const bsx_meth_opts *o, uint64_t n, const uint32_t *seq, const uint64_t *start, const uint64_t *end,
                               int fd);
+/* bsx_meth_regions, and pdr[r * 2 + {0 concordant, 1 discordant}]: the sums over the PDR file's lines in region r (with
+ * PDR on, bsx_meth_write_regions adds them and their PDR to the report).  BSX_ERR_ARG when PDR was not enabled. */
+int bsx_meth_regions_pdr(bsx_meth *m, const bsx_meth_opts *o, uint64_t n, const uint32_t *seq, const uint64_t *start, const uint64_t *end,
+                         uint64_t *out, uint64_t *pdr);
 /* the methratio.py command line: -o -d [-c -u -p -z -q -r -t -g -m -s] files... (SAM, BAM and BSP; -s is ignored);
  * extensions: --mbias FILE (the M-bias report) and --mbias-ignore A,B,C,D (bsx_meth_set_ignore), SAM and BAM only;
  * --ct-snp no-action|correct|skip (bsx_meth_enable_ct_snp); --conversion-filter N and --conversion-report FILE
  * (bsx_meth_enable_conversion_filter, bsx_meth_write_conversion); --region-report FILE with --regions BED or --tiles W
- * (bsx_meth_write_regions) */
+ * (bsx_meth_write_regions); --pdr FILE [--pdr-min-cpg K] (bsx_meth_enable_pdr, bsx_meth_write_pdr) */
 int bsx_methratio_main(int argc, char **argv);
 
 /* --- the bsmap command line (main.cpp:441-476): same options, same output files -------------- */
