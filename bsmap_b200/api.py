@@ -516,6 +516,36 @@ class Meth:
             check(1)
         return w
 
+    def enable_epialleles(self):
+        """count the methylation patterns of every alignment over windows of four consecutive CpG sites (include/
+        bsmap_b200.h); builds the CpG rank index on the device; before the first add / mapped batch, once"""
+        check(load().bsx_meth_enable_epialleles(self.h))
+
+    def epiallele_counters(self, k: int):
+        """-> (uint32 [n]: 0-based position of each CpG site's C on reference sequence k, uint32 [n, 16]: row j the
+        alignments by pattern over the window starting at site j, pattern 0 = UUUU, the first site the high bit)"""
+        n = C.c_uint64(0)
+        check(load().bsx_meth_cpg_sites(self.h, k, C.byref(n)))
+        pos, counts = np.zeros(n.value, dtype=np.uint32), np.zeros((n.value, 16), dtype=np.uint32)
+        check(load().bsx_meth_download_epialleles(self.h, k, pos.ctypes.data, counts.ctypes.data))
+        return pos, counts
+
+    def epialleles(self):
+        """-> (alignments with at least one window, windows counted)"""
+        spanning, windows = C.c_uint64(0), C.c_uint64(0)
+        check(load().bsx_meth_epialleles(self.h, C.byref(spanning), C.byref(windows)))
+        return spanning.value, windows.value
+
+    def write_epialleles(self, seqs, fd: int, chroms=None, threads=0) -> int:
+        """the epiallele file (include/bsmap_b200.h) to fd; seqs and chroms as in write; returns bytes written"""
+        keep = [s if isinstance(s, bytes) else bytes(s) for s in seqs]
+        lens = np.array([len(s) for s in keep], dtype=np.uint32)
+        sel = None if chroms is None else np.ascontiguousarray(np.asarray(chroms, dtype=np.uint8))
+        w = load().bsx_meth_write_epialleles(self.h, C.byref(self.o), strs(keep), lens.ctypes.data, _ptr(sel), threads, fd)
+        if w == 0:
+            check(1)
+        return w
+
     @staticmethod
     def _regions(chr_idx, start, end):
         arr = lambda a, t: np.ascontiguousarray(np.asarray(a, dtype=t).reshape(-1))

@@ -10,7 +10,9 @@
 // (--meth-conversion-filter N, --meth-conversion-report FILE: drop alignments with N or more methylated non-CpG calls),
 // and methylation levels per region and context reduced on the device (--meth-region-report FILE with --meth-regions BED
 // or --meth-tiles W), and the proportion of discordant reads per CpG from the CpG calls of each alignment (--meth-pdr
-// FILE, --meth-pdr-min-cpg K: the CpG calls an alignment needs to be scored, default 4).
+// FILE, --meth-pdr-min-cpg K: the CpG calls an alignment needs to be scored, default 4), and the methylation patterns of
+// the alignments over every window of four consecutive CpG sites, with methylation entropy and epipolymorphism
+// (--meth-epialleles FILE).
 // Out of scope (errors out): SAM text input (broken in the reference too: it is opened as BAM), -q quality
 // trimming, -M other than TC.
 #include <cerrno>
@@ -49,6 +51,7 @@ struct Opts {
     long long meth_tiles = 0;                // --meth-tiles W; 0 = none
     std::string meth_pdr;                    // --meth-pdr FILE
     int meth_pdr_min_cpg = 0;                // --meth-pdr-min-cpg K (1..255); 0 = not given (4); -1 = out of range
+    std::string meth_epialleles;             // --meth-epialleles FILE
     unsigned batch = 1u << 17;   // reads per GPU batch: small enough to keep the three host stages overlapped
     std::string gpus;            // -g: number of devices (default: all visible) or a comma list of device ids; output stays in input order
 };
@@ -104,7 +107,9 @@ void usage() {
            "       --meth-tiles <int>  tiles of this many bases over every sequence\n"
            "       --meth-pdr <str>    with --methratio: write the proportion of discordant reads per CpG (alignments with\n"
            "                           both methylated and unmethylated CpG calls among those with enough CpG calls)\n"
-           "       --meth-pdr-min-cpg <int>  with --meth-pdr: the CpG calls an alignment needs to count, 1..255 (default 4)\n\n");
+           "       --meth-pdr-min-cpg <int>  with --meth-pdr: the CpG calls an alignment needs to count, 1..255 (default 4)\n"
+           "       --meth-epialleles <str>  with --methratio: write the alignments' methylation patterns over every window of\n"
+           "                           four consecutive CpG sites, with methylation entropy and epipolymorphism\n\n");
     exit(1);
 }
 
@@ -162,6 +167,7 @@ int get_options(int argc, char **argv, Opts &o) {
                 o.meth_tiles = x;
             }
             else if (a == "meth-pdr" && i + 1 < argc) o.meth_pdr = argv[++i];
+            else if (a == "meth-epialleles" && i + 1 < argc) o.meth_epialleles = argv[++i];
             else if (a == "meth-pdr-min-cpg" && i + 1 < argc) {
                 const char *v = argv[++i]; char *e; const long x = strtol(v, &e, 10);
                 o.meth_pdr_min_cpg = (*e || e == v || x < 1 || x > 255) ? -1 : (int)x;
@@ -335,6 +341,7 @@ extern "C" int bsx_cli_main(int argc, char **argv) {
     if (o.meth_pdr_min_cpg && o.meth_pdr.empty()) { fprintf(stderr, "--meth-pdr-min-cpg needs --meth-pdr FILE\n"); return 2; }
     if (o.meth_out.empty() && !o.meth_pdr.empty()) { fprintf(stderr, "--meth-pdr needs --methratio\n"); return 2; }
     if (!o.meth_pdr.empty() && !o.meth_pdr_min_cpg) o.meth_pdr_min_cpg = 4;
+    if (o.meth_out.empty() && !o.meth_epialleles.empty()) { fprintf(stderr, "--meth-epialleles needs --methratio\n"); return 2; }
     if (o.qual_threshold != 0) { fprintf(stderr, "-q quality trimming is not supported by the GPU path\n"); return 1; }
     if (o.o.size() > 4) {
         if (o.o.compare(o.o.size() - 4, 4, ".sam") == 0) o.p.out_sam = 1;
@@ -441,6 +448,7 @@ extern "C" int bsx_cli_main(int argc, char **argv) {
             (o.meth_ct_snp && bsx_meth_enable_ct_snp(mh, o.meth_ct_snp) != BSX_OK) ||
             (o.meth_conv >= 0 && bsx_meth_enable_conversion_filter(mh, o.meth_conv) != BSX_OK) ||
             (!o.meth_pdr.empty() && bsx_meth_enable_pdr(mh, o.meth_pdr_min_cpg) != BSX_OK) ||
+            (!o.meth_epialleles.empty() && bsx_meth_enable_epialleles(mh) != BSX_OK) ||
             bsx_mapper_attach_meth(mp, mh, &o.mo, (p.out_sam || no_text) ? 1 : 0) != BSX_OK) {
             fprintf(stderr, "%s\n", bsx_last_error()); return 1; }
     }
@@ -598,6 +606,8 @@ extern "C" int bsx_cli_main(int argc, char **argv) {
         if (!o.meth_mbias.empty() && bsx_meth_write_mbias_file(mh, o.meth_mbias.c_str()) != BSX_OK) return 1;
         if (o.meth_conv >= 0 && bsx_meth_write_conversion_file(mh, o.meth_conv_report.empty() ? nullptr : o.meth_conv_report.c_str()) != BSX_OK) return 1;
         if (!o.meth_pdr.empty() && bsx_meth_write_pdr_file(mh, &o.mo, sp.data(), ln.data(), nullptr, threads, o.meth_pdr.c_str()) != BSX_OK) return 1;
+        if (!o.meth_epialleles.empty() &&
+            bsx_meth_write_epialleles_file(mh, &o.mo, sp.data(), ln.data(), nullptr, threads, o.meth_epialleles.c_str()) != BSX_OK) return 1;
         if (!o.meth_region_report.empty() && bsx_meth_write_regions_file(mh, &o.mo, regions, o.meth_region_report.c_str()) != BSX_OK) return 1;
         if (timing) fprintf(stderr, "[bsx timing] methratio report %.3f s\n", now() - t);
         bsx_meth_destroy(mh);

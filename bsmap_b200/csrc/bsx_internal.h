@@ -123,6 +123,10 @@ int bsx_meth_write_regions_file(bsx_meth *m, const bsx_meth_opts *o, const bsx_r
 // informative (>= K CpG calls), D discordant"; errors are printed (bsx_meth.cu)
 int bsx_meth_write_pdr_file(bsx_meth *m, const bsx_meth_opts *o, const char *const *seqs, const uint32_t *lens, const uint8_t *chroms, int threads,
                             const char *path);
+// the command lines' epiallele output: bsx_meth_write_epialleles to a new file at path, and on stderr "epialleles: S of V
+// valid mappings span a 4-CpG window, W window patterns counted"; errors are printed (bsx_meth.cu)
+int bsx_meth_write_epialleles_file(bsx_meth *m, const bsx_meth_opts *o, const char *const *seqs, const uint32_t *lens, const uint8_t *chroms, int threads,
+                                   const char *path);
 // "no-action" / "correct" / "skip" -> BSX_CT_SNP_*, anything else 0 (bsx_meth.cu)
 int bsx_ct_snp_mode(const char *name);
 int bsx_inflate_file(const char *path, std::vector<char> &out);   // gzip / BGZF members -> bytes (bsx_reads.cpp)

@@ -36,6 +36,14 @@
 // least K of them the second pass adds every CpG call to `concordant` (all methylated or all unmethylated) or
 // `discordant`, two more u32 arrays over the positions.  The informative and discordant alignments go into two per-CTA
 // shared counters, flushed like the histograms.
+//
+// 4-CpG epialleles (bsx_meth_enable_epialleles) switch them to their `Epi` instantiation, again only with `Cycles`.  A
+// CpG rank index over the packed reference (one u32 per word: the CpG sites before it; built on the device by a counting
+// kernel and a scan) numbers the sites, and 16 u32 counters per site count the methylation patterns of the alignments
+// that carry a call at that site and the next three.  The first pass counts the alignment's CpG calls; one with at least
+// four walks its span again, 32 positions a step, with three ballots (site, call, methylated) and the last three sites'
+// bits carried from step to step in warp-uniform registers.  The lane whose call closes a fully called run of four adds
+// the pattern to the first site's row: one global atomic per window.
 #include <algorithm>
 #include <cmath>
 #include <cstdio>
@@ -74,6 +82,11 @@ struct bsx_meth {
     uint32_t pdr_min_cpg = 0;                         // K; 0 = off
     uint32_t *d_conc = nullptr, *d_disc = nullptr;    // n_words * 16 counters each, like d_meth / d_depth
     unsigned long long *d_pdr = nullptr;              // informative, discordant alignments; NULL = PDR off
+    // epialleles: fixed before the first alignment is piled up
+    uint32_t *d_cpg_rank = nullptr;                   // n_words + 1: the CpG sites before each word (the last: all of them)
+    uint32_t *d_epi = nullptr;                        // 16 counters per site, by pattern; NULL = epialleles off
+    unsigned long long *d_epi_count = nullptr;        // alignments with a window, windows counted
+    uint64_t cpg_sites = 0;
 };
 
 namespace {
@@ -101,13 +114,93 @@ struct PdrArgs {
     uint32_t min_cpg;                    // K: an alignment with K or more CpG calls is informative
 };
 
+// what the Epi instantiation needs beyond the Cycles one
+struct EpiArgs {
+    const uint32_t *rank;                // per packed word: the CpG sites before it
+    uint32_t *counts;                    // 16 per site: the windows starting there, by pattern
+    unsigned long long *count;           // alignments with a window, windows counted
+};
+
 // Conv: the CTA's alignments by score, zeroed before and flushed (non-zero bins) after them.  At file scope, so that the
 // pile-up addresses it directly; only the Conv kernels reference it, and only they are given its 1 KB.
 __shared__ uint32_t conv_hist[BSX_CONV_BINS];
 // Pdr: the CTA's informative and discordant alignments, zeroed and flushed the same way
 __shared__ uint32_t pdr_count[2];
+// Epi: the CTA's alignments with a window and its windows, zeroed and flushed the same way
+__shared__ uint32_t epi_count[2];
 
 __device__ __forceinline__ uint32_t ref_code(const uint32_t *refcat, uint32_t q) { return (refcat[q >> 4] >> (30 - 2 * (q & 15))) & 3u; }
+
+// the CpG sites of a packed word w: bit 30 - 2j set when base j is C and base j + 1 is G (for j = 15, the first base of
+// the next word nx)
+__host__ __device__ __forceinline__ uint32_t cpg_mask(uint32_t w, uint32_t nx) {
+    const uint32_t lo = w & 0x55555555u, hi = (w >> 1) & 0x55555555u;
+    return (lo & ~hi) & (((hi & ~lo) << 2) | ((nx >> 30) == 2u ? 1u : 0u));
+}
+// the rank of CpG site c (its C's position): the sites before its word, then those before it in the word (they end
+// inside the word, so the next word is not needed)
+__device__ __forceinline__ uint32_t cpg_rank(const uint32_t *__restrict__ refcat, const uint32_t *__restrict__ rank, uint32_t c) {
+    return __ldg(rank + (c >> 4)) + __popc(cpg_mask(__ldg(refcat + (c >> 4)), 0u) & ~(0xffffffffu >> (2 * (c & 15))));
+}
+
+// Epi's third pass over an alignment's trimmed span [0, len) (read offset start + i, printed length L; calls of cycles
+// outside [lo, hi) are excluded), 32 positions a step with every lane active.  A site of the alignment's strand is a
+// '+' C whose next base is G (the site is the C) or a '-' G whose previous base is C (the site is that C); its call is
+// the read's methylated or converted letter in the cycle bounds, anything else breaks the windows through the site.
+// Three ballots mark the step's sites, calls and methylated calls; c3 / m3 carry the called / methylated bits of the last
+// three sites before the step (bit t: the (t + 1)-th latest), warp-uniform.  A called lane whose three previous sites are
+// called closes a window: its pattern is the four methylated bits, the earliest site the most significant, and its row
+// the earliest site's rank, so rank - 3.  Lane 0 counts the alignment and its windows in epi_count (shared).
+template <class GetC>
+__device__ __forceinline__ void epi_windows(const uint32_t *__restrict__ refcat, uint32_t base, int len, int start, int L, bool rev, int lo, int hi,
+                                            bool first_minus, uint32_t match, char cm, char cc, int lane, GetC getc, const EpiArgs &ep) {
+    const uint32_t want = 3u - match, below = (1u << lane) - 1u;
+    uint32_t c3 = 0u, m3 = 0u, mine = 0u;
+    // the called / methylated bits of the three latest sites among `sites`, then those carried in
+    auto last3 = [&](uint32_t sites, uint32_t calls, uint32_t meths, uint32_t &c, uint32_t &mm) {
+        uint32_t cn = 0u, mn = 0u, t = 0u;
+#pragma unroll
+        for (int r = 0; r < 3; r++) {
+            if (!sites) break;
+            const int p = 31 - __clz(sites);
+            sites &= ~(1u << p);
+            cn |= ((calls >> p) & 1u) << t; mn |= ((meths >> p) & 1u) << t; t++;
+        }
+        c = (cn | (c3 << t)) & 7u; mm = (mn | (m3 << t)) & 7u;
+    };
+#pragma unroll 1
+    for (int i0 = 0; i0 < len; i0 += 32) {
+        const int i = i0 + lane;
+        const uint32_t q = base + (uint32_t)i;
+        bool site = false, called = false, is_m = false;
+        if (i < len && ref_code(refcat, q) == match) {
+            site = (first_minus ? ref_code(refcat, q - 1u) : ref_code(refcat, q + 1u)) == want;
+            if (site) {
+                const int j = start + i;
+                const char c = getc(j);
+                const int cyc = rev ? L - 1 - j : j;
+                called = (c == cm || c == cc) && cyc >= lo && cyc < hi;
+                is_m = called && c == cm;
+            }
+        }
+        const uint32_t sites = __ballot_sync(0xffffffffu, site), calls = __ballot_sync(0xffffffffu, called), meths = __ballot_sync(0xffffffffu, is_m);
+        if (!sites) continue;
+        if (called) {
+            uint32_t c, mm;
+            last3(sites & below, calls, meths, c, mm);
+            if (c == 7u) {
+                const uint32_t row = cpg_rank(refcat, ep.rank, first_minus ? q - 1u : q) - 3u;
+                atomicAdd(ep.counts + (size_t)row * 16 + ((mm << 1) | (is_m ? 1u : 0u)), 1u);
+                mine++;
+            }
+        }
+        uint32_t c, mm;
+        last3(sites, calls, meths, c, mm);
+        c3 = c; m3 = mm;
+    }
+    mine = __reduce_add_sync(0xffffffffu, mine);
+    if (lane == 0 && mine) { atomicAdd(&epi_count[0], 1u); atomicAdd(&epi_count[1], mine); }
+}
 
 // One alignment, executed by a warp: get_alignment's trimming (methratio.py:56-64), the bounds test (105) and the
 // pile-up (107-118).  getc(i) = i-th character of SEQ as printed.  Filters (-u / -p) were applied by the caller.
@@ -120,13 +213,15 @@ __device__ __forceinline__ uint32_t ref_code(const uint32_t *refcat, uint32_t q)
 // Pdr (with Cycles): the first pass also counts the methylated (pm) and unmethylated (pu) CpG calls; when the alignment is
 // kept and pm + pu >= pd.min_cpg, the second pass adds each CpG call to pd.concordant (pm == 0 or pu == 0) or
 // pd.discordant, and lane 0 counts the alignment in pdr_count (shared).
-template <bool Cycles, bool Snp, bool Conv, bool Pdr, class GetC>
+// Epi (with Cycles): the first pass also counts the CpG calls; with BSX_EPI_CPGS or more, a third pass (epi_windows)
+// adds every fully called window of four consecutive sites to ep.counts.
+template <bool Cycles, bool Snp, bool Conv, bool Pdr, bool Epi, class GetC>
 __device__ __forceinline__ void pile_alignment(const uint32_t *__restrict__ refcat, const uint32_t *__restrict__ seqinfo, uint32_t n_seq,
                                                uint32_t *meth, uint32_t *depth, unsigned long long *n_valid, const bsx_meth_opts &o,
                                                uint32_t k, long long pos, long long len, int st, int ins, long long mate_pos, bool sam, int lane, GetC getc,
                                                const MbiasArgs &mb = MbiasArgs{}, int read2 = 0, uint32_t *hist = nullptr,
                                                uint32_t *confirm = nullptr, uint32_t *snp = nullptr, const ConvArgs &cv = ConvArgs{},
-                                               const PdrArgs &pd = PdrArgs{}) {
+                                               const PdrArgs &pd = PdrArgs{}, const EpiArgs &ep = EpiArgs{}) {
     const int L = (int)len;                                  // printed length, before trimming
     const uint32_t *anchor = seqinfo, *size = seqinfo + n_seq + 1;
     long long start = 0;
@@ -172,7 +267,8 @@ __device__ __forceinline__ void pile_alignment(const uint32_t *__restrict__ refc
         const bool rev = ((st ^ (st >> 1)) & 1) != 0;
         const int lo = read2 ? mb.ignore[2] : mb.ignore[0], hi = L - (read2 ? mb.ignore[3] : mb.ignore[1]);
         uint32_t *pdr_to = nullptr;                          // Pdr: where the second pass adds the CpG calls; NULL = nowhere
-        if constexpr (Conv || Pdr) {
+        bool epi_walk = false;                               // Epi: the alignment has enough CpG calls for a window
+        if constexpr (Conv || Pdr || Epi) {
             // the score: a methylated call (read C on '+', G on '-') inside the cycle bounds whose next base on the call's
             // strand is not the CpG partner (CHG and CHH alike, so the second context code is not needed).  The bounds
             // [lo, hi) on the cycle are a range of i: cycle j = start + i, or L - 1 - j when reversed.  Pdr counts the
@@ -183,7 +279,7 @@ __device__ __forceinline__ void pile_alignment(const uint32_t *__restrict__ refc
 #pragma unroll 1
             for (int i = max(rev ? L - s0 - hi : lo - s0, 0) + lane; i < i_end; i += 32) {
                 const uint32_t q = base + (uint32_t)i;
-                if constexpr (!Pdr) {
+                if constexpr (!Pdr && !Epi) {
                     if (ref_code(refcat, q) != match || getc(s0 + i) != cm) continue;
                     const uint32_t c1 = first_minus ? ref_code(refcat, q - 1u) : ref_code(refcat, q + 1u);
                     score += c1 != 3u - match;
@@ -211,6 +307,7 @@ __device__ __forceinline__ void pile_alignment(const uint32_t *__restrict__ refc
                     if (lane == 0) { atomicAdd(&pdr_count[0], 1u); if (disc) atomicAdd(&pdr_count[1], 1u); }
                 }
             }
+            if constexpr (Epi) epi_walk = (Pdr ? pm + pu : __reduce_add_sync(0xffffffffu, pm + pu)) >= (uint32_t)BSX_EPI_CPGS;
         }
         uint32_t *h = hist + read2 * (3 * BSX_MBIAS_CYCLES * 2);
         for (int i = lane; i < (int)len; i += 32) {
@@ -246,6 +343,9 @@ __device__ __forceinline__ void pile_alignment(const uint32_t *__restrict__ refc
             if (!mb.hist) continue;
             if (cyc < BSX_MBIAS_CYCLES) atomicAdd(h + (ctx * BSX_MBIAS_CYCLES + cyc) * 2 + (is_m ? 0 : 1), 1u);
             else atomicAdd(mb.hist + MBIAS_BINS, 1ull);
+        }
+        if constexpr (Epi) {
+            if (epi_walk) epi_windows(refcat, base, (int)len, (int)start, L, rev, lo, hi, first_minus, match, cm, cc, lane, getc, ep);
         }
     }
 }
@@ -316,18 +416,19 @@ __global__ void __launch_bounds__(256) meth_claim_kernel(const uint32_t *__restr
 
 // alignments parsed from SAM / BSP text on the host: one warp per alignment (Cycles: a grid-stride loop of them).
 // Conv asks for 4 resident CTAs per SM: without that floor, ptxas squeezes its instantiations to 32 or 40 registers
-// and spills; with it they take 38 - 44 and none.  Pdr takes the same floor.  The other instantiations keep the plain
-// bound (0 = none).
-template <bool Cycles, bool Snp, bool Conv, bool Pdr>
-__global__ void __launch_bounds__(256, (Conv || Pdr) ? 4 : 0) meth_pileup_kernel(const uint32_t *__restrict__ refcat, const uint32_t *__restrict__ seqinfo, uint32_t n_seq,
+// and spills; with it they take 38 - 44 and none.  Pdr and Epi take the same floor.  The other instantiations keep the
+// plain bound (0 = none).
+template <bool Cycles, bool Snp, bool Conv, bool Pdr, bool Epi>
+__global__ void __launch_bounds__(256, (Conv || Pdr || Epi) ? 4 : 0) meth_pileup_kernel(const uint32_t *__restrict__ refcat, const uint32_t *__restrict__ seqinfo, uint32_t n_seq,
                                                           uint32_t *meth, uint32_t *depth, unsigned long long *n_valid, uint32_t *first, bsx_meth_opts o, uint32_t n,
                                                           const char *__restrict__ seqs, uint32_t stride, const uint16_t *__restrict__ lens,
                                                           const uint32_t *__restrict__ chr, const uint32_t *__restrict__ pos0,
                                                           const uint8_t *__restrict__ strand, const int32_t *__restrict__ insert,
                                                           const int32_t *__restrict__ mate_pos, const uint8_t *__restrict__ flags, MbiasArgs mb,
-                                                          uint32_t *confirm, uint32_t *snp, ConvArgs cv, PdrArgs pd) {
+                                                          uint32_t *confirm, uint32_t *snp, ConvArgs cv, PdrArgs pd, EpiArgs ep) {
     static_assert(Cycles || !Conv, "the conversion filter runs in the Cycles kernels");
     static_assert(Cycles || !Pdr, "PDR runs in the Cycles kernels");
+    static_assert(Cycles || !Epi, "epialleles run in the Cycles kernels");
     const uint32_t w = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     const int lane = threadIdx.x & 31;
     auto one = [&](uint32_t a, uint32_t *hist) {
@@ -335,8 +436,8 @@ __global__ void __launch_bounds__(256, (Conv || Pdr) ? 4 : 0) meth_pileup_kernel
         if (!parsed_alignment(o, n_seq, a, lens, chr, pos0, strand, insert, mate_pos, flags, v)) return;
         if (first && !dup_holds(first, seqinfo, n_seq, v, a, lane)) return;
         const char *sq = seqs + (size_t)a * stride;
-        pile_alignment<Cycles, Snp, Conv, Pdr>(refcat, seqinfo, n_seq, meth, depth, n_valid, o, v.k, v.pos, v.len, v.st, v.ins, v.mate_pos, v.sam, lane,
-                                               [sq](int i) { return sq[i]; }, mb, (flags[a] & BSX_METH_READ2) ? 1 : 0, hist, confirm, snp, cv, pd);
+        pile_alignment<Cycles, Snp, Conv, Pdr, Epi>(refcat, seqinfo, n_seq, meth, depth, n_valid, o, v.k, v.pos, v.len, v.st, v.ins, v.mate_pos, v.sam, lane,
+                                                    [sq](int i) { return sq[i]; }, mb, (flags[a] & BSX_METH_READ2) ? 1 : 0, hist, confirm, snp, cv, pd, ep);
     };
     if constexpr (!Cycles) {
         if (w >= n) return;
@@ -346,10 +447,12 @@ __global__ void __launch_bounds__(256, (Conv || Pdr) ? 4 : 0) meth_pileup_kernel
         hist_zero<MBIAS_BINS>(hist, mb.hist);
         if constexpr (Conv) hist_zero<BSX_CONV_BINS>(conv_hist, cv.hist);
         if constexpr (Pdr) hist_zero<2>(pdr_count, pd.count);
+        if constexpr (Epi) hist_zero<2>(epi_count, ep.count);
         for (uint32_t a = w; a < n; a += (gridDim.x * blockDim.x) >> 5) one(a, hist);
         hist_flush<MBIAS_BINS>(hist, mb.hist);
         if constexpr (Conv) hist_flush<BSX_CONV_BINS>(conv_hist, cv.hist);
         if constexpr (Pdr) hist_flush<2>(pdr_count, pd.count);
+        if constexpr (Epi) hist_flush<2>(epi_count, ep.count);
     }
 }
 
@@ -407,18 +510,19 @@ __global__ void __launch_bounds__(256) meth_claim_mapped_kernel(const uint32_t *
         atomicMin(first + key, u + 1u);
 }
 
-// pile-up of the mapped batch: one warp per read (PE: per mate; Cycles: a grid-stride loop of them); Conv's and Pdr's
-// bound as above
-template <bool Cycles, bool Snp, bool Conv, bool Pdr>
-__global__ void __launch_bounds__(256, (Conv || Pdr) ? 4 : 0) meth_pileup_mapped_kernel(const uint32_t *__restrict__ refcat, const uint32_t *__restrict__ seqinfo, uint32_t n_seq,
+// pile-up of the mapped batch: one warp per read (PE: per mate; Cycles: a grid-stride loop of them); Conv's, Pdr's and
+// Epi's bound as above
+template <bool Cycles, bool Snp, bool Conv, bool Pdr, bool Epi>
+__global__ void __launch_bounds__(256, (Conv || Pdr || Epi) ? 4 : 0) meth_pileup_mapped_kernel(const uint32_t *__restrict__ refcat, const uint32_t *__restrict__ seqinfo, uint32_t n_seq,
                                                                  uint32_t *meth, uint32_t *depth, unsigned long long *n_valid, uint32_t *first, bsx_meth_opts o,
                                                                  int sam, int report_repeat_hits, uint32_t n, int mates, uint32_t stride,
                                                                  const uint8_t *__restrict__ seq_a, const uint8_t *__restrict__ seq_b,
                                                                  const bsx_rec *__restrict__ out_a, const bsx_rec *__restrict__ out_b,
                                                                  const bsx_pair_rec *__restrict__ out_pair, MbiasArgs mb, uint32_t *confirm, uint32_t *snp,
-                                                                 ConvArgs cv, PdrArgs pd) {
+                                                                 ConvArgs cv, PdrArgs pd, EpiArgs ep) {
     static_assert(Cycles || !Conv, "the conversion filter runs in the Cycles kernels");
     static_assert(Cycles || !Pdr, "PDR runs in the Cycles kernels");
+    static_assert(Cycles || !Epi, "epialleles run in the Cycles kernels");
     const uint32_t w = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     const int lane = threadIdx.x & 31;
     auto one = [&](uint32_t u, uint32_t *hist) {
@@ -429,9 +533,9 @@ __global__ void __launch_bounds__(256, (Conv || Pdr) ? 4 : 0) meth_pileup_mapped
         const uint8_t *rd = ((mates == 2 && (u & 1u)) ? seq_b : seq_a) + (size_t)r * stride;
         const int lp = (int)v.len;
         const int read2 = mates == 2 ? (int)(u & 1u) : (mb.readset == 2 ? 1 : 0);     // mate b / readset 2 print FLAG 0x80
-        pile_alignment<true, Snp, Conv, Pdr>(refcat, seqinfo, n_seq, meth, depth, n_valid, o, v.k, v.pos, v.len, v.st, v.ins, v.mate_pos, v.sam, lane,
-                                             [rd, rev, lp](int i) { return rev ? comp_char((char)rd[lp - 1 - i]) : (char)rd[i]; }, mb, read2, hist, confirm, snp, cv,
-                                             pd);
+        pile_alignment<true, Snp, Conv, Pdr, Epi>(refcat, seqinfo, n_seq, meth, depth, n_valid, o, v.k, v.pos, v.len, v.st, v.ins, v.mate_pos, v.sam, lane,
+                                                  [rd, rev, lp](int i) { return rev ? comp_char((char)rd[lp - 1 - i]) : (char)rd[i]; }, mb, read2, hist, confirm, snp,
+                                                  cv, pd, ep);
     };
     if constexpr (!Cycles) {
         // the same steps as `one`, written out: through the lambda, ptxas allocates this instantiation differently
@@ -443,17 +547,19 @@ __global__ void __launch_bounds__(256, (Conv || Pdr) ? 4 : 0) meth_pileup_mapped
         const uint32_t r = mates == 2 ? u >> 1 : u;
         const uint8_t *rd = ((mates == 2 && (u & 1u)) ? seq_b : seq_a) + (size_t)r * stride;
         const int lp = (int)v.len;
-        pile_alignment<false, Snp, false, false>(refcat, seqinfo, n_seq, meth, depth, n_valid, o, v.k, v.pos, v.len, v.st, v.ins, v.mate_pos, v.sam, lane,
+        pile_alignment<false, Snp, false, false, false>(refcat, seqinfo, n_seq, meth, depth, n_valid, o, v.k, v.pos, v.len, v.st, v.ins, v.mate_pos, v.sam, lane,
                                    [rd, rev, lp](int i) { return rev ? comp_char((char)rd[lp - 1 - i]) : (char)rd[i]; }, MbiasArgs{}, 0, nullptr, confirm, snp);
     } else {
         __shared__ uint32_t hist[MBIAS_BINS];
         hist_zero<MBIAS_BINS>(hist, mb.hist);
         if constexpr (Conv) hist_zero<BSX_CONV_BINS>(conv_hist, cv.hist);
         if constexpr (Pdr) hist_zero<2>(pdr_count, pd.count);
+        if constexpr (Epi) hist_zero<2>(epi_count, ep.count);
         for (uint32_t u = w; u < n * (uint32_t)mates; u += (gridDim.x * blockDim.x) >> 5) one(u, hist);
         hist_flush<MBIAS_BINS>(hist, mb.hist);
         if constexpr (Conv) hist_flush<BSX_CONV_BINS>(conv_hist, cv.hist);
         if constexpr (Pdr) hist_flush<2>(pdr_count, pd.count);
+        if constexpr (Epi) hist_flush<2>(epi_count, ep.count);
     }
 }
 
@@ -577,6 +683,62 @@ auto region_kernel_of(bool combine, int snp_mode) {
 }
 auto region_kernel(bool combine, int snp_mode, bool pdr) { return pdr ? region_kernel_of<true>(combine, snp_mode) : region_kernel_of<false>(combine, snp_mode); }
 
+// Epi's rank index, first step: the CpG sites of each packed word (x[n_words] = 0, so that the scan ends in the total)
+__global__ void __launch_bounds__(256) cpg_count_kernel(const uint32_t *__restrict__ refcat, uint64_t n_words, uint32_t *x) {
+    const uint64_t a = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (a > n_words) return;
+    x[a] = a < n_words ? (uint32_t)__popc(cpg_mask(refcat[a], a + 1 < n_words ? refcat[a + 1] : 0u)) : 0u;
+}
+
+// exclusive scan of u32 in place: each CTA scans a tile of SCAN_TILE (8 per thread, then the warps, then the CTA's 8
+// warp sums) and writes the tile's total to sums; the tiles' totals are scanned the same way (recursively) and added
+constexpr int SCAN_TILE = 256 * 8;
+__global__ void __launch_bounds__(256) scan_tile_kernel(uint32_t *x, uint64_t n, uint32_t *sums) {
+    __shared__ uint32_t warp_sum[8];
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const uint64_t b = (uint64_t)blockIdx.x * SCAN_TILE + (uint64_t)threadIdx.x * 8;
+    uint32_t v[8], t = 0;
+#pragma unroll
+    for (int k = 0; k < 8; k++) { const uint32_t y = b + k < n ? x[b + k] : 0u; v[k] = t; t += y; }
+    uint32_t inc = t;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) { const uint32_t y = __shfl_up_sync(0xffffffffu, inc, o); if (lane >= o) inc += y; }
+    if (lane == 31) warp_sum[warp] = inc;
+    __syncthreads();
+    if (warp == 0) {
+        uint32_t w = lane < 8 ? warp_sum[lane] : 0u, wi = w;
+#pragma unroll
+        for (int o = 1; o < 8; o <<= 1) { const uint32_t y = __shfl_up_sync(0xffffffffu, wi, o); if (lane >= o) wi += y; }
+        __syncwarp();
+        if (lane < 8) warp_sum[lane] = wi - w;
+    }
+    __syncthreads();
+    const uint32_t off = warp_sum[warp] + inc - t;
+#pragma unroll
+    for (int k = 0; k < 8; k++) if (b + k < n) x[b + k] = v[k] + off;
+    if (threadIdx.x == blockDim.x - 1) sums[blockIdx.x] = off + t;
+}
+__global__ void __launch_bounds__(256) scan_add_kernel(uint32_t *x, uint64_t n, const uint32_t *__restrict__ tile_off) {
+    const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < n) x[i] += tile_off[i / SCAN_TILE];
+}
+int scan_exclusive(uint32_t *x, uint64_t n) {
+    const uint64_t tiles = (n + SCAN_TILE - 1) / SCAN_TILE;
+    uint32_t *sums = nullptr;
+    if (cudaMalloc(&sums, tiles * 4) != cudaSuccess) { cudaGetLastError(); bsx_set_error("epialleles: out of device memory (%llu bytes for the scan)", (unsigned long long)tiles * 4); return BSX_ERR_CUDA; }
+    scan_tile_kernel<<<(unsigned)tiles, 256>>>(x, n, sums);
+    int rc = cudaGetLastError() == cudaSuccess ? BSX_OK : BSX_ERR_CUDA;
+    if (rc) bsx_set_error("epialleles: scan kernel failed");
+    if (!rc && tiles > 1) rc = scan_exclusive(sums, tiles);
+    if (!rc && tiles > 1) {
+        scan_add_kernel<<<(unsigned)((n + 255) / 256), 256>>>(x, n, sums);
+        if (cudaGetLastError() != cudaSuccess) { bsx_set_error("epialleles: scan kernel failed"); rc = BSX_ERR_CUDA; }
+    }
+    cudaDeviceSynchronize();
+    cudaFree(sums);
+    return rc;
+}
+
 int ensure_staging(bsx_meth *m, size_t n, uint32_t stride) {
     if (n <= m->cap && stride <= m->stride) return BSX_OK;
     cudaFree(m->d_seq); cudaFree(m->d_len); cudaFree(m->d_chr); cudaFree(m->d_pos); cudaFree(m->d_strand); cudaFree(m->d_flags); cudaFree(m->d_ins); cudaFree(m->d_mate);
@@ -603,26 +765,36 @@ int ensure_dup_table(bsx_meth *m) {
     return BSX_OK;
 }
 
-// the instantiation for a combination of options (the kernels of one combination share a signature); conv and pdr
+// the instantiation for a combination of options (the kernels of one combination share a signature); conv, pdr and epi
 // imply cycles
-auto text_kernel(bool cycles, bool snp, bool conv, bool pdr) {
-    if (pdr) return conv ? (snp ? meth_pileup_kernel<true, true, true, true> : meth_pileup_kernel<true, false, true, true>)
-                         : (snp ? meth_pileup_kernel<true, true, false, true> : meth_pileup_kernel<true, false, false, true>);
-    if (conv) return snp ? meth_pileup_kernel<true, true, true, false> : meth_pileup_kernel<true, false, true, false>;
-    return cycles ? (snp ? meth_pileup_kernel<true, true, false, false> : meth_pileup_kernel<true, false, false, false>)
-                  : (snp ? meth_pileup_kernel<false, true, false, false> : meth_pileup_kernel<false, false, false, false>);
+auto text_kernel(bool cycles, bool snp, bool conv, bool pdr, bool epi) {
+    if (epi) return pdr ? (conv ? (snp ? meth_pileup_kernel<true, true, true, true, true> : meth_pileup_kernel<true, false, true, true, true>)
+                                : (snp ? meth_pileup_kernel<true, true, false, true, true> : meth_pileup_kernel<true, false, false, true, true>))
+                        : (conv ? (snp ? meth_pileup_kernel<true, true, true, false, true> : meth_pileup_kernel<true, false, true, false, true>)
+                                : (snp ? meth_pileup_kernel<true, true, false, false, true> : meth_pileup_kernel<true, false, false, false, true>));
+    if (pdr) return conv ? (snp ? meth_pileup_kernel<true, true, true, true, false> : meth_pileup_kernel<true, false, true, true, false>)
+                         : (snp ? meth_pileup_kernel<true, true, false, true, false> : meth_pileup_kernel<true, false, false, true, false>);
+    if (conv) return snp ? meth_pileup_kernel<true, true, true, false, false> : meth_pileup_kernel<true, false, true, false, false>;
+    return cycles ? (snp ? meth_pileup_kernel<true, true, false, false, false> : meth_pileup_kernel<true, false, false, false, false>)
+                  : (snp ? meth_pileup_kernel<false, true, false, false, false> : meth_pileup_kernel<false, false, false, false, false>);
 }
-auto mapped_kernel(bool cycles, bool snp, bool conv, bool pdr) {
-    if (pdr) return conv ? (snp ? meth_pileup_mapped_kernel<true, true, true, true> : meth_pileup_mapped_kernel<true, false, true, true>)
-                         : (snp ? meth_pileup_mapped_kernel<true, true, false, true> : meth_pileup_mapped_kernel<true, false, false, true>);
-    if (conv) return snp ? meth_pileup_mapped_kernel<true, true, true, false> : meth_pileup_mapped_kernel<true, false, true, false>;
-    return cycles ? (snp ? meth_pileup_mapped_kernel<true, true, false, false> : meth_pileup_mapped_kernel<true, false, false, false>)
-                  : (snp ? meth_pileup_mapped_kernel<false, true, false, false> : meth_pileup_mapped_kernel<false, false, false, false>);
+auto mapped_kernel(bool cycles, bool snp, bool conv, bool pdr, bool epi) {
+    if (epi) return pdr ? (conv ? (snp ? meth_pileup_mapped_kernel<true, true, true, true, true> : meth_pileup_mapped_kernel<true, false, true, true, true>)
+                                : (snp ? meth_pileup_mapped_kernel<true, true, false, true, true> : meth_pileup_mapped_kernel<true, false, false, true, true>))
+                        : (conv ? (snp ? meth_pileup_mapped_kernel<true, true, true, false, true> : meth_pileup_mapped_kernel<true, false, true, false, true>)
+                                : (snp ? meth_pileup_mapped_kernel<true, true, false, false, true> : meth_pileup_mapped_kernel<true, false, false, false, true>));
+    if (pdr) return conv ? (snp ? meth_pileup_mapped_kernel<true, true, true, true, false> : meth_pileup_mapped_kernel<true, false, true, true, false>)
+                         : (snp ? meth_pileup_mapped_kernel<true, true, false, true, false> : meth_pileup_mapped_kernel<true, false, false, true, false>);
+    if (conv) return snp ? meth_pileup_mapped_kernel<true, true, true, false, false> : meth_pileup_mapped_kernel<true, false, true, false, false>;
+    return cycles ? (snp ? meth_pileup_mapped_kernel<true, true, false, false, false> : meth_pileup_mapped_kernel<true, false, false, false, false>)
+                  : (snp ? meth_pileup_mapped_kernel<false, true, false, false, false> : meth_pileup_mapped_kernel<false, false, false, false, false>);
 }
 
-// the Cycles kernels run for M-bias, exclusion, the conversion filter or PDR (with M-bias and exclusion off, Cycles is
-// the classification alone: no histogram, bounds [0, L))
-bool cycles_on(const bsx_meth *m) { return m->mbias || m->ignore[0] || m->ignore[1] || m->ignore[2] || m->ignore[3] || m->d_conv || m->d_pdr; }
+// the Cycles kernels run for M-bias, exclusion, the conversion filter, PDR or epialleles (with M-bias and exclusion off,
+// Cycles is the classification alone: no histogram, bounds [0, L))
+bool cycles_on(const bsx_meth *m) {
+    return m->mbias || m->ignore[0] || m->ignore[1] || m->ignore[2] || m->ignore[3] || m->d_conv || m->d_pdr || m->d_epi;
+}
 
 // the Cycles kernels' grid cap and, with M-bias on, their histogram (zeroed), on the first pile-up that needs them
 int ensure_cycles(bsx_meth *m) {
@@ -634,8 +806,8 @@ int ensure_cycles(bsx_meth *m) {
     int dev = 0, sms = 0, per_sm[2] = {0, 0};
     BSX_CUDA_CHECK(cudaGetDevice(&dev));
     BSX_CUDA_CHECK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
-    BSX_CUDA_CHECK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm[0], text_kernel(true, m->ct_snp != 0, m->d_conv != nullptr, m->d_pdr != nullptr), 256, 0));
-    BSX_CUDA_CHECK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm[1], mapped_kernel(true, m->ct_snp != 0, m->d_conv != nullptr, m->d_pdr != nullptr), 256, 0));
+    BSX_CUDA_CHECK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm[0], text_kernel(true, m->ct_snp != 0, m->d_conv != nullptr, m->d_pdr != nullptr, m->d_epi != nullptr), 256, 0));
+    BSX_CUDA_CHECK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm[1], mapped_kernel(true, m->ct_snp != 0, m->d_conv != nullptr, m->d_pdr != nullptr, m->d_epi != nullptr), 256, 0));
     for (int i = 0; i < 2; i++) m->resident[i] = std::max(per_sm[i], 1) * sms;
     BSX_CUDA_CHECK(cudaDeviceSynchronize());
     return BSX_OK;
@@ -648,6 +820,7 @@ MbiasArgs mbias_args(const bsx_meth *m, int readset) {
 }
 ConvArgs conv_args(const bsx_meth *m) { return ConvArgs{m->d_conv, (uint32_t)m->conv_threshold}; }
 PdrArgs pdr_args(const bsx_meth *m) { return PdrArgs{m->d_conc, m->d_disc, m->d_pdr, m->pdr_min_cpg}; }
+EpiArgs epi_args(const bsx_meth *m) { return EpiArgs{m->d_cpg_rank, m->d_epi, m->d_epi_count}; }
 
 int combine_once(bsx_meth *m, const bsx_meth_opts *o) {
     if (!o->combine_cpg || m->combined) return BSX_OK;
@@ -668,6 +841,7 @@ struct Sink {
     void putu(unsigned long long v) { char b[24]; char *e = b + 24, *q = e; do { *--q = (char)('0' + v % 10); v /= 10; } while (v); put(q, (size_t)(e - q)); }
     void putf3(double v) { char b[48]; const int l = snprintf(b, sizeof b, "%.3f", v); put(b, (size_t)l); }
     void putf2(double v) { char b[48]; const int l = snprintf(b, sizeof b, "%.2f", v); put(b, (size_t)l); }
+    void putf4(double v) { char b[48]; const int l = snprintf(b, sizeof b, "%.4f", v); put(b, (size_t)l); }
 };
 
 }  // namespace
@@ -697,7 +871,7 @@ extern "C" int bsx_meth_create(const bsx_index *ix, bsx_meth **out) {
 extern "C" int bsx_meth_destroy(bsx_meth *m) {
     if (!m) return BSX_OK;
     cudaFree(m->d_meth); cudaFree(m->d_depth); cudaFree(m->d_valid); cudaFree(m->d_first); cudaFree(m->d_mbias); cudaFree(m->d_confirm); cudaFree(m->d_snp); cudaFree(m->d_conv);
-    cudaFree(m->d_conc); cudaFree(m->d_disc); cudaFree(m->d_pdr);
+    cudaFree(m->d_conc); cudaFree(m->d_disc); cudaFree(m->d_pdr); cudaFree(m->d_cpg_rank); cudaFree(m->d_epi); cudaFree(m->d_epi_count);
     if (m->dup_order) cudaEventDestroy(m->dup_order);
     cudaFree(m->d_seq); cudaFree(m->d_len); cudaFree(m->d_chr); cudaFree(m->d_pos); cudaFree(m->d_strand); cudaFree(m->d_flags); cudaFree(m->d_ins); cudaFree(m->d_mate);
     delete m;
@@ -730,10 +904,10 @@ extern "C" int bsx_meth_add(bsx_meth *m, const bsx_meth_opts *o, uint32_t n, con
         const unsigned blocks = (unsigned)(((uint64_t)n * 32 + 255) / 256);
         const bool cyc = cycles_on(m);
         if (cyc) { rc = ensure_cycles(m); if (rc) return rc; }
-        text_kernel(cyc, m->ct_snp != 0, m->d_conv != nullptr, m->d_pdr != nullptr)<<<cyc ? std::min<unsigned>(blocks, (unsigned)m->resident[0]) : blocks, 256>>>(
+        text_kernel(cyc, m->ct_snp != 0, m->d_conv != nullptr, m->d_pdr != nullptr, m->d_epi != nullptr)<<<cyc ? std::min<unsigned>(blocks, (unsigned)m->resident[0]) : blocks, 256>>>(
             m->ix->d_refcat, m->ix->d_seqinfo, m->ix->n_seq, m->d_meth, m->d_depth, m->d_valid, o->rm_dup ? m->d_first : nullptr, *o, n, m->d_seq,
             m->stride, m->d_len, m->d_chr, m->d_pos, m->d_strand, m->d_ins, m->d_mate, m->d_flags, cyc ? mbias_args(m, 0) : MbiasArgs{}, m->d_confirm, m->d_snp,
-            conv_args(m), pdr_args(m));
+            conv_args(m), pdr_args(m), epi_args(m));
         BSX_CUDA_CHECK(cudaGetLastError());
     }
     if (n_valid) {
@@ -764,10 +938,10 @@ int bsx_meth_pile_mapped(bsx_meth *m, const bsx_meth_opts *o, int sam, int repor
         BSX_CUDA_CHECK(cudaGetLastError());
     }
     const unsigned blocks = (unsigned)(((uint64_t)n * (uint64_t)mates * 32 + 255) / 256);
-    mapped_kernel(cyc, m->ct_snp != 0, m->d_conv != nullptr, m->d_pdr != nullptr)<<<cyc ? std::min<unsigned>(blocks, (unsigned)m->resident[1]) : blocks, 256, 0, st>>>(
+    mapped_kernel(cyc, m->ct_snp != 0, m->d_conv != nullptr, m->d_pdr != nullptr, m->d_epi != nullptr)<<<cyc ? std::min<unsigned>(blocks, (unsigned)m->resident[1]) : blocks, 256, 0, st>>>(
         m->ix->d_refcat, m->ix->d_seqinfo, m->ix->n_seq, m->d_meth, m->d_depth, m->d_valid, o->rm_dup ? m->d_first : nullptr, *o, sam,
         report_repeat_hits, n, mates, stride, seq_a, seq_b, out_a, out_b, out_pair, cyc ? mbias_args(m, readset) : MbiasArgs{}, m->d_confirm, m->d_snp,
-        conv_args(m), pdr_args(m));
+        conv_args(m), pdr_args(m), epi_args(m));
     BSX_CUDA_CHECK(cudaGetLastError());
     if (o->rm_dup) BSX_CUDA_CHECK(cudaEventRecord(m->dup_order, st));
     return BSX_OK;
@@ -1116,6 +1290,174 @@ int bsx_meth_write_pdr_file(bsx_meth *m, const bsx_meth_opts *o, const char *con
     if (bsx_meth_pdr(m, &inf, &disc) != BSX_OK || bsx_meth_valid_count(m, &valid) != BSX_OK) { fprintf(stderr, "%s\n", bsx_last_error()); return BSX_ERR_CUDA; }
     fprintf(stderr, "PDR: %llu of %llu valid mappings informative (>= %u CpG calls), %llu discordant\n", (unsigned long long)inf, (unsigned long long)valid,
             m->pdr_min_cpg, (unsigned long long)disc);
+    return BSX_OK;
+}
+
+extern "C" int bsx_meth_enable_epialleles(bsx_meth *m) {
+    if (!m) { bsx_set_error("bsx_meth_enable_epialleles: bad argument"); return BSX_ERR_ARG; }
+    if (m->started) { bsx_set_error("bsx_meth_enable_epialleles: alignments were already piled up; enable epialleles first"); return BSX_ERR_ARG; }
+    if (m->d_epi) { bsx_set_error("bsx_meth_enable_epialleles: epialleles are already enabled"); return BSX_ERR_ARG; }
+    BSX_CUDA_CHECK(cudaSetDevice(m->ix->device));
+    const uint64_t nw = m->ix->n_words;
+    if (cudaMalloc(&m->d_cpg_rank, (nw + 1) * 4) != cudaSuccess) {
+        cudaGetLastError(); m->d_cpg_rank = nullptr;
+        bsx_set_error("epialleles: out of device memory (%llu bytes for the CpG rank index)", (unsigned long long)(nw + 1) * 4); return BSX_ERR_CUDA; }
+    auto undo = [m]() { cudaFree(m->d_cpg_rank); cudaFree(m->d_epi); cudaFree(m->d_epi_count); m->d_cpg_rank = m->d_epi = nullptr; m->d_epi_count = nullptr; };
+    cpg_count_kernel<<<(unsigned)((nw + 1 + 255) / 256), 256>>>(m->ix->d_refcat, nw, m->d_cpg_rank);
+    if (cudaGetLastError() != cudaSuccess) { undo(); bsx_set_error("epialleles: CpG count kernel failed"); return BSX_ERR_CUDA; }
+    const int rc = scan_exclusive(m->d_cpg_rank, nw + 1);
+    if (rc) { undo(); return rc; }
+    uint32_t sites = 0;
+    if (cudaMemcpy(&sites, m->d_cpg_rank + nw, 4, cudaMemcpyDeviceToHost) != cudaSuccess) { cudaGetLastError(); undo(); bsx_set_error("epialleles: rank index download failed"); return BSX_ERR_CUDA; }
+    const size_t bytes = (size_t)std::max<uint32_t>(sites, 1u) * 16 * sizeof(uint32_t);
+    if (cudaMalloc(&m->d_epi, bytes) != cudaSuccess || cudaMalloc(&m->d_epi_count, 2 * sizeof(unsigned long long)) != cudaSuccess) {
+        cudaGetLastError(); undo();
+        bsx_set_error("epialleles: out of device memory (%zu bytes for the pattern counters of %u CpG sites)", bytes, sites); return BSX_ERR_CUDA; }
+    if (cudaMemset(m->d_epi, 0, bytes) != cudaSuccess || cudaMemset(m->d_epi_count, 0, 2 * sizeof(unsigned long long)) != cudaSuccess) {
+        cudaGetLastError(); undo(); bsx_set_error("epialleles: cudaMemset failed"); return BSX_ERR_CUDA; }
+    m->cpg_sites = sites;
+    return BSX_OK;
+}
+
+// the CpG sites of sequence k: their positions in the sequence (may be NULL), their number and the rank of the first,
+// from the device's packed reference and rank index (the rule of cpg_rank, so that the ranks line up)
+static int epi_sites(bsx_meth *m, uint32_t k, std::vector<uint32_t> *pos, uint64_t *n, uint64_t *rank0) {
+    const bsx_index *ix = m->ix;
+    const uint64_t a0 = ix->anchor[k], L = ix->size[k];
+    const uint64_t w0 = a0 >> 4, w1 = std::min<uint64_t>((a0 + L) >> 4, ix->n_words - 1);   // the words holding [a0, a0 + L], and the next
+    std::vector<uint32_t> w((size_t)(w1 - w0 + 2), 0u);
+    BSX_CUDA_CHECK(cudaMemcpy(w.data(), ix->d_refcat + w0, (size_t)(w1 - w0 + 1) * 4, cudaMemcpyDeviceToHost));
+    uint32_t r = 0;
+    BSX_CUDA_CHECK(cudaMemcpy(&r, m->d_cpg_rank + w0, 4, cudaMemcpyDeviceToHost));
+    const uint32_t lead = (uint32_t)(a0 & 15);
+    r += (uint32_t)__builtin_popcount(cpg_mask(w[0], 0u) & ~(0xffffffffu >> (2 * lead)));
+    uint64_t cnt = 0;
+    for (uint64_t q = a0 - (a0 & 15); q < a0 + L; q += 16) {
+        const size_t wi = (size_t)((q >> 4) - w0);
+        uint32_t s = cpg_mask(w[wi], w[wi + 1]);
+        while (s) {
+            const int b = 31 - __builtin_clz(s);
+            s &= ~(1u << b);
+            const uint64_t c = q + (uint64_t)((30 - b) >> 1);
+            if (c < a0 || c >= a0 + L) continue;
+            if (pos) pos->push_back((uint32_t)(c - a0));
+            cnt++;
+        }
+    }
+    *n = cnt; *rank0 = r;
+    return BSX_OK;
+}
+
+extern "C" int bsx_meth_cpg_sites(bsx_meth *m, uint32_t k, uint64_t *n) {
+    if (!m || !n || k >= m->ix->n_seq) { bsx_set_error("bsx_meth_cpg_sites: bad argument"); return BSX_ERR_ARG; }
+    if (!m->d_epi) { bsx_set_error("bsx_meth_cpg_sites: epialleles were not enabled (bsx_meth_enable_epialleles)"); return BSX_ERR_ARG; }
+    BSX_CUDA_CHECK(cudaSetDevice(m->ix->device));
+    uint64_t r0 = 0;
+    return epi_sites(m, k, nullptr, n, &r0);
+}
+
+extern "C" int bsx_meth_download_epialleles(bsx_meth *m, uint32_t k, uint32_t *site_pos, uint32_t *counts) {
+    if (!m || k >= m->ix->n_seq) { bsx_set_error("bsx_meth_download_epialleles: bad argument"); return BSX_ERR_ARG; }
+    if (!m->d_epi) { bsx_set_error("bsx_meth_download_epialleles: epialleles were not enabled (bsx_meth_enable_epialleles)"); return BSX_ERR_ARG; }
+    BSX_CUDA_CHECK(cudaSetDevice(m->ix->device));
+    BSX_CUDA_CHECK(cudaDeviceSynchronize());           // in-process batches pile up from two streams
+    std::vector<uint32_t> pos;
+    uint64_t n = 0, r0 = 0;
+    int rc = epi_sites(m, k, &pos, &n, &r0); if (rc) return rc;
+    if (site_pos && n) memcpy(site_pos, pos.data(), n * 4);
+    if (counts && n) BSX_CUDA_CHECK(cudaMemcpy(counts, m->d_epi + r0 * 16, n * 16 * 4, cudaMemcpyDeviceToHost));
+    return BSX_OK;
+}
+
+extern "C" int bsx_meth_epialleles(bsx_meth *m, uint64_t *spanning, uint64_t *windows) {
+    if (!m) { bsx_set_error("bsx_meth_epialleles: bad argument"); return BSX_ERR_ARG; }
+    if (!m->d_epi) { bsx_set_error("bsx_meth_epialleles: epialleles were not enabled (bsx_meth_enable_epialleles)"); return BSX_ERR_ARG; }
+    BSX_CUDA_CHECK(cudaSetDevice(m->ix->device));
+    BSX_CUDA_CHECK(cudaDeviceSynchronize());           // in-process batches flush from two streams
+    unsigned long long h[2];
+    BSX_CUDA_CHECK(cudaMemcpy(h, m->d_epi_count, sizeof h, cudaMemcpyDeviceToHost));
+    if (spanning) *spanning = h[0];
+    if (windows) *windows = h[1];
+    return BSX_OK;
+}
+
+extern "C" size_t bsx_meth_write_epialleles(bsx_meth *m, const bsx_meth_opts *o, const char *const *seqs, const uint32_t *lens, const uint8_t *chroms,
+                                            int threads, int fd) {
+    if (!m || !o || !seqs || !lens) { bsx_set_error("bsx_meth_write_epialleles: bad argument"); return 0; }
+    if (!m->d_epi) { bsx_set_error("bsx_meth_write_epialleles: epialleles were not enabled (bsx_meth_enable_epialleles)"); return 0; }
+    const bsx_index *ix = m->ix;
+    if (cudaSetDevice(ix->device) != cudaSuccess || cudaDeviceSynchronize() != cudaSuccess) {   // in-process batches pile up from two streams
+        bsx_set_error("bsx_meth_write_epialleles: %s", cudaGetErrorString(cudaGetLastError())); return 0; }
+    threads = bsx_host_threads(threads);
+    size_t written = 0;
+    auto out = [&](const std::string &s) {
+        size_t off = 0;
+        while (off < s.size()) { const ssize_t w = write(fd, s.data() + off, s.size() - off); if (w <= 0) return false; off += (size_t)w; written += (size_t)w; }
+        return true;
+    };
+    if (!out("chr\tstart\tend\treads\tlevel\tentropy\tEPM\tpatterns\n")) return 0;
+    std::vector<uint32_t> order;
+    for (uint32_t k = 0; k < ix->n_seq; k++) if (!chroms || chroms[k]) order.push_back(k);
+    std::sort(order.begin(), order.end(), [&](uint32_t a, uint32_t b) { return ix->names[a] < ix->names[b]; });   // the table's order
+    // `correct` cannot rescale a pattern, so both SNP modes drop a window with SNP evidence at any of its eight bases
+    const bool snp_drop = m->ct_snp == BSX_CT_SNP_SKIP || m->ct_snp == BSX_CT_SNP_CORRECT;
+    const uint64_t min_n = (uint64_t)std::max(o->min_depth, 1);
+    std::vector<uint32_t> pos, cnt, ec, es;
+    for (uint32_t k : order) {
+        const uint32_t L = ix->size[k];
+        if (lens[k] != L) { bsx_set_error("bsx_meth_write_epialleles: sequence %u has %u bases, the index %u", k, lens[k], L); return 0; }
+        uint64_t n = 0, r0 = 0;
+        pos.clear();
+        if (epi_sites(m, k, &pos, &n, &r0) != BSX_OK) return 0;
+        if (n < BSX_EPI_CPGS) continue;
+        cnt.resize(n * 16);
+        if (cudaMemcpy(cnt.data(), m->d_epi + r0 * 16, n * 16 * 4, cudaMemcpyDeviceToHost) != cudaSuccess) {
+            bsx_set_error("bsx_meth_write_epialleles: counter download failed: %s", cudaGetErrorString(cudaGetLastError())); return 0; }
+        if (snp_drop) { ec.resize(L); es.resize(L); if (bsx_meth_download_ct_snp(m, o, k, ec.data(), es.data()) != BSX_OK) return 0; }
+        const std::string &name = ix->names[k];
+        std::vector<std::string> chunk((size_t)threads);
+        bsx_parallel(threads, (size_t)(n - (BSX_EPI_CPGS - 1)), [&](int t, size_t b, size_t e) {
+            Sink s{&chunk[t]};
+            for (size_t j = b; j < e; j++) {
+                const uint32_t *c = &cnt[j * 16];
+                uint64_t reads = 0, meth = 0;
+                for (int i = 0; i < 16; i++) { reads += c[i]; meth += (uint64_t)c[i] * (uint64_t)__builtin_popcount((unsigned)i); }
+                if (reads < min_n) continue;
+                if (snp_drop) {
+                    bool ev = false;
+                    for (int t4 = 0; t4 < BSX_EPI_CPGS; t4++) ev = ev || es[pos[j + t4]] || es[pos[j + t4] + 1];
+                    if (ev) continue;
+                }
+                // ascending i in double, as the oracle sums them
+                double h = 0.0, sq = 0.0;
+                for (int i = 0; i < 16; i++) {
+                    if (!c[i]) continue;
+                    const double p = (double)c[i] / (double)reads;
+                    h += p * log2(p); sq += p * p;
+                }
+                s.put(name.data(), name.size()); s.putc('\t'); s.putu(pos[j] + 1ull); s.putc('\t'); s.putu(pos[j + BSX_EPI_CPGS - 1] + 2ull); s.putc('\t');
+                s.putu(reads); s.putc('\t'); s.putf4((double)meth / (double)(4 * reads)); s.putc('\t'); s.putf4((0.0 - h) / 4.0); s.putc('\t');
+                s.putf4(1.0 - sq); s.putc('\t');
+                for (int i = 0; i < 16; i++) { if (i) s.putc(','); s.putu(c[i]); }
+                s.putc('\n');
+            }
+        });
+        for (int t = 0; t < threads; t++) if (!out(chunk[t])) return 0;
+    }
+    return written;
+}
+
+int bsx_meth_write_epialleles_file(bsx_meth *m, const bsx_meth_opts *o, const char *const *seqs, const uint32_t *lens, const uint8_t *chroms, int threads,
+                                   const char *path) {
+    const int fd = open(path, O_WRONLY | O_CREAT | O_TRUNC, 0644);
+    if (fd < 0) { fprintf(stderr, "failed to open epiallele output file: %s\n", path); return BSX_ERR_IO; }
+    const size_t w = bsx_meth_write_epialleles(m, o, seqs, lens, chroms, threads, fd);
+    close(fd);
+    if (w == 0) { fprintf(stderr, "%s\n", bsx_last_error()); return BSX_ERR_IO; }
+    uint64_t spanning = 0, windows = 0, valid = 0;
+    if (bsx_meth_epialleles(m, &spanning, &windows) != BSX_OK || bsx_meth_valid_count(m, &valid) != BSX_OK) { fprintf(stderr, "%s\n", bsx_last_error()); return BSX_ERR_CUDA; }
+    fprintf(stderr, "epialleles: %llu of %llu valid mappings span a %d-CpG window, %llu window patterns counted\n", (unsigned long long)spanning,
+            (unsigned long long)valid, BSX_EPI_CPGS, (unsigned long long)windows);
     return BSX_OK;
 }
 

@@ -27,6 +27,10 @@
 //                              mappings informative (>= K CpG calls), D discordant" to stderr; with --region-report the
 //                              report gains the columns concordant, discordant and PDR
 //   --pdr-min-cpg K            CpG calls an alignment needs to be informative, 1..255 (default 4)
+//   --epialleles FILE          4-CpG epialleles: per window of four consecutive CpG sites the alignments with a call at
+//                              all four, by methylation pattern, with their level, methylation entropy and
+//                              epipolymorphism; prints "epialleles: S of V valid mappings span a 4-CpG window, W window
+//                              patterns counted" to stderr
 #include <chrono>
 #include <cstdio>
 #include <cstdlib>
@@ -57,6 +61,7 @@ struct MOpts {
     long long tiles = 0;                     // --tiles W; 0 = none
     std::string pdr;                         // --pdr FILE
     int pdr_min_cpg = 0;                     // --pdr-min-cpg K; 0 = not given (4)
+    std::string epialleles;                  // --epialleles FILE
     std::vector<std::string> files;
 };
 
@@ -80,7 +85,8 @@ void parse(int argc, char **argv, MOpts &m) {
                                {'t', "trim-fillin", true}, {'g', "combine-CpG", false}, {'m', "min-depth", true}, {'h', "help", false},
                                {'\1', "mbias", true}, {'\2', "mbias-ignore", true}, {'\3', "ct-snp", true},
                                {'\4', "conversion-filter", true}, {'\5', "conversion-report", true}, {'\6', "region-report", true},
-                               {'\7', "regions", true}, {'\10', "tiles", true}, {'\11', "pdr", true}, {'\12', "pdr-min-cpg", true}};   // long only
+                               {'\7', "regions", true}, {'\10', "tiles", true}, {'\11', "pdr", true}, {'\12', "pdr-min-cpg", true},
+                               {'\13', "epialleles", true}};   // long only
     auto apply = [&](char c, const char *v) {
         if (!v) v = "";
         switch (c) {
@@ -123,9 +129,11 @@ void parse(int argc, char **argv, MOpts &m) {
             case '\12': { char *e; const long x = strtol(v, &e, 10);
                 if (*e || e == v || x < 1 || x > 255) usage_error("option --pdr-min-cpg: expected an integer 1..255");
                 m.pdr_min_cpg = (int)x; } break;
+            case '\13': m.epialleles = v; break;
             case 'h': printf("Usage: methratio [options] BSMAP_MAPPING_FILES\n  -o FILE -d FILE [-c CHR] [-u] [-p] [-z] [-q] [-r] [-t N] [-g] [-m FOLD] [--mbias FILE] [--mbias-ignore A,B,C,D]\n"
                              "  [--ct-snp no-action|correct|skip] [--conversion-filter N] [--conversion-report FILE]\n"
-                             "  [--region-report FILE (--regions BED | --tiles W)] [--pdr FILE [--pdr-min-cpg K]]\n"); exit(0);
+                             "  [--region-report FILE (--regions BED | --tiles W)] [--pdr FILE [--pdr-min-cpg K]]\n"
+                             "  [--epialleles FILE]\n"); exit(0);
         }
     };
     for (int i = 1; i < argc; i++) {
@@ -365,7 +373,8 @@ extern "C" int bsx_methratio_main(int argc, char **argv) {
         fprintf(stderr, "%s\n", bsx_last_error()); return 1; }
     if ((!m.mbias.empty() && bsx_meth_enable_mbias(mh) != BSX_OK) || (m.ignore_set && bsx_meth_set_ignore(mh, m.ignore) != BSX_OK) ||
         (m.ct_snp && bsx_meth_enable_ct_snp(mh, m.ct_snp) != BSX_OK) || (m.conv >= 0 && bsx_meth_enable_conversion_filter(mh, m.conv) != BSX_OK) ||
-        (!m.pdr.empty() && bsx_meth_enable_pdr(mh, m.pdr_min_cpg) != BSX_OK)) {
+        (!m.pdr.empty() && bsx_meth_enable_pdr(mh, m.pdr_min_cpg) != BSX_OK) ||
+        (!m.epialleles.empty() && bsx_meth_enable_epialleles(mh) != BSX_OK)) {
         fprintf(stderr, "%s\n", bsx_last_error()); return 1; }
     bsx_regions regions;                                      // read before the pile-up, so that a bad BED fails early
     if ((!m.regions.empty() && bsx_regions_bed(ix, selected.data(), m.regions.c_str(), regions) != BSX_OK) ||
@@ -467,6 +476,10 @@ extern "C" int bsx_methratio_main(int argc, char **argv) {
     if (!m.pdr.empty()) {
         disp(m, ("writing " + m.pdr + " ...").c_str());
         if (bsx_meth_write_pdr_file(mh, &m.o, sp.data(), ln.data(), selected.data(), threads, m.pdr.c_str()) != BSX_OK) return 1;
+    }
+    if (!m.epialleles.empty()) {
+        disp(m, ("writing " + m.epialleles + " ...").c_str());
+        if (bsx_meth_write_epialleles_file(mh, &m.o, sp.data(), ln.data(), selected.data(), threads, m.epialleles.c_str()) != BSX_OK) return 1;
     }
     if (!m.region_report.empty()) {
         disp(m, ("writing " + m.region_report + " ...").c_str());

@@ -399,6 +399,49 @@ int bsx_meth_pdr(bsx_meth *m, uint64_t *informative, uint64_t *discordant);
  * Returns bytes written (0 on error). */
 size_t bsx_meth_write_pdr(bsx_meth *m, const bsx_meth_opts *o, const char *const *seqs, const uint32_t *lens,
                           const uint8_t *chroms /* n_seq flags or NULL */, int threads, int fd);
+/* --- 4-CpG epialleles: methylation patterns of reads over consecutive CpG sites -------------------------------------
+ * PDR says whether the reads at a CpG are discordant, but not whether a few fixed patterns (clones) or random ones
+ * (disorder) make them so.  The patterns themselves, over windows of four consecutive CpG sites, tell the two apart:
+ * methylation entropy (Xie et al., NAR 2011) and epipolymorphism (Landau et al., Cancer Cell 2014).
+ *   site         a position c of the packed reference with ref[c] = C and ref[c+1] = G (upper-cased; N reads as A, so a
+ *                site never crosses sequences).  Sites are numbered by rank in reference order.  Both strands share a
+ *                site: a '+' CpG call at q belongs to site q, a '-' CpG call at q to site q - 1.
+ *   call         the PDR / M-bias call, after every other rule: -u / -p, -r, -t, mate-overlap removal, the bounds test
+ *                and bsx_meth_set_ignore's cycle rule; only CpG calls matter
+ *   read's sites the sites whose call position (the C on '+', the G on '-') lies in the alignment's trimmed span; such a
+ *                site without a call (N, a mismatch, an excluded cycle) breaks every window through it
+ *   window       sites s, s+1, s+2, s+3.  An alignment with a call at all four adds 1 to counts[s][i], i = sum of
+ *                m_k * 2^(3-k), k = 0 for site s, m_k = 1 when the call is methylated (i = 0: UUUU).  Each mate on its
+ *                own calls; mate-overlap removal keeps a CpG from counting twice.  Strands are always pooled, so -g
+ *                does not change the counters.
+ *   other rules  an alignment dropped by the conversion filter and a -r loser are not scored; the counters, the M-bias,
+ *                the C/T SNP evidence, the conversion histogram, the PDR counters and "valid mappings" do not change
+ *   summary      the alignments with at least one window, and the windows counted
+ *   file         header "chr start end reads level entropy EPM patterns" (tab-separated); one line per window with
+ *                reads = sum of its 16 counts >= max(-m, 1), sequences selected and sorted by name, windows ascending.
+ *                start = the 1-based position of the first site's C, end = that of the fourth site's G; level =
+ *                methylated calls / (4 reads); entropy = -(1/4) sum over n_i > 0 of (n_i/N) log2(n_i/N); EPM = 1 - sum
+ *                (n_i/N)^2; the three %.4f, summed in ascending i in double; patterns = the 16 counts, comma-separated,
+ *                i = 0 first.  BSX_CT_SNP_SKIP and BSX_CT_SNP_CORRECT drop a window with SNP evidence (snp > 0) at any
+ *                of its eight bases (`correct` cannot rescale a pattern); -z is ignored.
+ * HBM: 4 bytes per 16 positions for the rank index, and 64 bytes per CpG site. */
+#define BSX_EPI_CPGS 4
+/* build the CpG rank index and the pattern counters, and count windows from now on.  Must precede the first alignment
+ * piled up, once; a late or second call: BSX_ERR_ARG; no device memory: BSX_ERR_CUDA (the message names the size). */
+int bsx_meth_enable_epialleles(bsx_meth *m);
+/* the number of CpG sites of sequence k; BSX_ERR_ARG when epialleles were not enabled */
+int bsx_meth_cpg_sites(bsx_meth *m, uint32_t k, uint64_t *n);
+/* the sites of sequence k (n = bsx_meth_cpg_sites): site_pos[j] = 0-based position of site j's C in the sequence, and
+ * counts[j * 16 + i] the alignments with pattern i over the window that starts at site j (rows whose window would leave
+ * the sequence are zero).  Either may be NULL.  Synchronises the device; BSX_ERR_ARG when epialleles were not enabled. */
+int bsx_meth_download_epialleles(bsx_meth *m, uint32_t k, uint32_t *site_pos, uint32_t *counts);
+/* the alignments with at least one window and the windows counted so far (synchronises the device; either may be
+ * NULL); BSX_ERR_ARG when epialleles were not enabled */
+int bsx_meth_epialleles(bsx_meth *m, uint64_t *spanning, uint64_t *windows);
+/* write the epiallele file to fd for the sequences selected by `chroms` (NULL = all); seqs / lens as in bsx_meth_write
+ * (lens must match the index).  Returns bytes written (0 on error). */
+size_t bsx_meth_write_epialleles(bsx_meth *m, const bsx_meth_opts *o, const char *const *seqs, const uint32_t *lens,
+                                 const uint8_t *chroms /* n_seq flags or NULL */, int threads, int fd);
 /* --- methylation levels over regions, reduced on the device from the counters ----------------------------------------
  *   region   (sequence, start, end), 0-based and half-open as in BED; start == end is empty; an end past the sequence end
  *            is clipped when counting.  Each region is reported for the contexts CpG, CHG, CHH (ctx 0, 1, 2).
@@ -433,7 +476,8 @@ int bsx_meth_regions_pdr(bsx_meth *m, const bsx_meth_opts *o, uint64_t n, const 
  * extensions: --mbias FILE (the M-bias report) and --mbias-ignore A,B,C,D (bsx_meth_set_ignore), SAM and BAM only;
  * --ct-snp no-action|correct|skip (bsx_meth_enable_ct_snp); --conversion-filter N and --conversion-report FILE
  * (bsx_meth_enable_conversion_filter, bsx_meth_write_conversion); --region-report FILE with --regions BED or --tiles W
- * (bsx_meth_write_regions); --pdr FILE [--pdr-min-cpg K] (bsx_meth_enable_pdr, bsx_meth_write_pdr) */
+ * (bsx_meth_write_regions); --pdr FILE [--pdr-min-cpg K] (bsx_meth_enable_pdr, bsx_meth_write_pdr); --epialleles FILE
+ * (bsx_meth_enable_epialleles, bsx_meth_write_epialleles) */
 int bsx_methratio_main(int argc, char **argv);
 
 /* --- the bsmap command line (main.cpp:441-476): same options, same output files -------------- */
