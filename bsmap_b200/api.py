@@ -7,7 +7,7 @@ import os
 import numpy as np
 
 from . import lib as _l
-from .lib import CONV_BINS, CT_SNP_MODES, MBIAS_CYCLES, METH_READ2, PAIR_REC, REC, BsxError, IndexInfo, MethOpts, Params, Stats, check, load, strs
+from .lib import CONV_BINS, CT_SNP_MODES, MBIAS_CYCLES, METH_READ2, MHL_MAX_LEN, PAIR_REC, REC, BsxError, IndexInfo, MethOpts, Params, Stats, check, load, strs
 
 
 def make_params(s=16, I=4, v=2, w=1000, r=1, m=28, x=500, n=0, pairend=0, S=0, f=5, L=144,
@@ -575,6 +575,45 @@ class Meth:
         """the region report (include/bsmap_b200.h) to fd; returns bytes written"""
         c, s, e = self._regions(chr_idx, start, end)
         w = load().bsx_meth_write_regions(self.h, C.byref(self.o), len(c), c.ctypes.data, s.ctypes.data, e.ctypes.data, fd)
+        if w == 0:
+            check(1)
+        return w
+
+    def enable_mhl(self):
+        """count, per CpG site, the alignments' runs of consecutive called / methylated / unmethylated CpG sites ending
+        there, for the methylation haplotype load (include/bsmap_b200.h); builds the CpG rank index on the device unless
+        enable_epialleles did; before the first add / mapped batch, once"""
+        check(load().bsx_meth_enable_mhl(self.h))
+
+    def mhl_counters(self, k: int):
+        """-> (uint32 [n]: 0-based position of each CpG site's C on reference sequence k, uint32 [n, 3, 16]: the
+        alignments whose run of family f (0 called, 1 methylated, 2 unmethylated) ending at the site has length
+        min(r + 1, 16) at [j, f, r])"""
+        n = C.c_uint64(0)
+        check(load().bsx_meth_cpg_sites(self.h, k, C.byref(n)))
+        pos, counts = np.zeros(n.value, dtype=np.uint32), np.zeros((n.value, 3, MHL_MAX_LEN), dtype=np.uint32)
+        check(load().bsx_meth_download_mhl(self.h, k, pos.ctypes.data, counts.ctypes.data))
+        return pos, counts
+
+    def mhl(self):
+        """-> (alignments with at least one CpG call, their CpG calls)"""
+        a, c = C.c_uint64(0), C.c_uint64(0)
+        check(load().bsx_meth_mhl(self.h, C.byref(a), C.byref(c)))
+        return a.value, c.value
+
+    def mhl_regions(self, chr_idx, start, end):
+        """-> (uint64 [n]: the CpG sites of each region, uint64 [n, 3, 16]: T_l, M_l, U_l at [r, f, l - 1]) over the
+        0-based half-open regions; needs enable_mhl"""
+        c, s, e = self._regions(chr_idx, start, end)
+        sites, out = np.zeros(len(c), dtype=np.uint64), np.zeros((len(c), 3, MHL_MAX_LEN), dtype=np.uint64)
+        check(load().bsx_meth_regions_mhl(self.h, C.byref(self.o), len(c), c.ctypes.data, s.ctypes.data, e.ctypes.data, sites.ctypes.data,
+                                          out.ctypes.data))
+        return sites, out
+
+    def write_mhl(self, fd: int, chr_idx, start, end) -> int:
+        """the MHL file (include/bsmap_b200.h) for the regions to fd; returns bytes written"""
+        c, s, e = self._regions(chr_idx, start, end)
+        w = load().bsx_meth_write_mhl(self.h, C.byref(self.o), len(c), c.ctypes.data, s.ctypes.data, e.ctypes.data, fd)
         if w == 0:
             check(1)
         return w

@@ -12,7 +12,8 @@
 // or --meth-tiles W), and the proportion of discordant reads per CpG from the CpG calls of each alignment (--meth-pdr
 // FILE, --meth-pdr-min-cpg K: the CpG calls an alignment needs to be scored, default 4), and the methylation patterns of
 // the alignments over every window of four consecutive CpG sites, with methylation entropy and epipolymorphism
-// (--meth-epialleles FILE).
+// (--meth-epialleles FILE), and the methylation haplotype load per region of --meth-regions or --meth-tiles
+// (--meth-mhl FILE).
 // Out of scope (errors out): SAM text input (broken in the reference too: it is opened as BAM), -q quality
 // trimming, -M other than TC.
 #include <cerrno>
@@ -52,6 +53,7 @@ struct Opts {
     std::string meth_pdr;                    // --meth-pdr FILE
     int meth_pdr_min_cpg = 0;                // --meth-pdr-min-cpg K (1..255); 0 = not given (4); -1 = out of range
     std::string meth_epialleles;             // --meth-epialleles FILE
+    std::string meth_mhl;                    // --meth-mhl FILE
     unsigned batch = 1u << 17;   // reads per GPU batch: small enough to keep the three host stages overlapped
     std::string gpus;            // -g: number of devices (default: all visible) or a comma list of device ids; output stays in input order
 };
@@ -109,7 +111,9 @@ void usage() {
            "                           both methylated and unmethylated CpG calls among those with enough CpG calls)\n"
            "       --meth-pdr-min-cpg <int>  with --meth-pdr: the CpG calls an alignment needs to count, 1..255 (default 4)\n"
            "       --meth-epialleles <str>  with --methratio: write the alignments' methylation patterns over every window of\n"
-           "                           four consecutive CpG sites, with methylation entropy and epipolymorphism\n\n");
+           "                           four consecutive CpG sites, with methylation entropy and epipolymorphism\n"
+           "       --meth-mhl <str>    with --methratio and --meth-regions or --meth-tiles: write the methylation haplotype\n"
+           "                           load (MHL, uMHL) per region\n\n");
     exit(1);
 }
 
@@ -168,6 +172,7 @@ int get_options(int argc, char **argv, Opts &o) {
             }
             else if (a == "meth-pdr" && i + 1 < argc) o.meth_pdr = argv[++i];
             else if (a == "meth-epialleles" && i + 1 < argc) o.meth_epialleles = argv[++i];
+            else if (a == "meth-mhl" && i + 1 < argc) o.meth_mhl = argv[++i];
             else if (a == "meth-pdr-min-cpg" && i + 1 < argc) {
                 const char *v = argv[++i]; char *e; const long x = strtol(v, &e, 10);
                 o.meth_pdr_min_cpg = (*e || e == v || x < 1 || x > 255) ? -1 : (int)x;
@@ -332,11 +337,14 @@ extern "C" int bsx_cli_main(int argc, char **argv) {
     if (o.meth_out.empty() && (o.meth_conv >= 0 || !o.meth_conv_report.empty())) {
         fprintf(stderr, "--meth-conversion-filter and --meth-conversion-report need --methratio\n"); return 1; }
     if (!o.meth_conv_report.empty() && o.meth_conv < 0) o.meth_conv = 0;
+    if (o.meth_out.empty() && !o.meth_mhl.empty()) { fprintf(stderr, "--meth-mhl needs --methratio\n"); return 2; }
+    if (!o.meth_mhl.empty() && o.meth_regions.empty() && !o.meth_tiles) { fprintf(stderr, "--meth-mhl needs --meth-regions BED or --meth-tiles W\n"); return 2; }
     const bool region_opts = !o.meth_region_report.empty() || !o.meth_regions.empty() || o.meth_tiles;
     if (o.meth_out.empty() && region_opts) { fprintf(stderr, "--meth-region-report, --meth-regions and --meth-tiles need --methratio\n"); return 1; }
     if (!o.meth_regions.empty() && o.meth_tiles) { fprintf(stderr, "--meth-regions and --meth-tiles exclude each other\n"); return 1; }
-    if (region_opts && o.meth_region_report.empty()) { fprintf(stderr, "--meth-regions / --meth-tiles need --meth-region-report FILE\n"); return 1; }
-    if (region_opts && o.meth_regions.empty() && !o.meth_tiles) { fprintf(stderr, "--meth-region-report needs --meth-regions BED or --meth-tiles W\n"); return 1; }
+    if (region_opts && o.meth_region_report.empty() && o.meth_mhl.empty()) {
+        fprintf(stderr, "--meth-regions / --meth-tiles need --meth-region-report FILE or --meth-mhl FILE\n"); return 1; }
+    if (!o.meth_region_report.empty() && o.meth_regions.empty() && !o.meth_tiles) { fprintf(stderr, "--meth-region-report needs --meth-regions BED or --meth-tiles W\n"); return 1; }
     if (o.meth_pdr_min_cpg < 0) { fprintf(stderr, "--meth-pdr-min-cpg: expected an integer 1..255\n"); return 2; }
     if (o.meth_pdr_min_cpg && o.meth_pdr.empty()) { fprintf(stderr, "--meth-pdr-min-cpg needs --meth-pdr FILE\n"); return 2; }
     if (o.meth_out.empty() && !o.meth_pdr.empty()) { fprintf(stderr, "--meth-pdr needs --methratio\n"); return 2; }
@@ -449,6 +457,7 @@ extern "C" int bsx_cli_main(int argc, char **argv) {
             (o.meth_conv >= 0 && bsx_meth_enable_conversion_filter(mh, o.meth_conv) != BSX_OK) ||
             (!o.meth_pdr.empty() && bsx_meth_enable_pdr(mh, o.meth_pdr_min_cpg) != BSX_OK) ||
             (!o.meth_epialleles.empty() && bsx_meth_enable_epialleles(mh) != BSX_OK) ||
+            (!o.meth_mhl.empty() && bsx_meth_enable_mhl(mh) != BSX_OK) ||
             bsx_mapper_attach_meth(mp, mh, &o.mo, (p.out_sam || no_text) ? 1 : 0) != BSX_OK) {
             fprintf(stderr, "%s\n", bsx_last_error()); return 1; }
     }
@@ -608,6 +617,7 @@ extern "C" int bsx_cli_main(int argc, char **argv) {
         if (!o.meth_pdr.empty() && bsx_meth_write_pdr_file(mh, &o.mo, sp.data(), ln.data(), nullptr, threads, o.meth_pdr.c_str()) != BSX_OK) return 1;
         if (!o.meth_epialleles.empty() &&
             bsx_meth_write_epialleles_file(mh, &o.mo, sp.data(), ln.data(), nullptr, threads, o.meth_epialleles.c_str()) != BSX_OK) return 1;
+        if (!o.meth_mhl.empty() && bsx_meth_write_mhl_file(mh, &o.mo, regions, o.meth_mhl.c_str()) != BSX_OK) return 1;
         if (!o.meth_region_report.empty() && bsx_meth_write_regions_file(mh, &o.mo, regions, o.meth_region_report.c_str()) != BSX_OK) return 1;
         if (timing) fprintf(stderr, "[bsx timing] methratio report %.3f s\n", now() - t);
         bsx_meth_destroy(mh);

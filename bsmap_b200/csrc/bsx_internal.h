@@ -127,6 +127,9 @@ int bsx_meth_write_pdr_file(bsx_meth *m, const bsx_meth_opts *o, const char *con
 // valid mappings span a 4-CpG window, W window patterns counted"; errors are printed (bsx_meth.cu)
 int bsx_meth_write_epialleles_file(bsx_meth *m, const bsx_meth_opts *o, const char *const *seqs, const uint32_t *lens, const uint8_t *chroms, int threads,
                                    const char *path);
+// the command lines' MHL output: bsx_meth_write_mhl over the regions to a new file at path, and on stderr "MHL: A of V
+// valid mappings carry a CpG call, C CpG calls in haplotypes"; errors are printed (bsx_meth.cu)
+int bsx_meth_write_mhl_file(bsx_meth *m, const bsx_meth_opts *o, const bsx_regions &rg, const char *path);
 // "no-action" / "correct" / "skip" -> BSX_CT_SNP_*, anything else 0 (bsx_meth.cu)
 int bsx_ct_snp_mode(const char *name);
 int bsx_inflate_file(const char *path, std::vector<char> &out);   // gzip / BGZF members -> bytes (bsx_reads.cpp)

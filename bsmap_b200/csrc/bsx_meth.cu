@@ -44,6 +44,13 @@
 // four walks its span again, 32 positions a step, with three ballots (site, call, methylated) and the last three sites'
 // bits carried from step to step in warp-uniform registers.  The lane whose call closes a fully called run of four adds
 // the pattern to the first site's row: one global atomic per window.
+//
+// Methylation haplotype load (bsx_meth_enable_mhl) rides on the same walk (the Epi instantiation, with EpiArgs::mhl
+// set; an alignment with one CpG call is walked): 48 u32 counters per site count, by run length capped at 16, the
+// alignments in which a run of called / methylated / unmethylated sites ends there.  A called lane's runs are the sites
+// since the step's last break below it, plus the warp-uniform carries when there is none; it adds to family 0 and to 1
+// or 2: two global atomics per call.  meth_mhl_region_kernel reduces them over regions: each region's rank range from
+// the index, chunks of MHL_CHUNK ranks per warp, lanes over (site, run length), and a suffix sum over the run lengths.
 #include <algorithm>
 #include <cmath>
 #include <cstdio>
@@ -87,6 +94,9 @@ struct bsx_meth {
     uint32_t *d_epi = nullptr;                        // 16 counters per site, by pattern; NULL = epialleles off
     unsigned long long *d_epi_count = nullptr;        // alignments with a window, windows counted
     uint64_t cpg_sites = 0;
+    // MHL: fixed before the first alignment is piled up
+    uint32_t *d_mhl = nullptr;                        // 48 counters per site, [family][run length - 1]; NULL = MHL off
+    unsigned long long *d_mhl_count = nullptr;        // alignments with a CpG call, CpG calls
 };
 
 namespace {
@@ -117,8 +127,10 @@ struct PdrArgs {
 // what the Epi instantiation needs beyond the Cycles one
 struct EpiArgs {
     const uint32_t *rank;                // per packed word: the CpG sites before it
-    uint32_t *counts;                    // 16 per site: the windows starting there, by pattern
+    uint32_t *counts;                    // 16 per site: the windows starting there, by pattern; NULL = MHL only
     unsigned long long *count;           // alignments with a window, windows counted
+    uint32_t *mhl;                       // 48 per site: runs ending there, [family][length - 1]; NULL = MHL off
+    unsigned long long *mhl_count;       // alignments with a CpG call, CpG calls
 };
 
 // Conv: the CTA's alignments by score, zeroed before and flushed (non-zero bins) after them.  At file scope, so that the
@@ -128,6 +140,8 @@ __shared__ uint32_t conv_hist[BSX_CONV_BINS];
 __shared__ uint32_t pdr_count[2];
 // Epi: the CTA's alignments with a window and its windows, zeroed and flushed the same way
 __shared__ uint32_t epi_count[2];
+// MHL (Epi with EpiArgs::mhl): the CTA's alignments with a CpG call and their calls, zeroed and flushed the same way
+__shared__ uint32_t mhl_count[2];
 
 __device__ __forceinline__ uint32_t ref_code(const uint32_t *refcat, uint32_t q) { return (refcat[q >> 4] >> (30 - 2 * (q & 15))) & 3u; }
 
@@ -151,11 +165,14 @@ __device__ __forceinline__ uint32_t cpg_rank(const uint32_t *__restrict__ refcat
 // three sites before the step (bit t: the (t + 1)-th latest), warp-uniform.  A called lane whose three previous sites are
 // called closes a window: its pattern is the four methylated bits, the earliest site the most significant, and its row
 // the earliest site's rank, so rank - 3.  Lane 0 counts the alignment and its windows in epi_count (shared).
+// MHL (ep.mhl): run[f] carries the length (capped at 16) of the run of family f (called, methylated, unmethylated) that
+// ends at the last site before the step; a called lane's run is the sites after the latest break below it in the step,
+// plus run[f] when there is none, plus itself.  ep.counts NULL: no windows.
 template <class GetC>
 __device__ __forceinline__ void epi_windows(const uint32_t *__restrict__ refcat, uint32_t base, int len, int start, int L, bool rev, int lo, int hi,
                                             bool first_minus, uint32_t match, char cm, char cc, int lane, GetC getc, const EpiArgs &ep) {
     const uint32_t want = 3u - match, below = (1u << lane) - 1u;
-    uint32_t c3 = 0u, m3 = 0u, mine = 0u;
+    uint32_t c3 = 0u, m3 = 0u, mine = 0u, run[3] = {0u, 0u, 0u}, ncalls = 0u;
     // the called / methylated bits of the three latest sites among `sites`, then those carried in
     auto last3 = [&](uint32_t sites, uint32_t calls, uint32_t meths, uint32_t &c, uint32_t &mm) {
         uint32_t cn = 0u, mn = 0u, t = 0u;
@@ -185,21 +202,44 @@ __device__ __forceinline__ void epi_windows(const uint32_t *__restrict__ refcat,
         }
         const uint32_t sites = __ballot_sync(0xffffffffu, site), calls = __ballot_sync(0xffffffffu, called), meths = __ballot_sync(0xffffffffu, is_m);
         if (!sites) continue;
+        const uint32_t good[3] = {calls, meths, calls & ~meths};   // MHL: the sites that continue each family's run
         if (called) {
-            uint32_t c, mm;
-            last3(sites & below, calls, meths, c, mm);
-            if (c == 7u) {
-                const uint32_t row = cpg_rank(refcat, ep.rank, first_minus ? q - 1u : q) - 3u;
-                atomicAdd(ep.counts + (size_t)row * 16 + ((mm << 1) | (is_m ? 1u : 0u)), 1u);
-                mine++;
+            uint32_t c = 0u, mm = 0u;
+            if (ep.counts) last3(sites & below, calls, meths, c, mm);
+            if (c == 7u || ep.mhl) {
+                const uint32_t rank = cpg_rank(refcat, ep.rank, first_minus ? q - 1u : q);
+                if (c == 7u) {
+                    atomicAdd(ep.counts + (size_t)(rank - 3u) * 16 + ((mm << 1) | (is_m ? 1u : 0u)), 1u);
+                    mine++;
+                }
+                if (ep.mhl) {
+#pragma unroll
+                    for (int t = 0; t < 2; t++) {
+                        const int f = t == 0 ? 0 : (is_m ? 1 : 2);
+                        const uint32_t mine_sites = sites & below, brk = mine_sites & ~good[f];
+                        const uint32_t len = 1u + (brk ? (uint32_t)__popc(mine_sites >> (31 - __clz(brk))) - 1u : (uint32_t)__popc(mine_sites) + run[f]);
+                        atomicAdd(ep.mhl + ((size_t)rank * 3 + f) * BSX_MHL_MAX_LEN + min(len, (uint32_t)BSX_MHL_MAX_LEN) - 1u, 1u);
+                    }
+                }
             }
         }
-        uint32_t c, mm;
-        last3(sites, calls, meths, c, mm);
-        c3 = c; m3 = mm;
+        if (ep.counts) {
+            uint32_t c, mm;
+            last3(sites, calls, meths, c, mm);
+            c3 = c; m3 = mm;
+        }
+        if (ep.mhl) {
+#pragma unroll
+            for (int f = 0; f < 3; f++) {
+                const uint32_t brk = sites & ~good[f];
+                run[f] = min(brk ? (uint32_t)__popc(sites >> (31 - __clz(brk))) - 1u : run[f] + (uint32_t)__popc(sites), (uint32_t)BSX_MHL_MAX_LEN);
+            }
+            ncalls += (uint32_t)__popc(calls);
+        }
     }
     mine = __reduce_add_sync(0xffffffffu, mine);
     if (lane == 0 && mine) { atomicAdd(&epi_count[0], 1u); atomicAdd(&epi_count[1], mine); }
+    if (lane == 0 && ncalls) { atomicAdd(&mhl_count[0], 1u); atomicAdd(&mhl_count[1], ncalls); }
 }
 
 // One alignment, executed by a warp: get_alignment's trimming (methratio.py:56-64), the bounds test (105) and the
@@ -213,8 +253,9 @@ __device__ __forceinline__ void epi_windows(const uint32_t *__restrict__ refcat,
 // Pdr (with Cycles): the first pass also counts the methylated (pm) and unmethylated (pu) CpG calls; when the alignment is
 // kept and pm + pu >= pd.min_cpg, the second pass adds each CpG call to pd.concordant (pm == 0 or pu == 0) or
 // pd.discordant, and lane 0 counts the alignment in pdr_count (shared).
-// Epi (with Cycles): the first pass also counts the CpG calls; with BSX_EPI_CPGS or more, a third pass (epi_windows)
-// adds every fully called window of four consecutive sites to ep.counts.
+// Epi (with Cycles): the first pass also counts the CpG calls; with BSX_EPI_CPGS or more (MHL: one or more), a third
+// pass (epi_windows) adds every fully called window of four consecutive sites to ep.counts and, with MHL, every call's
+// runs to ep.mhl.
 template <bool Cycles, bool Snp, bool Conv, bool Pdr, bool Epi, class GetC>
 __device__ __forceinline__ void pile_alignment(const uint32_t *__restrict__ refcat, const uint32_t *__restrict__ seqinfo, uint32_t n_seq,
                                                uint32_t *meth, uint32_t *depth, unsigned long long *n_valid, const bsx_meth_opts &o,
@@ -267,7 +308,7 @@ __device__ __forceinline__ void pile_alignment(const uint32_t *__restrict__ refc
         const bool rev = ((st ^ (st >> 1)) & 1) != 0;
         const int lo = read2 ? mb.ignore[2] : mb.ignore[0], hi = L - (read2 ? mb.ignore[3] : mb.ignore[1]);
         uint32_t *pdr_to = nullptr;                          // Pdr: where the second pass adds the CpG calls; NULL = nowhere
-        bool epi_walk = false;                               // Epi: the alignment has enough CpG calls for a window
+        bool epi_walk = false;                               // Epi: the alignment has enough CpG calls for a window (MHL: one)
         if constexpr (Conv || Pdr || Epi) {
             // the score: a methylated call (read C on '+', G on '-') inside the cycle bounds whose next base on the call's
             // strand is not the CpG partner (CHG and CHH alike, so the second context code is not needed).  The bounds
@@ -307,7 +348,7 @@ __device__ __forceinline__ void pile_alignment(const uint32_t *__restrict__ refc
                     if (lane == 0) { atomicAdd(&pdr_count[0], 1u); if (disc) atomicAdd(&pdr_count[1], 1u); }
                 }
             }
-            if constexpr (Epi) epi_walk = (Pdr ? pm + pu : __reduce_add_sync(0xffffffffu, pm + pu)) >= (uint32_t)BSX_EPI_CPGS;
+            if constexpr (Epi) epi_walk = (Pdr ? pm + pu : __reduce_add_sync(0xffffffffu, pm + pu)) >= (ep.mhl ? 1u : (uint32_t)BSX_EPI_CPGS);
         }
         uint32_t *h = hist + read2 * (3 * BSX_MBIAS_CYCLES * 2);
         for (int i = lane; i < (int)len; i += 32) {
@@ -448,11 +489,13 @@ __global__ void __launch_bounds__(256, (Conv || Pdr || Epi) ? 4 : 0) meth_pileup
         if constexpr (Conv) hist_zero<BSX_CONV_BINS>(conv_hist, cv.hist);
         if constexpr (Pdr) hist_zero<2>(pdr_count, pd.count);
         if constexpr (Epi) hist_zero<2>(epi_count, ep.count);
+        if constexpr (Epi) hist_zero<2>(mhl_count, ep.mhl_count);
         for (uint32_t a = w; a < n; a += (gridDim.x * blockDim.x) >> 5) one(a, hist);
         hist_flush<MBIAS_BINS>(hist, mb.hist);
         if constexpr (Conv) hist_flush<BSX_CONV_BINS>(conv_hist, cv.hist);
         if constexpr (Pdr) hist_flush<2>(pdr_count, pd.count);
         if constexpr (Epi) hist_flush<2>(epi_count, ep.count);
+        if constexpr (Epi) hist_flush<2>(mhl_count, ep.mhl_count);
     }
 }
 
@@ -555,11 +598,13 @@ __global__ void __launch_bounds__(256, (Conv || Pdr || Epi) ? 4 : 0) meth_pileup
         if constexpr (Conv) hist_zero<BSX_CONV_BINS>(conv_hist, cv.hist);
         if constexpr (Pdr) hist_zero<2>(pdr_count, pd.count);
         if constexpr (Epi) hist_zero<2>(epi_count, ep.count);
+        if constexpr (Epi) hist_zero<2>(mhl_count, ep.mhl_count);
         for (uint32_t u = w; u < n * (uint32_t)mates; u += (gridDim.x * blockDim.x) >> 5) one(u, hist);
         hist_flush<MBIAS_BINS>(hist, mb.hist);
         if constexpr (Conv) hist_flush<BSX_CONV_BINS>(conv_hist, cv.hist);
         if constexpr (Pdr) hist_flush<2>(pdr_count, pd.count);
         if constexpr (Epi) hist_flush<2>(epi_count, ep.count);
+        if constexpr (Epi) hist_flush<2>(mhl_count, ep.mhl_count);
     }
 }
 
@@ -683,6 +728,96 @@ auto region_kernel_of(bool combine, int snp_mode) {
 }
 auto region_kernel(bool combine, int snp_mode, bool pdr) { return pdr ? region_kernel_of<true>(combine, snp_mode) : region_kernel_of<false>(combine, snp_mode); }
 
+// MHL's region reduction (bsx_meth_regions_mhl).  A region's sites are a rank range [a, b); it is cut into chunks of
+// MHL_CHUNK ranks, and scan[r] is the exclusive sum of chunks over the regions before r, as for meth_region_kernel.  A
+// slice of regions takes 48 u64 sums each, so it holds a quarter of REGION_SLICE's regions (96 MB of sums again).
+constexpr uint32_t MHL_CHUNK = 256;
+constexpr uint64_t MHL_SLICE = REGION_SLICE / 4;
+
+// the rank of the first site at or after position c (c may be the end of the packed reference: then no word is read)
+__device__ __forceinline__ uint32_t cpg_rank_at(const uint32_t *__restrict__ refcat, const uint32_t *__restrict__ rank, uint32_t c) {
+    return (c & 15u) ? cpg_rank(refcat, rank, c) : __ldg(rank + (c >> 4));
+}
+
+// one thread per region: its rank range from its clipped positions, and its chunks (chunks[n] = 0 ends the scan)
+__global__ void __launch_bounds__(256) mhl_span_kernel(const uint32_t *__restrict__ refcat, const uint32_t *__restrict__ rank,
+                                                       const uint2 *__restrict__ pos, uint32_t n, uint2 *span, uint32_t *chunks) {
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i > n) return;
+    if (i == n) { chunks[n] = 0u; return; }
+    const uint2 p = pos[i];
+    const uint32_t a = cpg_rank_at(refcat, rank, p.x), b = cpg_rank_at(refcat, rank, p.y);
+    span[i] = make_uint2(a, b);
+    chunks[i] = (b - a + MHL_CHUNK - 1) / MHL_CHUNK;
+}
+
+// the SNP modes' cut sites: bit s of cut set when site s has SNP evidence (snp > 0) at its C or its G.  One thread per
+// packed word; its sites, in ascending rank.
+__global__ void __launch_bounds__(256) mhl_cut_kernel(const uint32_t *__restrict__ refcat, uint64_t n_words, const uint32_t *__restrict__ rank,
+                                                      const uint32_t *__restrict__ snp, uint32_t *cut) {
+    const uint64_t a = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (a >= n_words) return;
+    uint32_t s = cpg_mask(refcat[a], a + 1 < n_words ? refcat[a + 1] : 0u), r = rank[a];
+    while (s) {
+        const int b = 31 - __clz(s);
+        s &= ~(1u << b);
+        const uint64_t c = a * 16 + (uint64_t)((30 - b) >> 1);
+        if (snp[c] || snp[c + 1]) atomicOr(cut + (r >> 5), 1u << (r & 31u));
+        r++;
+    }
+}
+
+// One warp per chunk (a grid-stride loop of them), two sites a step: lanes 0-15 take site s, 16-31 site s + 1, lane
+// l - 1 of each half the run length r = l.  Per family, the half's 16 counters are summed over r >= l (a suffix sum by
+// shuffles; in u32, as it is bounded by the alignments with a call at the site, which the u32 depth counter also
+// counts), and added to the lane's T_l / M_l / U_l while l <= lim: the region's sites up to s and, with cuts, those
+// since the last cut (0 at a cut site), capped at 16, carried warp-uniformly from site to site.  The halves are added
+// and lanes 0-15 add the 48 sums to out[(r * 3 + f) * 16 + l - 1] (u64 atomics: exact and independent of the schedule).
+__global__ void __launch_bounds__(256) meth_mhl_region_kernel(const uint32_t *__restrict__ counts, const uint32_t *__restrict__ cut,
+                                                              const uint32_t *__restrict__ scan, const uint2 *__restrict__ span, uint32_t n,
+                                                              unsigned long long *out) {
+    const int lane = threadIdx.x & 31, half = lane >> 4, l1 = lane & 15;
+    const uint32_t total = scan[n], warps = (gridDim.x * blockDim.x) >> 5;
+    auto is_cut = [&](uint32_t s) { return cut && ((__ldg(cut + (s >> 5)) >> (s & 31u)) & 1u); };
+    for (uint32_t c = (blockIdx.x * blockDim.x + threadIdx.x) >> 5; c < total; c += warps) {
+        uint32_t lo = 0, hi = n;                                // the chunk's region, as in meth_region_kernel
+        while (hi - lo > 1) {
+            const uint32_t step = (hi - lo + 31) / 32, idx = lo + (uint32_t)lane * step;
+            const unsigned ball = __ballot_sync(0xffffffffu, idx < hi && scan[idx] <= c);
+            lo += (uint32_t)(31 - __clz(ball)) * step;
+            hi = min(hi, lo + step);
+        }
+        const uint2 sp = span[lo];
+        const uint32_t b = sp.x + (c - scan[lo]) * MHL_CHUNK, e = min(b + MHL_CHUNK, sp.y);
+        uint32_t run = min(b - sp.x, (uint32_t)BSX_MHL_MAX_LEN);  // lim of site b - 1
+        for (uint32_t t = 1; t <= run; t++) if (is_cut(b - t)) { run = t - 1; break; }
+        unsigned long long acc[3] = {0ull, 0ull, 0ull};
+        for (uint32_t s0 = b; s0 < e; s0 += 2) {
+            const uint32_t r0 = is_cut(s0) ? 0u : min(run + 1u, (uint32_t)BSX_MHL_MAX_LEN);
+            const bool two = s0 + 1 < e;
+            const uint32_t r1 = (!two || is_cut(s0 + 1)) ? 0u : min(r0 + 1u, (uint32_t)BSX_MHL_MAX_LEN);
+            run = two ? r1 : r0;
+            const uint32_t lim = half ? r1 : r0;
+            const uint32_t *row = counts + (size_t)(s0 + (uint32_t)half) * (3 * BSX_MHL_MAX_LEN) + l1;
+#pragma unroll
+            for (int f = 0; f < 3; f++) {
+                uint32_t v = lim ? __ldg(row + f * BSX_MHL_MAX_LEN) : 0u;
+#pragma unroll
+                for (int o = 1; o < 16; o <<= 1) {
+                    const uint32_t y = __shfl_down_sync(0xffffffffu, v, o, 16);
+                    if (l1 + o < 16) v += y;
+                }
+                if ((uint32_t)l1 < lim) acc[f] += v;
+            }
+        }
+#pragma unroll
+        for (int f = 0; f < 3; f++) {
+            acc[f] += __shfl_xor_sync(0xffffffffu, acc[f], 16);
+            if (lane < 16 && acc[f]) atomicAdd(out + ((size_t)lo * 3 + f) * BSX_MHL_MAX_LEN + l1, acc[f]);
+        }
+    }
+}
+
 // Epi's rank index, first step: the CpG sites of each packed word (x[n_words] = 0, so that the scan ends in the total)
 __global__ void __launch_bounds__(256) cpg_count_kernel(const uint32_t *__restrict__ refcat, uint64_t n_words, uint32_t *x) {
     const uint64_t a = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -739,6 +874,24 @@ int scan_exclusive(uint32_t *x, uint64_t n) {
     return rc;
 }
 
+// the CpG rank index, built once for epialleles and MHL; `what` names the option in messages
+int ensure_cpg_rank(bsx_meth *m, const char *what) {
+    if (m->d_cpg_rank) return BSX_OK;
+    const uint64_t nw = m->ix->n_words;
+    if (cudaMalloc(&m->d_cpg_rank, (nw + 1) * 4) != cudaSuccess) {
+        cudaGetLastError(); m->d_cpg_rank = nullptr;
+        bsx_set_error("%s: out of device memory (%llu bytes for the CpG rank index)", what, (unsigned long long)(nw + 1) * 4); return BSX_ERR_CUDA; }
+    auto undo = [m]() { cudaFree(m->d_cpg_rank); m->d_cpg_rank = nullptr; };
+    cpg_count_kernel<<<(unsigned)((nw + 1 + 255) / 256), 256>>>(m->ix->d_refcat, nw, m->d_cpg_rank);
+    if (cudaGetLastError() != cudaSuccess) { undo(); bsx_set_error("%s: CpG count kernel failed", what); return BSX_ERR_CUDA; }
+    const int rc = scan_exclusive(m->d_cpg_rank, nw + 1);
+    if (rc) { undo(); return rc; }
+    uint32_t sites = 0;
+    if (cudaMemcpy(&sites, m->d_cpg_rank + nw, 4, cudaMemcpyDeviceToHost) != cudaSuccess) { cudaGetLastError(); undo(); bsx_set_error("%s: rank index download failed", what); return BSX_ERR_CUDA; }
+    m->cpg_sites = sites;
+    return BSX_OK;
+}
+
 int ensure_staging(bsx_meth *m, size_t n, uint32_t stride) {
     if (n <= m->cap && stride <= m->stride) return BSX_OK;
     cudaFree(m->d_seq); cudaFree(m->d_len); cudaFree(m->d_chr); cudaFree(m->d_pos); cudaFree(m->d_strand); cudaFree(m->d_flags); cudaFree(m->d_ins); cudaFree(m->d_mate);
@@ -790,11 +943,13 @@ auto mapped_kernel(bool cycles, bool snp, bool conv, bool pdr, bool epi) {
                   : (snp ? meth_pileup_mapped_kernel<false, true, false, false, false> : meth_pileup_mapped_kernel<false, false, false, false, false>);
 }
 
-// the Cycles kernels run for M-bias, exclusion, the conversion filter, PDR or epialleles (with M-bias and exclusion off,
+// the Cycles kernels run for M-bias, exclusion, the conversion filter, PDR, epialleles or MHL (with M-bias and exclusion off,
 // Cycles is the classification alone: no histogram, bounds [0, L))
 bool cycles_on(const bsx_meth *m) {
-    return m->mbias || m->ignore[0] || m->ignore[1] || m->ignore[2] || m->ignore[3] || m->d_conv || m->d_pdr || m->d_epi;
+    return m->mbias || m->ignore[0] || m->ignore[1] || m->ignore[2] || m->ignore[3] || m->d_conv || m->d_pdr || m->d_epi || m->d_mhl;
 }
+// the Epi instantiation serves epialleles, MHL or both
+bool epi_on(const bsx_meth *m) { return m->d_epi || m->d_mhl; }
 
 // the Cycles kernels' grid cap and, with M-bias on, their histogram (zeroed), on the first pile-up that needs them
 int ensure_cycles(bsx_meth *m) {
@@ -806,8 +961,8 @@ int ensure_cycles(bsx_meth *m) {
     int dev = 0, sms = 0, per_sm[2] = {0, 0};
     BSX_CUDA_CHECK(cudaGetDevice(&dev));
     BSX_CUDA_CHECK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
-    BSX_CUDA_CHECK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm[0], text_kernel(true, m->ct_snp != 0, m->d_conv != nullptr, m->d_pdr != nullptr, m->d_epi != nullptr), 256, 0));
-    BSX_CUDA_CHECK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm[1], mapped_kernel(true, m->ct_snp != 0, m->d_conv != nullptr, m->d_pdr != nullptr, m->d_epi != nullptr), 256, 0));
+    BSX_CUDA_CHECK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm[0], text_kernel(true, m->ct_snp != 0, m->d_conv != nullptr, m->d_pdr != nullptr, epi_on(m)), 256, 0));
+    BSX_CUDA_CHECK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm[1], mapped_kernel(true, m->ct_snp != 0, m->d_conv != nullptr, m->d_pdr != nullptr, epi_on(m)), 256, 0));
     for (int i = 0; i < 2; i++) m->resident[i] = std::max(per_sm[i], 1) * sms;
     BSX_CUDA_CHECK(cudaDeviceSynchronize());
     return BSX_OK;
@@ -820,7 +975,7 @@ MbiasArgs mbias_args(const bsx_meth *m, int readset) {
 }
 ConvArgs conv_args(const bsx_meth *m) { return ConvArgs{m->d_conv, (uint32_t)m->conv_threshold}; }
 PdrArgs pdr_args(const bsx_meth *m) { return PdrArgs{m->d_conc, m->d_disc, m->d_pdr, m->pdr_min_cpg}; }
-EpiArgs epi_args(const bsx_meth *m) { return EpiArgs{m->d_cpg_rank, m->d_epi, m->d_epi_count}; }
+EpiArgs epi_args(const bsx_meth *m) { return EpiArgs{m->d_cpg_rank, m->d_epi, m->d_epi_count, m->d_mhl, m->d_mhl_count}; }
 
 int combine_once(bsx_meth *m, const bsx_meth_opts *o) {
     if (!o->combine_cpg || m->combined) return BSX_OK;
@@ -872,6 +1027,7 @@ extern "C" int bsx_meth_destroy(bsx_meth *m) {
     if (!m) return BSX_OK;
     cudaFree(m->d_meth); cudaFree(m->d_depth); cudaFree(m->d_valid); cudaFree(m->d_first); cudaFree(m->d_mbias); cudaFree(m->d_confirm); cudaFree(m->d_snp); cudaFree(m->d_conv);
     cudaFree(m->d_conc); cudaFree(m->d_disc); cudaFree(m->d_pdr); cudaFree(m->d_cpg_rank); cudaFree(m->d_epi); cudaFree(m->d_epi_count);
+    cudaFree(m->d_mhl); cudaFree(m->d_mhl_count);
     if (m->dup_order) cudaEventDestroy(m->dup_order);
     cudaFree(m->d_seq); cudaFree(m->d_len); cudaFree(m->d_chr); cudaFree(m->d_pos); cudaFree(m->d_strand); cudaFree(m->d_flags); cudaFree(m->d_ins); cudaFree(m->d_mate);
     delete m;
@@ -904,7 +1060,7 @@ extern "C" int bsx_meth_add(bsx_meth *m, const bsx_meth_opts *o, uint32_t n, con
         const unsigned blocks = (unsigned)(((uint64_t)n * 32 + 255) / 256);
         const bool cyc = cycles_on(m);
         if (cyc) { rc = ensure_cycles(m); if (rc) return rc; }
-        text_kernel(cyc, m->ct_snp != 0, m->d_conv != nullptr, m->d_pdr != nullptr, m->d_epi != nullptr)<<<cyc ? std::min<unsigned>(blocks, (unsigned)m->resident[0]) : blocks, 256>>>(
+        text_kernel(cyc, m->ct_snp != 0, m->d_conv != nullptr, m->d_pdr != nullptr, epi_on(m))<<<cyc ? std::min<unsigned>(blocks, (unsigned)m->resident[0]) : blocks, 256>>>(
             m->ix->d_refcat, m->ix->d_seqinfo, m->ix->n_seq, m->d_meth, m->d_depth, m->d_valid, o->rm_dup ? m->d_first : nullptr, *o, n, m->d_seq,
             m->stride, m->d_len, m->d_chr, m->d_pos, m->d_strand, m->d_ins, m->d_mate, m->d_flags, cyc ? mbias_args(m, 0) : MbiasArgs{}, m->d_confirm, m->d_snp,
             conv_args(m), pdr_args(m), epi_args(m));
@@ -938,7 +1094,7 @@ int bsx_meth_pile_mapped(bsx_meth *m, const bsx_meth_opts *o, int sam, int repor
         BSX_CUDA_CHECK(cudaGetLastError());
     }
     const unsigned blocks = (unsigned)(((uint64_t)n * (uint64_t)mates * 32 + 255) / 256);
-    mapped_kernel(cyc, m->ct_snp != 0, m->d_conv != nullptr, m->d_pdr != nullptr, m->d_epi != nullptr)<<<cyc ? std::min<unsigned>(blocks, (unsigned)m->resident[1]) : blocks, 256, 0, st>>>(
+    mapped_kernel(cyc, m->ct_snp != 0, m->d_conv != nullptr, m->d_pdr != nullptr, epi_on(m))<<<cyc ? std::min<unsigned>(blocks, (unsigned)m->resident[1]) : blocks, 256, 0, st>>>(
         m->ix->d_refcat, m->ix->d_seqinfo, m->ix->n_seq, m->d_meth, m->d_depth, m->d_valid, o->rm_dup ? m->d_first : nullptr, *o, sam,
         report_repeat_hits, n, mates, stride, seq_a, seq_b, out_a, out_b, out_pair, cyc ? mbias_args(m, readset) : MbiasArgs{}, m->d_confirm, m->d_snp,
         conv_args(m), pdr_args(m), epi_args(m));
@@ -1298,24 +1454,16 @@ extern "C" int bsx_meth_enable_epialleles(bsx_meth *m) {
     if (m->started) { bsx_set_error("bsx_meth_enable_epialleles: alignments were already piled up; enable epialleles first"); return BSX_ERR_ARG; }
     if (m->d_epi) { bsx_set_error("bsx_meth_enable_epialleles: epialleles are already enabled"); return BSX_ERR_ARG; }
     BSX_CUDA_CHECK(cudaSetDevice(m->ix->device));
-    const uint64_t nw = m->ix->n_words;
-    if (cudaMalloc(&m->d_cpg_rank, (nw + 1) * 4) != cudaSuccess) {
-        cudaGetLastError(); m->d_cpg_rank = nullptr;
-        bsx_set_error("epialleles: out of device memory (%llu bytes for the CpG rank index)", (unsigned long long)(nw + 1) * 4); return BSX_ERR_CUDA; }
-    auto undo = [m]() { cudaFree(m->d_cpg_rank); cudaFree(m->d_epi); cudaFree(m->d_epi_count); m->d_cpg_rank = m->d_epi = nullptr; m->d_epi_count = nullptr; };
-    cpg_count_kernel<<<(unsigned)((nw + 1 + 255) / 256), 256>>>(m->ix->d_refcat, nw, m->d_cpg_rank);
-    if (cudaGetLastError() != cudaSuccess) { undo(); bsx_set_error("epialleles: CpG count kernel failed"); return BSX_ERR_CUDA; }
-    const int rc = scan_exclusive(m->d_cpg_rank, nw + 1);
-    if (rc) { undo(); return rc; }
-    uint32_t sites = 0;
-    if (cudaMemcpy(&sites, m->d_cpg_rank + nw, 4, cudaMemcpyDeviceToHost) != cudaSuccess) { cudaGetLastError(); undo(); bsx_set_error("epialleles: rank index download failed"); return BSX_ERR_CUDA; }
-    const size_t bytes = (size_t)std::max<uint32_t>(sites, 1u) * 16 * sizeof(uint32_t);
+    const int rc = ensure_cpg_rank(m, "epialleles");
+    if (rc) return rc;
+    const uint64_t sites = m->cpg_sites;
+    auto undo = [m]() { cudaFree(m->d_epi); cudaFree(m->d_epi_count); m->d_epi = nullptr; m->d_epi_count = nullptr; };
+    const size_t bytes = (size_t)std::max<uint64_t>(sites, 1u) * 16 * sizeof(uint32_t);
     if (cudaMalloc(&m->d_epi, bytes) != cudaSuccess || cudaMalloc(&m->d_epi_count, 2 * sizeof(unsigned long long)) != cudaSuccess) {
         cudaGetLastError(); undo();
-        bsx_set_error("epialleles: out of device memory (%zu bytes for the pattern counters of %u CpG sites)", bytes, sites); return BSX_ERR_CUDA; }
+        bsx_set_error("epialleles: out of device memory (%zu bytes for the pattern counters of %llu CpG sites)", bytes, (unsigned long long)sites); return BSX_ERR_CUDA; }
     if (cudaMemset(m->d_epi, 0, bytes) != cudaSuccess || cudaMemset(m->d_epi_count, 0, 2 * sizeof(unsigned long long)) != cudaSuccess) {
         cudaGetLastError(); undo(); bsx_set_error("epialleles: cudaMemset failed"); return BSX_ERR_CUDA; }
-    m->cpg_sites = sites;
     return BSX_OK;
 }
 
@@ -1350,7 +1498,7 @@ static int epi_sites(bsx_meth *m, uint32_t k, std::vector<uint32_t> *pos, uint64
 
 extern "C" int bsx_meth_cpg_sites(bsx_meth *m, uint32_t k, uint64_t *n) {
     if (!m || !n || k >= m->ix->n_seq) { bsx_set_error("bsx_meth_cpg_sites: bad argument"); return BSX_ERR_ARG; }
-    if (!m->d_epi) { bsx_set_error("bsx_meth_cpg_sites: epialleles were not enabled (bsx_meth_enable_epialleles)"); return BSX_ERR_ARG; }
+    if (!m->d_cpg_rank) { bsx_set_error("bsx_meth_cpg_sites: epialleles or MHL were not enabled (bsx_meth_enable_epialleles, bsx_meth_enable_mhl)"); return BSX_ERR_ARG; }
     BSX_CUDA_CHECK(cudaSetDevice(m->ix->device));
     uint64_t r0 = 0;
     return epi_sites(m, k, nullptr, n, &r0);
@@ -1458,6 +1606,170 @@ int bsx_meth_write_epialleles_file(bsx_meth *m, const bsx_meth_opts *o, const ch
     if (bsx_meth_epialleles(m, &spanning, &windows) != BSX_OK || bsx_meth_valid_count(m, &valid) != BSX_OK) { fprintf(stderr, "%s\n", bsx_last_error()); return BSX_ERR_CUDA; }
     fprintf(stderr, "epialleles: %llu of %llu valid mappings span a %d-CpG window, %llu window patterns counted\n", (unsigned long long)spanning,
             (unsigned long long)valid, BSX_EPI_CPGS, (unsigned long long)windows);
+    return BSX_OK;
+}
+
+extern "C" int bsx_meth_enable_mhl(bsx_meth *m) {
+    if (!m) { bsx_set_error("bsx_meth_enable_mhl: bad argument"); return BSX_ERR_ARG; }
+    if (m->started) { bsx_set_error("bsx_meth_enable_mhl: alignments were already piled up; enable MHL first"); return BSX_ERR_ARG; }
+    if (m->d_mhl) { bsx_set_error("bsx_meth_enable_mhl: MHL is already enabled"); return BSX_ERR_ARG; }
+    BSX_CUDA_CHECK(cudaSetDevice(m->ix->device));
+    const int rc = ensure_cpg_rank(m, "MHL");
+    if (rc) return rc;
+    auto undo = [m]() { cudaFree(m->d_mhl); cudaFree(m->d_mhl_count); m->d_mhl = nullptr; m->d_mhl_count = nullptr; };
+    const size_t bytes = (size_t)std::max<uint64_t>(m->cpg_sites, 1u) * 3 * BSX_MHL_MAX_LEN * sizeof(uint32_t);
+    if (cudaMalloc(&m->d_mhl, bytes) != cudaSuccess || cudaMalloc(&m->d_mhl_count, 2 * sizeof(unsigned long long)) != cudaSuccess) {
+        cudaGetLastError(); undo();
+        bsx_set_error("MHL: out of device memory (%zu bytes for the run counters of %llu CpG sites)", bytes, (unsigned long long)m->cpg_sites); return BSX_ERR_CUDA; }
+    if (cudaMemset(m->d_mhl, 0, bytes) != cudaSuccess || cudaMemset(m->d_mhl_count, 0, 2 * sizeof(unsigned long long)) != cudaSuccess) {
+        cudaGetLastError(); undo(); bsx_set_error("MHL: cudaMemset failed"); return BSX_ERR_CUDA; }
+    return BSX_OK;
+}
+
+extern "C" int bsx_meth_download_mhl(bsx_meth *m, uint32_t k, uint32_t *site_pos, uint32_t *counts) {
+    if (!m || k >= m->ix->n_seq) { bsx_set_error("bsx_meth_download_mhl: bad argument"); return BSX_ERR_ARG; }
+    if (!m->d_mhl) { bsx_set_error("bsx_meth_download_mhl: MHL was not enabled (bsx_meth_enable_mhl)"); return BSX_ERR_ARG; }
+    BSX_CUDA_CHECK(cudaSetDevice(m->ix->device));
+    BSX_CUDA_CHECK(cudaDeviceSynchronize());           // in-process batches pile up from two streams
+    std::vector<uint32_t> pos;
+    uint64_t n = 0, r0 = 0;
+    int rc = epi_sites(m, k, &pos, &n, &r0); if (rc) return rc;
+    if (site_pos && n) memcpy(site_pos, pos.data(), n * 4);
+    if (counts && n) BSX_CUDA_CHECK(cudaMemcpy(counts, m->d_mhl + r0 * 3 * BSX_MHL_MAX_LEN, n * 3 * BSX_MHL_MAX_LEN * 4, cudaMemcpyDeviceToHost));
+    return BSX_OK;
+}
+
+extern "C" int bsx_meth_mhl(bsx_meth *m, uint64_t *alignments, uint64_t *calls) {
+    if (!m) { bsx_set_error("bsx_meth_mhl: bad argument"); return BSX_ERR_ARG; }
+    if (!m->d_mhl) { bsx_set_error("bsx_meth_mhl: MHL was not enabled (bsx_meth_enable_mhl)"); return BSX_ERR_ARG; }
+    BSX_CUDA_CHECK(cudaSetDevice(m->ix->device));
+    BSX_CUDA_CHECK(cudaDeviceSynchronize());           // in-process batches flush from two streams
+    unsigned long long h[2];
+    BSX_CUDA_CHECK(cudaMemcpy(h, m->d_mhl_count, sizeof h, cudaMemcpyDeviceToHost));
+    if (alignments) *alignments = h[0];
+    if (calls) *calls = h[1];
+    return BSX_OK;
+}
+
+extern "C" int bsx_meth_regions_mhl(bsx_meth *m, const bsx_meth_opts *o, uint64_t n, const uint32_t *seq, const uint64_t *start, const uint64_t *end,
+                                    uint64_t *sites, uint64_t *out) {
+    if (!m || !o || (n && (!seq || !start || !end || !sites || !out))) { bsx_set_error("bsx_meth_regions_mhl: bad argument"); return BSX_ERR_ARG; }
+    if (!m->d_mhl) { bsx_set_error("bsx_meth_regions_mhl: MHL was not enabled (bsx_meth_enable_mhl)"); return BSX_ERR_ARG; }
+    const bsx_index *ix = m->ix;
+    for (uint64_t r = 0; r < n; r++) {
+        if (seq[r] >= ix->n_seq) { bsx_set_error("bsx_meth_regions_mhl: region %llu: sequence %u of %u", (unsigned long long)r, seq[r], ix->n_seq); return BSX_ERR_ARG; }
+        if (start[r] > end[r]) { bsx_set_error("bsx_meth_regions_mhl: region %llu: start %llu > end %llu", (unsigned long long)r, (unsigned long long)start[r],
+                                               (unsigned long long)end[r]); return BSX_ERR_ARG; }
+    }
+    BSX_CUDA_CHECK(cudaSetDevice(ix->device));
+    BSX_CUDA_CHECK(cudaDeviceSynchronize());           // in-process batches pile up on the mapper's streams
+    if (n == 0) return BSX_OK;
+    const uint64_t cap = std::min<uint64_t>(n, MHL_SLICE);
+    const bool cuts = m->ct_snp == BSX_CT_SNP_SKIP || m->ct_snp == BSX_CT_SNP_CORRECT;
+    const size_t cut_words = (size_t)((m->cpg_sites + 31) / 32) + 1;
+    uint32_t *d_chunks = nullptr, *d_cut = nullptr; uint2 *d_pos = nullptr, *d_span = nullptr; unsigned long long *d_out = nullptr;
+    if (cudaMalloc(&d_chunks, (cap + 1) * 4) != cudaSuccess || cudaMalloc(&d_pos, cap * 8) != cudaSuccess || cudaMalloc(&d_span, cap * 8) != cudaSuccess ||
+        cudaMalloc(&d_out, cap * 48 * 8) != cudaSuccess || (cuts && cudaMalloc(&d_cut, cut_words * 4) != cudaSuccess)) {
+        cudaGetLastError(); cudaFree(d_chunks); cudaFree(d_pos); cudaFree(d_span); cudaFree(d_out); cudaFree(d_cut);
+        bsx_set_error("bsx_meth_regions_mhl: out of device memory"); return BSX_ERR_CUDA; }
+    auto run = [&]() -> int {
+        if (cuts) {
+            BSX_CUDA_CHECK(cudaMemset(d_cut, 0, cut_words * 4));
+            mhl_cut_kernel<<<(unsigned)((ix->n_words + 255) / 256), 256>>>(ix->d_refcat, ix->n_words, m->d_cpg_rank, m->d_snp, d_cut);
+            BSX_CUDA_CHECK(cudaGetLastError());
+        }
+        int dev = 0, sms = 0, per_sm = 0;
+        BSX_CUDA_CHECK(cudaGetDevice(&dev));
+        BSX_CUDA_CHECK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+        BSX_CUDA_CHECK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, meth_mhl_region_kernel, 256, 0));
+        std::vector<uint2> pos, span;
+        for (uint64_t r0 = 0; r0 < n; r0 += cap) {
+            const uint32_t k = (uint32_t)std::min(cap, n - r0);
+            pos.resize(k); span.resize(k);
+            for (uint32_t i = 0; i < k; i++) {
+                const uint32_t sq = seq[r0 + i], len = ix->size[sq];
+                const uint64_t lo = std::min<uint64_t>(start[r0 + i], len), hi = std::min<uint64_t>(end[r0 + i], len);   // clipped to the sequence
+                pos[i] = make_uint2(ix->anchor[sq] + (uint32_t)lo, ix->anchor[sq] + (uint32_t)hi);
+            }
+            BSX_CUDA_CHECK(cudaMemcpy(d_pos, pos.data(), (size_t)k * 8, cudaMemcpyHostToDevice));
+            mhl_span_kernel<<<(k + 1 + 255) / 256, 256>>>(ix->d_refcat, m->d_cpg_rank, d_pos, k, d_span, d_chunks);
+            BSX_CUDA_CHECK(cudaGetLastError());
+            int rc = scan_exclusive(d_chunks, (uint64_t)k + 1); if (rc) return rc;
+            uint32_t total = 0;
+            BSX_CUDA_CHECK(cudaMemcpy(&total, d_chunks + k, 4, cudaMemcpyDeviceToHost));
+            BSX_CUDA_CHECK(cudaMemset(d_out, 0, (size_t)k * 48 * 8));
+            if (total) {
+                const unsigned blocks = (unsigned)std::min<unsigned long long>((total + 7) / 8, (unsigned long long)std::max(per_sm, 1) * (unsigned)sms);
+                meth_mhl_region_kernel<<<blocks, 256>>>(m->d_mhl, cuts ? d_cut : nullptr, d_chunks, d_span, k, d_out);
+                BSX_CUDA_CHECK(cudaGetLastError());
+            }
+            BSX_CUDA_CHECK(cudaMemcpy(out + r0 * 48, d_out, (size_t)k * 48 * 8, cudaMemcpyDeviceToHost));
+            BSX_CUDA_CHECK(cudaMemcpy(span.data(), d_span, (size_t)k * 8, cudaMemcpyDeviceToHost));
+            for (uint32_t i = 0; i < k; i++) sites[r0 + i] = span[i].y - span[i].x;
+        }
+        return BSX_OK;
+    };
+    const int err = run();
+    cudaFree(d_chunks); cudaFree(d_pos); cudaFree(d_span); cudaFree(d_out); cudaFree(d_cut);
+    return err;
+}
+
+extern "C" size_t bsx_meth_write_mhl(bsx_meth *m, const bsx_meth_opts *o, uint64_t n, const uint32_t *seq, const uint64_t *start,
+                                     const uint64_t *end, int fd) {
+    if (!m || !o || (n && (!seq || !start || !end))) { bsx_set_error("bsx_meth_write_mhl: bad argument"); return 0; }
+    if (!m->d_mhl) { bsx_set_error("bsx_meth_write_mhl: MHL was not enabled (bsx_meth_enable_mhl)"); return 0; }
+    const bsx_index *ix = m->ix;
+    const int threads = bsx_host_threads(0);
+    size_t written = 0;
+    auto put = [&](const std::string &s) {
+        size_t off = 0;
+        while (off < s.size()) { const ssize_t w = write(fd, s.data() + off, s.size() - off); if (w <= 0) return false; off += (size_t)w; written += (size_t)w; }
+        return true;
+    };
+    if (!put("chr\tstart\tend\tsites\tcalls\tL\tMHL\tuMHL\thaplotypes\tmethylated\tunmethylated\n")) return 0;
+    std::vector<uint64_t> sites, sums;
+    for (uint64_t r0 = 0; r0 < n; r0 += MHL_SLICE) {
+        const uint64_t k = std::min<uint64_t>(MHL_SLICE, n - r0);
+        sites.resize(k); sums.resize(k * 48);
+        if (bsx_meth_regions_mhl(m, o, k, seq + r0, start + r0, end + r0, sites.data(), sums.data()) != BSX_OK) return 0;
+        std::vector<std::string> chunk((size_t)threads);
+        bsx_parallel(threads, (size_t)k, [&](int t, size_t b, size_t e) {
+            Sink s{&chunk[t]};
+            for (size_t i = b; i < e; i++) {
+                const uint64_t *T = &sums[i * 48], *M = T + BSX_MHL_MAX_LEN, *U = M + BSX_MHL_MAX_LEN;
+                int L = 0;
+                for (int l = 1; l <= BSX_MHL_MAX_LEN; l++) if (T[l - 1]) L = l;
+                const std::string &name = ix->names[seq[r0 + i]];
+                s.put(name.data(), name.size()); s.putc('\t'); s.putu(start[r0 + i]); s.putc('\t'); s.putu(end[r0 + i]); s.putc('\t');
+                s.putu(sites[i]); s.putc('\t'); s.putu(T[0]); s.putc('\t'); s.putu((unsigned long long)L); s.putc('\t');
+                if (!L) { s.put("NA\tNA\tNA\tNA\tNA\n", 15); continue; }
+                // ascending l in double, as the oracle sums them
+                double hm = 0.0, hu = 0.0;
+                for (int l = 1; l <= L; l++) { hm += (double)((uint64_t)l * M[l - 1]) / (double)T[l - 1]; hu += (double)((uint64_t)l * U[l - 1]) / (double)T[l - 1]; }
+                const double w = (double)(L * (L + 1) / 2);
+                s.putf4(hm / w); s.putc('\t'); s.putf4(hu / w);
+                for (const uint64_t *v : {T, M, U}) {
+                    s.putc('\t');
+                    for (int l = 1; l <= L; l++) { if (l > 1) s.putc(','); s.putu(v[l - 1]); }
+                }
+                s.putc('\n');
+            }
+        });
+        for (const std::string &c : chunk) if (!put(c)) return 0;
+    }
+    return written;
+}
+
+int bsx_meth_write_mhl_file(bsx_meth *m, const bsx_meth_opts *o, const bsx_regions &rg, const char *path) {
+    const int fd = open(path, O_WRONLY | O_CREAT | O_TRUNC, 0644);
+    if (fd < 0) { fprintf(stderr, "failed to open MHL output file: %s\n", path); return BSX_ERR_IO; }
+    const size_t w = bsx_meth_write_mhl(m, o, rg.seq.size(), rg.seq.data(), rg.start.data(), rg.end.data(), fd);
+    close(fd);
+    if (w == 0) { fprintf(stderr, "%s\n", bsx_last_error()); return BSX_ERR_IO; }
+    uint64_t alignments = 0, calls = 0, valid = 0;
+    if (bsx_meth_mhl(m, &alignments, &calls) != BSX_OK || bsx_meth_valid_count(m, &valid) != BSX_OK) { fprintf(stderr, "%s\n", bsx_last_error()); return BSX_ERR_CUDA; }
+    fprintf(stderr, "MHL: %llu of %llu valid mappings carry a CpG call, %llu CpG calls in haplotypes\n", (unsigned long long)alignments,
+            (unsigned long long)valid, (unsigned long long)calls);
     return BSX_OK;
 }
 

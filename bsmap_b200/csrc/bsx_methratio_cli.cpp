@@ -31,6 +31,9 @@
 //                              all four, by methylation pattern, with their level, methylation entropy and
 //                              epipolymorphism; prints "epialleles: S of V valid mappings span a 4-CpG window, W window
 //                              patterns counted" to stderr
+//   --mhl FILE                 methylation haplotype load (MHL, uMHL) per region of --regions or --tiles (shared with
+//                              --region-report), from the runs of consecutive CpG calls of each alignment; prints "MHL:
+//                              A of V valid mappings carry a CpG call, C CpG calls in haplotypes" to stderr
 #include <chrono>
 #include <cstdio>
 #include <cstdlib>
@@ -62,6 +65,7 @@ struct MOpts {
     std::string pdr;                         // --pdr FILE
     int pdr_min_cpg = 0;                     // --pdr-min-cpg K; 0 = not given (4)
     std::string epialleles;                  // --epialleles FILE
+    std::string mhl;                         // --mhl FILE
     std::vector<std::string> files;
 };
 
@@ -86,7 +90,7 @@ void parse(int argc, char **argv, MOpts &m) {
                                {'\1', "mbias", true}, {'\2', "mbias-ignore", true}, {'\3', "ct-snp", true},
                                {'\4', "conversion-filter", true}, {'\5', "conversion-report", true}, {'\6', "region-report", true},
                                {'\7', "regions", true}, {'\10', "tiles", true}, {'\11', "pdr", true}, {'\12', "pdr-min-cpg", true},
-                               {'\13', "epialleles", true}};   // long only
+                               {'\13', "epialleles", true}, {'\14', "mhl", true}};   // long only
     auto apply = [&](char c, const char *v) {
         if (!v) v = "";
         switch (c) {
@@ -130,10 +134,11 @@ void parse(int argc, char **argv, MOpts &m) {
                 if (*e || e == v || x < 1 || x > 255) usage_error("option --pdr-min-cpg: expected an integer 1..255");
                 m.pdr_min_cpg = (int)x; } break;
             case '\13': m.epialleles = v; break;
+            case '\14': m.mhl = v; break;
             case 'h': printf("Usage: methratio [options] BSMAP_MAPPING_FILES\n  -o FILE -d FILE [-c CHR] [-u] [-p] [-z] [-q] [-r] [-t N] [-g] [-m FOLD] [--mbias FILE] [--mbias-ignore A,B,C,D]\n"
                              "  [--ct-snp no-action|correct|skip] [--conversion-filter N] [--conversion-report FILE]\n"
                              "  [--region-report FILE (--regions BED | --tiles W)] [--pdr FILE [--pdr-min-cpg K]]\n"
-                             "  [--epialleles FILE]\n"); exit(0);
+                             "  [--epialleles FILE] [--mhl FILE (--regions BED | --tiles W)]\n"); exit(0);
         }
     };
     for (int i = 1; i < argc; i++) {
@@ -330,7 +335,8 @@ extern "C" int bsx_methratio_main(int argc, char **argv) {
     if (m.files.empty()) usage_error("Require at least one BSMAP_MAPPING_FILE.");
     if (!m.conv_report.empty() && m.conv < 0) m.conv = 0;
     if (!m.regions.empty() && m.tiles) usage_error("--regions and --tiles exclude each other");
-    if (m.region_report.empty() && (!m.regions.empty() || m.tiles)) usage_error("--regions / --tiles need --region-report FILE");
+    if (m.region_report.empty() && m.mhl.empty() && (!m.regions.empty() || m.tiles)) usage_error("--regions / --tiles need --region-report FILE or --mhl FILE");
+    if (!m.mhl.empty() && m.regions.empty() && !m.tiles) usage_error("--mhl needs --regions BED or --tiles W");
     if (!m.region_report.empty() && m.regions.empty() && !m.tiles) usage_error("--region-report needs --regions BED or --tiles W");
     if (m.pdr_min_cpg && m.pdr.empty()) usage_error("--pdr-min-cpg needs --pdr FILE");
     if (!m.pdr.empty() && !m.pdr_min_cpg) m.pdr_min_cpg = 4;
@@ -374,7 +380,7 @@ extern "C" int bsx_methratio_main(int argc, char **argv) {
     if ((!m.mbias.empty() && bsx_meth_enable_mbias(mh) != BSX_OK) || (m.ignore_set && bsx_meth_set_ignore(mh, m.ignore) != BSX_OK) ||
         (m.ct_snp && bsx_meth_enable_ct_snp(mh, m.ct_snp) != BSX_OK) || (m.conv >= 0 && bsx_meth_enable_conversion_filter(mh, m.conv) != BSX_OK) ||
         (!m.pdr.empty() && bsx_meth_enable_pdr(mh, m.pdr_min_cpg) != BSX_OK) ||
-        (!m.epialleles.empty() && bsx_meth_enable_epialleles(mh) != BSX_OK)) {
+        (!m.epialleles.empty() && bsx_meth_enable_epialleles(mh) != BSX_OK) || (!m.mhl.empty() && bsx_meth_enable_mhl(mh) != BSX_OK)) {
         fprintf(stderr, "%s\n", bsx_last_error()); return 1; }
     bsx_regions regions;                                      // read before the pile-up, so that a bad BED fails early
     if ((!m.regions.empty() && bsx_regions_bed(ix, selected.data(), m.regions.c_str(), regions) != BSX_OK) ||
@@ -480,6 +486,10 @@ extern "C" int bsx_methratio_main(int argc, char **argv) {
     if (!m.epialleles.empty()) {
         disp(m, ("writing " + m.epialleles + " ...").c_str());
         if (bsx_meth_write_epialleles_file(mh, &m.o, sp.data(), ln.data(), selected.data(), threads, m.epialleles.c_str()) != BSX_OK) return 1;
+    }
+    if (!m.mhl.empty()) {
+        disp(m, ("writing " + m.mhl + " ...").c_str());
+        if (bsx_meth_write_mhl_file(mh, &m.o, regions, m.mhl.c_str()) != BSX_OK) return 1;
     }
     if (!m.region_report.empty()) {
         disp(m, ("writing " + m.region_report + " ...").c_str());

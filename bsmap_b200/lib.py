@@ -72,12 +72,14 @@ EXPORTS = [
     "bsx_meth_regions", "bsx_meth_write_regions",
     "bsx_meth_enable_pdr", "bsx_meth_download_pdr", "bsx_meth_pdr", "bsx_meth_write_pdr", "bsx_meth_regions_pdr",
     "bsx_meth_enable_epialleles", "bsx_meth_cpg_sites", "bsx_meth_download_epialleles", "bsx_meth_epialleles", "bsx_meth_write_epialleles",
+    "bsx_meth_enable_mhl", "bsx_meth_download_mhl", "bsx_meth_mhl", "bsx_meth_regions_mhl", "bsx_meth_write_mhl",
 ]
 
 METH_READ2 = 8        # BSX_METH_READ2: alignment flag, read 2 (FLAG 0x80)
 MBIAS_CYCLES = 512    # BSX_MBIAS_CYCLES
 CONV_BINS = 256       # BSX_CONV_BINS
 EPI_CPGS = 4          # BSX_EPI_CPGS
+MHL_MAX_LEN = 16      # BSX_MHL_MAX_LEN
 CT_SNP_MODES = {"no-action": 1, "correct": 2, "skip": 3}   # BSX_CT_SNP_*
 
 _lib = None
@@ -185,6 +187,12 @@ def load():
     L.bsx_meth_epialleles.argtypes = [vp, C.POINTER(C.c_uint64), C.POINTER(C.c_uint64)]
     L.bsx_meth_write_epialleles.restype = sz
     L.bsx_meth_write_epialleles.argtypes = [vp, C.POINTER(MethOpts), pp, vp, vp, i32, i32]
+    L.bsx_meth_enable_mhl.argtypes = [vp]
+    L.bsx_meth_download_mhl.argtypes = [vp, u32, vp, vp]
+    L.bsx_meth_mhl.argtypes = [vp, C.POINTER(C.c_uint64), C.POINTER(C.c_uint64)]
+    L.bsx_meth_regions_mhl.argtypes = [vp, C.POINTER(MethOpts), C.c_uint64, vp, vp, vp, vp, vp]
+    L.bsx_meth_write_mhl.restype = sz
+    L.bsx_meth_write_mhl.argtypes = [vp, C.POINTER(MethOpts), C.c_uint64, vp, vp, vp, i32]
     L.bsx_packed_stride.restype = sz
     L.bsx_packed_stride.argtypes = [u32]
     L.bsx_pack_reads.argtypes = [u32, vp, u32, vp, vp, C.POINTER(C.c_uint64), i32]

@@ -429,7 +429,7 @@ size_t bsx_meth_write_pdr(bsx_meth *m, const bsx_meth_opts *o, const char *const
 /* build the CpG rank index and the pattern counters, and count windows from now on.  Must precede the first alignment
  * piled up, once; a late or second call: BSX_ERR_ARG; no device memory: BSX_ERR_CUDA (the message names the size). */
 int bsx_meth_enable_epialleles(bsx_meth *m);
-/* the number of CpG sites of sequence k; BSX_ERR_ARG when epialleles were not enabled */
+/* the number of CpG sites of sequence k; BSX_ERR_ARG when neither epialleles nor MHL (bsx_meth_enable_mhl) were enabled */
 int bsx_meth_cpg_sites(bsx_meth *m, uint32_t k, uint64_t *n);
 /* the sites of sequence k (n = bsx_meth_cpg_sites): site_pos[j] = 0-based position of site j's C in the sequence, and
  * counts[j * 16 + i] the alignments with pattern i over the window that starts at site j (rows whose window would leave
@@ -472,12 +472,57 @@ size_t bsx_meth_write_regions(bsx_meth *m, const bsx_meth_opts *o, uint64_t n, c
  * PDR on, bsx_meth_write_regions adds them and their PDR to the report).  BSX_ERR_ARG when PDR was not enabled. */
 int bsx_meth_regions_pdr(bsx_meth *m, const bsx_meth_opts *o, uint64_t n, const uint32_t *seq, const uint64_t *start, const uint64_t *end,
                          uint64_t *out, uint64_t *pdr);
+/* --- methylation haplotype load (MHL, uMHL) over regions, from per-read CpG runs ---------------------------------------
+ * MHL (Guo et al., Nat Genet 2017) asks how much of a region's methylation sits on the same molecules, over read
+ * haplotypes of every length l: MHL = sum_l l P(MH_l) / sum_l l, P(MH_l) the fraction of the region's length-l haplotypes
+ * that are fully methylated; uMHL the same for fully unmethylated ones.
+ *   site, call   exactly as for epialleles (above): the CpG call left after every rule, strands pooled, a '-' call at q
+ *                belongs to site q - 1, sites numbered by rank; conversion-filter drops and -r losers are not scored;
+ *                each mate on its own calls; -g changes nothing
+ *   haplotype    the alignment's sites in rank order (those whose call position lies in its trimmed span); a site
+ *                without a call breaks it.  A length-l haplotype is any l consecutive called sites of one alignment.
+ *   counters     counts[s][f][r - 1], BSX_MHL_MAX_LEN = 16: the alignments in which a run ends at site s, r = min(run
+ *                length, 16), the run taken over the alignment's consecutive sites ending at s that are f = 0 all called,
+ *                f = 1 all methylated, f = 2 all unmethylated.  A called site adds to family 0 and to 1 or 2.
+ *   region       (seq, start, end) as in the region report, clipped to the sequence; its sites are those whose C lies in
+ *                [start, end): the rank range [a, b).  A haplotype counts only when all its sites lie in [a, b).
+ *   SNP modes    under BSX_CT_SNP_SKIP and BSX_CT_SNP_CORRECT a site with snp > 0 at its C or its G cuts the region: it
+ *                and every haplotype through it are not counted
+ *   reduction    for l = 1..16, T_l, M_l, U_l are the sums over sites s in [a, b) of counts[s][0, 1, 2][r] over r >= l,
+ *                where l <= s - a + 1 and no cut site lies in [s - l + 1, s]
+ *   L, MHL       L = the largest l <= 16 with T_l > 0, or 0.  MHL = (sum over ascending l of l * M_l / T_l, in double)
+ *                / (L (L + 1) / 2); uMHL the same with U_l.
+ *   file         header "chr start end sites calls L MHL uMHL haplotypes methylated unmethylated" (tab-separated); one
+ *                line per region in region order, start and end as given; sites = the sites of the clipped region,
+ *                calls = T_1, MHL and uMHL %.4f or NA when L = 0, the last three columns T_l, M_l, U_l for l = 1..L,
+ *                comma-separated, or NA when L = 0.  -m and -z are ignored.
+ *   summary      the alignments with at least one CpG call, and their CpG calls
+ * HBM: the CpG rank index of epialleles (shared when both are on), and 192 bytes per CpG site. */
+#define BSX_MHL_MAX_LEN 16
+/* build the CpG rank index (unless epialleles did) and the run counters, and count runs from now on.  Must precede the
+ * first alignment piled up, once; a late or second call: BSX_ERR_ARG; no device memory: BSX_ERR_CUDA (with the size). */
+int bsx_meth_enable_mhl(bsx_meth *m);
+/* the sites of sequence k (n = bsx_meth_cpg_sites): site_pos[j] = 0-based position of site j's C in the sequence, and
+ * counts[(j * 3 + f) * 16 + r - 1] its run counters.  Either may be NULL.  Synchronises the device; BSX_ERR_ARG when MHL
+ * was not enabled. */
+int bsx_meth_download_mhl(bsx_meth *m, uint32_t k, uint32_t *site_pos, uint32_t *counts);
+/* the alignments with at least one CpG call and their CpG calls so far (synchronises the device; either may be NULL);
+ * BSX_ERR_ARG when MHL was not enabled */
+int bsx_meth_mhl(bsx_meth *m, uint64_t *alignments, uint64_t *calls);
+/* reduce the run counters over n regions on the device: sites[r] = the region's sites, out[(r * 3 + f) * 16 + l - 1] =
+ * T_l, M_l, U_l (f = 0, 1, 2).  Synchronises the device; BSX_ERR_ARG when MHL was not enabled or a region is invalid. */
+int bsx_meth_regions_mhl(bsx_meth *m, const bsx_meth_opts *o, uint64_t n, const uint32_t *seq, const uint64_t *start, const uint64_t *end,
+                         uint64_t *sites, uint64_t *out);
+/* write the MHL file for n regions to fd.  Returns bytes written (0 on error). */
+size_t bsx_meth_write_mhl(bsx_meth *m, const bsx_meth_opts *o, uint64_t n, const uint32_t *seq, const uint64_t *start, const uint64_t *end,
+                          int fd);
 /* the methratio.py command line: -o -d [-c -u -p -z -q -r -t -g -m -s] files... (SAM, BAM and BSP; -s is ignored);
  * extensions: --mbias FILE (the M-bias report) and --mbias-ignore A,B,C,D (bsx_meth_set_ignore), SAM and BAM only;
  * --ct-snp no-action|correct|skip (bsx_meth_enable_ct_snp); --conversion-filter N and --conversion-report FILE
  * (bsx_meth_enable_conversion_filter, bsx_meth_write_conversion); --region-report FILE with --regions BED or --tiles W
  * (bsx_meth_write_regions); --pdr FILE [--pdr-min-cpg K] (bsx_meth_enable_pdr, bsx_meth_write_pdr); --epialleles FILE
- * (bsx_meth_enable_epialleles, bsx_meth_write_epialleles) */
+ * (bsx_meth_enable_epialleles, bsx_meth_write_epialleles); --mhl FILE with --regions BED or --tiles W
+ * (bsx_meth_enable_mhl, bsx_meth_write_mhl) */
 int bsx_methratio_main(int argc, char **argv);
 
 /* --- the bsmap command line (main.cpp:441-476): same options, same output files -------------- */
